@@ -203,6 +203,30 @@ def run_reference(args):
 # -------------------------------------------------------------------------------------------------
 # this repo's CUDA path
 # -------------------------------------------------------------------------------------------------
+DUMP_VALUES = 1 << 21          # sampled evaluations: 16 MB of values + 16 MB of indices
+
+
+def dump_outputs(dirname, dcoef, out):
+    """Write what a caller of the timed path receives from its last step, so that two builds can be compared
+    output for output on the same seeded inputs: coef.npy (all coefficients), values.npy (the evaluated values at a
+    fixed, seeded sample of the queries, or all of them when there are at most DUMP_VALUES) and values_index.npy
+    (the query index of each sampled value, as float64).  The inputs are seeded, but the default fit adds in a
+    run-dependent order, so two runs differ in the last digits (about 1e-12 relative in the coefficients) unless
+    SPLPAK_B200_DETERMINISTIC=1."""
+    import torch
+
+    os.makedirs(dirname, exist_ok=True)
+    nq = out.numel()
+    if nq <= DUMP_VALUES:
+        idx = np.arange(nq)
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(nq, DUMP_VALUES, replace=False))
+    values = out[torch.from_numpy(idx).to(out.device)]
+    np.save(os.path.join(dirname, "coef.npy"), dcoef.cpu().numpy())
+    np.save(os.path.join(dirname, "values.npy"), values.cpu().numpy())
+    np.save(os.path.join(dirname, "values_index.npy"), idx.astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -306,6 +330,8 @@ def run_ours(args):
         t_wall = time.perf_counter() - t_wall0
         launches = sp.total_launches() - launches0
         clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dcoef, out)      # before the sub-records below overwrite dcoef and out
 
     fit_all = [a.elapsed_time(b) for a, b, _ in evs]
     eval_all = [b.elapsed_time(c) for _, b, c in evs]
@@ -595,7 +621,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-pageable", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's coefficients and a seeded sample of its evaluated values from the last timed "
+                         "step to DIR/*.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's results; it does not apply to --impl reference")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3                       # timing rule: W >= 3
     if args.impl == "reference":
