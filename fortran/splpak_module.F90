@@ -11,8 +11,9 @@
 !    f = s%evaluate(ndim,x,[nderiv,]coef,xmin,xmax,nodes,ierror)
 !    call s%destroy()
 !
-!  plus three additions that have no counterpart in the reference: `evaluate_batch`
-!  (batched splfe/splde) and the streaming pair `add_points` / `compute` named by the
+!  plus additions that have no counterpart in the reference: `evaluate_batch`
+!  (batched splfe/splde), `evaluate_derivs` (all partial derivatives up to order 1 or 2 in
+!  one pass) and the streaming pair `add_points` / `compute` named by the
 !  project brief.  The numerical work (bascmp, the splcw row loop, suprls, splde) is
 !  replaced; cfaerr (printing) stays on this side so stdout is unchanged.
 !
@@ -53,6 +54,7 @@
         generic,public   :: evaluate   => splfe, splde   !! evaluate the spline
         procedure,public :: destroy    => destroy_splpak
         procedure,public :: evaluate_batch               !! (new) batched splfe/splde
+        procedure,public :: evaluate_derivs              !! (new) every partial derivative up to order 1 or 2, one pass
         procedure,public :: evaluate_grid                !! (new) splfe/splde on a regular output grid
         procedure,public :: create                       !! (new) streaming fit: create
         procedure,public :: add_points                   !! (new) streaming fit: accumulate points
@@ -117,6 +119,17 @@
             integer(c_int),intent(out) :: ierror
             integer(c_int) :: rc
         end function c_eval
+        function c_eval_derivs(ndim,x,l1x,nq,order,coef,xmin,xmax,nodes,out,ierror) &
+                 bind(C,name='splpak_b200_eval_derivs') result(rc)
+            import :: c_int, c_int64_t, cwp
+            integer(c_int),value :: ndim, l1x, order
+            integer(c_int64_t),value :: nq
+            real(cwp),intent(in) :: x(*), coef(*), xmin(*), xmax(*)
+            integer(c_int),intent(in) :: nodes(*)
+            real(cwp) :: out(*)
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_eval_derivs
         function c_eval_grid(ndim,axes,naxis,nderiv,coef,xmin,xmax,nodes,out,ierror) &
                  bind(C,name='splpak_b200_eval_grid') result(rc)
             import :: c_int, c_int64_t, c_ptr, cwp
@@ -309,6 +322,24 @@
         ierror = ie
         call cfaerr(ierror,.true.)
     end subroutine evaluate_batch
+
+    !> (new) every partial derivative up to total order `order` (1 or 2) at nq points x(l1x,nq) in one pass:
+    !> f(ncomp,nq) with ncomp = ndim+1 (order 1: the value, d/dx1 .. d/dxn) or (ndim+1)*(ndim+2)/2 (order 2: then
+    !> d2/dxi dxj for i <= j in row order).  Component k equals evaluate_batch with the nderiv it names, bit for bit.
+    !> An order other than 1 or 2 sets ierror = 104 and leaves f unchanged.
+    subroutine evaluate_derivs(me,ndim,x,l1x,nq,order,coef,xmin,xmax,nodes,f,ierror)
+        class(splpak_type),intent(inout) :: me
+        integer,intent(in) :: ndim, l1x, order
+        integer(int64),intent(in) :: nq
+        real(wp),intent(in) :: x(l1x,nq), coef(*), xmin(ndim), xmax(ndim)
+        integer,intent(in) :: nodes(ndim)
+        real(wp),intent(inout) :: f(*)
+        integer,intent(out) :: ierror
+        integer(c_int) :: rc, ie
+        rc = c_eval_derivs(int(ndim,c_int),x,int(l1x,c_int),int(nq,c_int64_t),int(order,c_int),coef,xmin,xmax,nodes,f,ie)
+        ierror = ie
+        call cfaerr(ierror,.true.)
+    end subroutine evaluate_derivs
 
     !> (new) value or partial derivative on the tensor grid spanned by the ndim axes stored one after the other in
     !> `axes` (axis d has naxis(d) points); f(naxis(1),...,naxis(ndim)); nderiv absent => splfe.

@@ -112,6 +112,22 @@ int splpak_b200_eval_device(int ndim, const splpak_real *d_x, int l1x, int64_t n
                             const splpak_real *xmax, const int *nodes, splpak_real *d_out,
                             void *stream, int *ierror);
 
+/* Derivative sets: for every point, all partial derivatives up to total order `order` in one pass (one gather of
+ * the point's 4^ndim coefficients for all of them).  out(ncomp, nq): the ncomp results of one point are contiguous.
+ *   order 1: ncomp = ndim + 1                 the value, d/dx1 .. d/dxn
+ *   order 2: ncomp = (ndim + 1)(ndim + 2) / 2 the order-1 set, then d2/dxi dxj for i <= j in row order
+ *            (1,1), (1,2), .., (1,n), (2,2), .., (n,n)
+ * Component k is bit-identical to splpak_b200_eval on the same batch with the nderiv it names.  Errors 101..103
+ * as splpak_b200_eval; an order other than 1 or 2 returns 104 and writes nothing.  HOST arrays (same staging as
+ * splpak_b200_eval) / DEVICE arrays (asynchronous on stream).  The REAL32 library keeps float I/O with float64
+ * arithmetic here, as splde does. */
+int splpak_b200_eval_derivs(int ndim, const splpak_real *x, int l1x, int64_t nq, int order,
+                            const splpak_real *coef, const splpak_real *xmin, const splpak_real *xmax,
+                            const int *nodes, splpak_real *out, int *ierror);
+int splpak_b200_eval_derivs_device(int ndim, const splpak_real *d_x, int l1x, int64_t nq, int order,
+                                   const splpak_real *d_coef, const splpak_real *xmin, const splpak_real *xmax,
+                                   const int *nodes, splpak_real *d_out, void *stream, int *ierror);
+
 /* Evaluation on a REGULAR OUTPUT GRID (new; the upstream fit-then-grid use, README.md:60): the value (nderiv NULL)
  * or partial derivative of the spline at every point (a1[i1], .., aN[iN]) of the tensor grid spanned by ndim axes.
  * axes = the axes concatenated (axis d has naxis[d] points, any order, inside or outside [xmin, xmax]);

@@ -10,8 +10,11 @@ from .api import (  # noqa: F401
     SplpakError,
     SplpakType,
     cfaerr_text,
+    derivs_ncomp,
     eval_batch,
     eval_batch_device,
+    eval_derivs,
+    eval_derivs_device,
     eval_grid,
     eval_grid_device,
     measure_peaks,
@@ -24,6 +27,6 @@ from .api import (  # noqa: F401
 
 __all__ = [
     "SplpakType", "FitHandle", "SplpakError", "splcc", "splcw", "splfe", "splde", "eval_batch",
-    "eval_batch_device", "eval_grid", "eval_grid_device", "measure_peaks", "total_launches", "cfaerr_text", "build", "load",
-    "lib_path", "SYMBOLS",
+    "eval_batch_device", "eval_derivs", "eval_derivs_device", "eval_grid", "eval_grid_device", "measure_peaks",
+    "total_launches", "cfaerr_text", "derivs_ncomp", "build", "load", "lib_path", "SYMBOLS",
 ]

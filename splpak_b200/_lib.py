@@ -25,6 +25,8 @@ SYMBOLS = [
     "splpak_b200_splfe",
     "splpak_b200_eval",
     "splpak_b200_eval_device",
+    "splpak_b200_eval_derivs",
+    "splpak_b200_eval_derivs_device",
     "splpak_b200_eval_grid",
     "splpak_b200_eval_grid_device",
     "splpak_b200_fit_create",
@@ -116,6 +118,8 @@ def load(real32: bool = False) -> C.CDLL:
         "splpak_b200_splfe": (real, [C.c_int, rp, vp, rp, rp, ip, ip]),
         "splpak_b200_eval": (C.c_int, [C.c_int, vp, C.c_int, i64, ip, vp, rp, rp, ip, vp, ip]),
         "splpak_b200_eval_device": (C.c_int, [C.c_int, vp, C.c_int, i64, ip, vp, rp, rp, ip, vp, vp, ip]),
+        "splpak_b200_eval_derivs": (C.c_int, [C.c_int, vp, C.c_int, i64, C.c_int, vp, rp, rp, ip, vp, ip]),
+        "splpak_b200_eval_derivs_device": (C.c_int, [C.c_int, vp, C.c_int, i64, C.c_int, vp, rp, rp, ip, vp, vp, ip]),
         "splpak_b200_eval_grid": (C.c_int, [C.c_int, vp, C.POINTER(i64), ip, vp, rp, rp, ip, vp, ip]),
         "splpak_b200_eval_grid_device": (C.c_int, [C.c_int, vp, C.POINTER(i64), ip, vp, rp, rp, ip, vp, vp, ip]),
         "splpak_b200_fit_create": (C.c_int, [C.c_int, rp, rp, ip, real, C.POINTER(vp), ip]),

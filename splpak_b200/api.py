@@ -16,7 +16,8 @@ Array convention: xdata is passed as a C-ordered numpy array of shape (ndata, l1
 memory image of Fortran's xdata(l1xdat, ndata).  coef is 1-D, dimension 1 fastest (:661-666).
 
 New, non-reference entry points (named by the north star): `FitHandle.add_points / compute`
-(streaming assembly / solve split), `eval_batch` (batched splfe/splde) and device-pointer variants
+(streaming assembly / solve split), `eval_batch` (batched splfe/splde), `eval_derivs` (every partial derivative up
+to order 1 or 2 in one pass) and device-pointer variants
 that take torch CUDA tensors so benchmarks can run device-resident.
 """
 from __future__ import annotations
@@ -179,6 +180,43 @@ def eval_batch_device(ndim, d_x, l1x, nq, d_coef, xmin, xmax, nodes, d_out, nder
     ierr = C.c_int(0)
     lib.splpak_b200_eval_device(int(ndim), _dev_ptr(d_x), int(l1x), int(nq), ndp, _dev_ptr(d_coef), mnp, mxp,
                                 nop, _dev_ptr(d_out), _stream_ptr(stream), C.byref(ierr))
+    return ierr.value
+
+
+def derivs_ncomp(ndim, order):
+    """Outputs per query of eval_derivs: ndim + 1 (order 1) or (ndim + 1)(ndim + 2) / 2 (order 2); 0 for another order."""
+    n = max(int(ndim), 0)
+    return {1: n + 1, 2: (n + 1) * (n + 2) // 2}.get(int(order), 0)
+
+
+def eval_derivs(ndim, x, coef, xmin, xmax, nodes, order=1, *, quiet=True, real32=False):
+    """Every partial derivative up to total order `order` (1 or 2) at HOST points x (nq, l1x), in one pass.
+    Returns (out[nq, ncomp], ierror).  Columns: the value, d/dx1 .. d/dxn, then (order 2) d2/dxi dxj for i <= j in row
+    order.  Column k is bit-identical to eval_batch with the nderiv it names; an order other than 1 or 2 gives 104."""
+    lib = _lib.load(real32)
+    dt = _np_dtype(real32)
+    xa = np.ascontiguousarray(x, dtype=dt)
+    if xa.ndim == 1:
+        xa = xa.reshape(-1, 1)
+    nq, l1x = xa.shape
+    cf = _vec(coef, dt)
+    out = np.zeros((nq, derivs_ncomp(ndim, order)), dtype=dt)
+    keep, (mnp, mxp, nop) = _grid_args(lib, ndim, xmin, xmax, nodes, real32)
+    ierr = C.c_int(0)
+    lib.splpak_b200_eval_derivs(int(ndim), _ptr(xa), int(l1x), int(nq), int(order), _ptr(cf), mnp, mxp, nop, _ptr(out),
+                                C.byref(ierr))
+    _report(ierr.value, True, quiet, real32)
+    return out, ierr.value
+
+
+def eval_derivs_device(ndim, d_x, l1x, nq, d_coef, xmin, xmax, nodes, d_out, order=1, stream=None, *, real32=False):
+    """eval_derivs with torch CUDA tensors (or raw device pointers); d_out holds nq * ncomp values, the ncomp of one
+    query contiguous.  Asynchronous on `stream`.  Returns ierror."""
+    lib = _lib.load(real32)
+    keep, (mnp, mxp, nop) = _grid_args(lib, ndim, xmin, xmax, nodes, real32)
+    ierr = C.c_int(0)
+    lib.splpak_b200_eval_derivs_device(int(ndim), _dev_ptr(d_x), int(l1x), int(nq), int(order), _dev_ptr(d_coef), mnp,
+                                       mxp, nop, _dev_ptr(d_out), _stream_ptr(stream), C.byref(ierr))
     return ierr.value
 
 

@@ -18,11 +18,12 @@ unsigned long long g_spl_launches = 0;
 // ---- kernels' host launchers (other translation units) ----
 int spl_assemble_scratch_init(const GridParams &gp, AssembleScratch &sc, cudaStream_t st);
 void spl_assemble_scratch_free(AssembleScratch &sc);
-int spl_eval_launch(const GridParams &gp, const int *nderiv, const real_t *d_x, int l1x, long long nq,
+int spl_eval_launch(const GridParams &gp, const int *nderiv, int order, const real_t *d_x, int l1x, long long nq,
                     const double *d_coef, long long ncol_padded, real_t *d_out, cudaStream_t stream,
                     int nsm, size_t smem_optin, unsigned long long *d_counter, double *d_pad);
 long long spl_eval_regroup_elems(const GridParams &gp, long long nq, int nsm, size_t smem_optin);
-long long spl_eval_scratch_elems(const GridParams &gp, const int *nderiv, long long nq, int nsm, size_t smem_optin);
+long long spl_eval_scratch_elems(const GridParams &gp, const int *nderiv, int order, long long nq, int nsm,
+                                 size_t smem_optin);
 #ifdef SPLPAK_REAL32
 int spl_eval_f32_launch(const GridParams &gp, const real_t *d_x, int l1x, long long nq, const real_t *d_coef,
                         real_t *d_out, cudaStream_t stream, int nsm, size_t smem_optin, unsigned long long *d_counter);
@@ -438,13 +439,15 @@ static unsigned long long *eval_counter_slot(int device) {
     return pool[device] + (next[device]++ % EVAL_COUNTERS);
 }
 
-static int eval_device_impl(const GridParams &gp, const DeviceInfo &di, const int *nderiv,
+// order 0: one output per query (nderiv, NULL = splfe); order 1 / 2: the derivative sets, ncomp outputs per query
+static int eval_device_impl(const GridParams &gp, const DeviceInfo &di, const int *nderiv, int order,
                             const real_t *d_x, int l1x, long long nq, const real_t *d_coef,
                             real_t *d_out, cudaStream_t st) {
 #ifdef SPLPAK_REAL32
     {
-        // splfe of the REAL32 library runs in working precision (float), like the reference built with -DREAL32
-        bool value = true;
+        // splfe of the REAL32 library runs in working precision (float), like the reference built with -DREAL32; the
+        // derivative sets keep float I/O with float64 arithmetic, as splde does
+        bool value = order == 0;
         for (int d = 0; d < gp.ndim; ++d)
             if (nderiv && nderiv[d] != 0) value = false;
         const char *mode = getenv("SPLPAK_B200_R32");
@@ -510,7 +513,7 @@ static int eval_device_impl(const GridParams &gp, const DeviceInfo &di, const in
     if (!counter) return SPLPAK_ERR_ALLOC;
     // image of the table the kernels read: extended (uniform form) and/or padded (regrouping kernel) copy
     double *pad = nullptr;
-    const long long pad_elems = spl_eval_scratch_elems(gp, nderiv, nq, di.nsm, di.smem_optin);
+    const long long pad_elems = spl_eval_scratch_elems(gp, nderiv, order, nq, di.nsm, di.smem_optin);
     if (pad_elems > 0) {
         cudaMemPool_t pool = eval_scratch_pool(di.dev);
         cudaError_t e = pool ? cudaMallocFromPoolAsync((void **)&pad, sizeof(double) * (size_t)(pad_elems + 2), pool, st)
@@ -520,7 +523,7 @@ static int eval_device_impl(const GridParams &gp, const DeviceInfo &di, const in
             pad = nullptr;                                     // the exact plain kernel needs no scratch
         }
     }
-    int rc = spl_eval_launch(gp, nderiv, d_x, l1x, nq, coef64, npad, d_out, st, di.nsm, di.smem_optin, counter, pad);
+    int rc = spl_eval_launch(gp, nderiv, order, d_x, l1x, nq, coef64, npad, d_out, st, di.nsm, di.smem_optin, counter, pad);
     if (pad) cudaFreeAsync(pad, st);
     if (tmp) cudaFreeAsync(tmp, st);
     return rc;
@@ -537,7 +540,7 @@ extern "C" int splpak_b200_eval_device(int ndim, const real_t *d_x, int l1x, int
         DeviceInfo di;
         rc = get_device(di);
         if (rc == SPLPAK_OK)
-            rc = eval_device_impl(gp, di, nderiv, d_x, l1x, nq, d_coef, d_out, (cudaStream_t)stream);
+            rc = eval_device_impl(gp, di, nderiv, 0, d_x, l1x, nq, d_coef, d_out, (cudaStream_t)stream);
     }
     if (rc == SPLPAK_OK && soft) rc = SPLPAK_ERR_NDERIV;
     if (ierror) *ierror = rc;
@@ -694,22 +697,11 @@ static EvalHostCtx &eval_host_ctx(int device) {
     return ctx[(device >= 0 && device < 64) ? device : 0];
 }
 
-extern "C" int splpak_b200_eval(int ndim, const real_t *x, int l1x, int64_t nq, const int *nderiv,
-                                const real_t *coef, const real_t *xmin, const real_t *xmax,
-                                const int *nodes, real_t *out, int *ierror) {
-    GridParams gp;
-    int soft = 0;
-    int rc = make_grid(ndim, xmin, xmax, nodes, nderiv, gp, &soft);
-    if (rc != SPLPAK_OK || nq <= 0) {
-        if (ierror) *ierror = rc;
-        return rc;
-    }
-    DeviceInfo di;
-    rc = get_device(di);
-    if (rc != SPLPAK_OK) {
-        if (ierror) *ierror = rc;
-        return rc;
-    }
+// The host-array path of splpak_b200_eval / splpak_b200_eval_derivs: ncomp outputs per query, launch(d_x, nc, d_coef,
+// d_out, st) evaluates nc staged queries.  Returns the code of the call (ierror is the caller's business).
+template <class Launch>
+static int eval_host_staged(const GridParams &gp, const DeviceInfo &di, const real_t *x, int l1x, long long nq,
+                            const real_t *coef, real_t *out, int ncomp, Launch launch) {
     // Streams, events and device staging buffers of the host path are cached per device (grow-only) and
     // the call holds the device's lock: creating and freeing ~270 MB of device memory per call made
     // identical calls take anywhere between 52 and 900 ms.
@@ -721,7 +713,6 @@ extern "C" int splpak_b200_eval(int ndim, const real_t *x, int l1x, int64_t nq, 
     do {                                                    \
         if ((expr) != cudaSuccess) {                        \
             cudaGetLastError();                             \
-            if (ierror) *ierror = SPLPAK_ERR_CUDA;          \
             return SPLPAK_ERR_CUDA;                         \
         }                                                   \
     } while (0)
@@ -741,7 +732,7 @@ extern "C" int splpak_b200_eval(int ndim, const real_t *x, int l1x, int64_t nq, 
         cx.coef_cap = (size_t)(gp.ncol + 2);
         cx.coef_valid = false;
     }
-    const size_t xneed = (size_t)chunk * l1x, oneed = (size_t)chunk;
+    const size_t xneed = (size_t)chunk * l1x, oneed = (size_t)chunk * ncomp;
     for (int k = 0; k < nbuf; ++k) {
         if (xneed > cx.x_cap[k]) {
             if (cx.d_x[k]) cudaFree(cx.d_x[k]);
@@ -767,7 +758,6 @@ extern "C" int splpak_b200_eval(int ndim, const real_t *x, int l1x, int64_t nq, 
             try {
                 cx.coef_shadow.assign(reinterpret_cast<const char *>(coef), reinterpret_cast<const char *>(coef) + cbytes);
             } catch (...) {                                        // no C++ exception may cross the C ABI
-                if (ierror) *ierror = SPLPAK_ERR_ALLOC;
                 return SPLPAK_ERR_ALLOC;
             }
             // from the shadow, not from the caller's array: the copy may still be in flight when we return on an error path
@@ -776,16 +766,15 @@ extern "C" int splpak_b200_eval(int ndim, const real_t *x, int l1x, int64_t nq, 
             cx.coef_valid = true;
         }
     }
+    int rc = SPLPAK_OK;
     if (nq <= 4096) {
         // latency path (scalar splfe / splde and small batches): one stream, one synchronisation
         EV_TRY(cudaMemcpyAsync(cx.d_x[0], x, sizeof(real_t) * (size_t)nq * l1x, cudaMemcpyHostToDevice, st));
-        rc = eval_device_impl(gp, di, nderiv, cx.d_x[0], l1x, nq, d_coef, cx.d_out[0], st);
+        rc = launch(cx.d_x[0], nq, d_coef, cx.d_out[0], st);
         if (rc == SPLPAK_OK) {
-            EV_TRY(cudaMemcpyAsync(out, cx.d_out[0], sizeof(real_t) * (size_t)nq, cudaMemcpyDeviceToHost, st));
+            EV_TRY(cudaMemcpyAsync(out, cx.d_out[0], sizeof(real_t) * (size_t)nq * ncomp, cudaMemcpyDeviceToHost, st));
             EV_TRY(cudaStreamSynchronize(st));
         }
-        if (rc == SPLPAK_OK && soft) rc = SPLPAK_ERR_NDERIV;
-        if (ierror) *ierror = rc;
         return rc;
     }
     // chunked, double-buffered: H2D of chunk k+1 (st2) overlaps the kernel + D2H of chunk k (st)
@@ -796,16 +785,76 @@ extern "C" int splpak_b200_eval(int ndim, const real_t *x, int l1x, int64_t nq, 
         EV_TRY(spl_h2d(cx.d_x[k], x + q0 * (long long)l1x, sizeof(real_t) * (size_t)nc * l1x, st2, di.dev));
         EV_TRY(cudaEventRecord(cx.ev_in[k], st2));
         EV_TRY(cudaStreamWaitEvent(st, cx.ev_in[k], 0));
-        rc = eval_device_impl(gp, di, nderiv, cx.d_x[k], l1x, nc, d_coef, cx.d_out[k], st);
+        rc = launch(cx.d_x[k], nc, d_coef, cx.d_out[k], st);
         if (rc != SPLPAK_OK) break;
-        EV_TRY(spl_d2h(out + q0, cx.d_out[k], sizeof(real_t) * (size_t)nc, st, di.dev));
+        EV_TRY(spl_d2h(out + q0 * ncomp, cx.d_out[k], sizeof(real_t) * (size_t)nc * ncomp, st, di.dev));
         EV_TRY(cudaEventRecord(cx.ev_done[k], st));
     }
     EV_TRY(spl_d2h_flush(di.dev));
     EV_TRY(cudaStreamSynchronize(st));
     EV_TRY(cudaStreamSynchronize(st2));
 #undef EV_TRY
+    return rc;
+}
+
+extern "C" int splpak_b200_eval(int ndim, const real_t *x, int l1x, int64_t nq, const int *nderiv,
+                                const real_t *coef, const real_t *xmin, const real_t *xmax,
+                                const int *nodes, real_t *out, int *ierror) {
+    GridParams gp;
+    int soft = 0;
+    int rc = make_grid(ndim, xmin, xmax, nodes, nderiv, gp, &soft);
+    if (rc != SPLPAK_OK || nq <= 0) {
+        if (ierror) *ierror = rc;
+        return rc;
+    }
+    DeviceInfo di;
+    rc = get_device(di);
+    if (rc == SPLPAK_OK)
+        rc = eval_host_staged(gp, di, x, l1x, nq, coef, out, 1,
+                              [&](const real_t *d_x, long long n, const real_t *d_coef, real_t *d_out, cudaStream_t st) {
+                                  return eval_device_impl(gp, di, nderiv, 0, d_x, l1x, n, d_coef, d_out, st);
+                              });
     if (rc == SPLPAK_OK && soft) rc = SPLPAK_ERR_NDERIV;
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+// ------------------------------------------------------------------------------------------
+// derivative sets: every partial derivative up to total order `order` of each query in one pass
+// ------------------------------------------------------------------------------------------
+static int derivs_ncomp(int ndim, int order) { return order == 1 ? ndim + 1 : (ndim + 1) * (ndim + 2) / 2; }
+
+extern "C" int splpak_b200_eval_derivs_device(int ndim, const real_t *d_x, int l1x, int64_t nq, int order,
+                                              const real_t *d_coef, const real_t *xmin, const real_t *xmax,
+                                              const int *nodes, real_t *d_out, void *stream, int *ierror) {
+    GridParams gp;
+    int rc = make_grid(ndim, xmin, xmax, nodes, nullptr, gp, nullptr);
+    if (rc == SPLPAK_OK && order != 1 && order != 2) rc = SPLPAK_ERR_NDERIV;
+    if (rc == SPLPAK_OK && nq > 0) {
+        DeviceInfo di;
+        rc = get_device(di);
+        if (rc == SPLPAK_OK)
+            rc = eval_device_impl(gp, di, nullptr, order, d_x, l1x, nq, d_coef, d_out, (cudaStream_t)stream);
+    }
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+extern "C" int splpak_b200_eval_derivs(int ndim, const real_t *x, int l1x, int64_t nq, int order, const real_t *coef,
+                                       const real_t *xmin, const real_t *xmax, const int *nodes, real_t *out,
+                                       int *ierror) {
+    GridParams gp;
+    int rc = make_grid(ndim, xmin, xmax, nodes, nullptr, gp, nullptr);
+    if (rc == SPLPAK_OK && order != 1 && order != 2) rc = SPLPAK_ERR_NDERIV;
+    if (rc == SPLPAK_OK && nq > 0) {
+        DeviceInfo di;
+        rc = get_device(di);
+        if (rc == SPLPAK_OK)
+            rc = eval_host_staged(gp, di, x, l1x, nq, coef, out, derivs_ncomp(ndim, order),
+                                  [&](const real_t *d_x, long long n, const real_t *d_c, real_t *d_out, cudaStream_t st) {
+                                      return eval_device_impl(gp, di, nullptr, order, d_x, l1x, n, d_c, d_out, st);
+                                  });
+    }
     if (ierror) *ierror = rc;
     return rc;
 }
@@ -1476,7 +1525,7 @@ static int refine_device_chunk(splpak_b200_fit_t h, const real_t *d_x, int l1x, 
         h->res_cap = n;
     }
     // s(x_i) with the current coefficients, then r_i = y_i - s(x_i), then g += sum (w phi)(w r)
-    rc = eval_device_impl(h->gp, h->di, nullptr, d_x, l1x, n, reinterpret_cast<const real_t *>(h->d_coef64), h->d_res,
+    rc = eval_device_impl(h->gp, h->di, nullptr, 0, d_x, l1x, n, reinterpret_cast<const real_t *>(h->d_coef64), h->d_res,
                           h->st);
     if (rc != SPLPAK_OK) return rc;
     spl_residual_kernel<<<spl_div_up(n, 256), 256, 0, h->st>>>(d_y, h->d_res, n);

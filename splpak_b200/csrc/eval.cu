@@ -231,8 +231,256 @@ __device__ __forceinline__ double spl_eval_point_uni(const GridParams &gp, const
     return spl_eval_point_uni_at<NDIM, VALUE>(dp, tl, cf, f, base, scale);
 }
 
-template <int NDIM> struct EvalCfg {
-    static constexpr int THREADS = (NDIM <= 3) ? 1024 : 512;
+// ------------------------------------------------------------------------------------------
+// Fused derivative sets (splpak_b200_eval_derivs): every partial derivative of total order <= ORDER of one query from
+// ONE gather of its 4^ndim coefficients.  Output order: the value, d/dx1 .. d/dxn, then (ORDER 2) d2/dxi dxj for i <= j
+// in row order.  Component k is bit-identical to the single-nderiv evaluation: each is the nested contraction of
+// spl_contract_at with that component's weights per dimension, in the same fma order; what is shared is the gather
+// and every partial sum over dimensions 1..m that components agree on (weight SET s of a dimension: derivative order
+// s, and in the exact form set ORDER + 1 = the x8 value weights of spl_window_weights_value, which splfe uses and
+// which only combine with each other).
+// ------------------------------------------------------------------------------------------
+__host__ __device__ constexpr int spl_ncomp(int ndim, int order) {
+    return order == 1 ? ndim + 1 : (ndim + 1) * (ndim + 2) / 2;
+}
+// a prefix s[0..m-1] of weight sets that some output component extends
+template <int ORDER>
+__device__ constexpr bool spl_dprefix(int m, int s0, int s1 = 0, int s2 = 0, int s3 = 0) {
+    const int s[4] = {s0, s1, s2, s3};
+    int nv = 0, tot = 0;
+    for (int i = 0; i < m; ++i) {
+        nv += s[i] > ORDER;
+        tot += s[i] > ORDER ? 0 : s[i];
+    }
+    return (nv == 0 || nv == m) && tot <= ORDER;
+}
+// output component of a full set of weight sets (-1: none; VSET: the exact form, whose value is the all-x8 set)
+template <int NDIM, int ORDER, bool VSET>
+__device__ constexpr int spl_dcomp(int s0, int s1 = 0, int s2 = 0, int s3 = 0) {
+    const int s[4] = {s0, s1, s2, s3};
+    if (!spl_dprefix<ORDER>(NDIM, s0, s1, s2, s3)) return -1;
+    int tot = 0, i1 = -1, i2 = -1;
+    for (int d = 0; d < NDIM; ++d) {
+        if (s[d] > ORDER) return 0;
+        tot += s[d];
+        if (s[d] == 2) i1 = i2 = d;
+        else if (s[d] == 1) (i1 < 0 ? i1 : i2) = d;
+    }
+    if (tot == 0) return VSET ? -1 : 0;
+    if (tot == 1) return 1 + i1;
+    return 1 + NDIM + i1 * NDIM - i1 * (i1 - 1) / 2 + (i2 - i1);
+}
+// derivative order of dimension d in component c (inverse of spl_dcomp)
+__device__ __forceinline__ int spl_dorder(int ndim, int c, int d) {
+    if (c == 0) return 0;
+    if (c <= ndim) return c - 1 == d ? 1 : 0;
+    int r = c - 1 - ndim, i = 0;
+    while (r >= ndim - i) r -= ndim - i++;
+    const int j = i + r;
+    return (i == d) + (j == d);
+}
+
+// res[c] (NS weight sets per dimension, b[d][s][k]): the contraction of every component, dimension 1 innermost
+template <int NDIM, int ORDER, int NS>
+__device__ __forceinline__ void spl_contract_multi(const TableLayout &tl, const double *__restrict__ p0,
+                                                   const double (*b)[NS][4], double *res) {
+    constexpr bool VSET = NS > ORDER + 1;
+#pragma unroll
+    for (int c = 0; c < spl_ncomp(NDIM, ORDER); ++c) res[c] = 0.0;
+    if constexpr (NDIM == 1) {
+#pragma unroll
+        for (int a = 0; a < NS; ++a) {
+            const int c = spl_dcomp<1, ORDER, VSET>(a);
+            if (c < 0) continue;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) res[c] = fma(p0[i], b[0][a][i], res[c]);
+        }
+    } else if constexpr (NDIM == 2) {
+        const int n0 = tl.s1;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const double *p = p0 + n0 * j;
+            double v[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) v[i] = p[i];
+#pragma unroll
+            for (int a = 0; a < NS; ++a) {
+                if (!spl_dprefix<ORDER>(1, a)) continue;
+                double sj = 0.0;
+#pragma unroll
+                for (int i = 0; i < 4; ++i) sj = fma(v[i], b[0][a][i], sj);
+#pragma unroll
+                for (int e = 0; e < NS; ++e) {
+                    const int c = spl_dcomp<2, ORDER, VSET>(a, e);
+                    if (c >= 0) res[c] = fma(sj, b[1][e][j], res[c]);
+                }
+            }
+        }
+    } else if constexpr (NDIM == 3) {
+        const int n0 = tl.s1;
+        const int n01 = tl.s2;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            double sk[NS][NS];
+#pragma unroll
+            for (int a = 0; a < NS; ++a)
+#pragma unroll
+                for (int e = 0; e < NS; ++e) sk[a][e] = 0.0;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const double *p = p0 + n0 * j + n01 * k;
+                double v[4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i) v[i] = p[i];
+#pragma unroll
+                for (int a = 0; a < NS; ++a) {
+                    if (!spl_dprefix<ORDER>(1, a)) continue;
+                    double sj = 0.0;
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) sj = fma(v[i], b[0][a][i], sj);
+#pragma unroll
+                    for (int e = 0; e < NS; ++e)
+                        if (spl_dprefix<ORDER>(2, a, e)) sk[a][e] = fma(sj, b[1][e][j], sk[a][e]);
+                }
+            }
+#pragma unroll
+            for (int a = 0; a < NS; ++a)
+#pragma unroll
+                for (int e = 0; e < NS; ++e)
+#pragma unroll
+                    for (int g = 0; g < NS; ++g) {
+                        const int c = spl_dcomp<3, ORDER, VSET>(a, e, g);
+                        if (c >= 0) res[c] = fma(sk[a][e], b[2][g][k], res[c]);
+                    }
+        }
+    } else {
+        const int n0 = tl.s1;
+        const int n01 = tl.s2;
+        const long long n012 = tl.s3;
+#pragma unroll
+        for (int l = 0; l < 4; ++l) {
+            double sl[NS][NS][NS];
+#pragma unroll
+            for (int a = 0; a < NS; ++a)
+#pragma unroll
+                for (int e = 0; e < NS; ++e)
+#pragma unroll
+                    for (int g = 0; g < NS; ++g) sl[a][e][g] = 0.0;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                double sk[NS][NS];
+#pragma unroll
+                for (int a = 0; a < NS; ++a)
+#pragma unroll
+                    for (int e = 0; e < NS; ++e) sk[a][e] = 0.0;
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    const double *p = p0 + n0 * j + n01 * k + n012 * l;
+                    double v[4];
+#pragma unroll
+                    for (int i = 0; i < 4; ++i) v[i] = p[i];
+#pragma unroll
+                    for (int a = 0; a < NS; ++a) {
+                        if (!spl_dprefix<ORDER>(1, a)) continue;
+                        double sj = 0.0;
+#pragma unroll
+                        for (int i = 0; i < 4; ++i) sj = fma(v[i], b[0][a][i], sj);
+#pragma unroll
+                        for (int e = 0; e < NS; ++e)
+                            if (spl_dprefix<ORDER>(2, a, e)) sk[a][e] = fma(sj, b[1][e][j], sk[a][e]);
+                    }
+                }
+#pragma unroll
+                for (int a = 0; a < NS; ++a)
+#pragma unroll
+                    for (int e = 0; e < NS; ++e)
+#pragma unroll
+                        for (int g = 0; g < NS; ++g)
+                            if (spl_dprefix<ORDER>(3, a, e, g)) sl[a][e][g] = fma(sk[a][e], b[2][g][k], sl[a][e][g]);
+            }
+#pragma unroll
+            for (int a = 0; a < NS; ++a)
+#pragma unroll
+                for (int e = 0; e < NS; ++e)
+#pragma unroll
+                    for (int g = 0; g < NS; ++g)
+#pragma unroll
+                        for (int h = 0; h < NS; ++h) {
+                            const int c = spl_dcomp<4, ORDER, VSET>(a, e, g, h);
+                            if (c >= 0) res[c] = fma(sl[a][e][g], b[3][h][l], res[c]);
+                        }
+        }
+    }
+}
+
+// one query, exact form (bascmp's node-by-node formulas): the ncomp results to o[0 .. ncomp-1]
+template <int NDIM, int ORDER>
+__device__ __forceinline__ void spl_eval_derivs_point(const GridParams &gp, const TableLayout &tl,
+                                                      const double *__restrict__ cf, const double *xv,
+                                                      real_t *__restrict__ o) {
+    constexpr int NS = ORDER + 2;
+    double b[NDIM][NS][4];
+    int ws[NDIM];
+#pragma unroll
+    for (int d = 0; d < NDIM; ++d) {
+#pragma unroll
+        for (int s = 0; s <= ORDER; ++s)
+            spl_window_weights(xv[d], gp.xmin[d], gp.dx[d], gp.dxin[d], gp.nodes[d], s, ws[d], b[d][s]);
+        spl_window_weights_value<true>(xv[d], gp.xmin[d], gp.dx[d], gp.dxin[d], gp.nodes[d], ws[d], b[d][ORDER + 1]);
+    }
+    const double *p0 = cf + ws[0];
+    if constexpr (NDIM >= 2) p0 += tl.s1 * ws[1];
+    if constexpr (NDIM >= 3) p0 += (long long)tl.s2 * ws[2];
+    if constexpr (NDIM >= 4) p0 += tl.s3 * ws[3];
+    double res[spl_ncomp(NDIM, ORDER)];
+    spl_contract_multi<NDIM, ORDER, NS>(tl, p0, b, res);
+    // the value as spl_eval_point<VALUE = true>: 8^-ndim, and 0 for a NaN coordinate
+    res[0] *= 1.0 / (double)spl_ipow(8, NDIM);
+    bool isnan_q = false;
+#pragma unroll
+    for (int d = 0; d < NDIM; ++d) isnan_q |= (xv[d] != xv[d]);
+    if (isnan_q) res[0] = 0.0;
+#pragma unroll
+    for (int c = 0; c < spl_ncomp(NDIM, ORDER); ++c) o[c] = (real_t)res[c];
+}
+// one query, uniform form, from its fractional coordinates and window base (spl_uni_locate); scale[c]: the factor
+// spl_uni_scale gives component c
+template <int NDIM, int ORDER>
+__device__ __forceinline__ void spl_eval_derivs_uni_at(const TableLayout &tl, const double *__restrict__ cf,
+                                                       const double *f, unsigned base, const double *scale,
+                                                       real_t *__restrict__ o) {
+    constexpr int NS = ORDER + 1;
+    double b[NDIM][NS][4];
+    const bool oob = (base & SPL_UNI_OOB) != 0u;
+#pragma unroll
+    for (int d = 0; d < NDIM; ++d)
+#pragma unroll
+        for (int s = 0; s < NS; ++s) spl_uni_weights<false>(f[d], oob, s, b[d][s]);
+    double res[spl_ncomp(NDIM, ORDER)];
+    spl_contract_multi<NDIM, ORDER, NS>(tl, cf + (base & ~SPL_UNI_OOB), b, res);
+    bool isnan_q = false;
+#pragma unroll
+    for (int d = 0; d < NDIM; ++d) isnan_q |= (f[d] != f[d]);
+#pragma unroll
+    for (int c = 0; c < spl_ncomp(NDIM, ORDER); ++c) o[c] = (real_t)(isnan_q ? 0.0 : res[c] * scale[c]);
+}
+// spl_uni_scale of every component, same multiplication order (one entry per thread c < ncomp)
+template <int NDIM, int ORDER>
+__device__ __forceinline__ double spl_uni_dscale(const GridParams &gp, int c) {
+    double sc = 1.0 / (double)spl_ipow(4, NDIM);
+#pragma unroll
+    for (int d = 0; d < NDIM; ++d) {
+        const int nd = spl_dorder(NDIM, c, d);
+        if (nd >= 1) sc *= gp.dxin[d];
+        if (nd >= 2) sc *= gp.dxin[d];
+    }
+    return sc;
+}
+
+// threads per CTA of the plain kernel; ORDER > 0: the derivative sets, which carry (ORDER + 1..2) x 4 weights per dimension
+// and up to 15 accumulators -- sized so that ptxas needs no spills (eval.ptxas.log)
+template <int NDIM, int ORDER = 0> struct EvalCfg {
+    static constexpr int THREADS = ORDER == 0 ? ((NDIM <= 3) ? 1024 : 512) : (NDIM <= 2 ? 512 : 256);
 };
 
 // ------------------------------------------------------------------------------------------
@@ -242,20 +490,25 @@ template <int NDIM> struct EvalCfg {
 // ------------------------------------------------------------------------------------------
 #define EVAL_WCHUNK 256   // queries a warp claims per atomic (8 per lane)
 
-template <int NDIM, bool SMEM, bool VALUE, bool UNI = false>
-__global__ void __launch_bounds__(EvalCfg<NDIM>::THREADS, 1)
+// ORDER > 0: the derivative sets of spl_eval_derivs_point / spl_eval_derivs_uni_at, out(ncomp, nq); VALUE is false
+template <int NDIM, bool SMEM, bool VALUE, bool UNI = false, int ORDER = 0>
+__global__ void __launch_bounds__(EvalCfg<NDIM, ORDER>::THREADS, 1)
 spl_eval_kernel(const __grid_constant__ GridParams gp, const DerivParams dp, const TableLayout tl,
                 const real_t *__restrict__ x, int l1x, long long nq,
                 const double *__restrict__ coef, long long ncol_padded, real_t *__restrict__ out,
                 unsigned long long *__restrict__ chunk_counter, const int *__restrict__ order_flag) {
+    constexpr int NC = ORDER > 0 ? spl_ncomp(NDIM, ORDER) : 1;
     extern __shared__ __align__(128) double s_dyn[];
     __shared__ __align__(8) uint64_t mbar;
     __shared__ unsigned long long s_chunk;
+    __shared__ double s_dscale[NC];
     // order_flag (spl_eval_probe_kernel): 1 = the batch is scattered and the regrouping kernel evaluates it
     if (order_flag && *order_flag == 1) return;
     const int tid = threadIdx.x;
     const int lane = tid & 31;
     if (tid == 0) s_chunk = 0ULL;
+    if constexpr (ORDER > 0 && UNI)
+        if (tid < NC) s_dscale[tid] = spl_uni_dscale<NDIM, ORDER>(gp, tid);
     if (!SMEM) __syncthreads();
     const double *cf = coef;
     const double uscale = UNI ? spl_uni_scale<NDIM>(gp, dp, VALUE) : 1.0;
@@ -322,7 +575,15 @@ spl_eval_kernel(const __grid_constant__ GridParams gp, const DerivParams dp, con
 #pragma unroll
             for (int k = 0; k < KQ; ++k) {
                 const long long q = cbase + k * 32 + lane;
-                if (q < q_hi) out[q] = (real_t)spl_eval_point_uni<NDIM, VALUE>(gp, dp, tl, cf, cur[k], uscale);
+                if constexpr (ORDER > 0) {
+                    if (q < q_hi) {
+                        double f[NDIM];
+                        const unsigned base = spl_uni_locate<NDIM>(gp, tl, cur[k], f);
+                        spl_eval_derivs_uni_at<NDIM, ORDER>(tl, cf, f, base, s_dscale, out + q * NC);
+                    }
+                } else if (q < q_hi) {
+                    out[q] = (real_t)spl_eval_point_uni<NDIM, VALUE>(gp, dp, tl, cf, cur[k], uscale);
+                }
             }
         }
         return;
@@ -355,9 +616,20 @@ spl_eval_kernel(const __grid_constant__ GridParams gp, const DerivParams dp, con
 #pragma unroll
                 for (int d = 0; d < NDIM; ++d) xn[d] = (q2 < q_hi) ? (double)x[q2 * (long long)l1x + d] : 0.0;
             }
-            if (q < q_hi)
+            if constexpr (ORDER > 0) {
+                if (q < q_hi) {
+                    if (UNI) {
+                        double f[NDIM];
+                        const unsigned base = spl_uni_locate<NDIM>(gp, tl, xv, f);
+                        spl_eval_derivs_uni_at<NDIM, ORDER>(tl, cf, f, base, s_dscale, out + q * NC);
+                    } else {
+                        spl_eval_derivs_point<NDIM, ORDER>(gp, tl, cf, xv, out + q * NC);
+                    }
+                }
+            } else if (q < q_hi) {
                 out[q] = UNI ? (real_t)spl_eval_point_uni<NDIM, VALUE>(gp, dp, tl, cf, xv, uscale)
                              : (real_t)spl_eval_point<NDIM, VALUE>(gp, dp, tl, cf, xv);
+            }
         }
     }
 }
@@ -367,9 +639,10 @@ spl_eval_kernel(const __grid_constant__ GridParams gp, const DerivParams dp, con
 // ------------------------------------------------------------------------------------------
 #define RG_CHUNK 256u     // raw queries a warp claims from its CTA's range per shared-memory atomic
 
-template <int NDIM> struct RegroupCfg {
-    // warps per CTA (one CTA per SM): the register budget per thread is 64 K / threads
-    static constexpr int NWARPS = (NDIM <= 2) ? 32 : (NDIM == 3 ? 24 : 16);
+template <int NDIM, int ORDER = 0> struct RegroupCfg {
+    // warps per CTA (one CTA per SM): the register budget per thread is 64 K / threads; the derivative sets (ORDER > 0)
+    // need more registers than the value kernel, so fewer warps (and deeper FIFOs: regroup_plan)
+    static constexpr int NWARPS = ORDER == 0 ? ((NDIM <= 2) ? 32 : (NDIM == 3 ? 24 : 16)) : (NDIM <= 2 ? 16 : 8);
 };
 
 // Order probe: are the queries scattered (regrouping kernel) or do they arrive in coherent runs, e.g. the raster order of
@@ -484,18 +757,23 @@ __global__ void spl_uni_table_kernel(const __grid_constant__ GridParams gp, cons
     }
 }
 
-template <int NDIM, bool VALUE, int NWARPS = RegroupCfg<NDIM>::NWARPS, bool UNI = false>
+// ORDER > 0: the derivative sets, out(ncomp, nq), as spl_eval_kernel
+template <int NDIM, bool VALUE, int NWARPS = RegroupCfg<NDIM>::NWARPS, bool UNI = false, int ORDER = 0>
 __global__ void __launch_bounds__(NWARPS * 32, 1)
 spl_eval_regroup_kernel(const __grid_constant__ GridParams gp, const DerivParams dp, const TableLayout tl,
                         const real_t *__restrict__ x, int l1x, long long nq,
                         const double *__restrict__ coef_padded, unsigned table_doubles, int cap,
                         real_t *__restrict__ out, const int *__restrict__ order_flag) {
+    constexpr int NC = ORDER > 0 ? spl_ncomp(NDIM, ORDER) : 1;
     extern __shared__ __align__(128) double s_dyn[];
     __shared__ __align__(8) uint64_t mbar;
     __shared__ unsigned s_chunk;
+    __shared__ double s_dscale[NC];
     // order_flag (spl_eval_probe_kernel): 0 = the batch arrives in coherent runs and the plain kernel evaluates it
     if (order_flag && *order_flag == 0) return;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if constexpr (ORDER > 0 && UNI)
+        if (tid < NC) s_dscale[tid] = spl_uni_dscale<NDIM, ORDER>(gp, tid);
     if (tid == 0) {
         s_chunk = 0;
         mbar_init(&mbar, 1);
@@ -520,7 +798,7 @@ spl_eval_regroup_kernel(const __grid_constant__ GridParams gp, const DerivParams
     const long long q_hi = nq * ((long long)blockIdx.x + 1) / (long long)gridDim.x;
     const unsigned range = (unsigned)(q_hi - q_lo);
     const real_t *xb = x + q_lo * (long long)l1x;
-    real_t *ob = out + q_lo;
+    real_t *ob = out + q_lo * NC;
 
     const unsigned full = 0xffffffffu, lt = (1u << lane) - 1u;
     const int dc = lane & 15, hf = lane >> 4;                        // dedicated class, half-warp
@@ -649,7 +927,12 @@ spl_eval_regroup_kernel(const __grid_constant__ GridParams gp, const DerivParams
             __syncwarp();
         }
         refill();
-        if (take) {
+        if constexpr (ORDER > 0) {
+            if (take) {
+                if (UNI) spl_eval_derivs_uni_at<NDIM, ORDER>(tl, cf, ex, ebase, s_dscale, ob + (size_t)etag * NC);
+                else spl_eval_derivs_point<NDIM, ORDER>(gp, tl, cf, ex, ob + (size_t)etag * NC);
+            }
+        } else if (take) {
             if (UNI) ob[etag] = (real_t)spl_eval_point_uni_at<NDIM, VALUE>(dp, tl, cf, ex, ebase, uscale);
             else ob[etag] = (real_t)spl_eval_point<NDIM, VALUE>(gp, dp, tl, cf, ex);
         }
@@ -696,7 +979,9 @@ static double class_pmax(const GridParams &gp, const long long *st, bool uni, in
     return m;
 }
 // warps per CTA of the regrouping kernel (SPLPAK_B200_RG_WARPS = 16 | 24 | 32 overrides the default for experiments)
-static int regroup_warps(int ndim, bool uni) {
+static int regroup_warps(int ndim, bool uni, int order) {
+    if (order == 1) return ndim == 2 ? RegroupCfg<2, 1>::NWARPS : (ndim == 3 ? RegroupCfg<3, 1>::NWARPS : RegroupCfg<4, 1>::NWARPS);
+    if (order == 2) return ndim == 2 ? RegroupCfg<2, 2>::NWARPS : (ndim == 3 ? RegroupCfg<3, 2>::NWARPS : RegroupCfg<4, 2>::NWARPS);
     int nw = ndim == 2 ? RegroupCfg<2>::NWARPS : (ndim == 3 ? RegroupCfg<3>::NWARPS : RegroupCfg<4>::NWARPS);
     // uniform form, 3-D: the larger extended table leaves less room for the FIFOs; 16 warps keep them 9 deep
     // (measured 8 / 12 / 16 / 24 / 32 warps: 28.4 / 24.2 / 22.9 / 24.3 / 24.1 ms per 1e9 scattered queries)
@@ -708,11 +993,12 @@ static int regroup_warps(int ndim, bool uni) {
     return nw;
 }
 // f32: the float kernel of the REAL32 library (uniform form only): 4-byte table entries, 32 bank classes, one FIFO
-// column per lane
-static const RegroupPlan &regroup_plan(const GridParams &gp, size_t smem_optin, bool uni, bool f32 = false) {
-    static thread_local RegroupPlan plans[3];
-    RegroupPlan &plan = plans[f32 ? 2 : (uni ? 1 : 0)];
-    const int nwarps = f32 ? 16 : regroup_warps(gp.ndim, uni);
+// column per lane.  order: 0 = single-component evaluation, 1 / 2 = the derivative-set kernels (their own warp counts,
+// so a plan per order is cached and alternating value and derivative calls do not redo the search)
+static const RegroupPlan &regroup_plan(const GridParams &gp, size_t smem_optin, bool uni, bool f32 = false, int order = 0) {
+    static thread_local RegroupPlan plans[7];
+    RegroupPlan &plan = plans[f32 ? 6 : 2 * order + (uni ? 1 : 0)];
+    const int nwarps = f32 ? 16 : regroup_warps(gp.ndim, uni, order);
     bool same = plan.key_ndim == gp.ndim && plan.key_smem == smem_optin && plan.key_warps == nwarps;
     for (int d = 0; d < SPL_MAXDIM && same; ++d) same = plan.key_nodes[d] == gp.nodes[d];
     if (same) return plan;
@@ -827,10 +1113,29 @@ static EvalRoute eval_route(const GridParams &gp, const int *nderiv, long long n
     }
     return r;
 }
+// derivative sets of order 1 / 2: the same decisions as a single-component batch -- in particular the same basis form,
+// so that every component is bit-identical to it -- with the regrouping plan of the derivative kernels; when that plan
+// does not fit, the plain kernel in the SAME form
+static EvalRoute eval_route_derivs(const GridParams &gp, int order, long long nq, int nsm, size_t smem_optin) {
+    EvalRoute r = eval_route(gp, nullptr, nq, nsm, smem_optin);
+    if (!r.regroup) return r;
+    const RegroupPlan &pl = regroup_plan(gp, smem_optin, r.uni, false, order);
+    if (pl.ok) {
+        r.tl = pl.tl;
+        r.table_doubles = pl.table_doubles;
+        return r;
+    }
+    r.regroup = r.force_regroup = false;
+    r.tl = natural_layout(gp, r.uni ? 2 : 0);
+    r.table_doubles = r.uni ? natural_doubles(gp, 2) : 0;
+    return r;
+}
 
 // doubles of device scratch the evaluation of this batch needs behind the caller's table (+ 2 for the order flag): the
-// extended and/or padded copy of the table.  0: none.
-long long spl_eval_scratch_elems(const GridParams &gp, const int *nderiv, long long nq, int nsm, size_t smem_optin) {
+// extended and/or padded copy of the table.  0: none.  order 1 / 2: the derivative sets (nderiv unused)
+long long spl_eval_scratch_elems(const GridParams &gp, const int *nderiv, int order, long long nq, int nsm,
+                                 size_t smem_optin) {
+    if (order > 0) return eval_route_derivs(gp, order, nq, nsm, smem_optin).table_doubles;
     return eval_route(gp, nderiv, nq, nsm, smem_optin).table_doubles;
 }
 // the exact-form regrouping kernel alone (REAL32 library, 4-D): 0 or the number of doubles of its padded table
@@ -855,21 +1160,23 @@ static void launch_table(const GridParams &gp, const TableLayout &tl, long long 
 }
 
 // d_tab: the table image launch_table() made for this plan
-template <int NDIM, bool VALUE, bool UNI>
+template <int NDIM, bool VALUE, bool UNI, int ORDER = 0>
 static int launch_eval_regroup(const GridParams &gp, const DerivParams &dp, const real_t *d_x, int l1x, long long nq,
                                const double *d_tab, real_t *d_out, cudaStream_t stream, int nsm,
                                size_t smem_optin, int *d_flag) {
-    const RegroupPlan &pl = regroup_plan(gp, smem_optin, UNI);
+    const RegroupPlan &pl = regroup_plan(gp, smem_optin, UNI, false, ORDER);
     if (d_flag) {
         spl_eval_probe_kernel<NDIM, UNI><<<1, 1024, 0, stream>>>(gp, pl.tl, d_x, l1x, nq, d_flag);
         ++g_spl_launches;
     }
     void (*kern)(GridParams, DerivParams, TableLayout, const real_t *, int, long long, const double *, unsigned, int,
-                 real_t *, const int *) = spl_eval_regroup_kernel<NDIM, VALUE, RegroupCfg<NDIM>::NWARPS, UNI>;
-    if (NDIM == 3 && pl.nwarps == 8) kern = spl_eval_regroup_kernel<NDIM, VALUE, (NDIM == 3 ? 8 : RegroupCfg<NDIM>::NWARPS), UNI>;
-    if (NDIM == 3 && pl.nwarps == 12) kern = spl_eval_regroup_kernel<NDIM, VALUE, (NDIM == 3 ? 12 : RegroupCfg<NDIM>::NWARPS), UNI>;
-    if (NDIM == 3 && pl.nwarps == 16) kern = spl_eval_regroup_kernel<NDIM, VALUE, (NDIM == 3 ? 16 : RegroupCfg<NDIM>::NWARPS), UNI>;
-    if (NDIM == 3 && pl.nwarps == 32) kern = spl_eval_regroup_kernel<NDIM, VALUE, (NDIM == 3 ? 32 : RegroupCfg<NDIM>::NWARPS), UNI>;
+                 real_t *, const int *) = spl_eval_regroup_kernel<NDIM, VALUE, RegroupCfg<NDIM, ORDER>::NWARPS, UNI, ORDER>;
+    if constexpr (ORDER == 0) {
+        if (NDIM == 3 && pl.nwarps == 8) kern = spl_eval_regroup_kernel<NDIM, VALUE, (NDIM == 3 ? 8 : RegroupCfg<NDIM>::NWARPS), UNI>;
+        if (NDIM == 3 && pl.nwarps == 12) kern = spl_eval_regroup_kernel<NDIM, VALUE, (NDIM == 3 ? 12 : RegroupCfg<NDIM>::NWARPS), UNI>;
+        if (NDIM == 3 && pl.nwarps == 16) kern = spl_eval_regroup_kernel<NDIM, VALUE, (NDIM == 3 ? 16 : RegroupCfg<NDIM>::NWARPS), UNI>;
+        if (NDIM == 3 && pl.nwarps == 32) kern = spl_eval_regroup_kernel<NDIM, VALUE, (NDIM == 3 ? 32 : RegroupCfg<NDIM>::NWARPS), UNI>;
+    }
     SPL_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem));
     long long grid = nsm;
     const long long per_cta_min = 4096;                 // tiny batches: fewer CTAs, each with a useful range
@@ -1375,12 +1682,12 @@ int spl_eval_f32_mixed4_launch(const GridParams &gp, const real_t *d_x, int l1x,
 // host side
 // ------------------------------------------------------------------------------------------
 // d_tab: the table the kernel reads, tab_doubles (even) entries laid out as tl
-template <int NDIM, bool VALUE, bool UNI>
+template <int NDIM, bool VALUE, bool UNI, int ORDER = 0>
 static int launch_eval(const GridParams &gp, const DerivParams &dp, const TableLayout &tl, const real_t *d_x, int l1x,
                        long long nq, const double *d_tab, long long tab_doubles, real_t *d_out,
                        cudaStream_t stream, int nsm, size_t smem_optin, unsigned long long *d_counter,
                        const int *d_flag = nullptr) {
-    constexpr int THREADS = EvalCfg<NDIM>::THREADS;
+    constexpr int THREADS = EvalCfg<NDIM, ORDER>::THREADS;
     const size_t coef_bytes = (size_t)tab_doubles * sizeof(double);
     const size_t static_reserve = 2048;
     SPL_CUDA_TRY(cudaMemsetAsync(d_counter, 0, sizeof(unsigned long long), stream));
@@ -1391,14 +1698,14 @@ static int launch_eval(const GridParams &gp, const DerivParams &dp, const TableL
     long long ctas = (chunks + THREADS / 32 - 1) / (THREADS / 32);
     if (ctas < 1) ctas = 1;
     if (use_smem) {
-        auto kern = spl_eval_kernel<NDIM, true, VALUE, UNI>;
+        auto kern = spl_eval_kernel<NDIM, true, VALUE, UNI, ORDER>;
         SPL_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coef_bytes));
         long long grid = nsm;
         if (grid > ctas) grid = ctas;
         kern<<<(unsigned)grid, THREADS, coef_bytes, stream>>>(gp, dp, tl, d_x, l1x, nq, d_tab, tab_doubles, d_out,
                                                               d_counter, d_flag);
     } else {
-        auto kern = spl_eval_kernel<NDIM, false, VALUE, UNI>;
+        auto kern = spl_eval_kernel<NDIM, false, VALUE, UNI, ORDER>;
         long long grid = (long long)nsm * (2048 / THREADS);
         if (grid > ctas) grid = ctas;
         kern<<<(unsigned)grid, THREADS, 0, stream>>>(gp, dp, tl, d_x, l1x, nq, d_tab, tab_doubles, d_out, d_counter, d_flag);
@@ -1408,7 +1715,7 @@ static int launch_eval(const GridParams &gp, const DerivParams &dp, const TableL
     return SPLPAK_OK;
 }
 
-template <int NDIM, bool VALUE, bool UNI>
+template <int NDIM, bool VALUE, bool UNI, int ORDER = 0>
 static int eval_dispatch(const GridParams &gp, const DerivParams &dp, const EvalRoute &rt, const real_t *d_x, int l1x,
                          long long nq, const double *d_coef, long long ncol_padded, real_t *d_out, cudaStream_t stream,
                          int nsm, size_t smem_optin, unsigned long long *d_counter, double *d_scratch) {
@@ -1424,47 +1731,48 @@ static int eval_dispatch(const GridParams &gp, const DerivParams &dp, const Eval
             // forced ("regroup"): the regrouping kernel alone.  Default: order probe, then BOTH kernels -- the probe's flag
             // (behind the table image in d_scratch) makes the wrong one exit immediately.
             int *d_flag = rt.force_regroup ? nullptr : reinterpret_cast<int *>(d_scratch + rt.table_doubles);
-            int rc = launch_eval_regroup<NDIM, VALUE, UNI>(gp, dp, d_x, l1x, nq, tab, d_out, stream, nsm, smem_optin, d_flag);
+            int rc = launch_eval_regroup<NDIM, VALUE, UNI, ORDER>(gp, dp, d_x, l1x, nq, tab, d_out, stream, nsm, smem_optin, d_flag);
             if (rc != SPLPAK_OK || !d_flag) return rc;
             // the plain kernel reads the same (padded) image when it is the extended table; the exact form reads the caller's
-            if (UNI) return launch_eval<NDIM, VALUE, UNI>(gp, dp, rt.tl, d_x, l1x, nq, tab, tab_doubles, d_out, stream, nsm,
-                                                          smem_optin, d_counter, d_flag);
-            return launch_eval<NDIM, VALUE, false>(gp, dp, natural_layout(gp, 0), d_x, l1x, nq, d_coef, ncol_padded, d_out,
-                                                   stream, nsm, smem_optin, d_counter, d_flag);
+            if (UNI) return launch_eval<NDIM, VALUE, UNI, ORDER>(gp, dp, rt.tl, d_x, l1x, nq, tab, tab_doubles, d_out, stream,
+                                                                 nsm, smem_optin, d_counter, d_flag);
+            return launch_eval<NDIM, VALUE, false, ORDER>(gp, dp, natural_layout(gp, 0), d_x, l1x, nq, d_coef, ncol_padded,
+                                                          d_out, stream, nsm, smem_optin, d_counter, d_flag);
         }
     }
-    return launch_eval<NDIM, VALUE, UNI>(gp, dp, rt.tl, d_x, l1x, nq, tab, tab_doubles, d_out, stream, nsm, smem_optin,
-                                         d_counter);
+    return launch_eval<NDIM, VALUE, UNI, ORDER>(gp, dp, rt.tl, d_x, l1x, nq, tab, tab_doubles, d_out, stream, nsm,
+                                                smem_optin, d_counter);
 }
 
 // d_coef: float64 device table with ncol_padded (even, >= ncol) entries; d_counter: 8-byte scratch; d_scratch: scratch of
 // spl_eval_scratch_elems() + 2 doubles (or NULL when that is 0, or when the allocation failed: exact plain kernel).
-int spl_eval_launch(const GridParams &gp, const int *nderiv, const real_t *d_x, int l1x, long long nq,
+// order 0: one output per query, the derivative nderiv (NULL: splfe); order 1 / 2: the derivative sets, out(ncomp, nq).
+int spl_eval_launch(const GridParams &gp, const int *nderiv, int order, const real_t *d_x, int l1x, long long nq,
                     const double *d_coef, long long ncol_padded, real_t *d_out, cudaStream_t stream,
                     int nsm, size_t smem_optin, unsigned long long *d_counter, double *d_scratch) {
     DerivParams dp;
     bool value = true;
     for (int d = 0; d < SPL_MAXDIM; ++d) {
-        dp.nd[d] = (nderiv && d < gp.ndim) ? nderiv[d] : 0;
+        dp.nd[d] = (nderiv && d < gp.ndim && order == 0) ? nderiv[d] : 0;
         if (dp.nd[d] != 0) value = false;
     }
     if (nq <= 0) return SPLPAK_OK;
-    EvalRoute rt = eval_route(gp, nderiv, nq, nsm, smem_optin);
+    if (order < 0 || order > 2) return SPLPAK_ERR_NDERIV;
+    EvalRoute rt = order > 0 ? eval_route_derivs(gp, order, nq, nsm, smem_optin) : eval_route(gp, nderiv, nq, nsm, smem_optin);
     if (!d_scratch && rt.table_doubles > 0) {
         rt = EvalRoute();                         // no scratch: the exact plain kernel on the caller's table
         rt.tl = natural_layout(gp, 0);
     }
+#define SPL_EVAL_ARGS gp, dp, rt, d_x, l1x, nq, d_coef, ncol_padded, d_out, stream, nsm, smem_optin, d_counter, d_scratch
 #define SPL_EVAL_CASE(N)                                                                                              \
     case N:                                                                                                           \
+        if (order == 1)                                                                                               \
+            return rt.uni ? eval_dispatch<N, false, true, 1>(SPL_EVAL_ARGS) : eval_dispatch<N, false, false, 1>(SPL_EVAL_ARGS); \
+        if (order == 2)                                                                                               \
+            return rt.uni ? eval_dispatch<N, false, true, 2>(SPL_EVAL_ARGS) : eval_dispatch<N, false, false, 2>(SPL_EVAL_ARGS); \
         if (rt.uni)                                                                                                   \
-            return value ? eval_dispatch<N, true, true>(gp, dp, rt, d_x, l1x, nq, d_coef, ncol_padded, d_out, stream, nsm, \
-                                                        smem_optin, d_counter, d_scratch)                             \
-                         : eval_dispatch<N, false, true>(gp, dp, rt, d_x, l1x, nq, d_coef, ncol_padded, d_out, stream, nsm, \
-                                                         smem_optin, d_counter, d_scratch);                           \
-        return value ? eval_dispatch<N, true, false>(gp, dp, rt, d_x, l1x, nq, d_coef, ncol_padded, d_out, stream, nsm, \
-                                                     smem_optin, d_counter, d_scratch)                                \
-                     : eval_dispatch<N, false, false>(gp, dp, rt, d_x, l1x, nq, d_coef, ncol_padded, d_out, stream, nsm, \
-                                                      smem_optin, d_counter, d_scratch);
+            return value ? eval_dispatch<N, true, true>(SPL_EVAL_ARGS) : eval_dispatch<N, false, true>(SPL_EVAL_ARGS);    \
+        return value ? eval_dispatch<N, true, false>(SPL_EVAL_ARGS) : eval_dispatch<N, false, false>(SPL_EVAL_ARGS);
     switch (gp.ndim) {
         SPL_EVAL_CASE(1)
         SPL_EVAL_CASE(2)
@@ -1472,5 +1780,6 @@ int spl_eval_launch(const GridParams &gp, const int *nderiv, const real_t *d_x, 
         SPL_EVAL_CASE(4)
     }
 #undef SPL_EVAL_CASE
+#undef SPL_EVAL_ARGS
     return SPLPAK_ERR_NDIM;
 }

@@ -91,6 +91,14 @@ public:
         splpak_b200_eval(ndim, x, l1x, nq, nderiv, coef, xmin, xmax, nodes, out, &ierror);
         cfaerr(ierror, true);
     }
+    // every partial derivative up to total order `order` (1 or 2) in one pass: out(ncomp, nq), ncomp = ndim + 1 or
+    // (ndim + 1)(ndim + 2) / 2 (new entry point; component k == evaluate_batch with the nderiv it names)
+    void evaluate_derivs(int ndim, const wp *x, int l1x, std::int64_t nq, int order, const wp *coef, const wp *xmin,
+                         const wp *xmax, const int *nodes, wp *out, int &ierror) {
+        mdim_ = ndim;
+        splpak_b200_eval_derivs(ndim, x, l1x, nq, order, coef, xmin, xmax, nodes, out, &ierror);
+        cfaerr(ierror, true);
+    }
 
 private:
     int mdim_ = 0;
