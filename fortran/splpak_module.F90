@@ -61,6 +61,7 @@
         procedure,public :: compute                      !! (new) streaming fit: constraints + solve
         procedure,public :: refine                       !! (new) streaming fit: one refinement pass over the same points
         procedure,public :: set_solver                   !! (new) streaming fit: 0 = band Cholesky (default), 1 = orthogonal (Householder)
+        procedure,public :: set_smoothing                !! (new) streaming fit: roughness penalty lambda (0 = curvature, 1 = thin plate)
         procedure,private :: splcc
         procedure,private :: splcw
         procedure,private :: splfe
@@ -195,6 +196,13 @@
             integer(c_int),value :: solver
             integer(c_int) :: rc
         end function c_fit_set_solver
+        function c_fit_set_smoothing(h,lambda,penalty) bind(C,name='splpak_b200_fit_set_smoothing') result(rc)
+            import :: c_int, c_double, c_ptr
+            type(c_ptr),value :: h
+            real(c_double),value :: lambda
+            integer(c_int),value :: penalty
+            integer(c_int) :: rc
+        end function c_fit_set_smoothing
         function c_fit_destroy(h) bind(C,name='splpak_b200_fit_destroy') result(rc)
             import :: c_int, c_ptr
             type(c_ptr),value :: h
@@ -385,6 +393,19 @@
         integer,intent(out) :: ierror
         ierror = int(c_fit_set_solver(me%handle,int(solver,c_int)))
     end subroutine set_solver
+
+    !> (new) smoothing of a streaming fit, after create and before compute: the Cholesky fit adds
+    !  lambda * the integral over [xmin, xmax] of the penalty to the least-squares objective.
+    !  penalty 0 = sum of squared second derivatives (curvature), 1 = thin plate (mixed ones too).
+    !  lambda = 0 (default) is the unsmoothed fit.  ierror = 203 for lambda < 0 or not finite, an
+    !  unknown penalty, or lambda > 0 with the orthogonal solver.
+    subroutine set_smoothing(me,lambda,penalty,ierror)
+        class(splpak_type),intent(inout) :: me
+        real(c_double),intent(in) :: lambda
+        integer,intent(in) :: penalty
+        integer,intent(out) :: ierror
+        ierror = int(c_fit_set_smoothing(me%handle,lambda,int(penalty,c_int)))
+    end subroutine set_smoothing
 
     !> (new) accumulate n more points; wdata absent (or wdata(1)<0) => all weights 1.
     subroutine add_points(me,xdata,l1xdat,ydata,ndata,ierror,wdata)

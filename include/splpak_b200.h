@@ -206,6 +206,19 @@ int splpak_b200_fit_compute_device(splpak_b200_fit_t h, splpak_real *d_coef, int
 #define SPLPAK_SOLVER_ORTHOGONAL 1
 int splpak_b200_fit_set_solver(splpak_b200_fit_t h, int solver);
 int splpak_b200_fit_get_solver(splpak_b200_fit_t h);
+/* Smoothing -- (new) no counterpart in the reference.  The Cholesky fit then minimises
+ *     sum_i (w_i (y_i - s(x_i)))^2  [+ the constraint rows when xtrap != 0]  +  lambda * integral over [xmin, xmax] of P(s)
+ * with P(s) = sum_d (d2s/dx_d^2)^2 (SPLPAK_PENALTY_CURVATURE; multilinear functions are not penalised) or that plus
+ * 2 sum_{i<j} (d2s/dx_i dx_j)^2 (SPLPAK_PENALTY_THIN_PLATE; affine functions are not penalised), in the caller's
+ * coordinates.  fit_compute solves (G + lambda R) c = g; fit_get_normal_equations then returns S + lambda R, and the
+ * refinement steps keep the penalty.  With lambda > 0, fewer points than columns is not an error (the penalty makes the
+ * system well posed); a non-positive pivot still returns 107.  lambda = 0 (the default) is exactly the unsmoothed fit.
+ * The setting persists across fit_reset.  Any time before fit_compute.  Returns 203 for an invalid or finalized handle, for
+ * lambda < 0, NaN or inf, for an unknown penalty, and for lambda > 0 on the orthogonal solver (set_solver(ORTHOGONAL) on a
+ * handle with lambda > 0 returns 203 too). */
+#define SPLPAK_PENALTY_CURVATURE  0
+#define SPLPAK_PENALTY_THIN_PLATE 1
+int splpak_b200_fit_set_smoothing(splpak_b200_fit_t h, double lambda, int penalty);
 /* Parity-test hook of the orthogonal path: which = 0 -> per-window triangles [nwindows][4^ndim][4^ndim + 1] (R_w | z_w),
  * which = 1 -> band factor [ncol][b + 2] (row i: R[i][i..i+b], then (Q^T r)_i).  out may be NULL to query *count. */
 int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity, int64_t *count);
@@ -238,13 +251,14 @@ int splpak_b200_fit_reset(splpak_b200_fit_t h);
 /* cudaStream_t (as void*) the handle launches on. */
 void *splpak_b200_fit_stream(splpak_b200_fit_t h);
 /* Device-time split of everything since create/reset, milliseconds:
- * ms[0] classify+histogram, ms[1] scan+scatter (binning), ms[2] accumulate, ms[3] constraints,
- * ms[4] band expand, ms[5] factor, ms[6] back-substitution.  Synchronises the stream. */
+ * ms[0] classify+histogram, ms[1] scan+scatter (binning), ms[2] accumulate, ms[3] constraints (and, with smoothing,
+ * the penalty tables and S += lambda R), ms[4] band expand, ms[5] factor, ms[6] back-substitution.  Synchronises the stream. */
 int splpak_b200_fit_timings(splpak_b200_fit_t h, double *ms, int n);
 /* Kernels this handle has launched since create/reset (for bench.py's gpu_launches). */
 int64_t splpak_b200_fit_launch_count(splpak_b200_fit_t h);
 /* Debug/parity access: copy the assembled G (stencil storage, ncol*4^ndim float64), g (ncol),
- * node histogram (ncol) and [totlwt, nrows] to HOST arrays (any may be NULL). */
+ * node histogram (ncol) and [totlwt, nrows] to HOST arrays (any may be NULL).  After a compute with smoothing
+ * (lambda > 0), S holds G + lambda R. */
 int splpak_b200_fit_get_normal_equations(splpak_b200_fit_t h, double *S, double *g, double *cnt,
                                          double *totals);
 int splpak_b200_fit_destroy(splpak_b200_fit_t h);

@@ -317,6 +317,21 @@ class FitHandle:
         self._check()
         return {0: "cholesky", 1: "orthogonal"}.get(self.lib.splpak_b200_fit_get_solver(self.h))
 
+    PENALTIES = {"curvature": 0, "thin_plate": 1}
+
+    def set_smoothing(self, lam, penalty="curvature"):
+        """Smoothing of the Cholesky fit: minimise the weighted squared residuals (+ the constraint rows) + lam times the
+        integral over [xmin, xmax] of the penalty, "curvature" (sum of squared second derivatives d2s/dx_d^2) or
+        "thin_plate" (that + 2 x the squared mixed second derivatives).  Any time before compute; persists across reset.
+        Returns the library code: 203 for lam < 0, NaN or inf, an unknown penalty code, a finalized handle, or lam > 0
+        with the orthogonal solver.  An unknown penalty name raises SplpakError."""
+        self._check()
+        if isinstance(penalty, str):
+            if penalty not in self.PENALTIES:
+                raise SplpakError(f"unknown penalty {penalty!r}: expected one of {sorted(self.PENALTIES)}")
+            penalty = self.PENALTIES[penalty]
+        return self.lib.splpak_b200_fit_set_smoothing(self.h, float(lam), int(penalty))
+
     def orthogonal_factor(self, which):
         """Parity-test hook: which = 0 -> per-window triangles (nwindows, 4^ndim, 4^ndim + 1); 1 -> band factor (ncol, b + 2)."""
         self._check()

@@ -4,6 +4,7 @@
 // usable CUDA device every compute entry point returns SPLPAK_ERR_CUDA.
 #include <condition_variable>
 #include <dlfcn.h>
+#include <math.h>
 #include <mutex>
 #include <new>
 #include <stdlib.h>
@@ -58,6 +59,11 @@ int spl_resolve_launch(const GridParams &gp, const double *d_AB, double *d_g, do
 int spl_constraints_residual_launch(const GridParams &gp, double xtrap, const double *d_cnt,
                                     const double *d_totals_in, const double *d_coef, double *d_g,
                                     cudaStream_t st, int nsm);
+long long spl_penalty_table_len(const GridParams &gp);
+int spl_penalty_add_launch(const GridParams &gp, double lambda, int penalty, double *d_tab, double *d_S,
+                           cudaStream_t st, int nsm);
+int spl_penalty_residual_launch(const GridParams &gp, double lambda, int penalty, const double *d_tab,
+                                const double *d_coef, double *d_g, cudaStream_t st, int nsm);
 int spl_measure_peaks_impl(double *out, int n);
 int spl_ortho_supported(const GridParams &gp);
 void spl_ortho_free(OrthoScratch &os);
@@ -919,6 +925,10 @@ struct splpak_b200_fit_s {
     real_t *d_out_tmp;            // ncol reals: working-precision copy of the solution for the D2H of real32 builds
     int refining;
     int constraints_fired;        // derivative-constraint rows were added by compute
+    // smoothing (penalty.cu): lambda * R is added to S by compute when lambda > 0; kept across fit_reset
+    double lambda;
+    int penalty;                  // SPLPAK_PENALTY_CURVATURE or SPLPAK_PENALTY_THIN_PLATE
+    double *d_pen;                // 1-D penalty tables (spl_penalty_table_len doubles), allocated by the first lambda > 0
     // timing: accumulated event pairs
     double ms[NTIMER];
     cudaEvent_t ev[12];           // 0-3 assembly, 4-5 constraints, 8-11 solve stages
@@ -956,6 +966,7 @@ static void free_handle(splpak_b200_fit_t h) {
     if (h->d_res) cudaFree(h->d_res);
     if (h->d_dummy_tot) cudaFree(h->d_dummy_tot);
     if (h->d_out_tmp) cudaFree(h->d_out_tmp);
+    if (h->d_pen) cudaFree(h->d_pen);
     if (h->os) {
         spl_ortho_free(*h->os);
         delete h->os;
@@ -1435,6 +1446,16 @@ static int fit_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_on_devic
             return rc;
         }
     }
+    // smoothing: S += lambda R after the constraint rows (and the fixed-point finish of the deterministic mode); after the
+    // all-reduce of a multi-GPU fit, so the penalty counts once.  Timed in the constraints slot.
+    if (h->lambda > 0.0) {
+        rc = spl_penalty_add_launch(gp, h->lambda, h->penalty, h->d_pen, h->d_S, st, h->di.nsm);
+        if (rc != SPLPAK_OK) {
+            h->finalized = 1;
+            if (ierror) *ierror = rc;
+            return rc;
+        }
+    }
     FC_TRY(cudaEventRecord(h->ev[5], st));
     FC_TRY(cudaMemsetAsync(h->d_AB, 0, sizeof(double) * (size_t)need, st));
     FC_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
@@ -1474,8 +1495,9 @@ static int fit_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_on_devic
         add_ms(h, 4, sev[0], sev[1]);
         add_ms(h, 5, sev[1], sev[2]);
         add_ms(h, 6, sev[2], sev[3]);
-        // fewer rows than columns (suprls error 33, :1650) or a non-positive pivot -> 107
-        if (fail || totals[1] < (double)gp.ncol) rc = SPLPAK_ERR_SOLVER;
+        // fewer rows than columns (suprls error 33, :1650; not an error with smoothing, whose penalty makes such a fit
+        // well posed) or a non-positive pivot -> 107
+        if (fail || (h->lambda == 0.0 && totals[1] < (double)gp.ncol)) rc = SPLPAK_ERR_SOLVER;
         h->solved = (rc == SPLPAK_OK);
         h->cond_est = (prange[0] > 0.0 && prange[1] > 0.0) ? (prange[1] / prange[0]) * (prange[1] / prange[0]) : 0.0;
         h->factor_valid = h->solved;
@@ -1611,6 +1633,14 @@ static int fit_refine_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_o
                 return rc;
             }
         }
+        if (h->lambda > 0.0) {
+            // the penalty's share of the residual, -lambda R c: without it the steps would converge to the unsmoothed fit
+            rc = spl_penalty_residual_launch(gp, h->lambda, h->penalty, h->d_pen, h->d_coef64, h->d_g, st, h->di.nsm);
+            if (rc != SPLPAK_OK) {
+                if (ierror) *ierror = rc;
+                return rc;
+            }
+        }
         const int bw = spl_half_bandwidth(gp);
         const long long lda = spl_band_lda(bw);
         const long long band_elems = (gp.ncol * (lda + 1) + 64 + 1) & ~1LL;     // even: the workspace behind stays 16-byte aligned
@@ -1672,13 +1702,29 @@ extern "C" int splpak_b200_fit_set_solver(splpak_b200_fit_t h, int solver) {
         h->solver = solver;
         return SPLPAK_OK;
     }
-    if (solver == SPLPAK_SOLVER_ORTHOGONAL && spl_ortho_supported(h->gp)) {
+    // the penalty couples nodes across the windows of the orthogonal path: no smoothing there
+    if (solver == SPLPAK_SOLVER_ORTHOGONAL && spl_ortho_supported(h->gp) && h->lambda == 0.0) {
         h->solver = solver;
         return SPLPAK_OK;
     }
     return SPLPAK_ERR_HANDLE;
 }
 extern "C" int splpak_b200_fit_get_solver(splpak_b200_fit_t h) { return valid(h) ? h->solver : -1; }
+extern "C" int splpak_b200_fit_set_smoothing(splpak_b200_fit_t h, double lambda, int penalty) {
+    if (!valid(h) || h->finalized) return SPLPAK_ERR_HANDLE;
+    if (!(lambda >= 0.0) || !isfinite(lambda)) return SPLPAK_ERR_HANDLE;                  // negative, NaN, inf
+    if (penalty != SPLPAK_PENALTY_CURVATURE && penalty != SPLPAK_PENALTY_THIN_PLATE) return SPLPAK_ERR_HANDLE;
+    if (lambda > 0.0 && h->solver == SPLPAK_SOLVER_ORTHOGONAL) return SPLPAK_ERR_HANDLE;
+    if (lambda > 0.0 && !h->d_pen &&
+        cudaMalloc((void **)&h->d_pen, sizeof(double) * (size_t)spl_penalty_table_len(h->gp)) != cudaSuccess) {
+        cudaGetLastError();
+        h->d_pen = nullptr;
+        return SPLPAK_ERR_ALLOC;
+    }
+    h->lambda = lambda;
+    h->penalty = penalty;
+    return SPLPAK_OK;
+}
 // Parity-test hook of the orthogonal path: which = 0 -> the per-window triangles [nwindows][ncw][ncw + 1] (R_w | z_w),
 // which = 1 -> the band factor [ncol][bw + 2] (row i: R[i][i..i+bw], then (Q^T r)_i).  *count returns the size.
 extern "C" int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity,
