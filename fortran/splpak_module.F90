@@ -62,6 +62,9 @@
         procedure,public :: refine                       !! (new) streaming fit: one refinement pass over the same points
         procedure,public :: set_solver                   !! (new) streaming fit: 0 = band Cholesky (default), 1 = orthogonal (Householder)
         procedure,public :: set_smoothing                !! (new) streaming fit: roughness penalty lambda (0 = curvature, 1 = thin plate)
+        procedure,public :: enable_gcv                   !! (new) streaming fit: collect what the GCV score needs (before add_points)
+        procedure,public :: smoothing_score              !! (new) streaming fit: GCV score {V, RSS, edf, N, ywy} of one lambda
+        procedure,public :: select_smoothing             !! (new) streaming fit: lambda minimising the GCV score, set on the fit
         procedure,private :: splcc
         procedure,private :: splcw
         procedure,private :: splfe
@@ -203,6 +206,33 @@
             integer(c_int),value :: penalty
             integer(c_int) :: rc
         end function c_fit_set_smoothing
+        function c_fit_enable_gcv(h) bind(C,name='splpak_b200_fit_enable_gcv') result(rc)
+            import :: c_int, c_ptr
+            type(c_ptr),value :: h
+            integer(c_int) :: rc
+        end function c_fit_enable_gcv
+        function c_fit_smoothing_score(h,lambda,penalty,out,nout,ierror) &
+                 bind(C,name='splpak_b200_fit_smoothing_score') result(rc)
+            import :: c_int, c_double, c_ptr
+            type(c_ptr),value :: h
+            real(c_double),value :: lambda
+            integer(c_int),value :: penalty, nout
+            real(c_double),intent(out) :: out(*)
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_smoothing_score
+        function c_fit_select_smoothing(h,penalty,lambda_lo,lambda_hi,lambda,out,nout,trace,trace_cap,ntrace,ierror) &
+                 bind(C,name='splpak_b200_fit_select_smoothing') result(rc)
+            import :: c_int, c_int64_t, c_double, c_ptr
+            type(c_ptr),value :: h
+            integer(c_int),value :: penalty, nout
+            real(c_double),value :: lambda_lo, lambda_hi
+            real(c_double),intent(out) :: lambda, out(*), trace(*)
+            integer(c_int64_t),value :: trace_cap
+            integer(c_int64_t),intent(out) :: ntrace
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_select_smoothing
         function c_fit_destroy(h) bind(C,name='splpak_b200_fit_destroy') result(rc)
             import :: c_int, c_ptr
             type(c_ptr),value :: h
@@ -406,6 +436,43 @@
         integer,intent(out) :: ierror
         ierror = int(c_fit_set_smoothing(me%handle,lambda,int(penalty,c_int)))
     end subroutine set_smoothing
+
+    !> (new) generalized cross-validation: call before the first add_points (ierror = 203 otherwise,
+    !  or with the orthogonal solver).  Persists across reset.
+    subroutine enable_gcv(me,ierror)
+        class(splpak_type),intent(inout) :: me
+        integer,intent(out) :: ierror
+        ierror = int(c_fit_enable_gcv(me%handle))
+    end subroutine enable_gcv
+
+    !> (new) GCV score of smoothing lambda after the assembly, before compute (changes nothing compute
+    !  sees): score = [V, RSS, edf, N, ywy].  ierror = 107 for a non-positive pivot, 203 when refused.
+    subroutine smoothing_score(me,lambda,penalty,score,ierror)
+        class(splpak_type),intent(inout) :: me
+        real(c_double),intent(in) :: lambda
+        integer,intent(in) :: penalty
+        real(c_double),intent(out) :: score(5)
+        integer,intent(out) :: ierror
+        integer(c_int) :: ierr, rc
+        rc = c_fit_smoothing_score(me%handle,lambda,int(penalty,c_int),score,5_c_int,ierr)
+        ierror = int(rc)
+    end subroutine smoothing_score
+
+    !> (new) lambda minimising the GCV score over [lambda_lo, lambda_hi] (either <= 0: the default range),
+    !  then set on the fit, so the next compute is the selected fit.  score as smoothing_score.
+    subroutine select_smoothing(me,penalty,lambda_lo,lambda_hi,lambda,score,ierror)
+        class(splpak_type),intent(inout) :: me
+        integer,intent(in) :: penalty
+        real(c_double),intent(in) :: lambda_lo, lambda_hi
+        real(c_double),intent(out) :: lambda, score(5)
+        integer,intent(out) :: ierror
+        integer(c_int) :: ierr, rc
+        integer(c_int64_t) :: ntrace
+        real(c_double) :: trace(4)
+        rc = c_fit_select_smoothing(me%handle,int(penalty,c_int),lambda_lo,lambda_hi,lambda,score,5_c_int, &
+                                    trace,0_c_int64_t,ntrace,ierr)
+        ierror = int(rc)
+    end subroutine select_smoothing
 
     !> (new) accumulate n more points; wdata absent (or wdata(1)<0) => all weights 1.
     subroutine add_points(me,xdata,l1xdat,ydata,ndata,ierror,wdata)

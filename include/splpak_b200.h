@@ -219,6 +219,35 @@ int splpak_b200_fit_get_solver(splpak_b200_fit_t h);
 #define SPLPAK_PENALTY_CURVATURE  0
 #define SPLPAK_PENALTY_THIN_PLATE 1
 int splpak_b200_fit_set_smoothing(splpak_b200_fit_t h, double lambda, int penalty);
+/* Choosing lambda by generalized cross-validation -- (new).  With M = G0 + C + lambda R (G0 the assembled data rows, C the
+ * constraint rows, R the penalty) and c = M^-1 g:
+ *     RSS = sum_i (w_i (y_i - s(x_i)))^2 = ywy - 2 c.g + c^T G0 c,   edf = tr(M^-1 G0),   V = N RSS / (N - edf)^2
+ * (N: the data rows counted, V = +inf when N <= edf).  edf is exact: Sigma = M^-1 is formed on the band of the Cholesky
+ * factor (selected inverse).  RSS carries a cancellation: its relative error is about eps * ywy / RSS.
+ *   enable_gcv          before the first add_points (203 otherwise): every add_points chunk also sums ywy = sum (w y)^2
+ *                       into one more slot at the END of the partial buffer, [S | g | cnt | totlwt | nrows | ywy]
+ *                       (fit_partial_buffer reports one more double, and the multi-GPU all-reduce sums it too).  Persists
+ *                       across fit_reset, which zeroes ywy.  Not with the orthogonal solver (203, in either order).
+ *   smoothing_score     after the (all-reduced) assembly, before fit_compute: out[0..4] = {V, RSS, edf, N, ywy}, nout >= 5.
+ *                       Changes neither S, g, the counts nor the totals: a later compute is unaffected.  lambda = 0 is
+ *                       allowed; a non-positive pivot returns 107.
+ *   select_smoothing    V minimised over log10 lambda: a grid at 2 points per decade over [lambda_lo, lambda_hi], then
+ *                       golden-section refinement around the best grid point down to 0.02 decades; ties go to the larger
+ *                       lambda.  lambda_lo <= 0 or lambda_hi <= 0: rho * [1e-10, 1e4], rho = sum G0_ii / sum R_ii.  Points
+ *                       with a non-positive pivot count as V = +inf (107 when all do).  On success it calls
+ *                       set_smoothing(best, penalty), writes *lambda, the best point's out, and the evaluated
+ *                       [lambda, V, RSS, edf] rows in evaluation order into trace (up to trace_cap rows; *ntrace = count).
+ *   get_selected_inverse  parity hook, valid after a score call: out[ncol][b + 1], row i = Sigma(i, i..i+b) of the last
+ *                       lambda scored (after select_smoothing: the selected lambda); out may be NULL to query *count.
+ * All in FP64 (the REAL32 library too).  Given the same summed partial buffer, every output is bit-identical across calls,
+ * handles and ranks, so every rank of a multi-GPU fit selects the same lambda.  203: invalid or finalized handle, GCV
+ * not enabled, unknown penalty, lambda < 0 / NaN / inf, lambda_lo > lambda_hi. */
+int splpak_b200_fit_enable_gcv(splpak_b200_fit_t h);
+int splpak_b200_fit_smoothing_score(splpak_b200_fit_t h, double lambda, int penalty, double *out, int nout, int *ierror);
+int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty, double lambda_lo, double lambda_hi, double *lambda,
+                                     double *out, int nout, double *trace, int64_t trace_cap, int64_t *ntrace,
+                                     int *ierror);
+int splpak_b200_fit_get_selected_inverse(splpak_b200_fit_t h, double *out, int64_t capacity, int64_t *count);
 /* Parity-test hook of the orthogonal path: which = 0 -> per-window triangles [nwindows][4^ndim][4^ndim + 1] (R_w | z_w),
  * which = 1 -> band factor [ncol][b + 2] (row i: R[i][i..i+b], then (Q^T r)_i).  out may be NULL to query *count. */
 int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity, int64_t *count);

@@ -51,6 +51,10 @@ SYMBOLS = [
     "splpak_b200_fit_set_solver",
     "splpak_b200_fit_get_solver",
     "splpak_b200_fit_set_smoothing",
+    "splpak_b200_fit_enable_gcv",
+    "splpak_b200_fit_smoothing_score",
+    "splpak_b200_fit_select_smoothing",
+    "splpak_b200_fit_get_selected_inverse",
     "splpak_b200_fit_get_orthogonal_factor",
     "splpak_b200_fit_condition_estimate",
     "splpak_b200_fit_constraints_fired",
@@ -145,6 +149,11 @@ def load(real32: bool = False) -> C.CDLL:
         "splpak_b200_fit_set_solver": (C.c_int, [vp, C.c_int]),
         "splpak_b200_fit_get_solver": (C.c_int, [vp]),
         "splpak_b200_fit_set_smoothing": (C.c_int, [vp, C.c_double, C.c_int]),
+        "splpak_b200_fit_enable_gcv": (C.c_int, [vp]),
+        "splpak_b200_fit_smoothing_score": (C.c_int, [vp, C.c_double, C.c_int, vp, C.c_int, ip]),
+        "splpak_b200_fit_select_smoothing": (C.c_int, [vp, C.c_int, C.c_double, C.c_double, C.POINTER(C.c_double), vp,
+                                                       C.c_int, vp, i64, C.POINTER(i64), ip]),
+        "splpak_b200_fit_get_selected_inverse": (C.c_int, [vp, vp, i64, C.POINTER(i64)]),
         "splpak_b200_fit_get_orthogonal_factor": (C.c_int, [vp, C.c_int, vp, i64, C.POINTER(i64)]),
         "splpak_b200_fit_condition_estimate": (C.c_int, [vp, C.POINTER(C.c_double)]),
         "splpak_b200_fit_constraints_fired": (C.c_int, [vp]),

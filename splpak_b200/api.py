@@ -332,6 +332,64 @@ class FitHandle:
             penalty = self.PENALTIES[penalty]
         return self.lib.splpak_b200_fit_set_smoothing(self.h, float(lam), int(penalty))
 
+    def _penalty_code(self, penalty):
+        if isinstance(penalty, str):
+            if penalty not in self.PENALTIES:
+                raise SplpakError(f"unknown penalty {penalty!r}: expected one of {sorted(self.PENALTIES)}")
+            return self.PENALTIES[penalty]
+        return int(penalty)
+
+    def enable_gcv(self):
+        """Generalized cross-validation: before the first add_points (203 otherwise).  Every chunk then also sums
+        (w y)^2 into one more slot at the end of the partial buffer.  Persists across reset.  Returns the library code."""
+        self._check()
+        return self.lib.splpak_b200_fit_enable_gcv(self.h)
+
+    _SCORE_KEYS = ("gcv", "rss", "edf", "n", "ywy")
+
+    def smoothing_score(self, lam, penalty="curvature"):
+        """GCV score of the fit with smoothing `lam`, after the (all-reduced) assembly and before compute; changes
+        nothing a later compute sees.  Returns {gcv, rss, edf, n, ywy}; raises SplpakError on a non-zero code (107: a
+        non-positive pivot, 203: refused)."""
+        self._check()
+        out = np.zeros(5)
+        ierr = C.c_int(0)
+        rc = self.lib.splpak_b200_fit_smoothing_score(self.h, float(lam), self._penalty_code(penalty), _ptr(out), 5,
+                                                      C.byref(ierr))
+        if rc != 0:
+            raise SplpakError(f"smoothing_score failed: {rc}", rc)
+        return dict(zip(self._SCORE_KEYS, (float(v) for v in out)))
+
+    def select_smoothing(self, penalty="curvature", lo=None, hi=None, trace_cap=512):
+        """lambda minimising the GCV score over [lo, hi] (default: rho * [1e-10, 1e4], rho = tr G0 / tr R); sets it on
+        the handle (set_smoothing), so the next compute is the selected fit.  Returns (lam, score dict, trace), trace:
+        (k, 4) rows [lambda, V, RSS, edf] in evaluation order.  Raises SplpakError on a non-zero code."""
+        self._check()
+        lam = C.c_double(0.0)
+        out = np.zeros(5)
+        trace = np.zeros((int(trace_cap), 4))
+        nt = C.c_int64(0)
+        ierr = C.c_int(0)
+        rc = self.lib.splpak_b200_fit_select_smoothing(self.h, self._penalty_code(penalty),
+                                                       0.0 if lo is None else float(lo), 0.0 if hi is None else float(hi),
+                                                       C.byref(lam), _ptr(out), 5, _ptr(trace), int(trace_cap),
+                                                       C.byref(nt), C.byref(ierr))
+        if rc != 0:
+            raise SplpakError(f"select_smoothing failed: {rc}", rc)
+        return lam.value, dict(zip(self._SCORE_KEYS, (float(v) for v in out))), trace[: min(nt.value, int(trace_cap))]
+
+    def selected_inverse(self):
+        """Parity hook, after a score call: (ncol, b + 1), row i = Sigma(i, i..i+b), Sigma = (G0 + C + lambda R)^-1."""
+        self._check()
+        n = C.c_int64(0)
+        if self.lib.splpak_b200_fit_get_selected_inverse(self.h, None, 0, C.byref(n)) != 0:
+            raise SplpakError("no selected inverse on this handle (call smoothing_score first)")
+        out = np.zeros(n.value)
+        rc = self.lib.splpak_b200_fit_get_selected_inverse(self.h, _ptr(out), n.value, C.byref(n))
+        if rc != 0:
+            raise SplpakError(f"get_selected_inverse failed: {rc}")
+        return out.reshape(self.ncol, -1)
+
     def orthogonal_factor(self, which):
         """Parity-test hook: which = 0 -> per-window triangles (nwindows, 4^ndim, 4^ndim + 1); 1 -> band factor (ncol, b + 2)."""
         self._check()

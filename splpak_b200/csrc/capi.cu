@@ -75,6 +75,17 @@ int spl_ortho_add_chunk(const GridParams &gp, const real_t *d_x, int l1x, const 
 int spl_ortho_compute(const GridParams &gp, double xtrap, OrthoScratch &os, const double *d_cnt, double *d_totals,
                       int *d_fail, cudaStream_t st, int nsm);
 int spl_pivot_range_launch(const GridParams &gp, const double *d_work, double *d_out2, cudaStream_t st);
+int spl_penalty_diag_launch(const GridParams &gp, int penalty, double *d_tab, const double *d_S, double *d_out2,
+                            cudaStream_t st);
+long long spl_selinv_scratch(const GridParams &gp);
+int spl_selinv_launch(const GridParams &gp, double *d_AB, const double *d_work, double *d_scr, cudaStream_t st,
+                      void **cache);
+void spl_selinv_cache_free(void *cache);
+int spl_gcv_ywy_launch(const real_t *d_y, const real_t *d_w, int weighted, long long n, double *d_part, double *d_ywy,
+                       cudaStream_t st);
+long long spl_gcv_part_len();
+int spl_gcv_stencil_launch(const GridParams &gp, const double *d_S, const double *d_AB, const double *d_c,
+                           const double *d_g0, double *d_part, double *d_out3, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------
 // small conversion kernels
@@ -929,6 +940,16 @@ struct splpak_b200_fit_s {
     double lambda;
     int penalty;                  // SPLPAK_PENALTY_CURVATURE or SPLPAK_PENALTY_THIN_PLATE
     double *d_pen;                // 1-D penalty tables (spl_penalty_table_len doubles), allocated by the first lambda > 0
+    // generalized cross-validation (selinv.cu): enable_gcv; kept across fit_reset
+    int gcv;
+    double *d_ywy;                // the last slot of the partial buffer: sum (w y)^2
+    double *d_ywy_part;           // per-CTA partials of one chunk's sum
+    double *d_gcv;                // score scratch: S1 = G0 + C, S2 = S1 + lambda R, g2, totals1, results, reductions,
+                                  // selected-inverse scratch (allocated by the first score call)
+    int s1_valid;                 // d_gcv holds S1 of the current assembly
+    int sigma_valid;              // d_AB holds Sigma of the last score call
+    void *score_cache;            // solve graphs of the score calls (their own buffers: compute keeps its graphs)
+    void *selinv_cache;           // graph of the selected inverse
     // timing: accumulated event pairs
     double ms[NTIMER];
     cudaEvent_t ev[12];           // 0-3 assembly, 4-5 constraints, 8-11 solve stages
@@ -967,6 +988,10 @@ static void free_handle(splpak_b200_fit_t h) {
     if (h->d_dummy_tot) cudaFree(h->d_dummy_tot);
     if (h->d_out_tmp) cudaFree(h->d_out_tmp);
     if (h->d_pen) cudaFree(h->d_pen);
+    if (h->d_ywy_part) cudaFree(h->d_ywy_part);
+    if (h->d_gcv) cudaFree(h->d_gcv);
+    if (h->score_cache) spl_solve_cache_free(h->score_cache);
+    if (h->selinv_cache) spl_selinv_cache_free(h->selinv_cache);
     if (h->os) {
         spl_ortho_free(*h->os);
         delete h->os;
@@ -1053,6 +1078,7 @@ extern "C" int splpak_b200_fit_reset(splpak_b200_fit_t h) {
     h->timers_pending = 0;
     h->total_points = 0;
     h->solved = h->refining = h->constraints_fired = h->factor_valid = 0;
+    h->s1_valid = h->sigma_valid = 0;
     h->cond_est = 0.0;
     if (h->os) return spl_ortho_reset(h->gp, *h->os, h->st);
     return SPLPAK_OK;
@@ -1138,6 +1164,10 @@ static int add_device_chunk(splpak_b200_fit_t h, const real_t *d_x, int l1x, con
     h->timers_pending = 1;
     rc = spl_assemble_chunk(h->gp, d_x, l1x, d_y, d_w, weighted, n, h->xtrap != 0.0, 0, h->sc, h->d_S,
                             h->d_g, h->d_cnt, h->d_totals, h->st, h->di.nsm, h->ev);
+    if (rc == SPLPAK_OK && h->gcv) {
+        h->s1_valid = h->sigma_valid = 0;
+        rc = spl_gcv_ywy_launch(d_y, weighted ? d_w : nullptr, weighted, n, h->d_ywy_part, h->d_ywy, h->st);
+    }
     return rc;
 }
 
@@ -1233,6 +1263,7 @@ extern "C" int splpak_b200_fit_add_points(splpak_b200_fit_t h, const real_t *x, 
 
 extern "C" int splpak_b200_fit_partial_buffer(splpak_b200_fit_t h, void **d_ptr, int64_t *count) {
     if (!valid(h)) return SPLPAK_ERR_HANDLE;
+    h->s1_valid = 0;                  // the caller may write the sums through the pointer (all-reduce)
     if (d_ptr) *d_ptr = h->d_part;
     if (count) *count = h->n_part;
     return SPLPAK_OK;
@@ -1280,6 +1311,7 @@ extern "C" int splpak_b200_fit_allreduce(splpak_b200_fit_t h, void *nccl_comm) {
     NcclApi &api = nccl_api();
     if (!api.ok) return SPLPAK_ERR_NCCL;
     // ncclFloat64 = 8, ncclSum = 0 (nccl.h)
+    h->s1_valid = h->sigma_valid = 0;
     const int rc = api.AllReduce(h->d_part, h->d_part, (size_t)h->n_part, 8, 0, nccl_comm, h->st);
     return rc == 0 ? SPLPAK_OK : SPLPAK_ERR_NCCL;
 }
@@ -1324,6 +1356,27 @@ extern "C" int splpak_b200_comm_group_start(void) {
 extern "C" int splpak_b200_comm_group_end(void) {
     NcclApi &api = nccl_api();
     return api.ok && api.GroupEnd() == 0 ? SPLPAK_OK : SPLPAK_ERR_NCCL;
+}
+
+// the band matrix and the solve workspace behind it (grow-only): *band_elems doubles of band, *need in all
+static int ensure_band(splpak_b200_fit_t h, long long *band_elems, long long *need) {
+    const GridParams &gp = h->gp;
+    const int bw = spl_half_bandwidth(gp);
+    const long long lda = spl_band_lda(bw);
+    // element (i, j) lives at i + j*lda, so the last one, (n-1, n-1), is at (n-1)*(lda+1)
+    *band_elems = (gp.ncol * (lda + 1) + 64 + 1) & ~1LL;     // even: the workspace behind stays 16-byte aligned
+    *need = *band_elems + spl_solve_workspace(gp);
+    if (*need > h->ab_elems) {
+        if (h->d_AB) cudaFree(h->d_AB);
+        h->d_AB = nullptr;
+        h->ab_elems = 0;
+        if (cudaMalloc((void **)&h->d_AB, sizeof(double) * (size_t)*need) != cudaSuccess) {
+            cudaGetLastError();
+            return SPLPAK_ERR_ALLOC;
+        }
+        h->ab_elems = *need;
+    }
+    return SPLPAK_OK;
 }
 
 static int fit_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_on_device, int64_t ncf,
@@ -1405,21 +1458,11 @@ static int fit_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_on_devic
         if (ierror) *ierror = rc;
         return rc;
     }
-    const int bw = spl_half_bandwidth(gp);
-    const long long lda = spl_band_lda(bw);
-    // element (i, j) lives at i + j*lda, so the last one, (n-1, n-1), is at (n-1)*(lda+1)
-    const long long band_elems = (gp.ncol * (lda + 1) + 64 + 1) & ~1LL;     // even: the workspace behind stays 16-byte aligned
-    const long long need = band_elems + spl_solve_workspace(gp);
-    if (need > h->ab_elems) {
-        if (h->d_AB) cudaFree(h->d_AB);
-        h->d_AB = nullptr;
-        h->ab_elems = 0;
-        if (cudaMalloc((void **)&h->d_AB, sizeof(double) * (size_t)need) != cudaSuccess) {
-            cudaGetLastError();
-            if (ierror) *ierror = SPLPAK_ERR_ALLOC;
-            return SPLPAK_ERR_ALLOC;
-        }
-        h->ab_elems = need;
+    long long band_elems = 0, need = 0;
+    rc = ensure_band(h, &band_elems, &need);
+    if (rc != SPLPAK_OK) {
+        if (ierror) *ierror = rc;
+        return rc;
     }
     // A CUDA failure below must reach the caller through *ierror (the Fortran shim and api.py read nothing
     // else) and leave the handle finalized.
@@ -1459,6 +1502,7 @@ static int fit_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_on_devic
     FC_TRY(cudaEventRecord(h->ev[5], st));
     FC_TRY(cudaMemsetAsync(h->d_AB, 0, sizeof(double) * (size_t)need, st));
     FC_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
+    h->sigma_valid = 0;
     cudaEvent_t *sev = h->ev + 8;
     // the solve destroys g; the solution comes back in the workspace behind the band matrix
     double *d_sol = nullptr;
@@ -1703,7 +1747,7 @@ extern "C" int splpak_b200_fit_set_solver(splpak_b200_fit_t h, int solver) {
         return SPLPAK_OK;
     }
     // the penalty couples nodes across the windows of the orthogonal path: no smoothing there
-    if (solver == SPLPAK_SOLVER_ORTHOGONAL && spl_ortho_supported(h->gp) && h->lambda == 0.0) {
+    if (solver == SPLPAK_SOLVER_ORTHOGONAL && spl_ortho_supported(h->gp) && h->lambda == 0.0 && !h->gcv) {
         h->solver = solver;
         return SPLPAK_OK;
     }
@@ -1725,6 +1769,290 @@ extern "C" int splpak_b200_fit_set_smoothing(splpak_b200_fit_t h, double lambda,
     h->penalty = penalty;
     return SPLPAK_OK;
 }
+// ---- generalized cross-validation (selinv.cu; DESIGN §4.12) ----
+extern "C" int splpak_b200_fit_enable_gcv(splpak_b200_fit_t h) {
+    if (!valid(h) || h->finalized || h->total_points != 0 || h->solver == SPLPAK_SOLVER_ORTHOGONAL)
+        return SPLPAK_ERR_HANDLE;
+    if (h->gcv) return SPLPAK_OK;
+    // one more slot at the end of the partial buffer, so that the one all-reduce sums ywy too
+    double *part = nullptr;
+    if (cudaMalloc((void **)&part, sizeof(double) * (size_t)(h->n_part + 1)) != cudaSuccess ||
+        (!h->d_ywy_part && cudaMalloc((void **)&h->d_ywy_part, sizeof(double) * 256) != cudaSuccess)) {
+        cudaGetLastError();
+        if (part) cudaFree(part);
+        return SPLPAK_ERR_ALLOC;
+    }
+    SPL_CUDA_TRY(cudaStreamSynchronize(h->st));
+    cudaFree(h->d_part);
+    h->d_part = part;
+    h->n_part += 1;
+    const GridParams &gp = h->gp;
+    h->d_S = h->d_part;
+    h->d_g = h->d_S + gp.ncol * gp.nsten;
+    h->d_cnt = h->d_g + gp.ncol;
+    h->d_totals = h->d_cnt + gp.ncol;
+    h->d_ywy = h->d_totals + 2;
+    SPL_CUDA_TRY(cudaMemsetAsync(h->d_part, 0, sizeof(double) * (size_t)h->n_part, h->st));
+    h->gcv = 1;
+    h->s1_valid = h->sigma_valid = 0;
+    return SPLPAK_OK;
+}
+
+// Score scratch layout: S1, S2 (ncol * nsten each), g2 (ncol), totals1 (2), results (8), reductions, selected-inverse
+// scratch.  Every part starts at a multiple of 32 doubles (256 bytes): the selected inverse stages its X panel with
+// 16-byte cp.async, and with ncol odd an unpadded layout would put it at an odd double offset.
+struct GcvScratch {
+    long long S1, S2, g2, tot1, res, red, sel, len;
+};
+static GcvScratch gcv_scratch_layout(const GridParams &gp) {
+    auto up = [](long long v) { return (v + 31) & ~31LL; };
+    const long long ns = gp.ncol * gp.nsten;
+    GcvScratch L;
+    L.S1 = 0;
+    L.S2 = up(L.S1 + ns);
+    L.g2 = up(L.S2 + ns);
+    L.tot1 = up(L.g2 + gp.ncol);
+    L.res = up(L.tot1 + 2);
+    L.red = up(L.res + 8);
+    L.sel = up(L.red + spl_gcv_part_len());
+    L.len = L.sel + spl_selinv_scratch(gp);
+    return L;
+}
+
+// {V, RSS, edf, N, ywy} of one lambda.  Leaves S, g, cnt and totals as they are; d_AB then holds Sigma.
+static int gcv_score_impl(splpak_b200_fit_t h, double lambda, int penalty, double out5[5]) {
+    const GridParams &gp = h->gp;
+    cudaStream_t st = h->st;
+    long long band_elems = 0, need = 0;
+    int rc = ensure_band(h, &band_elems, &need);
+    if (rc != SPLPAK_OK) return rc;
+    const GcvScratch L = gcv_scratch_layout(gp);
+    if (!h->d_gcv) {
+        if (cudaMalloc((void **)&h->d_gcv, sizeof(double) * (size_t)L.len) != cudaSuccess) {
+            cudaGetLastError();
+            h->d_gcv = nullptr;
+            return SPLPAK_ERR_ALLOC;
+        }
+        h->s1_valid = 0;
+    }
+    if (lambda > 0.0 && !h->d_pen) {
+        if (cudaMalloc((void **)&h->d_pen, sizeof(double) * (size_t)spl_penalty_table_len(gp)) != cudaSuccess) {
+            cudaGetLastError();
+            h->d_pen = nullptr;
+            return SPLPAK_ERR_ALLOC;
+        }
+    }
+    const long long ns = gp.ncol * gp.nsten;
+    double *d_S1 = h->d_gcv + L.S1, *d_S2 = h->d_gcv + L.S2, *d_g2 = h->d_gcv + L.g2, *d_tot1 = h->d_gcv + L.tot1;
+    double *d_res = h->d_gcv + L.res, *d_red = h->d_gcv + L.red, *d_sel = h->d_gcv + L.sel;
+    h->sigma_valid = 0;
+    if (!h->s1_valid) {
+        // S1 = G0 + C: the constraint rows through the fixed-point limbs, as in compute, on copies of S and the totals
+        SPL_CUDA_TRY(cudaMemcpyAsync(d_S1, h->d_S, sizeof(double) * (size_t)ns, cudaMemcpyDeviceToDevice, st));
+        SPL_CUDA_TRY(cudaMemcpyAsync(d_tot1, h->d_totals, sizeof(double) * 2, cudaMemcpyDeviceToDevice, st));
+        if (h->xtrap != 0.0) {
+            rc = spl_constraints_launch(h->gp_fx.fxS ? h->gp_fx : gp, h->xtrap, h->d_cnt, d_tot1, d_S1, d_tot1, st,
+                                        h->di.nsm);
+            if (rc != SPLPAK_OK) return rc;
+        }
+        h->s1_valid = 1;
+    }
+    SPL_CUDA_TRY(cudaMemcpyAsync(d_S2, d_S1, sizeof(double) * (size_t)ns, cudaMemcpyDeviceToDevice, st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(d_g2, h->d_g, sizeof(double) * (size_t)gp.ncol, cudaMemcpyDeviceToDevice, st));
+    if (lambda > 0.0) {
+        rc = spl_penalty_add_launch(gp, lambda, penalty, h->d_pen, d_S2, st, h->di.nsm);
+        if (rc != SPLPAK_OK) return rc;
+    }
+    SPL_CUDA_TRY(cudaMemsetAsync(h->d_AB, 0, sizeof(double) * (size_t)need, st));
+    SPL_CUDA_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
+    h->factor_valid = 0;
+    double *d_sol = nullptr;
+    rc = spl_solve_launch(gp, d_S2, h->d_AB, d_g2, h->d_AB + band_elems, &d_sol, h->d_fail, st, h->st_aux, h->di.nsm,
+                          nullptr, &h->score_cache);
+    if (rc != SPLPAK_OK) return rc;
+    int fail = 0;
+    SPL_CUDA_TRY(cudaMemcpyAsync(&fail, h->d_fail, sizeof(int), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaStreamSynchronize(st));
+    if (fail) return SPLPAK_ERR_SOLVER;
+    rc = spl_selinv_launch(gp, h->d_AB, h->d_AB + band_elems, d_sel, st, &h->selinv_cache);
+    if (rc != SPLPAK_OK) return rc;
+    rc = spl_gcv_stencil_launch(gp, h->d_S, h->d_AB, d_sol, h->d_g, d_red, d_res, st);
+    if (rc != SPLPAK_OK) return rc;
+    double r[3], totals[2], ywy = 0.0;
+    SPL_CUDA_TRY(cudaMemcpyAsync(r, d_res, sizeof(r), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(totals, h->d_totals, sizeof(totals), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(&ywy, h->d_ywy, sizeof(double), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaStreamSynchronize(st));
+    const double edf = r[0], N = totals[1];
+    // the cancellation of ywy - 2 c.g + c^T G0 c: relative error ~ eps ywy / RSS
+    const double rss = ywy - 2.0 * r[2] + r[1];
+    const double dof = N - edf;
+    out5[0] = dof > 0.0 ? N * rss / (dof * dof) : INFINITY;
+    out5[1] = rss;
+    out5[2] = edf;
+    out5[3] = N;
+    out5[4] = ywy;
+    h->sigma_valid = 1;
+    return SPLPAK_OK;
+}
+
+static int gcv_check(splpak_b200_fit_t h, int penalty) {
+    if (!valid(h) || h->finalized || !h->gcv || h->solver == SPLPAK_SOLVER_ORTHOGONAL) return SPLPAK_ERR_HANDLE;
+    if (penalty != SPLPAK_PENALTY_CURVATURE && penalty != SPLPAK_PENALTY_THIN_PLATE) return SPLPAK_ERR_HANDLE;
+    return SPLPAK_OK;
+}
+
+extern "C" int splpak_b200_fit_smoothing_score(splpak_b200_fit_t h, double lambda, int penalty, double *out, int nout,
+                                               int *ierror) {
+    int rc = gcv_check(h, penalty);
+    if (rc == SPLPAK_OK && (!(lambda >= 0.0) || !isfinite(lambda) || !out || nout < 5)) rc = SPLPAK_ERR_HANDLE;
+    if (rc == SPLPAK_OK) rc = gcv_score_impl(h, lambda, penalty, out);
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+extern "C" int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty, double lambda_lo, double lambda_hi,
+                                                double *lambda, double *out, int nout, double *trace, int64_t trace_cap,
+                                                int64_t *ntrace, int *ierror) {
+    int rc = gcv_check(h, penalty);
+    if (rc == SPLPAK_OK && (isnan(lambda_lo) || isnan(lambda_hi) || isinf(lambda_lo) || isinf(lambda_hi)))
+        rc = SPLPAK_ERR_HANDLE;
+    if (rc == SPLPAK_OK && lambda_lo > lambda_hi) rc = SPLPAK_ERR_HANDLE;
+    if (rc == SPLPAK_OK && out && nout < 5) rc = SPLPAK_ERR_HANDLE;
+    if (rc != SPLPAK_OK) {
+        if (ierror) *ierror = rc;
+        return rc;
+    }
+    if (ntrace) *ntrace = 0;
+    if (!(lambda_lo > 0.0) || !(lambda_hi > 0.0)) {
+        // default range rho * [1e-10, 1e4], rho = sum G0_ii / sum R_ii on the device
+        if (!h->d_pen &&
+            cudaMalloc((void **)&h->d_pen, sizeof(double) * (size_t)spl_penalty_table_len(h->gp)) != cudaSuccess) {
+            cudaGetLastError();
+            h->d_pen = nullptr;
+            if (ierror) *ierror = SPLPAK_ERR_ALLOC;
+            return SPLPAK_ERR_ALLOC;
+        }
+        double sums[2] = {0.0, 0.0};
+        rc = spl_penalty_diag_launch(h->gp, penalty, h->d_pen, h->d_S, h->d_dummy_tot, h->st);
+        if (rc == SPLPAK_OK && (cudaMemcpyAsync(sums, h->d_dummy_tot, sizeof(sums), cudaMemcpyDeviceToHost, h->st) !=
+                                    cudaSuccess ||
+                                cudaStreamSynchronize(h->st) != cudaSuccess))
+            rc = SPLPAK_ERR_CUDA;
+        if (rc != SPLPAK_OK) {
+            if (ierror) *ierror = rc;
+            return rc;
+        }
+        const double rho = (sums[0] > 0.0 && sums[1] > 0.0) ? sums[0] / sums[1] : 1.0;
+        lambda_lo = rho * 1e-10;
+        lambda_hi = rho * 1e4;
+    }
+    // every evaluated point, in order; the best is the smallest V, ties to the larger lambda
+    int64_t neval = 0;
+    double best_t = 0.0, best_v = INFINITY, best_out[5] = {0, 0, 0, 0, 0}, last_t = 0.0;
+    bool any_ok = false, have_best = false;
+    auto eval = [&](double t, double *v) -> int {
+        const double lam = pow(10.0, t);
+        last_t = t;
+        double o[5];
+        const int r = gcv_score_impl(h, lam, penalty, o);
+        if (r != SPLPAK_OK && r != SPLPAK_ERR_SOLVER) return r;
+        if (r == SPLPAK_ERR_SOLVER) {
+            o[0] = INFINITY;
+            o[1] = o[2] = NAN;
+        } else {
+            any_ok = true;
+        }
+        if (trace && neval < trace_cap) {
+            trace[4 * neval + 0] = lam;
+            trace[4 * neval + 1] = o[0];
+            trace[4 * neval + 2] = o[1];
+            trace[4 * neval + 3] = o[2];
+        }
+        ++neval;
+        if (r == SPLPAK_OK && (!have_best || o[0] < best_v || (o[0] == best_v && t > best_t))) {
+            have_best = true;
+            best_t = t;
+            best_v = o[0];
+            memcpy(best_out, o, sizeof(o));
+        }
+        *v = o[0];
+        return SPLPAK_OK;
+    };
+    const double t_lo = log10(lambda_lo), t_hi = log10(lambda_hi);
+    int K = (int)ceil(2.0 * (t_hi - t_lo) - 1e-9);
+    if (K < 0) K = 0;
+    int kbest = 0;
+    double vbest = INFINITY;
+    for (int k = 0; k <= K && rc == SPLPAK_OK; ++k) {
+        const double t = K > 0 ? t_lo + (t_hi - t_lo) * k / K : t_lo;
+        double v = 0.0;
+        rc = eval(t, &v);
+        if (rc == SPLPAK_OK && (k == 0 || v <= vbest)) {
+            vbest = v;
+            kbest = k;
+        }
+    }
+    if (rc == SPLPAK_OK && K > 0) {
+        // golden section on the grid bracket of the best point
+        auto grid_t = [&](int k) { return t_lo + (t_hi - t_lo) * k / K; };
+        double a = grid_t(kbest > 0 ? kbest - 1 : 0), b = grid_t(kbest < K ? kbest + 1 : K);
+        const double gr = 0.5 * (sqrt(5.0) - 1.0);
+        double c = b - gr * (b - a), d = a + gr * (b - a), fc = 0.0, fd = 0.0;
+        rc = eval(c, &fc);
+        if (rc == SPLPAK_OK) rc = eval(d, &fd);
+        while (rc == SPLPAK_OK && b - a > 0.02) {
+            if (fc < fd) {
+                b = d;
+                d = c;
+                fd = fc;
+                c = b - gr * (b - a);
+                rc = eval(c, &fc);
+            } else {
+                a = c;
+                c = d;
+                fc = fd;
+                d = a + gr * (b - a);
+                rc = eval(d, &fd);
+            }
+        }
+    }
+    if (ntrace) *ntrace = (trace && neval > trace_cap) ? trace_cap : neval;
+    if (rc == SPLPAK_OK && !any_ok) rc = SPLPAK_ERR_SOLVER;
+    if (rc == SPLPAK_OK && last_t != best_t) {
+        // d_AB holds Sigma of the last point evaluated: score the selected lambda again, so that get_selected_inverse
+        // returns the inverse of the system the handle now carries (the same inputs: the same scores, bit for bit)
+        double o[5];
+        rc = gcv_score_impl(h, pow(10.0, best_t), penalty, o);
+    }
+    if (rc == SPLPAK_OK) {
+        const double lam = pow(10.0, best_t);
+        rc = splpak_b200_fit_set_smoothing(h, lam, penalty);
+        if (rc == SPLPAK_OK) {
+            if (lambda) *lambda = lam;
+            if (out) memcpy(out, best_out, sizeof(best_out));
+        }
+    }
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+extern "C" int splpak_b200_fit_get_selected_inverse(splpak_b200_fit_t h, double *out, int64_t capacity, int64_t *count) {
+    if (!valid(h) || !h->sigma_valid) return SPLPAK_ERR_HANDLE;
+    const GridParams &gp = h->gp;
+    const int bw = spl_half_bandwidth(gp);
+    const long long lda = spl_band_lda(bw);
+    const int64_t n = (int64_t)gp.ncol * (bw + 1);
+    if (count) *count = n;
+    if (!out) return SPLPAK_OK;
+    if (capacity < n) return SPLPAK_ERR_HANDLE;
+    // row i = Sigma(i..i+b, i): b + 1 consecutive doubles from AB + i (lda + 1); the entries past n are zero
+    SPL_CUDA_TRY(cudaStreamSynchronize(h->st));
+    SPL_CUDA_TRY(cudaMemcpy2D(out, sizeof(double) * (size_t)(bw + 1), h->d_AB, sizeof(double) * (size_t)(lda + 1),
+                              sizeof(double) * (size_t)(bw + 1), (size_t)gp.ncol, cudaMemcpyDeviceToHost));
+    return SPLPAK_OK;
+}
+
 // Parity-test hook of the orthogonal path: which = 0 -> the per-window triangles [nwindows][ncw][ncw + 1] (R_w | z_w),
 // which = 1 -> the band factor [ncol][bw + 2] (row i: R[i][i..i+bw], then (Q^T r)_i).  *count returns the size.
 extern "C" int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity,

@@ -252,3 +252,59 @@ int spl_penalty_residual_launch(const GridParams &gp, double lambda, int penalty
     SPL_CUDA_TRY(cudaGetLastError());
     return SPLPAK_OK;
 }
+
+// rho = sum_i G0_ii / sum_i R_ii, the scale of the default lambda range of splpak_b200_fit_select_smoothing: one CTA,
+// every thread a fixed set of nodes, a fixed-order reduction.  out2 = {sum G0_ii, sum R_ii}.
+template <int NDIM>
+__global__ void __launch_bounds__(1024)
+spl_penalty_diag_kernel(const __grid_constant__ GridParams gp, const double *__restrict__ tab, int thin_plate,
+                        const double *__restrict__ S, double *__restrict__ out2) {
+    __shared__ double s_g[1024], s_r[1024];
+    double sg = 0.0, sr = 0.0;
+    for (long long node = threadIdx.x; node < gp.ncol; node += blockDim.x) {
+        int lo[NDIM], delta[NDIM];
+        long long k = node;
+#pragma unroll
+        for (int d = 0; d < NDIM; ++d) {
+            lo[d] = (int)(k % gp.nodes[d]);
+            k /= gp.nodes[d];
+            delta[d] = 0;
+        }
+        double a[NDIM][3];
+        spl_penalty_factors<NDIM>(tab, gp, lo, delta, a);
+        sr += spl_penalty_entry<NDIM>(a, thin_plate);
+        sg += S[node * gp.nsten];
+    }
+    s_g[threadIdx.x] = sg;
+    s_r[threadIdx.x] = sr;
+    __syncthreads();
+    for (int o = 512; o > 0; o >>= 1) {
+        if (threadIdx.x < o) {
+            s_g[threadIdx.x] += s_g[threadIdx.x + o];
+            s_r[threadIdx.x] += s_r[threadIdx.x + o];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        out2[0] = s_g[0];
+        out2[1] = s_r[0];
+    }
+}
+
+int spl_penalty_diag_launch(const GridParams &gp, int penalty, double *d_tab, const double *d_S, double *d_out2,
+                            cudaStream_t st) {
+    const long long ntab = spl_penalty_table_len(gp);
+    spl_penalty_gram_kernel<<<spl_div_up(ntab, 128), 128, 0, st>>>(gp, d_tab, ntab);
+    ++g_spl_launches;
+    const int tp = penalty == SPLPAK_PENALTY_THIN_PLATE;
+    switch (gp.ndim) {
+    case 1: spl_penalty_diag_kernel<1><<<1, 1024, 0, st>>>(gp, d_tab, tp, d_S, d_out2); break;
+    case 2: spl_penalty_diag_kernel<2><<<1, 1024, 0, st>>>(gp, d_tab, tp, d_S, d_out2); break;
+    case 3: spl_penalty_diag_kernel<3><<<1, 1024, 0, st>>>(gp, d_tab, tp, d_S, d_out2); break;
+    case 4: spl_penalty_diag_kernel<4><<<1, 1024, 0, st>>>(gp, d_tab, tp, d_S, d_out2); break;
+    default: return SPLPAK_ERR_NDIM;
+    }
+    ++g_spl_launches;
+    SPL_CUDA_TRY(cudaGetLastError());
+    return SPLPAK_OK;
+}

@@ -19,15 +19,20 @@ def shard_range(n: int, rank: int, world: int):
     return lo, hi
 
 
-def partial_layout(ndim: int, nodes):
-    """Offsets of the fields inside the partial buffer (float64 counts)."""
+def partial_layout(ndim: int, nodes, gcv=False):
+    """Offsets of the fields inside the partial buffer (float64 counts).  gcv: the handle called enable_gcv, which adds
+    the ywy = sum (w y)^2 slot at the end."""
     ncol = int(np.prod(np.asarray(nodes, dtype=np.int64)[:ndim]))
     nst = 4 ** ndim
     off = {"S": (0, ncol * nst), "g": (ncol * nst, ncol * nst + ncol),
            "cnt": (ncol * nst + ncol, ncol * nst + 2 * ncol),
            "totlwt": (ncol * nst + 2 * ncol, ncol * nst + 2 * ncol + 1),
            "nrows": (ncol * nst + 2 * ncol + 1, ncol * nst + 2 * ncol + 2)}
-    return off, ncol * nst + 2 * ncol + 2
+    total = ncol * nst + 2 * ncol + 2
+    if gcv:
+        off["ywy"] = (total, total + 1)
+        total += 1
+    return off, total
 
 
 def allreduce_partials(buf, group=None):
@@ -59,13 +64,16 @@ def _on_handle_stream(handle, fn, stream=None):
 
 
 def fit_sharded(handle, x, y, w, weighted=True, device_resident=False, l1x=None, n=None, group=None, stream=None,
-                broadcast_coef=False):
+                broadcast_coef=False, select_smoothing=None):
     """Every rank adds ITS shard to `handle`, the partial sums are all-reduced, every rank solves.
     Returns (coef, ierror).  The all-reduce is ordered against the handle's stream (see _on_handle_stream), so no
     host synchronisation is needed around it.  The replicated solves see identical inputs (the all-reduce hands every
     rank the same sums), add their constraint rows through order-independent integer limbs and solve deterministically,
     so the coefficients are bitwise identical on all ranks (tests/test_gpu_multi.py); `broadcast_coef` additionally
-    broadcasts rank 0's coefficients (8*ncol bytes) for hosts that want to rule out any divergence, e.g. mixed GPU types."""
+    broadcasts rank 0's coefficients (8*ncol bytes) for hosts that want to rule out any divergence, e.g. mixed GPU types.
+    `select_smoothing` (a penalty name; the handle must have called enable_gcv): after the all-reduce every rank
+    selects lambda by GCV on the summed buffer -- bit-identical inputs, so every rank selects the same lambda -- and
+    the solve is the selected fit."""
     import torch
     import torch.distributed as dist
 
@@ -77,6 +85,8 @@ def fit_sharded(handle, x, y, w, weighted=True, device_resident=False, l1x=None,
         return None, rc
     part = handle.partial_tensor()
     _on_handle_stream(handle, lambda: allreduce_partials(part, group), stream)
+    if select_smoothing is not None:
+        handle.select_smoothing(select_smoothing)
     coef, ierr = handle.compute()
     if broadcast_coef and dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
         t = torch.from_numpy(np.ascontiguousarray(coef, dtype=np.float64)).cuda()
