@@ -65,6 +65,8 @@
         procedure,public :: enable_gcv                   !! (new) streaming fit: collect what the GCV score needs (before add_points)
         procedure,public :: smoothing_score              !! (new) streaming fit: GCV score {V, RSS, edf, N, ywy} of one lambda
         procedure,public :: select_smoothing             !! (new) streaming fit: lambda minimising the GCV score, set on the fit
+        procedure,public :: prepare_variance             !! (new) streaming fit: tables of the posterior variances (before compute)
+        procedure,public :: variance                     !! (new) streaming fit: b(x)^T Sigma b(x) at a batch of points
         procedure,private :: splcc
         procedure,private :: splcw
         procedure,private :: splfe
@@ -233,6 +235,25 @@
             integer(c_int),intent(out) :: ierror
             integer(c_int) :: rc
         end function c_fit_select_smoothing
+        function c_fit_prepare_variance(h,out,nout,ierror) bind(C,name='splpak_b200_fit_prepare_variance') result(rc)
+            import :: c_int, c_double, c_ptr
+            type(c_ptr),value :: h
+            integer(c_int),value :: nout
+            real(c_double),intent(out) :: out(*)
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_prepare_variance
+        function c_fit_variance(h,x,l1x,nq,nderiv,out,ierror) bind(C,name='splpak_b200_fit_variance') result(rc)
+            import :: c_int, c_int64_t, c_ptr, cwp
+            type(c_ptr),value :: h
+            real(cwp),intent(in) :: x(*)
+            integer(c_int),value :: l1x
+            integer(c_int64_t),value :: nq
+            type(c_ptr),value :: nderiv                      !! c_null_ptr => values
+            real(cwp) :: out(*)
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_variance
         function c_fit_destroy(h) bind(C,name='splpak_b200_fit_destroy') result(rc)
             import :: c_int, c_ptr
             type(c_ptr),value :: h
@@ -473,6 +494,38 @@
                                     trace,0_c_int64_t,ntrace,ierr)
         ierror = int(rc)
     end subroutine select_smoothing
+
+    !> (new) posterior variances of a smoothing fit, after the assembly (and select_smoothing) and before
+    !  compute: builds the per-window tables from Sigma of the fit's current lambda (scoring once unless
+    !  select_smoothing left that Sigma behind).  score = [V, RSS, edf, N, ywy, sigma2], sigma2 = RSS / (N - edf).
+    !  ierror = 203 when refused (GCV not enabled, orthogonal solver, after compute), 204 allocation, 107 pivot.
+    subroutine prepare_variance(me,score,ierror)
+        class(splpak_type),intent(inout) :: me
+        real(c_double),intent(out) :: score(6)
+        integer,intent(out) :: ierror
+        integer(c_int) :: ierr, rc
+        rc = c_fit_prepare_variance(me%handle,score,6_c_int,ierr)
+        ierror = int(rc)
+    end subroutine prepare_variance
+
+    !> (new) q(i) = b(x_i)^T Sigma b(x_i) at the nq points x(:,i), after prepare_variance (any time, also after
+    !  compute): the posterior variance of the fitted value -- of the partial derivative nderiv when present --
+    !  divided by sigma2.  ierror = 203 without valid tables, 104 for nderiv outside 0..2.
+    subroutine variance(me,x,l1x,nq,q,ierror,nderiv)
+        class(splpak_type),intent(inout) :: me
+        integer,intent(in) :: l1x
+        integer(int64),intent(in) :: nq
+        real(wp),intent(in) :: x(l1x,nq)
+        real(wp),intent(out) :: q(nq)
+        integer,intent(out) :: ierror
+        integer,intent(in),optional,target :: nderiv(me%mdim)
+        integer(c_int) :: rc, ie
+        type(c_ptr) :: pn
+        pn = c_null_ptr
+        if (present(nderiv)) pn = c_loc(nderiv)
+        rc = c_fit_variance(me%handle,x,int(l1x,c_int),int(nq,c_int64_t),pn,q,ie)
+        ierror = int(rc)
+    end subroutine variance
 
     !> (new) accumulate n more points; wdata absent (or wdata(1)<0) => all weights 1.
     subroutine add_points(me,xdata,l1xdat,ydata,ndata,ierror,wdata)

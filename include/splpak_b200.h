@@ -248,6 +248,32 @@ int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty, double la
                                      double *out, int nout, double *trace, int64_t trace_cap, int64_t *ntrace,
                                      int *ierror);
 int splpak_b200_fit_get_selected_inverse(splpak_b200_fit_t h, double *out, int64_t capacity, int64_t *count);
+/* Pointwise posterior variances of a smoothing fit -- (new).  With Sigma = M^-1 as above and b_k(x) the row of basis
+ * values (nderiv = k: of their partial derivatives) at x,
+ *     q_k(x) = b_k(x)^T Sigma b_k(x),     Var[d^k s(x)] = sigma2 q_k(x)     (the Bayesian posterior variance)
+ * and w_i^2 q_0(x_i) is the leverage of data point i (the leverages sum to edf).
+ *   prepare_variance    after the (all-reduced) assembly, before fit_compute; GCV enabled, Cholesky solver.  Uses the
+ *                       handle's current (lambda, penalty): when the selected inverse of exactly that system is held
+ *                       (after select_smoothing) it does not score again, otherwise it runs one smoothing_score.  Then it
+ *                       builds one table of 10^ndim doubles per window (8 KB per window in 3-D, 80 KB in 4-D) into a
+ *                       buffer the handle owns, so the tables survive fit_compute and the refinement steps.
+ *                       out[0..5] = {V, RSS, edf, N, ywy, sigma2}, sigma2 = RSS / (N - edf) (+inf when N <= edf); nout >= 6.
+ *   variance            HOST arrays x(l1x, nq) -> out(nq) = q(x), unscaled: multiply by sigma2 (or a known noise
+ *                       variance).  nderiv: ndim entries in 0..2, NULL = values.
+ *   variance_device     the same with device arrays, asynchronous on `stream` (NULL: the handle's stream).
+ * Sequence: [select_smoothing ->] prepare_variance -> fit_compute -> variance*.  The tables become invalid with
+ * add_points, fit_partial_buffer / fit_allreduce, fit_reset, and set_smoothing to another (lambda, penalty).  Exterior
+ * queries use the clamped window and the linearly continued basis, as splde; a NaN coordinate gives NaN.  FP64 arithmetic
+ * (the REAL32 library: float I/O).  Bit-identical across calls, and across handles and ranks given the same summed
+ * partial buffer.  203: invalid handle, GCV not enabled, orthogonal solver, prepare_variance on a finalized handle or
+ * with nout < 6, variance* without valid tables or with l1x < ndim; 104: nderiv outside 0..2 (nothing is computed);
+ * 204: the tables cannot be allocated; 107: a non-positive pivot in the score.  nq <= 0 is a no-op.  A variance_device
+ * call on another stream must complete before the next prepare_variance of the handle. */
+int splpak_b200_fit_prepare_variance(splpak_b200_fit_t h, double *out, int nout, int *ierror);
+int splpak_b200_fit_variance(splpak_b200_fit_t h, const splpak_real *x, int l1x, int64_t nq, const int *nderiv,
+                             splpak_real *out, int *ierror);
+int splpak_b200_fit_variance_device(splpak_b200_fit_t h, const splpak_real *d_x, int l1x, int64_t nq, const int *nderiv,
+                                    splpak_real *d_out, void *stream, int *ierror);
 /* Parity-test hook of the orthogonal path: which = 0 -> per-window triangles [nwindows][4^ndim][4^ndim + 1] (R_w | z_w),
  * which = 1 -> band factor [ncol][b + 2] (row i: R[i][i..i+b], then (Q^T r)_i).  out may be NULL to query *count. */
 int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity, int64_t *count);

@@ -55,6 +55,9 @@ SYMBOLS = [
     "splpak_b200_fit_smoothing_score",
     "splpak_b200_fit_select_smoothing",
     "splpak_b200_fit_get_selected_inverse",
+    "splpak_b200_fit_prepare_variance",
+    "splpak_b200_fit_variance",
+    "splpak_b200_fit_variance_device",
     "splpak_b200_fit_get_orthogonal_factor",
     "splpak_b200_fit_condition_estimate",
     "splpak_b200_fit_constraints_fired",
@@ -154,6 +157,9 @@ def load(real32: bool = False) -> C.CDLL:
         "splpak_b200_fit_select_smoothing": (C.c_int, [vp, C.c_int, C.c_double, C.c_double, C.POINTER(C.c_double), vp,
                                                        C.c_int, vp, i64, C.POINTER(i64), ip]),
         "splpak_b200_fit_get_selected_inverse": (C.c_int, [vp, vp, i64, C.POINTER(i64)]),
+        "splpak_b200_fit_prepare_variance": (C.c_int, [vp, vp, C.c_int, ip]),
+        "splpak_b200_fit_variance": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, ip]),
+        "splpak_b200_fit_variance_device": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, vp, ip]),
         "splpak_b200_fit_get_orthogonal_factor": (C.c_int, [vp, C.c_int, vp, i64, C.POINTER(i64)]),
         "splpak_b200_fit_condition_estimate": (C.c_int, [vp, C.POINTER(C.c_double)]),
         "splpak_b200_fit_constraints_fired": (C.c_int, [vp]),

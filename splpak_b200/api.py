@@ -390,6 +390,46 @@ class FitHandle:
             raise SplpakError(f"get_selected_inverse failed: {rc}")
         return out.reshape(self.ncol, -1)
 
+    def prepare_variance(self):
+        """Posterior variances: after the (all-reduced) assembly and before compute, with the handle's current (lambda,
+        penalty).  Reuses the selected inverse select_smoothing left behind, otherwise scores once, then builds the
+        per-window tables the variance calls read.  Returns the smoothing_score dict plus sigma2 = rss / (n - edf) (+inf
+        when n <= edf); raises SplpakError on a non-zero code (107, 203, 204)."""
+        self._check()
+        out = np.zeros(6)
+        ierr = C.c_int(0)
+        rc = self.lib.splpak_b200_fit_prepare_variance(self.h, _ptr(out), 6, C.byref(ierr))
+        if rc != 0:
+            raise SplpakError(f"prepare_variance failed: {rc}", rc)
+        return dict(zip(self._SCORE_KEYS + ("sigma2",), (float(v) for v in out)))
+
+    def variance(self, x, nderiv=None):
+        """q(x) = b(x)^T Sigma b(x) at HOST points x (nq, l1x), after prepare_variance: the posterior variance of the
+        fitted value (nderiv: of that partial derivative) divided by sigma2.  Returns (q[nq], ierror)."""
+        self._check()
+        xa = np.ascontiguousarray(x, dtype=self.dt)
+        if xa.ndim == 1:
+            xa = xa.reshape(-1, 1)
+        nq, l1x = xa.shape
+        out = np.zeros(nq, dtype=self.dt)
+        nd = _vec(nderiv, np.int32, self.ndim) if nderiv is not None else None
+        ierr = C.c_int(0)
+        self.lib.splpak_b200_fit_variance(self.h, _ptr(xa), int(l1x), int(nq),
+                                          nd.ctypes.data_as(C.POINTER(C.c_int)) if nd is not None else None, _ptr(out),
+                                          C.byref(ierr))
+        return out, ierr.value
+
+    def variance_device(self, d_x, l1x, nq, d_out, nderiv=None, stream=None):
+        """variance with torch CUDA tensors (or raw device pointers); asynchronous on `stream` (None: the handle's
+        stream).  Returns ierror."""
+        self._check()
+        nd = _vec(nderiv, np.int32, self.ndim) if nderiv is not None else None
+        ierr = C.c_int(0)
+        self.lib.splpak_b200_fit_variance_device(self.h, _dev_ptr(d_x), int(l1x), int(nq),
+                                                 nd.ctypes.data_as(C.POINTER(C.c_int)) if nd is not None else None,
+                                                 _dev_ptr(d_out), _stream_ptr(stream), C.byref(ierr))
+        return ierr.value
+
     def orthogonal_factor(self, which):
         """Parity-test hook: which = 0 -> per-window triangles (nwindows, 4^ndim, 4^ndim + 1); 1 -> band factor (ncol, b + 2)."""
         self._check()

@@ -86,6 +86,11 @@ int spl_gcv_ywy_launch(const real_t *d_y, const real_t *d_w, int weighted, long 
 long long spl_gcv_part_len();
 int spl_gcv_stencil_launch(const GridParams &gp, const double *d_S, const double *d_AB, const double *d_c,
                            const double *d_g0, double *d_part, double *d_out3, cudaStream_t st);
+long long spl_variance_table_len(const GridParams &gp);
+int spl_variance_table_launch(const GridParams &gp, const double *d_AB, long long lda, double *d_W, cudaStream_t st,
+                              int nsm);
+int spl_variance_launch(const GridParams &gp, const int *nderiv, const real_t *d_x, int l1x, long long nq,
+                        const double *d_W, real_t *d_out, cudaStream_t st, int nsm);
 
 // ------------------------------------------------------------------------------------------
 // small conversion kernels
@@ -714,8 +719,10 @@ static EvalHostCtx &eval_host_ctx(int device) {
     return ctx[(device >= 0 && device < 64) ? device : 0];
 }
 
-// The host-array path of splpak_b200_eval / splpak_b200_eval_derivs: ncomp outputs per query, launch(d_x, nc, d_coef,
-// d_out, st) evaluates nc staged queries.  Returns the code of the call (ierror is the caller's business).
+// The host-array path of splpak_b200_eval / splpak_b200_eval_derivs / splpak_b200_fit_variance: ncomp outputs per query,
+// launch(d_x, nc, d_coef, d_out, st) evaluates nc staged queries.  coef == NULL: the launch reads no coefficient table
+// (the variance kernel reads the handle's tables), so none is uploaded and d_coef is NULL.  Returns the code of the
+// call (ierror is the caller's business).
 template <class Launch>
 static int eval_host_staged(const GridParams &gp, const DeviceInfo &di, const real_t *x, int l1x, long long nq,
                             const real_t *coef, real_t *out, int ncomp, Launch launch) {
@@ -741,7 +748,7 @@ static int eval_host_staged(const GridParams &gp, const DeviceInfo &di, const re
             EV_TRY(cudaEventCreateWithFlags(&cx.ev_done[k], cudaEventDisableTiming));
         }
     }
-    if ((size_t)(gp.ncol + 2) > cx.coef_cap) {
+    if (coef && (size_t)(gp.ncol + 2) > cx.coef_cap) {
         if (cx.d_coef) cudaFree(cx.d_coef);
         cx.d_coef = nullptr;
         cx.coef_cap = 0;
@@ -767,8 +774,8 @@ static int eval_host_staged(const GridParams &gp, const DeviceInfo &di, const re
         }
     }
     cudaStream_t st = cx.st, st2 = cx.st2;
-    real_t *d_coef = cx.d_coef;
-    {
+    real_t *d_coef = coef ? cx.d_coef : nullptr;
+    if (coef) {
         const size_t cbytes = sizeof(real_t) * (size_t)gp.ncol;
         if (!(cx.coef_valid && cx.coef_shadow.size() == cbytes && memcmp(cx.coef_shadow.data(), coef, cbytes) == 0)) {
             cx.coef_valid = false;
@@ -948,6 +955,13 @@ struct splpak_b200_fit_s {
                                   // selected-inverse scratch (allocated by the first score call)
     int s1_valid;                 // d_gcv holds S1 of the current assembly
     int sigma_valid;              // d_AB holds Sigma of the last score call
+    double sigma_lambda;          // (lambda, penalty) of that score call and its {V, RSS, edf, N, ywy}
+    int sigma_penalty;
+    double sigma_out[5];
+    // posterior variances (variance.cu): per-window tables of Sigma, built by prepare_variance, outside d_AB so that
+    // they survive compute and the refinement steps
+    double *d_var;                // spl_variance_table_len doubles, allocated by the first prepare_variance
+    int var_valid;                // d_var holds the tables of the current assembly and (lambda, penalty)
     void *score_cache;            // solve graphs of the score calls (their own buffers: compute keeps its graphs)
     void *selinv_cache;           // graph of the selected inverse
     // timing: accumulated event pairs
@@ -990,6 +1004,7 @@ static void free_handle(splpak_b200_fit_t h) {
     if (h->d_pen) cudaFree(h->d_pen);
     if (h->d_ywy_part) cudaFree(h->d_ywy_part);
     if (h->d_gcv) cudaFree(h->d_gcv);
+    if (h->d_var) cudaFree(h->d_var);
     if (h->score_cache) spl_solve_cache_free(h->score_cache);
     if (h->selinv_cache) spl_selinv_cache_free(h->selinv_cache);
     if (h->os) {
@@ -1078,7 +1093,7 @@ extern "C" int splpak_b200_fit_reset(splpak_b200_fit_t h) {
     h->timers_pending = 0;
     h->total_points = 0;
     h->solved = h->refining = h->constraints_fired = h->factor_valid = 0;
-    h->s1_valid = h->sigma_valid = 0;
+    h->s1_valid = h->sigma_valid = h->var_valid = 0;
     h->cond_est = 0.0;
     if (h->os) return spl_ortho_reset(h->gp, *h->os, h->st);
     return SPLPAK_OK;
@@ -1165,7 +1180,7 @@ static int add_device_chunk(splpak_b200_fit_t h, const real_t *d_x, int l1x, con
     rc = spl_assemble_chunk(h->gp, d_x, l1x, d_y, d_w, weighted, n, h->xtrap != 0.0, 0, h->sc, h->d_S,
                             h->d_g, h->d_cnt, h->d_totals, h->st, h->di.nsm, h->ev);
     if (rc == SPLPAK_OK && h->gcv) {
-        h->s1_valid = h->sigma_valid = 0;
+        h->s1_valid = h->sigma_valid = h->var_valid = 0;
         rc = spl_gcv_ywy_launch(d_y, weighted ? d_w : nullptr, weighted, n, h->d_ywy_part, h->d_ywy, h->st);
     }
     return rc;
@@ -1263,7 +1278,7 @@ extern "C" int splpak_b200_fit_add_points(splpak_b200_fit_t h, const real_t *x, 
 
 extern "C" int splpak_b200_fit_partial_buffer(splpak_b200_fit_t h, void **d_ptr, int64_t *count) {
     if (!valid(h)) return SPLPAK_ERR_HANDLE;
-    h->s1_valid = 0;                  // the caller may write the sums through the pointer (all-reduce)
+    h->s1_valid = h->var_valid = 0;   // the caller may write the sums through the pointer (all-reduce)
     if (d_ptr) *d_ptr = h->d_part;
     if (count) *count = h->n_part;
     return SPLPAK_OK;
@@ -1311,7 +1326,7 @@ extern "C" int splpak_b200_fit_allreduce(splpak_b200_fit_t h, void *nccl_comm) {
     NcclApi &api = nccl_api();
     if (!api.ok) return SPLPAK_ERR_NCCL;
     // ncclFloat64 = 8, ncclSum = 0 (nccl.h)
-    h->s1_valid = h->sigma_valid = 0;
+    h->s1_valid = h->sigma_valid = h->var_valid = 0;
     const int rc = api.AllReduce(h->d_part, h->d_part, (size_t)h->n_part, 8, 0, nccl_comm, h->st);
     return rc == 0 ? SPLPAK_OK : SPLPAK_ERR_NCCL;
 }
@@ -1765,6 +1780,7 @@ extern "C" int splpak_b200_fit_set_smoothing(splpak_b200_fit_t h, double lambda,
         h->d_pen = nullptr;
         return SPLPAK_ERR_ALLOC;
     }
+    if (lambda != h->lambda || (lambda > 0.0 && penalty != h->penalty)) h->var_valid = 0;   // another system
     h->lambda = lambda;
     h->penalty = penalty;
     return SPLPAK_OK;
@@ -1794,7 +1810,7 @@ extern "C" int splpak_b200_fit_enable_gcv(splpak_b200_fit_t h) {
     h->d_ywy = h->d_totals + 2;
     SPL_CUDA_TRY(cudaMemsetAsync(h->d_part, 0, sizeof(double) * (size_t)h->n_part, h->st));
     h->gcv = 1;
-    h->s1_valid = h->sigma_valid = 0;
+    h->s1_valid = h->sigma_valid = h->var_valid = 0;
     return SPLPAK_OK;
 }
 
@@ -1893,6 +1909,9 @@ static int gcv_score_impl(splpak_b200_fit_t h, double lambda, int penalty, doubl
     out5[3] = N;
     out5[4] = ywy;
     h->sigma_valid = 1;
+    h->sigma_lambda = lambda;
+    h->sigma_penalty = penalty;
+    memcpy(h->sigma_out, out5, sizeof(h->sigma_out));
     return SPLPAK_OK;
 }
 
@@ -2051,6 +2070,75 @@ extern "C" int splpak_b200_fit_get_selected_inverse(splpak_b200_fit_t h, double 
     SPL_CUDA_TRY(cudaMemcpy2D(out, sizeof(double) * (size_t)(bw + 1), h->d_AB, sizeof(double) * (size_t)(lda + 1),
                               sizeof(double) * (size_t)(bw + 1), (size_t)gp.ncol, cudaMemcpyDeviceToHost));
     return SPLPAK_OK;
+}
+
+// ---- posterior variances (variance.cu; DESIGN §4.13) ----
+extern "C" int splpak_b200_fit_prepare_variance(splpak_b200_fit_t h, double *out, int nout, int *ierror) {
+    int rc = SPLPAK_OK;
+    if (!valid(h) || h->finalized || !h->gcv || h->solver == SPLPAK_SOLVER_ORTHOGONAL || !out || nout < 6)
+        rc = SPLPAK_ERR_HANDLE;
+    double o[5];
+    if (rc == SPLPAK_OK) {
+        // Sigma of exactly the handle's current system is already in d_AB (after select_smoothing): no second score
+        const bool same = h->sigma_valid && h->s1_valid && h->sigma_lambda == h->lambda &&
+                          (h->lambda == 0.0 || h->sigma_penalty == h->penalty);
+        h->var_valid = 0;
+        if (same) memcpy(o, h->sigma_out, sizeof(o));
+        else rc = gcv_score_impl(h, h->lambda, h->penalty, o);
+    }
+    if (rc == SPLPAK_OK && !h->d_var &&
+        cudaMalloc((void **)&h->d_var, sizeof(double) * (size_t)spl_variance_table_len(h->gp)) != cudaSuccess) {
+        cudaGetLastError();
+        h->d_var = nullptr;
+        rc = SPLPAK_ERR_ALLOC;
+    }
+    if (rc == SPLPAK_OK) {
+        const long long lda = spl_band_lda(spl_half_bandwidth(h->gp));
+        rc = spl_variance_table_launch(h->gp, h->d_AB, lda, h->d_var, h->st, h->di.nsm);
+        // complete before returning: variance_device may run on any stream
+        if (rc == SPLPAK_OK && cudaStreamSynchronize(h->st) != cudaSuccess) {
+            cudaGetLastError();
+            rc = SPLPAK_ERR_CUDA;
+        }
+    }
+    if (rc == SPLPAK_OK) {
+        h->var_valid = 1;
+        const double dof = o[3] - o[2];
+        memcpy(out, o, sizeof(o));
+        out[5] = dof > 0.0 ? o[1] / dof : INFINITY;
+    }
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+static int variance_check(splpak_b200_fit_t h, int l1x, const int *nderiv) {
+    if (!valid(h) || !h->var_valid || l1x < h->gp.ndim) return SPLPAK_ERR_HANDLE;
+    for (int d = 0; d < h->gp.ndim && nderiv; ++d)
+        if (nderiv[d] < 0 || nderiv[d] > 2) return SPLPAK_ERR_NDERIV;
+    return SPLPAK_OK;
+}
+
+extern "C" int splpak_b200_fit_variance_device(splpak_b200_fit_t h, const real_t *d_x, int l1x, int64_t nq,
+                                               const int *nderiv, real_t *d_out, void *stream, int *ierror) {
+    int rc = variance_check(h, l1x, nderiv);
+    if (rc == SPLPAK_OK && nq > 0)
+        rc = spl_variance_launch(h->gp, nderiv, d_x, l1x, nq, h->d_var, d_out,
+                                 stream ? (cudaStream_t)stream : h->st, h->di.nsm);
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+extern "C" int splpak_b200_fit_variance(splpak_b200_fit_t h, const real_t *x, int l1x, int64_t nq, const int *nderiv,
+                                        real_t *out, int *ierror) {
+    int rc = variance_check(h, l1x, nderiv);
+    if (rc == SPLPAK_OK && nq > 0)
+        rc = eval_host_staged(h->gp, h->di, x, l1x, nq, nullptr, out, 1,
+                              [&](const real_t *d_x, long long n, const real_t *, real_t *d_out, cudaStream_t st) {
+                                  return spl_variance_launch(h->gp, nderiv, d_x, l1x, n, h->d_var, d_out, st,
+                                                             h->di.nsm);
+                              });
+    if (ierror) *ierror = rc;
+    return rc;
 }
 
 // Parity-test hook of the orthogonal path: which = 0 -> the per-window triangles [nwindows][ncw][ncw + 1] (R_w | z_w),
