@@ -65,6 +65,8 @@
         procedure,public :: enable_gcv                   !! (new) streaming fit: collect what the GCV score needs (before add_points)
         procedure,public :: smoothing_score              !! (new) streaming fit: GCV score {V, RSS, edf, N, ywy} of one lambda
         procedure,public :: select_smoothing             !! (new) streaming fit: lambda minimising the GCV score, set on the fit
+        procedure,public :: reml_score                   !! (new) streaming fit: REML score {V_R, D_p, log|M|, n, ywy, phi} of one lambda
+        procedure,public :: select_smoothing_reml        !! (new) streaming fit: lambda minimising the REML score, set on the fit
         procedure,public :: prepare_variance             !! (new) streaming fit: tables of the posterior variances (before compute)
         procedure,public :: variance                     !! (new) streaming fit: b(x)^T Sigma b(x) at a batch of points
         procedure,private :: splcc
@@ -235,6 +237,28 @@
             integer(c_int),intent(out) :: ierror
             integer(c_int) :: rc
         end function c_fit_select_smoothing
+        function c_fit_reml_score(h,lambda,penalty,out,nout,ierror) &
+                 bind(C,name='splpak_b200_fit_reml_score') result(rc)
+            import :: c_int, c_double, c_ptr
+            type(c_ptr),value :: h
+            real(c_double),value :: lambda
+            integer(c_int),value :: penalty, nout
+            real(c_double),intent(out) :: out(*)
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_reml_score
+        function c_fit_select_smoothing_reml(h,penalty,lambda_lo,lambda_hi,lambda,out,nout,trace,trace_cap,ntrace,ierror) &
+                 bind(C,name='splpak_b200_fit_select_smoothing_reml') result(rc)
+            import :: c_int, c_int64_t, c_double, c_ptr
+            type(c_ptr),value :: h
+            integer(c_int),value :: penalty, nout
+            real(c_double),value :: lambda_lo, lambda_hi
+            real(c_double),intent(out) :: lambda, out(*), trace(*)
+            integer(c_int64_t),value :: trace_cap
+            integer(c_int64_t),intent(out) :: ntrace
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_select_smoothing_reml
         function c_fit_prepare_variance(h,out,nout,ierror) bind(C,name='splpak_b200_fit_prepare_variance') result(rc)
             import :: c_int, c_double, c_ptr
             type(c_ptr),value :: h
@@ -494,6 +518,36 @@
                                     trace,0_c_int64_t,ntrace,ierr)
         ierror = int(rc)
     end subroutine select_smoothing
+
+    !> (new) REML score of smoothing lambda > 0 after the assembly, before compute (changes nothing compute
+    !  sees): score = [V_R, D_p, log|M|, n, ywy, phi], n counting the constraint rows, phi = D_p / (n - Mp).
+    !  ierror = 107 for a non-positive pivot, 203 when refused (also for lambda <= 0).
+    subroutine reml_score(me,lambda,penalty,score,ierror)
+        class(splpak_type),intent(inout) :: me
+        real(c_double),intent(in) :: lambda
+        integer,intent(in) :: penalty
+        real(c_double),intent(out) :: score(6)
+        integer,intent(out) :: ierror
+        integer(c_int) :: ierr, rc
+        rc = c_fit_reml_score(me%handle,lambda,int(penalty,c_int),score,6_c_int,ierr)
+        ierror = int(rc)
+    end subroutine reml_score
+
+    !> (new) lambda minimising the REML score over [lambda_lo, lambda_hi] (either <= 0: the default range),
+    !  then set on the fit, so the next compute is the selected fit.  score as reml_score.
+    subroutine select_smoothing_reml(me,penalty,lambda_lo,lambda_hi,lambda,score,ierror)
+        class(splpak_type),intent(inout) :: me
+        integer,intent(in) :: penalty
+        real(c_double),intent(in) :: lambda_lo, lambda_hi
+        real(c_double),intent(out) :: lambda, score(6)
+        integer,intent(out) :: ierror
+        integer(c_int) :: ierr, rc
+        integer(c_int64_t) :: ntrace
+        real(c_double) :: trace(4)
+        rc = c_fit_select_smoothing_reml(me%handle,int(penalty,c_int),lambda_lo,lambda_hi,lambda,score,6_c_int, &
+                                         trace,0_c_int64_t,ntrace,ierr)
+        ierror = int(rc)
+    end subroutine select_smoothing_reml
 
     !> (new) posterior variances of a smoothing fit, after the assembly (and select_smoothing) and before
     !  compute: builds the per-window tables from Sigma of the fit's current lambda (scoring once unless

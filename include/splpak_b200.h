@@ -248,6 +248,32 @@ int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty, double la
                                      double *out, int nout, double *trace, int64_t trace_cap, int64_t *ntrace,
                                      int *ierror);
 int splpak_b200_fit_get_selected_inverse(splpak_b200_fit_t h, double *out, int64_t capacity, int64_t *count);
+/* Choosing lambda by REML (restricted maximum likelihood) -- (new).  M = G0 + C + lambda R and c = M^-1 g as above,
+ * p = ncol, Mp the dimension of the penalty's null space (2^ndim for CURVATURE, ndim + 1 for THIN_PLATE, 2 for both in
+ * 1-D), n the rows of the system COUNTING THE CONSTRAINT ROWS: they enter the likelihood as observations with a zero
+ * response (GCV counts them as part of the regulariser instead; as data the score stays exact and needs only the factor).
+ *     D_p   = ywy - 2 c.g + c^T M c          (= weighted RSS + constraint-row residuals + lambda c^T R c)
+ *     phi   = D_p / (n - Mp)                 (the REML estimate of the noise variance)
+ *     V_R   = (n - Mp) log(D_p / (n - Mp)) + log|M| - (p - Mp) log lambda
+ * V_R is -2 x the restricted log-likelihood with the noise variance profiled out, WITHOUT its two lambda-independent
+ * terms + (n - Mp)(1 + log 2 pi) and - log|R|+ (|R|+ the product of the non-zero eigenvalues of R): compare V_R only
+ * across lambda for one grid and penalty.  log|M| = 2 sum log L_jj from the Cholesky factor; no selected inverse.
+ * V_R = +inf when n <= Mp.
+ *   reml_score          preconditions as smoothing_score (enable_gcv, Cholesky solver, after the all-reduced assembly,
+ *                       before fit_compute; S, g, the counts and the totals stay untouched).  lambda > 0 (V_R -> +inf as
+ *                       lambda -> 0).  out[0..5] = {V_R, D_p, log|M|, n, ywy, phi}, nout >= 6.  A non-positive pivot
+ *                       returns 107.  It overwrites the band storage with a factor: get_selected_inverse returns 203 after
+ *                       it, and a following prepare_variance scores by GCV once.
+ *   select_smoothing_reml  V_R minimised with the search, default range and tie rule of select_smoothing; points with a
+ *                       non-positive pivot count as +inf.  On success set_smoothing(best, penalty), the best point's six
+ *                       values in out, trace rows [lambda, V_R, D_p, log|M|].  prepare_variance after it returns GCV's
+ *                       sigma2 = RSS / (N - edf), not phi.
+ * FP64, fixed-order reductions: bit-identical across calls, handles and ranks given the same summed partial buffer.
+ * 203: as smoothing_score, and lambda <= 0. */
+int splpak_b200_fit_reml_score(splpak_b200_fit_t h, double lambda, int penalty, double *out, int nout, int *ierror);
+int splpak_b200_fit_select_smoothing_reml(splpak_b200_fit_t h, int penalty, double lambda_lo, double lambda_hi,
+                                          double *lambda, double *out, int nout, double *trace, int64_t trace_cap,
+                                          int64_t *ntrace, int *ierror);
 /* Pointwise posterior variances of a smoothing fit -- (new).  With Sigma = M^-1 as above and b_k(x) the row of basis
  * values (nderiv = k: of their partial derivatives) at x,
  *     q_k(x) = b_k(x)^T Sigma b_k(x),     Var[d^k s(x)] = sigma2 q_k(x)     (the Bayesian posterior variance)

@@ -55,6 +55,8 @@ SYMBOLS = [
     "splpak_b200_fit_smoothing_score",
     "splpak_b200_fit_select_smoothing",
     "splpak_b200_fit_get_selected_inverse",
+    "splpak_b200_fit_reml_score",
+    "splpak_b200_fit_select_smoothing_reml",
     "splpak_b200_fit_prepare_variance",
     "splpak_b200_fit_variance",
     "splpak_b200_fit_variance_device",
@@ -157,6 +159,9 @@ def load(real32: bool = False) -> C.CDLL:
         "splpak_b200_fit_select_smoothing": (C.c_int, [vp, C.c_int, C.c_double, C.c_double, C.POINTER(C.c_double), vp,
                                                        C.c_int, vp, i64, C.POINTER(i64), ip]),
         "splpak_b200_fit_get_selected_inverse": (C.c_int, [vp, vp, i64, C.POINTER(i64)]),
+        "splpak_b200_fit_reml_score": (C.c_int, [vp, C.c_double, C.c_int, vp, C.c_int, ip]),
+        "splpak_b200_fit_select_smoothing_reml": (C.c_int, [vp, C.c_int, C.c_double, C.c_double, C.POINTER(C.c_double),
+                                                            vp, C.c_int, vp, i64, C.POINTER(i64), ip]),
         "splpak_b200_fit_prepare_variance": (C.c_int, [vp, vp, C.c_int, ip]),
         "splpak_b200_fit_variance": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, ip]),
         "splpak_b200_fit_variance_device": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, vp, ip]),

@@ -360,23 +360,50 @@ class FitHandle:
             raise SplpakError(f"smoothing_score failed: {rc}", rc)
         return dict(zip(self._SCORE_KEYS, (float(v) for v in out)))
 
-    def select_smoothing(self, penalty="curvature", lo=None, hi=None, trace_cap=512):
-        """lambda minimising the GCV score over [lo, hi] (default: rho * [1e-10, 1e4], rho = tr G0 / tr R); sets it on
-        the handle (set_smoothing), so the next compute is the selected fit.  Returns (lam, score dict, trace), trace:
-        (k, 4) rows [lambda, V, RSS, edf] in evaluation order.  Raises SplpakError on a non-zero code."""
+    _REML_KEYS = ("reml", "dp", "logdet", "n", "ywy", "phi")
+
+    def reml_score(self, lam, penalty="curvature"):
+        """REML score of the fit with smoothing `lam` > 0, after the (all-reduced) assembly and before compute; changes
+        nothing a later compute sees.  Returns {reml, dp, logdet, n, ywy, phi}: V_R (-2 x the profiled restricted
+        log-likelihood up to terms that do not depend on lam), the penalised deviance, log|M|, the rows counted
+        (constraint rows included), ywy and phi = dp / (n - Mp), the REML estimate of the noise variance.  Raises
+        SplpakError on a non-zero code (107: a non-positive pivot, 203: refused)."""
         self._check()
+        out = np.zeros(6)
+        ierr = C.c_int(0)
+        rc = self.lib.splpak_b200_fit_reml_score(self.h, float(lam), self._penalty_code(penalty), _ptr(out), 6,
+                                                 C.byref(ierr))
+        if rc != 0:
+            raise SplpakError(f"reml_score failed: {rc}", rc)
+        return dict(zip(self._REML_KEYS, (float(v) for v in out)))
+
+    CRITERIA = ("gcv", "reml")
+
+    def _criterion_is_reml(self, criterion):
+        if criterion not in self.CRITERIA:
+            raise SplpakError(f"unknown criterion {criterion!r}: expected one of {list(self.CRITERIA)}")
+        return criterion == "reml"
+
+    def select_smoothing(self, penalty="curvature", lo=None, hi=None, trace_cap=512, criterion="gcv"):
+        """lambda minimising the GCV score (criterion="gcv") or the REML score (criterion="reml") over [lo, hi]
+        (default: rho * [1e-10, 1e4], rho = tr G0 / tr R); sets it on the handle (set_smoothing), so the next compute is
+        the selected fit.  Returns (lam, score dict, trace), trace: (k, 4) rows in evaluation order, [lambda, V, RSS, edf]
+        for GCV, [lambda, V_R, dp, logdet] for REML; the score dict is that of smoothing_score or reml_score.  Raises
+        SplpakError on a non-zero code or an unknown criterion."""
+        reml = self._criterion_is_reml(criterion)
+        self._check()
+        fn = self.lib.splpak_b200_fit_select_smoothing_reml if reml else self.lib.splpak_b200_fit_select_smoothing
+        keys = self._REML_KEYS if reml else self._SCORE_KEYS
         lam = C.c_double(0.0)
-        out = np.zeros(5)
+        out = np.zeros(len(keys))
         trace = np.zeros((int(trace_cap), 4))
         nt = C.c_int64(0)
         ierr = C.c_int(0)
-        rc = self.lib.splpak_b200_fit_select_smoothing(self.h, self._penalty_code(penalty),
-                                                       0.0 if lo is None else float(lo), 0.0 if hi is None else float(hi),
-                                                       C.byref(lam), _ptr(out), 5, _ptr(trace), int(trace_cap),
-                                                       C.byref(nt), C.byref(ierr))
+        rc = fn(self.h, self._penalty_code(penalty), 0.0 if lo is None else float(lo), 0.0 if hi is None else float(hi),
+                C.byref(lam), _ptr(out), len(keys), _ptr(trace), int(trace_cap), C.byref(nt), C.byref(ierr))
         if rc != 0:
             raise SplpakError(f"select_smoothing failed: {rc}", rc)
-        return lam.value, dict(zip(self._SCORE_KEYS, (float(v) for v in out))), trace[: min(nt.value, int(trace_cap))]
+        return lam.value, dict(zip(keys, (float(v) for v in out))), trace[: min(nt.value, int(trace_cap))]
 
     def selected_inverse(self):
         """Parity hook, after a score call: (ncol, b + 1), row i = Sigma(i, i..i+b), Sigma = (G0 + C + lambda R)^-1."""

@@ -84,6 +84,8 @@ void spl_selinv_cache_free(void *cache);
 int spl_gcv_ywy_launch(const real_t *d_y, const real_t *d_w, int weighted, long long n, double *d_part, double *d_ywy,
                        cudaStream_t st);
 long long spl_gcv_part_len();
+int spl_reml_stencil_launch(const GridParams &gp, const double *d_M, const double *d_c, const double *d_g,
+                            const double *d_linv, double *d_part, double *d_out3, cudaStream_t st);
 int spl_gcv_stencil_launch(const GridParams &gp, const double *d_S, const double *d_AB, const double *d_c,
                            const double *d_g0, double *d_part, double *d_out3, cudaStream_t st);
 long long spl_variance_table_len(const GridParams &gp);
@@ -1835,8 +1837,10 @@ static GcvScratch gcv_scratch_layout(const GridParams &gp) {
     return L;
 }
 
-// {V, RSS, edf, N, ywy} of one lambda.  Leaves S, g, cnt and totals as they are; d_AB then holds Sigma.
-static int gcv_score_impl(splpak_b200_fit_t h, double lambda, int penalty, double out5[5]) {
+// The part both scores share: M = S1 + lambda R into S2 (S1 = G0 + C cached per assembly), then the factor and solve
+// of M c = g in d_AB / the workspace behind it (band_elems doubles in), c at *d_sol.  Leaves S, g, cnt and totals as
+// they are.  Clears sigma_valid: d_AB no longer holds Sigma.  SPLPAK_ERR_SOLVER for a non-positive pivot.
+static int score_factor(splpak_b200_fit_t h, double lambda, int penalty, long long *band_elems_out, double **d_sol_out) {
     const GridParams &gp = h->gp;
     cudaStream_t st = h->st;
     long long band_elems = 0, need = 0;
@@ -1860,7 +1864,6 @@ static int gcv_score_impl(splpak_b200_fit_t h, double lambda, int penalty, doubl
     }
     const long long ns = gp.ncol * gp.nsten;
     double *d_S1 = h->d_gcv + L.S1, *d_S2 = h->d_gcv + L.S2, *d_g2 = h->d_gcv + L.g2, *d_tot1 = h->d_gcv + L.tot1;
-    double *d_res = h->d_gcv + L.res, *d_red = h->d_gcv + L.red, *d_sel = h->d_gcv + L.sel;
     h->sigma_valid = 0;
     if (!h->s1_valid) {
         // S1 = G0 + C: the constraint rows through the fixed-point limbs, as in compute, on copies of S and the totals
@@ -1890,6 +1893,21 @@ static int gcv_score_impl(splpak_b200_fit_t h, double lambda, int penalty, doubl
     SPL_CUDA_TRY(cudaMemcpyAsync(&fail, h->d_fail, sizeof(int), cudaMemcpyDeviceToHost, st));
     SPL_CUDA_TRY(cudaStreamSynchronize(st));
     if (fail) return SPLPAK_ERR_SOLVER;
+    *band_elems_out = band_elems;
+    *d_sol_out = d_sol;
+    return SPLPAK_OK;
+}
+
+// {V, RSS, edf, N, ywy} of one lambda.  Leaves S, g, cnt and totals as they are; d_AB then holds Sigma.
+static int gcv_score_impl(splpak_b200_fit_t h, double lambda, int penalty, double out5[5]) {
+    const GridParams &gp = h->gp;
+    cudaStream_t st = h->st;
+    long long band_elems = 0;
+    double *d_sol = nullptr;
+    int rc = score_factor(h, lambda, penalty, &band_elems, &d_sol);
+    if (rc != SPLPAK_OK) return rc;
+    const GcvScratch L = gcv_scratch_layout(gp);
+    double *d_res = h->d_gcv + L.res, *d_red = h->d_gcv + L.red, *d_sel = h->d_gcv + L.sel;
     rc = spl_selinv_launch(gp, h->d_AB, h->d_AB + band_elems, d_sel, st, &h->selinv_cache);
     if (rc != SPLPAK_OK) return rc;
     rc = spl_gcv_stencil_launch(gp, h->d_S, h->d_AB, d_sol, h->d_g, d_red, d_res, st);
@@ -1930,14 +1948,67 @@ extern "C" int splpak_b200_fit_smoothing_score(splpak_b200_fit_t h, double lambd
     return rc;
 }
 
-extern "C" int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty, double lambda_lo, double lambda_hi,
-                                                double *lambda, double *out, int nout, double *trace, int64_t trace_cap,
-                                                int64_t *ntrace, int *ierror) {
+// ---- REML (selinv.cu: spl_reml_stencil_kernel; DESIGN §4.14) ----
+// Dimension Mp of the penalty's null space: the multilinear functions (curvature), the affine ones (thin plate); 2 in 1-D.
+static int penalty_null_dim(int ndim, int penalty) {
+    return penalty == SPLPAK_PENALTY_CURVATURE ? 1 << ndim : ndim + 1;
+}
+
+// {V_R, D_p, log|M|, n, ywy, phi} of one lambda > 0.  Leaves S, g, cnt and totals as they are; d_AB then holds the
+// factor of M, not Sigma (score_factor clears sigma_valid).
+static int reml_score_impl(splpak_b200_fit_t h, double lambda, int penalty, double out6[6]) {
+    const GridParams &gp = h->gp;
+    cudaStream_t st = h->st;
+    long long band_elems = 0;
+    double *d_sol = nullptr;
+    int rc = score_factor(h, lambda, penalty, &band_elems, &d_sol);
+    if (rc != SPLPAK_OK) return rc;
+    const GcvScratch L = gcv_scratch_layout(gp);
+    double *d_res = h->d_gcv + L.res, *d_red = h->d_gcv + L.red;
+    // M = S2: the band expansion and the solve only read it
+    rc = spl_reml_stencil_launch(gp, h->d_gcv + L.S2, d_sol, h->d_g, h->d_AB + band_elems, d_red, d_res, st);
+    if (rc != SPLPAK_OK) return rc;
+    double r[3], tot1[2], ywy = 0.0;
+    SPL_CUDA_TRY(cudaMemcpyAsync(r, d_res, sizeof(r), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(tot1, h->d_gcv + L.tot1, sizeof(tot1), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(&ywy, h->d_ywy, sizeof(double), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaStreamSynchronize(st));
+    // n: the data rows and the constraint rows (their totals after the constraint kernel)
+    const double n = tot1[1], mp = (double)penalty_null_dim(gp.ndim, penalty), p = (double)gp.ncol;
+    // the quadratic form, not ywy - c.g: at the minimiser its error is second order in the solve's error
+    const double dp = ywy - 2.0 * r[1] + r[0];
+    const double logdet = 2.0 * r[2];
+    const double dof = n - mp;
+    out6[0] = dof > 0.0 ? dof * log(dp / dof) + logdet - (p - mp) * log(lambda) : INFINITY;
+    out6[1] = dp;
+    out6[2] = logdet;
+    out6[3] = n;
+    out6[4] = ywy;
+    out6[5] = dof > 0.0 ? dp / dof : INFINITY;
+    return SPLPAK_OK;
+}
+
+extern "C" int splpak_b200_fit_reml_score(splpak_b200_fit_t h, double lambda, int penalty, double *out, int nout,
+                                          int *ierror) {
+    int rc = gcv_check(h, penalty);
+    if (rc == SPLPAK_OK && (!(lambda > 0.0) || !isfinite(lambda) || !out || nout < 6)) rc = SPLPAK_ERR_HANDLE;
+    if (rc == SPLPAK_OK) rc = reml_score_impl(h, lambda, penalty, out);
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+// The search of select_smoothing and select_smoothing_reml: `score` writes nres outputs, the criterion first, and
+// returns SPLPAK_ERR_SOLVER for a non-positive pivot.  rescore: when the best point was not the last one evaluated,
+// score it again at the end (the GCV score leaves that point's Sigma behind).
+typedef int (*ScoreFn)(splpak_b200_fit_t, double, int, double *);
+static int select_smoothing_search(splpak_b200_fit_t h, int penalty, double lambda_lo, double lambda_hi, ScoreFn score,
+                                   int nres, bool rescore, double *lambda, double *out, int nout, double *trace,
+                                   int64_t trace_cap, int64_t *ntrace, int *ierror) {
     int rc = gcv_check(h, penalty);
     if (rc == SPLPAK_OK && (isnan(lambda_lo) || isnan(lambda_hi) || isinf(lambda_lo) || isinf(lambda_hi)))
         rc = SPLPAK_ERR_HANDLE;
     if (rc == SPLPAK_OK && lambda_lo > lambda_hi) rc = SPLPAK_ERR_HANDLE;
-    if (rc == SPLPAK_OK && out && nout < 5) rc = SPLPAK_ERR_HANDLE;
+    if (rc == SPLPAK_OK && out && nout < nres) rc = SPLPAK_ERR_HANDLE;
     if (rc != SPLPAK_OK) {
         if (ierror) *ierror = rc;
         return rc;
@@ -1968,13 +2039,13 @@ extern "C" int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty
     }
     // every evaluated point, in order; the best is the smallest V, ties to the larger lambda
     int64_t neval = 0;
-    double best_t = 0.0, best_v = INFINITY, best_out[5] = {0, 0, 0, 0, 0}, last_t = 0.0;
+    double best_t = 0.0, best_v = INFINITY, best_out[6] = {0, 0, 0, 0, 0, 0}, last_t = 0.0;
     bool any_ok = false, have_best = false;
     auto eval = [&](double t, double *v) -> int {
         const double lam = pow(10.0, t);
         last_t = t;
-        double o[5];
-        const int r = gcv_score_impl(h, lam, penalty, o);
+        double o[6];
+        const int r = score(h, lam, penalty, o);
         if (r != SPLPAK_OK && r != SPLPAK_ERR_SOLVER) return r;
         if (r == SPLPAK_ERR_SOLVER) {
             o[0] = INFINITY;
@@ -1993,7 +2064,7 @@ extern "C" int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty
             have_best = true;
             best_t = t;
             best_v = o[0];
-            memcpy(best_out, o, sizeof(o));
+            memcpy(best_out, o, sizeof(double) * (size_t)nres);
         }
         *v = o[0];
         return SPLPAK_OK;
@@ -2038,7 +2109,7 @@ extern "C" int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty
     }
     if (ntrace) *ntrace = (trace && neval > trace_cap) ? trace_cap : neval;
     if (rc == SPLPAK_OK && !any_ok) rc = SPLPAK_ERR_SOLVER;
-    if (rc == SPLPAK_OK && last_t != best_t) {
+    if (rescore && rc == SPLPAK_OK && last_t != best_t) {
         // d_AB holds Sigma of the last point evaluated: score the selected lambda again, so that get_selected_inverse
         // returns the inverse of the system the handle now carries (the same inputs: the same scores, bit for bit)
         double o[5];
@@ -2049,11 +2120,25 @@ extern "C" int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty
         rc = splpak_b200_fit_set_smoothing(h, lam, penalty);
         if (rc == SPLPAK_OK) {
             if (lambda) *lambda = lam;
-            if (out) memcpy(out, best_out, sizeof(best_out));
+            if (out) memcpy(out, best_out, sizeof(double) * (size_t)nres);
         }
     }
     if (ierror) *ierror = rc;
     return rc;
+}
+
+extern "C" int splpak_b200_fit_select_smoothing(splpak_b200_fit_t h, int penalty, double lambda_lo, double lambda_hi,
+                                                double *lambda, double *out, int nout, double *trace, int64_t trace_cap,
+                                                int64_t *ntrace, int *ierror) {
+    return select_smoothing_search(h, penalty, lambda_lo, lambda_hi, gcv_score_impl, 5, true, lambda, out, nout, trace,
+                                   trace_cap, ntrace, ierror);
+}
+
+extern "C" int splpak_b200_fit_select_smoothing_reml(splpak_b200_fit_t h, int penalty, double lambda_lo,
+                                                     double lambda_hi, double *lambda, double *out, int nout,
+                                                     double *trace, int64_t trace_cap, int64_t *ntrace, int *ierror) {
+    return select_smoothing_search(h, penalty, lambda_lo, lambda_hi, reml_score_impl, 6, false, lambda, out, nout,
+                                   trace, trace_cap, ntrace, ierror);
 }
 
 extern "C" int splpak_b200_fit_get_selected_inverse(splpak_b200_fit_t h, double *out, int64_t capacity, int64_t *count) {

@@ -1,5 +1,5 @@
 // selinv.cu -- exact band selected inverse of the Cholesky factor and the generalized cross-validation score of a
-// smoothing fit (splpak_b200_fit_smoothing_score; DESIGN §4.12).
+// smoothing fit (splpak_b200_fit_smoothing_score; DESIGN §4.12), and the reductions of the REML score (§4.14).
 //
 // After spl_solve_launch, AB holds L in band storage (below the 64 x 64 diagonal blocks) and the workspace behind it the
 // block inverses Linv_K = L_KK^-1 (row-major, 4096 doubles per panel).  Sigma = M^-1 = L^-T L^-1 is formed on the band
@@ -18,6 +18,9 @@
 // GCV (fixed-order reductions, FP64):
 //   spl_gcv_ywy_kernel      sum (w y)^2 of an add_points chunk (per-CTA partials, spl_gcv_ywy_finish adds them in order)
 //   spl_gcv_stencil_kernel  edf = sum Sigma_ij G0_ij, c^T G0 c and c.g0 over the 7^ndim stencil of every column
+//
+// REML (splpak_b200_fit_reml_score; DESIGN §4.14), on the factor alone (no selected inverse):
+//   spl_reml_stencil_kernel c^T M c over the same stencil walk, c.g, and sum log L_jj from the stored block inverses
 #include <stdlib.h>
 #include <string.h>
 #include <new>
@@ -328,6 +331,30 @@ int spl_gcv_ywy_launch(const real_t *d_y, const real_t *d_w, int weighted, long 
     return SPLPAK_OK;
 }
 
+// The stencil pair (i, j) of column j (node digits jd) at the signed offset tuple cc (base 7, one digit per dimension: the offset + 3),
+// the walk of spl_expand_band_kernel: false when node i lies outside the grid; otherwise *i and *slot, the position of
+// the pair's entry in orthant-stencil storage (node * nsten + sten).
+__device__ __forceinline__ bool gcv_stencil_pair(const GridParams &gp, const int (&jd)[SPL_MAXDIM], const long long j,
+                                                 int cc, long long *i, long long *slot) {
+    int sten = 0, sstride = 1;
+    long long off = 0, node = 0, nstride = 1;
+    bool inside = true;
+    for (int d = 0; d < gp.ndim; ++d) {
+        const int dd = cc % 7 - 3;
+        cc /= 7;
+        const int id = jd[d] + dd;
+        if (id < 0 || id >= gp.nodes[d]) inside = false;
+        off += (long long)dd * nstride;
+        node += (long long)(dd < 0 ? id : jd[d]) * nstride;
+        sten += (dd < 0 ? -dd : dd) * sstride;
+        nstride *= gp.nodes[d];
+        sstride *= 4;
+    }
+    *i = j + off;
+    *slot = node * gp.nsten + sten;
+    return inside;
+}
+
 // One CTA per column j (grid-stride), the threads over the 7^ndim signed offsets (the walk of spl_expand_band_kernel):
 // for every stencil neighbour i of j,  edf += Sigma_ij G0_ij,  cGc += c_i G0_ij c_j;  and c.g0 += c_j g0_j.
 __global__ void __launch_bounds__(256)
@@ -349,24 +376,10 @@ spl_gcv_stencil_kernel(const __grid_constant__ GridParams gp, const double *__re
         const double cj = c[j];
         if (threadIdx.x == 0) v[2] = fma(cj, g0[j], v[2]);
         for (int cc0 = threadIdx.x; cc0 < ncombo; cc0 += blockDim.x) {
-            int cc = cc0, sten = 0, sstride = 1;
-            long long off = 0, node = 0, nstride = 1;
-            bool inside = true;
-            for (int d = 0; d < gp.ndim; ++d) {
-                const int dd = cc % 7 - 3;
-                cc /= 7;
-                const int id = jd[d] + dd;
-                if (id < 0 || id >= gp.nodes[d]) inside = false;
-                off += (long long)dd * nstride;
-                node += (long long)(dd < 0 ? id : jd[d]) * nstride;
-                sten += (dd < 0 ? -dd : dd) * sstride;
-                nstride *= gp.nodes[d];
-                sstride *= 4;
-            }
-            if (!inside) continue;
-            const long long i = j + off;
-            const double gij = S[node * gp.nsten + sten];
-            const double sij = off >= 0 ? AB[i + j * lda] : AB[j + i * lda];
+            long long i, slot;
+            if (!gcv_stencil_pair(gp, jd, j, cc0, &i, &slot)) continue;
+            const double gij = S[slot];
+            const double sij = i >= j ? AB[i + j * lda] : AB[j + i * lda];
             v[0] = fma(sij, gij, v[0]);
             v[1] = fma(c[i] * gij, cj, v[1]);
         }
@@ -393,6 +406,58 @@ int spl_gcv_stencil_launch(const GridParams &gp, const double *d_S, const double
                            const double *d_g0, double *d_part, double *d_out3, cudaStream_t st) {
     const long long lda = spl_band_lda(spl_half_bandwidth(gp));
     spl_gcv_stencil_kernel<<<GCV_BLOCKS, 256, 0, st>>>(gp, d_S, d_AB, lda, d_c, d_g0, d_part);
+    spl_gcv_stencil_finish<<<1, 32, 0, st>>>(d_part, d_out3);
+    g_spl_launches += 2;
+    SPL_CUDA_TRY(cudaGetLastError());
+    return SPLPAK_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// REML reductions (splpak_b200_fit_reml_score; DESIGN §4.14)
+// ------------------------------------------------------------------------------------------
+// One CTA per column j (grid-stride), the threads over the 7^ndim signed offsets as spl_gcv_stencil_kernel:
+// for every stencil neighbour i of j,  cMc += c_i M_ij c_j  (M in stencil storage: the score's copy S1 + lambda R, which
+// the band expansion and the solve only read);  and  c.g += c_j g_j,  logL -= log Linv_jj = log L_jj, the diagonal of
+// the stored block inverses read as spl_pivot_range_kernel reads it (both solver paths store them).
+__global__ void __launch_bounds__(256)
+spl_reml_stencil_kernel(const __grid_constant__ GridParams gp, const double *__restrict__ M, const double *__restrict__ c,
+                        const double *__restrict__ g, const double *__restrict__ linv, double *__restrict__ part) {
+    int ncombo = 1;
+    for (int d = 0; d < gp.ndim; ++d) ncombo *= 7;
+    double v[3] = {0.0, 0.0, 0.0};
+    for (long long j = blockIdx.x; j < gp.ncol; j += gridDim.x) {
+        int jd[SPL_MAXDIM];
+        {
+            long long kj = j;
+            for (int d = 0; d < gp.ndim; ++d) {
+                jd[d] = (int)(kj % gp.nodes[d]);
+                kj /= gp.nodes[d];
+            }
+        }
+        const double cj = c[j];
+        if (threadIdx.x == 0) {
+            v[1] = fma(cj, g[j], v[1]);
+            v[2] -= log(linv[(j / SI_NB) * 4096 + (j % SI_NB) * 65]);
+        }
+        for (int cc0 = threadIdx.x; cc0 < ncombo; cc0 += blockDim.x) {
+            long long i, slot;
+            if (!gcv_stencil_pair(gp, jd, j, cc0, &i, &slot)) continue;
+            v[0] = fma(c[i] * M[slot], cj, v[0]);
+        }
+    }
+    gcv_block_sum<3>(v);
+    if (threadIdx.x == 0) {
+        part[blockIdx.x] = v[0];
+        part[GCV_BLOCKS + blockIdx.x] = v[1];
+        part[2 * GCV_BLOCKS + blockIdx.x] = v[2];
+    }
+}
+
+// out3 = {c^T M c, c.g, sum_j log L_jj}; M in stencil storage, d_linv the block inverses the solve left behind; d_part:
+// spl_gcv_part_len() doubles of scratch.  The partials are added in order by spl_gcv_stencil_finish.
+int spl_reml_stencil_launch(const GridParams &gp, const double *d_M, const double *d_c, const double *d_g,
+                            const double *d_linv, double *d_part, double *d_out3, cudaStream_t st) {
+    spl_reml_stencil_kernel<<<GCV_BLOCKS, 256, 0, st>>>(gp, d_M, d_c, d_g, d_linv, d_part);
     spl_gcv_stencil_finish<<<1, 32, 0, st>>>(d_part, d_out3);
     g_spl_launches += 2;
     SPL_CUDA_TRY(cudaGetLastError());

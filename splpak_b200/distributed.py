@@ -64,7 +64,7 @@ def _on_handle_stream(handle, fn, stream=None):
 
 
 def fit_sharded(handle, x, y, w, weighted=True, device_resident=False, l1x=None, n=None, group=None, stream=None,
-                broadcast_coef=False, select_smoothing=None, prepare_variance=False):
+                broadcast_coef=False, select_smoothing=None, prepare_variance=False, criterion="gcv"):
     """Every rank adds ITS shard to `handle`, the partial sums are all-reduced, every rank solves.
     Returns (coef, ierror).  The all-reduce is ordered against the handle's stream (see _on_handle_stream), so no
     host synchronisation is needed around it.  The replicated solves see identical inputs (the all-reduce hands every
@@ -72,8 +72,8 @@ def fit_sharded(handle, x, y, w, weighted=True, device_resident=False, l1x=None,
     so the coefficients are bitwise identical on all ranks (tests/test_gpu_multi.py); `broadcast_coef` additionally
     broadcasts rank 0's coefficients (8*ncol bytes) for hosts that want to rule out any divergence, e.g. mixed GPU types.
     `select_smoothing` (a penalty name; the handle must have called enable_gcv): after the all-reduce every rank
-    selects lambda by GCV on the summed buffer -- bit-identical inputs, so every rank selects the same lambda -- and
-    the solve is the selected fit.  `prepare_variance`: after the selection (if any) and before the solve, every rank
+    selects lambda by `criterion` ("gcv" or "reml") on the summed buffer -- bit-identical inputs, so every rank selects
+    the same lambda -- and the solve is the selected fit.  `prepare_variance`: after the selection (if any) and before the solve, every rank
     builds the posterior-variance tables from the same summed buffer -- bit-identical on every rank, so the queries of
     handle.variance / variance_device then shard without communication.  A refusal raises SplpakError."""
     import torch
@@ -88,7 +88,7 @@ def fit_sharded(handle, x, y, w, weighted=True, device_resident=False, l1x=None,
     part = handle.partial_tensor()
     _on_handle_stream(handle, lambda: allreduce_partials(part, group), stream)
     if select_smoothing is not None:
-        handle.select_smoothing(select_smoothing)
+        handle.select_smoothing(select_smoothing, criterion=criterion)
     if prepare_variance:
         handle.prepare_variance()
     coef, ierr = handle.compute()
