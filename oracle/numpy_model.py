@@ -187,23 +187,7 @@ class SplpakModel:
             nrect = 1
             for d in range(ndim):
                 nrect *= inmx[d]
-            work = [0.0] * ncol
-            totlwt = 0.0
-            for idata in range(ndata):                                          # :885-907
-                bump = 1.0
-                if weighted:
-                    bump = float(wdata[idata])
-                if bump == 0.0:
-                    continue
-                iin = 0
-                for idimc in range(1, ndim + 1):
-                    idim = ndim + 1 - idimc
-                    inidim = _trunc(self.dxin[idim - 1] * (float(xdata[idata][idim - 1]) - xmin[idim - 1]) + 0.5)
-                    if inidim < 0 or inidim > inmx[idim - 1]:
-                        continue                                                # the bare `cycle` of :899: this dimension is dropped
-                    iin = (inmx[idim - 1] + 1) * iin + inidim
-                work[iin] = work[iin] + bump
-                totlwt = totlwt + bump
+            work, totlwt = self.histogram(ndim, xdata, wdata, xmin, xmax, nodes)
             wtprrc = totlwt / float(nrect)                                      # :910
             inn = [0] * ndim
             iin = 0
@@ -260,6 +244,33 @@ class SplpakModel:
                 if done:
                     break
         return out, ncol
+
+    def histogram(self, ndim, xdata, wdata, xmin, xmax, nodes):
+        """The nearest-node weight histogram of :885-907: (work[ncol], totlwt).  Same weight convention as rows."""
+        nodes = [int(v) for v in nodes]
+        xmin = [float(v) for v in xmin]
+        xmax = [float(v) for v in xmax]
+        ncol = self._setup(ndim, xmin, xmax, nodes)
+        weighted = wdata is not None and len(wdata) > 0 and float(wdata[0]) >= 0.0
+        inmx = [nodes[d] - 1 for d in range(ndim)]
+        work = [0.0] * ncol
+        totlwt = 0.0
+        for idata in range(len(xdata)):                                         # :885-907
+            bump = 1.0
+            if weighted:
+                bump = float(wdata[idata])
+            if bump == 0.0:
+                continue
+            iin = 0
+            for idimc in range(1, ndim + 1):
+                idim = ndim + 1 - idimc
+                inidim = _trunc(self.dxin[idim - 1] * (float(xdata[idata][idim - 1]) - xmin[idim - 1]) + 0.5)
+                if inidim < 0 or inidim > inmx[idim - 1]:
+                    continue                                                    # the bare `cycle` of :899: this dimension is dropped
+                iin = (inmx[idim - 1] + 1) * iin + inidim
+            work[iin] = work[iin] + bump
+            totlwt = totlwt + bump
+        return work, totlwt
 
     # ------------------------------------------------------------------ suprls :1425-1693 (1-based scratch a[1..nn])
     def suprls(self, i, rowi, n, bi, a, nn, soln):

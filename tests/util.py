@@ -50,6 +50,37 @@ def dense_from_stencil(S, nodes):
     return G
 
 
+def stencil_scale(diag, nodes):
+    """sqrt(G_ii G_jj) for every entry S[node, sten] of the orthant-stencil storage (i = node, j = node + delta), 0
+    where j is off the grid.  By Cauchy-Schwarz it bounds the sum of |terms| of G_ij, so tau times it bounds the
+    rounding error of that entry summed in any order."""
+    nodes = [int(n) for n in nodes]
+    ndim = len(nodes)
+    ncol = int(np.prod(nodes))
+    strides = np.cumprod([1] + nodes[:-1])
+    k = np.arange(ncol)
+    multi = []
+    for d in range(ndim):
+        multi.append(k % nodes[d])
+        k = k // nodes[d]
+    multi = np.stack(multi, axis=1)
+    out = np.zeros((ncol, 4 ** ndim))
+    for sten in range(4 ** ndim):
+        jm = multi + np.array([(sten >> (2 * d)) & 3 for d in range(ndim)])
+        ok = (jm < np.array(nodes)).all(axis=1)
+        j = (jm[ok] * strides).sum(axis=1)
+        out[ok, sten] = np.sqrt(np.abs(diag[ok] * diag[j]))
+    return out
+
+
+def worst_ratio(got, want, tol):
+    """max |got - want| / tol; an entry with tol 0 must match exactly (inf otherwise)."""
+    err = np.abs(np.asarray(got) - np.asarray(want))
+    with np.errstate(divide="ignore", invalid="ignore"):
+        r = np.where(err == 0, 0.0, err / tol)
+    return float(r.max()) if r.size else 0.0
+
+
 def coef_tolerance(G, base=1e-10):
     """max(1e-10, 10 * eps * cond(G)): the north star's "~1e-10 relative, scaled by the system's condition
     estimate".  (SURVEY 8c guessed 0.1*eps*cond from a QR-vs-Cholesky comparison; two runs of THIS
