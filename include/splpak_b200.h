@@ -303,6 +303,18 @@ int splpak_b200_fit_variance_device(splpak_b200_fit_t h, const splpak_real *d_x,
 /* Parity-test hook of the orthogonal path: which = 0 -> per-window triangles [nwindows][4^ndim][4^ndim + 1] (R_w | z_w),
  * which = 1 -> band factor [ncol][b + 2] (row i: R[i][i..i+b], then (Q^T r)_i).  out may be NULL to query *count. */
 int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity, int64_t *count);
+/* Parity-test hook of the Cholesky path, valid after fit_compute and the refinement steps (203 otherwise, e.g. after a
+ * score call, which leaves Sigma or the factor of another M in the band storage).  G = L L^T in lower band storage with
+ * lda = (b + 65) rounded up to even, panels of 64 columns.  Columns first_col .. first_col + ncols - 1:
+ *   which = 0 -> out[ncols][lda], row j - first_col = the band column j, rows j .. j + lda - 1 (entry r: L(j + r, j)).
+ *                Outside the 64 x 64 diagonal blocks these are L, and exactly 0 where j + r >= ncol or r > b.  The
+ *                diagonal blocks are scratch and hold no part of L on any route: the panel kernels factor them in shared
+ *                memory and keep only L11^-1; what is left there (an updated A11) depends on the route.
+ *   which = 1 -> out[nblk][64][64], the block inverses L11^-1 (row-major) of the panels first_col / 64 .. (first_col +
+ *                ncols - 1) / 64; a last panel of nb < 64 columns is padded with the identity.
+ * out may be NULL to query *count.  203 also for which outside 0..1 or a column range outside 0..ncol-1. */
+int splpak_b200_fit_get_cholesky_factor(splpak_b200_fit_t h, int which, int64_t first_col, int64_t ncols, double *out,
+                                        int64_t capacity, int64_t *count);
 /* (max L_jj / min L_jj)^2 of the last Cholesky factor: a cheap LOWER bound of cond(G); 0 when unknown. */
 int splpak_b200_fit_condition_estimate(splpak_b200_fit_t h, double *cond_lower_bound);
 

@@ -61,6 +61,7 @@ SYMBOLS = [
     "splpak_b200_fit_variance",
     "splpak_b200_fit_variance_device",
     "splpak_b200_fit_get_orthogonal_factor",
+    "splpak_b200_fit_get_cholesky_factor",
     "splpak_b200_fit_condition_estimate",
     "splpak_b200_fit_constraints_fired",
     "splpak_b200_fit_rhs_buffer",
@@ -166,6 +167,7 @@ def load(real32: bool = False) -> C.CDLL:
         "splpak_b200_fit_variance": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, ip]),
         "splpak_b200_fit_variance_device": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, vp, ip]),
         "splpak_b200_fit_get_orthogonal_factor": (C.c_int, [vp, C.c_int, vp, i64, C.POINTER(i64)]),
+        "splpak_b200_fit_get_cholesky_factor": (C.c_int, [vp, C.c_int, i64, i64, vp, i64, C.POINTER(i64)]),
         "splpak_b200_fit_condition_estimate": (C.c_int, [vp, C.POINTER(C.c_double)]),
         "splpak_b200_fit_constraints_fired": (C.c_int, [vp]),
         "splpak_b200_fit_rhs_buffer": (C.c_int, [vp, C.POINTER(vp), C.POINTER(i64)]),

@@ -470,6 +470,24 @@ class FitHandle:
         ncw = 4 ** self.ndim
         return out.reshape(-1, ncw, ncw + 1) if which == 0 else out.reshape(self.ncol, -1)
 
+    def cholesky_factor(self, which, first_col=0, ncols=None):
+        """Parity-test hook of the Cholesky factor, after compute (header: fit_get_cholesky_factor).  which = 0 -> band
+        columns first_col.. (ncols, lda), row j - first_col = L(j .. j + lda - 1, j), the 64 x 64 diagonal blocks
+        excluded from the contract; 1 -> the block inverses L11^-1 of their panels (nblk, 64, 64)."""
+        self._check()
+        ncols = self.ncol - int(first_col) if ncols is None else int(ncols)
+        n = C.c_int64(0)
+        rc = self.lib.splpak_b200_fit_get_cholesky_factor(self.h, int(which), int(first_col), ncols, None, 0,
+                                                          C.byref(n))
+        if rc != 0:
+            raise SplpakError(f"get_cholesky_factor failed: {rc}", rc)
+        out = np.zeros(n.value)
+        rc = self.lib.splpak_b200_fit_get_cholesky_factor(self.h, int(which), int(first_col), ncols, _ptr(out),
+                                                          n.value, C.byref(n))
+        if rc != 0:
+            raise SplpakError(f"get_cholesky_factor failed: {rc}", rc)
+        return out.reshape(ncols, -1) if which == 0 else out.reshape(-1, 64, 64)
+
     def condition_estimate(self):
         """Pivot-ratio LOWER bound of cond(G) from the last Cholesky factor (0.0 when unknown)."""
         self._check()

@@ -2157,6 +2157,32 @@ extern "C" int splpak_b200_fit_get_selected_inverse(splpak_b200_fit_t h, double 
     return SPLPAK_OK;
 }
 
+// Parity-test hook of the Cholesky factor (layout: spl_solve_launch).  which = 0: columns first_col .. first_col+ncols-1
+// of the band, each its lda doubles AB[j (lda+1) ..], rows j .. j+lda-1; which = 1: the block inverses L11^-1 of the
+// panels those columns belong to, 64 x 64 row-major each.  *count returns the size.
+extern "C" int splpak_b200_fit_get_cholesky_factor(splpak_b200_fit_t h, int which, int64_t first_col, int64_t ncols,
+                                                   double *out, int64_t capacity, int64_t *count) {
+    if (!valid(h) || !h->factor_valid) return SPLPAK_ERR_HANDLE;
+    const GridParams &gp = h->gp;
+    if (which < 0 || which > 1 || first_col < 0 || ncols < 1 || first_col + ncols > gp.ncol) return SPLPAK_ERR_HANDLE;
+    const long long lda = spl_band_lda(spl_half_bandwidth(gp));
+    const long long band_elems = (gp.ncol * (lda + 1) + 64 + 1) & ~1LL;
+    const long long kb0 = first_col / 64, kb1 = (first_col + ncols - 1) / 64;
+    const int64_t n = which == 0 ? ncols * lda : (kb1 - kb0 + 1) * 4096;
+    if (count) *count = n;
+    if (!out) return SPLPAK_OK;
+    if (capacity < n) return SPLPAK_ERR_HANDLE;
+    SPL_CUDA_TRY(cudaStreamSynchronize(h->st));
+    if (which == 0)
+        SPL_CUDA_TRY(cudaMemcpy2D(out, sizeof(double) * (size_t)lda, h->d_AB + first_col * (lda + 1),
+                                  sizeof(double) * (size_t)(lda + 1), sizeof(double) * (size_t)lda, (size_t)ncols,
+                                  cudaMemcpyDeviceToHost));
+    else
+        SPL_CUDA_TRY(cudaMemcpy(out, h->d_AB + band_elems + kb0 * 4096, sizeof(double) * (size_t)n,
+                                cudaMemcpyDeviceToHost));
+    return SPLPAK_OK;
+}
+
 // ---- posterior variances (variance.cu; DESIGN §4.13) ----
 extern "C" int splpak_b200_fit_prepare_variance(splpak_b200_fit_t h, double *out, int nout, int *ierror) {
     int rc = SPLPAK_OK;
