@@ -1118,7 +1118,9 @@ int spl_fx_finish(const GridParams &gp, double *d_S, double *d_g, cudaStream_t s
 // ------------------------------------------------------------------------------------------
 #include "moments.cuh"
 
-int spl_acc_chunk_points(int ndim, int moments) {
+#define TWOLEVEL_MIN_POINTS (1LL << 21)   // smallest chunk of the two-level partition (pairs and keys are sized for it)
+
+static int spl_acc_chunk_points(int ndim, int moments) {
     if (moments) return MOM_CH;
     switch (ndim) {
     case 1: return AccTraits<1>::CH;
@@ -1188,7 +1190,40 @@ int spl_assemble_scratch_init(const GridParams &gp, AssembleScratch &sc, cudaStr
     return spl_hist_scratch_init(gp, sc.hist, st);
 }
 
+static void free_chunk_arrays(AssembleScratch &sc) {
+    unsigned *u[] = {sc.perm, sc.perm2, sc.keys, sc.item_win, sc.item_seg};
+    for (unsigned *p : u)
+        if (p) cudaFree(p);
+    if (sc.yw) cudaFree(sc.yw);
+    if (sc.pairs) cudaFree(sc.pairs);
+    sc.perm = sc.perm2 = sc.keys = sc.item_win = sc.item_seg = nullptr;
+    sc.yw = nullptr;
+    sc.pairs = nullptr;
+    sc.cap = 0;
+}
+
+// Grow-only: the chunk-sized arrays for chunks of up to n points.  The old arrays are released with the synchronising
+// cudaFree: the kernels of an earlier chunk may still be reading them.
+int spl_assemble_scratch_reserve(const GridParams &gp, AssembleScratch &sc, long long n) {
+    if (n <= sc.cap) return SPLPAK_OK;
+    free_chunk_arrays(sc);
+    sc.max_items = sc.nbins + n / spl_acc_chunk_points(gp.ndim, sc.moments) + 2;
+    SPL_CUDA_TRY(cudaMalloc((void **)&sc.perm, sizeof(unsigned) * (size_t)n));
+    // deterministic mode: second permutation buffer of the per-bin sort
+    if (sc.deterministic) SPL_CUDA_TRY(cudaMalloc((void **)&sc.perm2, sizeof(unsigned) * (size_t)n));
+    if (sc.moments) SPL_CUDA_TRY(cudaMalloc((void **)&sc.yw, 2 * sizeof(double) * (size_t)n));
+    if (sc.moments && n >= TWOLEVEL_MIN_POINTS) {
+        SPL_CUDA_TRY(cudaMalloc((void **)&sc.pairs, sizeof(unsigned long long) * (size_t)n));
+        SPL_CUDA_TRY(cudaMalloc((void **)&sc.keys, sizeof(unsigned) * (size_t)n));
+    }
+    SPL_CUDA_TRY(cudaMalloc((void **)&sc.item_win, sizeof(unsigned) * (size_t)sc.max_items));
+    SPL_CUDA_TRY(cudaMalloc((void **)&sc.item_seg, sizeof(unsigned) * (size_t)sc.max_items));
+    sc.cap = n;
+    return SPLPAK_OK;
+}
+
 void spl_assemble_scratch_free(AssembleScratch &sc) {
+    free_chunk_arrays(sc);
     unsigned *u[] = {sc.wincount, sc.winstart, sc.wincursor, sc.itemstart, sc.meta};
     for (unsigned *p : u)
         if (p) cudaFree(p);
@@ -1231,7 +1266,7 @@ static int assemble_chunk_t(const GridParams &gp, const real_t *d_x, int l1x, co
         // two-level partition for large chunks of many cells (SPLPAK_B200_BINNING=atomic keeps the per-point atomics)
         const char *bm = getenv("SPLPAK_B200_BINNING");
         // (beyond ~1e5 cells a tile of 8,192 points holds less than one point per cell of its buckets: nothing to aggregate)
-        twolevel = sc.pairs && sc.keys && n >= (1LL << 21) && nbins >= 2048 && nbins <= 48 * 2048 &&
+        twolevel = sc.pairs && sc.keys && n >= TWOLEVEL_MIN_POINTS && nbins >= 2048 && nbins <= 48 * 2048 &&
                    !(bm && strcmp(bm, "atomic") == 0);
     }
     unsigned *keys = twolevel ? sc.keys : nullptr;

@@ -18,6 +18,7 @@ unsigned long long g_spl_launches = 0;
 
 // ---- kernels' host launchers (other translation units) ----
 int spl_assemble_scratch_init(const GridParams &gp, AssembleScratch &sc, cudaStream_t st);
+int spl_assemble_scratch_reserve(const GridParams &gp, AssembleScratch &sc, long long n);
 void spl_assemble_scratch_free(AssembleScratch &sc);
 int spl_eval_launch(const GridParams &gp, const int *nderiv, int order, const real_t *d_x, int l1x, long long nq,
                     const double *d_coef, long long ncol_padded, real_t *d_out, cudaStream_t stream,
@@ -39,7 +40,6 @@ long long spl_grid_tmp_elems(const GridParams &gp, const long long *naxis);
 int spl_eval_grid_launch(const GridParams &gp, const int *nderiv, const real_t *const *d_axis, const long long *naxis,
                          const double *d_coef64, real_t *d_out, double *d_tmp, long long tmp_elems, int *d_iws,
                          double *d_w4, cudaStream_t st, int nsm);
-int spl_acc_chunk_points(int ndim, int moments);
 int spl_assemble_chunk(const GridParams &gp, const real_t *d_x, int l1x, const real_t *d_y,
                        const real_t *d_w, int weighted, long long n, int do_hist, int rhs_only,
                        const AssembleScratch &sc, double *d_S, double *d_g, double *d_cnt,
@@ -49,6 +49,7 @@ int spl_constraints_launch(const GridParams &gp, double xtrap, const double *d_c
                            cudaStream_t st, int nsm);
 long long spl_band_lda(int bw);
 int spl_half_bandwidth(const GridParams &gp);
+long long spl_band_elems(const GridParams &gp);
 long long spl_solve_workspace(const GridParams &gp);
 int spl_solve_launch(const GridParams &gp, const double *d_S, double *d_AB, double *d_g, double *d_work,
                      double **d_coef_out, int *d_fail, cudaStream_t st, cudaStream_t st_aux, int nsm, cudaEvent_t *ev,
@@ -705,12 +706,30 @@ extern "C" int splpak_b200_eval_grid(int ndim, const real_t *axes, const int64_t
     return rc;
 }
 
+// Grow-only device buffer: afterwards *p holds at least `need` elements (*cap of them).  The old buffer is released with
+// the synchronising cudaFree: the kernels of an earlier call may still be reading it.
+template <class T>
+static cudaError_t grow(T **p, long long *cap, long long need) {
+    if (need <= *cap) return cudaSuccess;
+    if (*p) cudaFree(*p);
+    *p = nullptr;
+    *cap = 0;
+    const cudaError_t e = cudaMalloc((void **)p, sizeof(T) * (size_t)need);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        *p = nullptr;
+        return e;
+    }
+    *cap = need;
+    return cudaSuccess;
+}
+
 struct EvalHostCtx {
     std::mutex mu;
     cudaStream_t st = nullptr, st2 = nullptr;
     cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
     real_t *d_coef = nullptr, *d_x[2] = {nullptr, nullptr}, *d_out[2] = {nullptr, nullptr};
-    size_t coef_cap = 0, x_cap[2] = {0, 0}, out_cap[2] = {0, 0};
+    long long coef_cap = 0, x_cap[2] = {0, 0}, out_cap[2] = {0, 0};
     // host shadow of the table that d_coef holds: a call with the same coefficients (the reference's usage is
     // `evaluate` once per point in a loop, test/splpak_test.f90:72-80) skips the upload after one memcmp
     std::vector<char> coef_shadow;
@@ -750,30 +769,13 @@ static int eval_host_staged(const GridParams &gp, const DeviceInfo &di, const re
             EV_TRY(cudaEventCreateWithFlags(&cx.ev_done[k], cudaEventDisableTiming));
         }
     }
-    if (coef && (size_t)(gp.ncol + 2) > cx.coef_cap) {
-        if (cx.d_coef) cudaFree(cx.d_coef);
-        cx.d_coef = nullptr;
-        cx.coef_cap = 0;
-        EV_TRY(cudaMalloc((void **)&cx.d_coef, sizeof(real_t) * (size_t)(gp.ncol + 2)));
-        cx.coef_cap = (size_t)(gp.ncol + 2);
-        cx.coef_valid = false;
+    if (coef && gp.ncol + 2 > cx.coef_cap) {
+        cx.coef_valid = false;                                   // a new buffer holds no table
+        EV_TRY(grow(&cx.d_coef, &cx.coef_cap, gp.ncol + 2));
     }
-    const size_t xneed = (size_t)chunk * l1x, oneed = (size_t)chunk * ncomp;
     for (int k = 0; k < nbuf; ++k) {
-        if (xneed > cx.x_cap[k]) {
-            if (cx.d_x[k]) cudaFree(cx.d_x[k]);
-            cx.d_x[k] = nullptr;
-            cx.x_cap[k] = 0;
-            EV_TRY(cudaMalloc((void **)&cx.d_x[k], sizeof(real_t) * xneed));
-            cx.x_cap[k] = xneed;
-        }
-        if (oneed > cx.out_cap[k]) {
-            if (cx.d_out[k]) cudaFree(cx.d_out[k]);
-            cx.d_out[k] = nullptr;
-            cx.out_cap[k] = 0;
-            EV_TRY(cudaMalloc((void **)&cx.d_out[k], sizeof(real_t) * oneed));
-            cx.out_cap[k] = oneed;
-        }
+        EV_TRY(grow(&cx.d_x[k], &cx.x_cap[k], chunk * l1x));
+        EV_TRY(grow(&cx.d_out[k], &cx.out_cap[k], chunk * ncomp));
     }
     cudaStream_t st = cx.st, st2 = cx.st2;
     real_t *d_coef = coef ? cx.d_coef : nullptr;
@@ -916,16 +918,14 @@ struct splpak_b200_fit_s {
     DeviceInfo di;
     double xtrap;
     cudaStream_t st, st_copy, st_aux;   // st_aux: look-ahead stream of the solve
-    // partial sums, one contiguous buffer: [S | g | cnt | totals(2)]
+    // partial sums, one contiguous buffer (layout_partial): [S | g | cnt | totals(2) (| ywy)]
     double *d_part;
     long long n_part;
     double *d_S, *d_g, *d_cnt, *d_totals;
     // chunk scratch
     AssembleScratch sc;
-    long long chunk_cap;          // points the scratch can take
     real_t *d_stage[2][3];        // host-path staging: x, y, w double-buffered
-    long long stage_cap;          // points the y / w staging buffers hold
-    long long stage_xcap;         // reals the x staging buffers hold (chunk * l1x of the call that sized them)
+    long long stage_cap[2][3];    // reals each staging buffer holds
     cudaEvent_t ev_stage_in[2], ev_stage_free[2];
     // solve
     double *d_AB;
@@ -948,7 +948,7 @@ struct splpak_b200_fit_s {
     // smoothing (penalty.cu): lambda * R is added to S by compute when lambda > 0; kept across fit_reset
     double lambda;
     int penalty;                  // SPLPAK_PENALTY_CURVATURE or SPLPAK_PENALTY_THIN_PLATE
-    double *d_pen;                // 1-D penalty tables (spl_penalty_table_len doubles), allocated by the first lambda > 0
+    double *d_pen;                // 1-D penalty tables (spl_penalty_table_len doubles): ensure_penalty_tables
     // generalized cross-validation (selinv.cu): enable_gcv; kept across fit_reset
     int gcv;
     double *d_ywy;                // the last slot of the partial buffer: sum (w y)^2
@@ -980,12 +980,6 @@ static bool valid(splpak_b200_fit_t h) { return h && h->magic == FIT_MAGIC; }
 static void free_handle(splpak_b200_fit_t h) {
     if (!h) return;
     if (h->d_part) cudaFree(h->d_part);
-    if (h->sc.yw) cudaFree(h->sc.yw);
-    if (h->sc.pairs) cudaFree(h->sc.pairs);
-    if (h->sc.keys) cudaFree(h->sc.keys);
-    unsigned *u[] = {h->sc.item_win, h->sc.item_seg, h->sc.perm, h->sc.perm2};
-    for (unsigned *p : u)
-        if (p) cudaFree(p);
     spl_assemble_scratch_free(h->sc);
     for (int k = 0; k < 2; ++k) {
         for (int a = 0; a < 3; ++a)
@@ -1018,6 +1012,16 @@ static void free_handle(splpak_b200_fit_t h) {
     if (h->st_aux) cudaStreamDestroy(h->st_aux);
     h->magic = 0;
     delete h;
+}
+
+// Pointers into the partial buffer [S | g | cnt | totals(2)], and with GCV one more slot: ywy = sum (w y)^2
+static void layout_partial(splpak_b200_fit_t h, bool ywy) {
+    const GridParams &gp = h->gp;
+    h->d_S = h->d_part;
+    h->d_g = h->d_S + gp.ncol * gp.nsten;
+    h->d_cnt = h->d_g + gp.ncol;
+    h->d_totals = h->d_cnt + gp.ncol;
+    h->d_ywy = ywy ? h->d_totals + 2 : nullptr;
 }
 
 extern "C" int splpak_b200_fit_create(int ndim, const real_t *xmin, const real_t *xmax,
@@ -1069,10 +1073,7 @@ extern "C" int splpak_b200_fit_create(int ndim, const real_t *xmin, const real_t
         ok = ok && cudaEventCreateWithFlags(&h->ev_stage_free[k], cudaEventDisableTiming) == cudaSuccess;
     }
     if (ok) {
-        h->d_S = h->d_part;
-        h->d_g = h->d_S + gp.ncol * gp.nsten;
-        h->d_cnt = h->d_g + gp.ncol;
-        h->d_totals = h->d_cnt + gp.ncol;
+        layout_partial(h, false);
         ok = cudaMemsetAsync(h->d_part, 0, sizeof(double) * (size_t)h->n_part, h->st) == cudaSuccess;
     }
     if (!ok) {
@@ -1101,56 +1102,26 @@ extern "C" int splpak_b200_fit_reset(splpak_b200_fit_t h) {
     return SPLPAK_OK;
 }
 
+// The assembly scratch for chunks of up to n points (assemble.cu), created by the first chunk.
 static int ensure_scratch(splpak_b200_fit_t h, long long n) {
-    if (n <= h->chunk_cap) return SPLPAK_OK;
-    GridParams &gp = h->gp;
     AssembleScratch &sc = h->sc;
-    if (sc.perm) cudaFree(sc.perm);
-    if (sc.perm2) cudaFree(sc.perm2);
-    sc.perm2 = nullptr;
-    if (sc.pairs) cudaFree(sc.pairs);
-    sc.pairs = nullptr;
-    if (sc.keys) cudaFree(sc.keys);
-    sc.keys = nullptr;
-    if (sc.yw) cudaFree(sc.yw);
-    sc.yw = nullptr;
-    if (sc.item_win) cudaFree(sc.item_win);
-    if (sc.item_seg) cudaFree(sc.item_seg);
-    sc.perm = nullptr;
-    sc.item_win = sc.item_seg = nullptr;
-    h->chunk_cap = 0;
     if (!sc.wincount) {
-        const int rc = spl_assemble_scratch_init(gp, sc, h->st);
+        const int rc = spl_assemble_scratch_init(h->gp, sc, h->st);
         if (rc != SPLPAK_OK) return rc;
     }
-    const int ch = spl_acc_chunk_points(gp.ndim, sc.moments);
-    sc.max_items = sc.nbins + n / ch + 2;
-    SPL_CUDA_TRY(cudaMalloc((void **)&sc.perm, sizeof(unsigned) * (size_t)n));
     // The constraint rows always go through the fixed-point limbs (tiny work): after an all-reduce every rank holds the
     // same S, adds the same rows in an order-independent way and -- the solver being deterministic -- gets the SAME
     // coefficients, bit for bit.  With unordered FP64 atomics the replicas differed by ~eps cond(G), every rank formed the
     // residual of its shard with its own coefficients, and a multi-GPU refinement stalled at that difference.
-    h->gp_fx = gp;
+    h->gp_fx = h->gp;
     h->gp_fx.fxS = sc.fxS;
     h->gp_fx.fxg = sc.fxg;
     h->gp_fx.fxmax = sc.fxmax;
     h->gp_fx.fxe = sc.fxe;
     h->gp_fx.fxpass = 0;
-    if (sc.deterministic) {
-        // SPLPAK_B200_DETERMINISTIC=1: the assembly too (second permutation buffer of the per-bin sort; the assembly
-        // kernels find the limb arrays in gp)
-        SPL_CUDA_TRY(cudaMalloc((void **)&sc.perm2, sizeof(unsigned) * (size_t)n));
-        gp = h->gp_fx;
-    }
-    if (sc.moments) SPL_CUDA_TRY(cudaMalloc((void **)&sc.yw, 2 * sizeof(double) * (size_t)n));
-    if (sc.moments && n >= (1LL << 21)) {
-        SPL_CUDA_TRY(cudaMalloc((void **)&sc.pairs, sizeof(unsigned long long) * (size_t)n));
-        SPL_CUDA_TRY(cudaMalloc((void **)&sc.keys, sizeof(unsigned) * (size_t)n));
-    }
-    SPL_CUDA_TRY(cudaMalloc((void **)&sc.item_win, sizeof(unsigned) * (size_t)sc.max_items));
-    SPL_CUDA_TRY(cudaMalloc((void **)&sc.item_seg, sizeof(unsigned) * (size_t)sc.max_items));
-    h->chunk_cap = n;
-    return SPLPAK_OK;
+    // SPLPAK_B200_DETERMINISTIC=1: the assembly too (the assembly kernels find the limb arrays in gp)
+    if (sc.deterministic) h->gp = h->gp_fx;
+    return spl_assemble_scratch_reserve(h->gp, sc, n);
 }
 
 static void collect_assemble_timers(splpak_b200_fit_t h);
@@ -1200,6 +1171,54 @@ static void collect_assemble_timers(splpak_b200_fit_t h) {
     add_ms(h, 2, h->ev[2], h->ev[3]);
 }
 
+// Device points in chunks of DEVICE_CHUNK; chunk(h, d_x, l1x, d_y, d_w, weighted, n) takes one chunk (add_device_chunk
+// or refine_device_chunk).
+template <class Chunk>
+static int feed_device(splpak_b200_fit_t h, const real_t *d_x, int l1x, const real_t *d_y, const real_t *d_w,
+                       int weighted, long long n, Chunk chunk) {
+    for (long long i0 = 0; i0 < n; i0 += DEVICE_CHUNK) {
+        const long long nc = (n - i0 < DEVICE_CHUNK) ? n - i0 : DEVICE_CHUNK;
+        const int rc = chunk(h, d_x + i0 * (long long)l1x, l1x, d_y + i0, weighted ? d_w + i0 : nullptr, weighted, nc);
+        if (rc != SPLPAK_OK) return rc;
+    }
+    return SPLPAK_OK;
+}
+
+// Host-path staging buffers, grow-only.  The x buffer is sized in REALS (chunk * l1x): a later call with
+// a larger leading dimension must not reuse a buffer sized for a smaller one.
+static int ensure_stage(splpak_b200_fit_t h, long long chunk, int l1x) {
+    for (int k = 0; k < 2; ++k)
+        for (int a = 0; a < 3; ++a)
+            SPL_CUDA_TRY(grow(&h->d_stage[k][a], &h->stage_cap[k][a], a == 0 ? chunk * (long long)l1x : chunk));
+    return SPLPAK_OK;
+}
+
+// Host points through the double-buffered staging buffers, HOST_CHUNK at a time: the copy stream uploads chunk k+1
+// while the handle's stream works on chunk k.  chunk: as in feed_device.
+template <class Chunk>
+static int feed_host(splpak_b200_fit_t h, const real_t *x, int l1x, const real_t *y, const real_t *w, int weighted,
+                     long long n, Chunk chunk) {
+    const long long nch = n < HOST_CHUNK ? n : HOST_CHUNK;
+    const int rcs = ensure_stage(h, nch, l1x);
+    if (rcs != SPLPAK_OK) return rcs;
+    int k = 0;
+    for (long long i0 = 0; i0 < n; i0 += nch, k ^= 1) {
+        const long long nc = (n - i0 < nch) ? n - i0 : nch;
+        real_t *const *buf = h->d_stage[k];
+        // copy stream: wait until the kernels that read staging buffer k have finished
+        SPL_CUDA_TRY(cudaStreamWaitEvent(h->st_copy, h->ev_stage_free[k], 0));
+        SPL_CUDA_TRY(spl_h2d(buf[0], x + i0 * (long long)l1x, sizeof(real_t) * (size_t)nc * l1x, h->st_copy, h->di.dev));
+        SPL_CUDA_TRY(spl_h2d(buf[1], y + i0, sizeof(real_t) * (size_t)nc, h->st_copy, h->di.dev));
+        if (weighted) SPL_CUDA_TRY(spl_h2d(buf[2], w + i0, sizeof(real_t) * (size_t)nc, h->st_copy, h->di.dev));
+        SPL_CUDA_TRY(cudaEventRecord(h->ev_stage_in[k], h->st_copy));
+        SPL_CUDA_TRY(cudaStreamWaitEvent(h->st, h->ev_stage_in[k], 0));
+        const int rc = chunk(h, buf[0], l1x, buf[1], weighted ? buf[2] : nullptr, weighted, nc);
+        if (rc != SPLPAK_OK) return rc;
+        SPL_CUDA_TRY(cudaEventRecord(h->ev_stage_free[k], h->st));
+    }
+    return SPLPAK_OK;
+}
+
 extern "C" int splpak_b200_fit_add_points_device(splpak_b200_fit_t h, const real_t *d_x, int l1x,
                                                  const real_t *d_y, const real_t *d_w, int weighted,
                                                  int64_t n) {
@@ -1207,44 +1226,10 @@ extern "C" int splpak_b200_fit_add_points_device(splpak_b200_fit_t h, const real
     if (n <= 0) return SPLPAK_OK;
     if (l1x < h->gp.ndim) return SPLPAK_ERR_HANDLE;
     if (!d_w) weighted = 0;
-    for (long long i0 = 0; i0 < n; i0 += DEVICE_CHUNK) {
-        const long long nc = (n - i0 < DEVICE_CHUNK) ? n - i0 : DEVICE_CHUNK;
-        int rc = add_device_chunk(h, d_x + i0 * (long long)l1x, l1x, d_y + i0, d_w ? d_w + i0 : nullptr,
-                                  weighted, nc);
-        if (rc != SPLPAK_OK) return rc;
-    }
+    const int rc = feed_device(h, d_x, l1x, d_y, d_w, weighted, n, add_device_chunk);
+    if (rc != SPLPAK_OK) return rc;
     h->total_points += n;
     return SPLPAK_OK;   // asynchronous: timers are harvested by the next chunk / compute / fit_timings
-}
-
-// Host-path staging buffers, grow-only.  The x buffer is sized in REALS (chunk * l1x): a later call with
-// a larger leading dimension must not reuse a buffer sized for a smaller one.
-static int ensure_stage(splpak_b200_fit_t h, long long chunk, int l1x) {
-    const long long xneed = chunk * (long long)l1x;
-    if (chunk > h->stage_cap) {
-        for (int k = 0; k < 2; ++k)
-            for (int a = 1; a < 3; ++a) {
-                if (h->d_stage[k][a]) cudaFree(h->d_stage[k][a]);
-                h->d_stage[k][a] = nullptr;
-            }
-        h->stage_cap = 0;
-        for (int k = 0; k < 2; ++k) {
-            SPL_CUDA_TRY(cudaMalloc((void **)&h->d_stage[k][1], sizeof(real_t) * (size_t)chunk));
-            SPL_CUDA_TRY(cudaMalloc((void **)&h->d_stage[k][2], sizeof(real_t) * (size_t)chunk));
-        }
-        h->stage_cap = chunk;
-    }
-    if (xneed > h->stage_xcap) {
-        for (int k = 0; k < 2; ++k) {
-            if (h->d_stage[k][0]) cudaFree(h->d_stage[k][0]);
-            h->d_stage[k][0] = nullptr;
-        }
-        h->stage_xcap = 0;
-        for (int k = 0; k < 2; ++k)
-            SPL_CUDA_TRY(cudaMalloc((void **)&h->d_stage[k][0], sizeof(real_t) * (size_t)xneed));
-        h->stage_xcap = xneed;
-    }
-    return SPLPAK_OK;
 }
 
 extern "C" int splpak_b200_fit_add_points(splpak_b200_fit_t h, const real_t *x, int l1x,
@@ -1253,26 +1238,8 @@ extern "C" int splpak_b200_fit_add_points(splpak_b200_fit_t h, const real_t *x, 
     if (n <= 0) return SPLPAK_OK;
     if (l1x < h->gp.ndim) return SPLPAK_ERR_HANDLE;
     if (!w) weighted = 0;
-    const long long chunk = n < HOST_CHUNK ? n : HOST_CHUNK;
-    int rcs = ensure_stage(h, chunk, l1x);
-    if (rcs != SPLPAK_OK) return rcs;
-    int k = 0;
-    for (long long i0 = 0; i0 < n; i0 += chunk, k ^= 1) {
-        const long long nc = (n - i0 < chunk) ? n - i0 : chunk;
-        // copy stream: wait until the kernels that read staging buffer k have finished
-        SPL_CUDA_TRY(cudaStreamWaitEvent(h->st_copy, h->ev_stage_free[k], 0));
-        SPL_CUDA_TRY(spl_h2d(h->d_stage[k][0], x + i0 * (long long)l1x, sizeof(real_t) * (size_t)nc * l1x, h->st_copy,
-                             h->di.dev));
-        SPL_CUDA_TRY(spl_h2d(h->d_stage[k][1], y + i0, sizeof(real_t) * (size_t)nc, h->st_copy, h->di.dev));
-        if (weighted)
-            SPL_CUDA_TRY(spl_h2d(h->d_stage[k][2], w + i0, sizeof(real_t) * (size_t)nc, h->st_copy, h->di.dev));
-        SPL_CUDA_TRY(cudaEventRecord(h->ev_stage_in[k], h->st_copy));
-        SPL_CUDA_TRY(cudaStreamWaitEvent(h->st, h->ev_stage_in[k], 0));
-        int rc = add_device_chunk(h, h->d_stage[k][0], l1x, h->d_stage[k][1],
-                                  weighted ? h->d_stage[k][2] : nullptr, weighted, nc);
-        if (rc != SPLPAK_OK) return rc;
-        SPL_CUDA_TRY(cudaEventRecord(h->ev_stage_free[k], h->st));
-    }
+    const int rc = feed_host(h, x, l1x, y, w, weighted, n, add_device_chunk);
+    if (rc != SPLPAK_OK) return rc;
     collect_assemble_timers(h);
     h->total_points += n;
     return SPLPAK_OK;
@@ -1377,195 +1344,135 @@ extern "C" int splpak_b200_comm_group_end(void) {
 
 // the band matrix and the solve workspace behind it (grow-only): *band_elems doubles of band, *need in all
 static int ensure_band(splpak_b200_fit_t h, long long *band_elems, long long *need) {
-    const GridParams &gp = h->gp;
-    const int bw = spl_half_bandwidth(gp);
-    const long long lda = spl_band_lda(bw);
-    // element (i, j) lives at i + j*lda, so the last one, (n-1, n-1), is at (n-1)*(lda+1)
-    *band_elems = (gp.ncol * (lda + 1) + 64 + 1) & ~1LL;     // even: the workspace behind stays 16-byte aligned
-    *need = *band_elems + spl_solve_workspace(gp);
-    if (*need > h->ab_elems) {
-        if (h->d_AB) cudaFree(h->d_AB);
-        h->d_AB = nullptr;
-        h->ab_elems = 0;
-        if (cudaMalloc((void **)&h->d_AB, sizeof(double) * (size_t)*need) != cudaSuccess) {
-            cudaGetLastError();
-            return SPLPAK_ERR_ALLOC;
-        }
-        h->ab_elems = *need;
+    *band_elems = spl_band_elems(h->gp);
+    *need = *band_elems + spl_solve_workspace(h->gp);
+    return grow(&h->d_AB, &h->ab_elems, *need) == cudaSuccess ? SPLPAK_OK : SPLPAK_ERR_ALLOC;
+}
+
+// The solution (ncol doubles at d_sol) to the caller's coef, on st: a device array, or a host array of real_t (REAL32:
+// through d_out_tmp; d_AB keeps the factor for refinement steps).  The host copy is complete at the next synchronisation.
+static int write_coef(splpak_b200_fit_t h, const double *d_sol, real_t *coef, int coef_on_device) {
+    const long long n = h->gp.ncol;
+    if (!coef_on_device && sizeof(real_t) == sizeof(double)) {
+        SPL_CUDA_TRY(cudaMemcpyAsync(coef, d_sol, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, h->st));
+        return SPLPAK_OK;
     }
+    real_t *dst = coef_on_device ? coef : h->d_out_tmp;
+    spl_from_double_kernel<<<spl_div_up(n, 256), 256, 0, h->st>>>(d_sol, dst, n);
+    ++g_spl_launches;
+    if (!coef_on_device)
+        SPL_CUDA_TRY(cudaMemcpyAsync(coef, dst, sizeof(real_t) * (size_t)n, cudaMemcpyDeviceToHost, h->st));
     return SPLPAK_OK;
 }
 
-static int fit_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_on_device, int64_t ncf,
-                            int64_t nwrk, int *ierror) {
-    int rc = SPLPAK_OK;
-    if (!valid(h)) {
-        if (ierror) *ierror = SPLPAK_ERR_HANDLE;
-        return SPLPAK_ERR_HANDLE;
-    }
-    const GridParams &gp = h->gp;
-    if (gp.ncol > ncf) rc = SPLPAK_ERR_NCF;                                    // :751
-    if (rc == SPLPAK_OK && nwrk >= 0) {
-        // :757-781 and suprls :1443-1454
-        const long long nwrk1 = (h->xtrap != 0.0) ? gp.ncol + 1 : 1;
-        const long long nwlft = (long long)nwrk - nwrk1 + 1;
-        const long long nreq = ((gp.ncol + 5) * gp.ncol + 2) / 2;
-        if (nwlft < 1) rc = SPLPAK_ERR_NWRK;
-        else if (nwlft < nreq) rc = SPLPAK_ERR_SOLVER;
-    }
-    if (rc != SPLPAK_OK) {
-        if (ierror) *ierror = rc;
-        return rc;
-    }
-    if (h->finalized) {
-        if (ierror) *ierror = SPLPAK_ERR_HANDLE;
-        return SPLPAK_ERR_HANDLE;
-    }
+// The end of both compute paths: read back the failure flag and the row counts (one synchronisation), set solved and
+// constraints_fired.  Not solved: a non-positive pivot, or fewer rows than columns (suprls error 33, :1650; not an error
+// with smoothing, whose penalty makes such a fit well posed).
+static int read_back_solve(splpak_b200_fit_t h) {
     cudaStream_t st = h->st;
-    if (h->solver == SPLPAK_SOLVER_ORTHOGONAL) {
-        // Householder path (ortho.cuh): constraint rows, band QR of the stacked window triangles, back-substitution
-#define FO_TRY(expr)                                                                        \
-    do {                                                                                    \
-        cudaError_t _e = (expr);                                                            \
-        if (_e != cudaSuccess) {                                                            \
-            fprintf(stderr, "splpak_b200: CUDA error %s at %s:%d (%s)\n", cudaGetErrorString(_e), __FILE__, \
-                    __LINE__, #expr);                                                       \
-            h->finalized = 1;                                                               \
-            h->solved = 0;                                                                  \
-            if (ierror) *ierror = SPLPAK_ERR_CUDA;                                          \
-            return SPLPAK_ERR_CUDA;                                                         \
-        }                                                                                   \
-    } while (0)
-        h->finalized = 1;
-        double totals[2] = {0.0, 0.0}, rows_before = 0.0;
-        int fail = 0;
-        if (!h->os || !h->os->ready) {
-            // no point was ever added: fewer rows than columns (suprls error 33)
-            if (ierror) *ierror = SPLPAK_ERR_SOLVER;
-            return SPLPAK_ERR_SOLVER;
-        }
-        FO_TRY(cudaMemcpyAsync(h->d_dummy_tot + 2, h->d_totals + 1, sizeof(double), cudaMemcpyDeviceToDevice, st));
-        FO_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
-        FO_TRY(cudaEventRecord(h->ev[8], st));
-        rc = spl_ortho_compute(gp, h->xtrap, *h->os, h->d_cnt, h->d_totals, h->d_fail, st, h->di.nsm);
-        FO_TRY(cudaEventRecord(h->ev[9], st));
-        if (rc == SPLPAK_OK) {
-            const double *d_sol = h->os->csol;
-            FO_TRY(cudaMemcpyAsync(h->d_coef64, d_sol, sizeof(double) * (size_t)gp.ncol, cudaMemcpyDeviceToDevice, st));
-            if (coef_on_device) {
-                spl_from_double_kernel<<<spl_div_up(gp.ncol, 256), 256, 0, st>>>(d_sol, coef, gp.ncol);
-                ++g_spl_launches;
-            } else if (sizeof(real_t) == sizeof(double)) {
-                FO_TRY(cudaMemcpyAsync(coef, d_sol, sizeof(double) * (size_t)gp.ncol, cudaMemcpyDeviceToHost, st));
-            } else {
-                spl_from_double_kernel<<<spl_div_up(gp.ncol, 256), 256, 0, st>>>(d_sol, h->d_out_tmp, gp.ncol);
-                ++g_spl_launches;
-                FO_TRY(cudaMemcpyAsync(coef, h->d_out_tmp, sizeof(real_t) * (size_t)gp.ncol, cudaMemcpyDeviceToHost, st));
-            }
-            FO_TRY(cudaMemcpyAsync(&fail, h->d_fail, sizeof(int), cudaMemcpyDeviceToHost, st));
-            FO_TRY(cudaMemcpyAsync(totals, h->d_totals, sizeof(double) * 2, cudaMemcpyDeviceToHost, st));
-            FO_TRY(cudaMemcpyAsync(&rows_before, h->d_dummy_tot + 2, sizeof(double), cudaMemcpyDeviceToHost, st));
-            FO_TRY(cudaStreamSynchronize(st));
-            add_ms(h, 5, h->ev[8], h->ev[9]);                      // reported in the "factor" slot
-            if (fail || totals[1] < (double)gp.ncol) rc = SPLPAK_ERR_SOLVER;     // :1650 (33), :1662 (34)
-            h->solved = (rc == SPLPAK_OK);
-            h->constraints_fired = (h->xtrap != 0.0) && (totals[1] > rows_before);
-        }
-#undef FO_TRY
-        if (ierror) *ierror = rc;
-        return rc;
-    }
-    long long band_elems = 0, need = 0;
-    rc = ensure_band(h, &band_elems, &need);
-    if (rc != SPLPAK_OK) {
-        if (ierror) *ierror = rc;
-        return rc;
-    }
-    // A CUDA failure below must reach the caller through *ierror (the Fortran shim and api.py read nothing
-    // else) and leave the handle finalized.
-#define FC_TRY(expr)                                                                        \
-    do {                                                                                    \
-        cudaError_t _e = (expr);                                                            \
-        if (_e != cudaSuccess) {                                                            \
-            fprintf(stderr, "splpak_b200: CUDA error %s at %s:%d (%s)\n", cudaGetErrorString(_e), __FILE__, \
-                    __LINE__, #expr);                                                       \
-            h->finalized = 1;                                                               \
-            h->solved = 0;                                                                  \
-            if (ierror) *ierror = SPLPAK_ERR_CUDA;                                          \
-            return SPLPAK_ERR_CUDA;                                                         \
-        }                                                                                   \
-    } while (0)
+    int fail = 0;
+    double totals[2] = {0.0, 0.0}, rows_before = 0.0;
+    SPL_CUDA_TRY(cudaMemcpyAsync(&fail, h->d_fail, sizeof(int), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(totals, h->d_totals, sizeof(double) * 2, cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(&rows_before, h->d_dummy_tot + 2, sizeof(double), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaStreamSynchronize(st));
+    h->solved = !fail && !(h->lambda == 0.0 && totals[1] < (double)h->gp.ncol);
+    h->constraints_fired = (h->xtrap != 0.0) && (totals[1] > rows_before);
+    return SPLPAK_OK;
+}
+
+// Householder path (ortho.cuh): constraint rows, band QR of the stacked window triangles, back-substitution
+static int compute_orthogonal(splpak_b200_fit_t h, real_t *coef, int coef_on_device) {
+    cudaStream_t st = h->st;
+    // no point was ever added: fewer rows than columns (suprls error 33)
+    if (!h->os || !h->os->ready) return SPLPAK_ERR_SOLVER;
+    SPL_CUDA_TRY(cudaMemcpyAsync(h->d_dummy_tot + 2, h->d_totals + 1, sizeof(double), cudaMemcpyDeviceToDevice, st));
+    SPL_CUDA_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
+    SPL_CUDA_TRY(cudaEventRecord(h->ev[8], st));
+    int rc = spl_ortho_compute(h->gp, h->xtrap, *h->os, h->d_cnt, h->d_totals, h->d_fail, st, h->di.nsm);
+    SPL_CUDA_TRY(cudaEventRecord(h->ev[9], st));
+    if (rc != SPLPAK_OK) return rc;
+    const double *d_sol = h->os->csol;
+    SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, d_sol, sizeof(double) * (size_t)h->gp.ncol, cudaMemcpyDeviceToDevice, st));
+    rc = write_coef(h, d_sol, coef, coef_on_device);
+    if (rc == SPLPAK_OK) rc = read_back_solve(h);
+    if (rc != SPLPAK_OK) return rc;
+    add_ms(h, 5, h->ev[8], h->ev[9]);                      // reported in the "factor" slot
+    return h->solved ? SPLPAK_OK : SPLPAK_ERR_SOLVER;
+}
+
+// Band Cholesky path: constraint rows and penalty into S, band expansion, factor and solve in d_AB (band_elems doubles
+// of band, need in all)
+static int compute_cholesky(splpak_b200_fit_t h, real_t *coef, int coef_on_device, long long band_elems,
+                            long long need) {
+    const GridParams &gp = h->gp;
+    cudaStream_t st = h->st;
     // row count before the constraint rows, kept on the device until the one synchronisation after the solve
-    FC_TRY(cudaMemcpyAsync(h->d_dummy_tot + 2, h->d_totals + 1, sizeof(double), cudaMemcpyDeviceToDevice, st));
-    FC_TRY(cudaEventRecord(h->ev[4], st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(h->d_dummy_tot + 2, h->d_totals + 1, sizeof(double), cudaMemcpyDeviceToDevice, st));
+    SPL_CUDA_TRY(cudaEventRecord(h->ev[4], st));
+    int rc = SPLPAK_OK;
     if (h->xtrap != 0.0) {
         rc = spl_constraints_launch(h->gp_fx.fxS ? h->gp_fx : gp, h->xtrap, h->d_cnt, h->d_totals, h->d_S, h->d_totals, st, h->di.nsm);
-        if (rc != SPLPAK_OK) {
-            h->finalized = 1;
-            if (ierror) *ierror = rc;
-            return rc;
-        }
+        if (rc != SPLPAK_OK) return rc;
     }
     // smoothing: S += lambda R after the constraint rows (and the fixed-point finish of the deterministic mode); after the
     // all-reduce of a multi-GPU fit, so the penalty counts once.  Timed in the constraints slot.
     if (h->lambda > 0.0) {
         rc = spl_penalty_add_launch(gp, h->lambda, h->penalty, h->d_pen, h->d_S, st, h->di.nsm);
-        if (rc != SPLPAK_OK) {
-            h->finalized = 1;
-            if (ierror) *ierror = rc;
-            return rc;
-        }
+        if (rc != SPLPAK_OK) return rc;
     }
-    FC_TRY(cudaEventRecord(h->ev[5], st));
-    FC_TRY(cudaMemsetAsync(h->d_AB, 0, sizeof(double) * (size_t)need, st));
-    FC_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
+    SPL_CUDA_TRY(cudaEventRecord(h->ev[5], st));
+    SPL_CUDA_TRY(cudaMemsetAsync(h->d_AB, 0, sizeof(double) * (size_t)need, st));
+    SPL_CUDA_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
     h->sigma_valid = 0;
     cudaEvent_t *sev = h->ev + 8;
     // the solve destroys g; the solution comes back in the workspace behind the band matrix
     double *d_sol = nullptr;
     rc = spl_solve_launch(gp, h->d_S, h->d_AB, h->d_g, h->d_AB + band_elems, &d_sol, h->d_fail, st, h->st_aux, h->di.nsm, sev,
                           &h->solve_cache);
-    int fail = 0;
-    double totals[2] = {0.0, 0.0}, rows_before = 0.0;
-    if (rc == SPLPAK_OK) {
-        FC_TRY(cudaMemcpyAsync(h->d_coef64, d_sol, sizeof(double) * (size_t)gp.ncol, cudaMemcpyDeviceToDevice, st));
-        if (coef_on_device) {
-            spl_from_double_kernel<<<spl_div_up(gp.ncol, 256), 256, 0, st>>>(d_sol, coef, gp.ncol);
-            ++g_spl_launches;
-        }
-        FC_TRY(cudaMemcpyAsync(&fail, h->d_fail, sizeof(int), cudaMemcpyDeviceToHost, st));
-        FC_TRY(cudaMemcpyAsync(totals, h->d_totals, sizeof(double) * 2, cudaMemcpyDeviceToHost, st));
-        FC_TRY(cudaMemcpyAsync(&rows_before, h->d_dummy_tot + 2, sizeof(double), cudaMemcpyDeviceToHost, st));
-        // smallest / largest diagonal entry of L (from the stored block inverses): a cheap LOWER bound of cond(G)
-        double prange[2] = {0.0, 0.0};
-        if (spl_pivot_range_launch(gp, h->d_AB + band_elems, h->d_dummy_tot, st) == SPLPAK_OK)
-            FC_TRY(cudaMemcpyAsync(prange, h->d_dummy_tot, sizeof(double) * 2, cudaMemcpyDeviceToHost, st));
-        if (!coef_on_device) {
-            if (sizeof(real_t) == sizeof(double)) {
-                FC_TRY(cudaMemcpyAsync(coef, d_sol, sizeof(double) * (size_t)gp.ncol, cudaMemcpyDeviceToHost, st));
-            } else {
-                real_t *tmp = h->d_out_tmp;                           // d_AB keeps the factor for refinement steps
-                spl_from_double_kernel<<<spl_div_up(gp.ncol, 256), 256, 0, st>>>(d_sol, tmp, gp.ncol);
-                ++g_spl_launches;
-                FC_TRY(cudaMemcpyAsync(coef, tmp, sizeof(real_t) * (size_t)gp.ncol, cudaMemcpyDeviceToHost, st));
-            }
-        }
-        FC_TRY(cudaStreamSynchronize(st));
-        collect_assemble_timers(h);
-        add_ms(h, 3, h->ev[4], h->ev[5]);
-        add_ms(h, 4, sev[0], sev[1]);
-        add_ms(h, 5, sev[1], sev[2]);
-        add_ms(h, 6, sev[2], sev[3]);
-        // fewer rows than columns (suprls error 33, :1650; not an error with smoothing, whose penalty makes such a fit
-        // well posed) or a non-positive pivot -> 107
-        if (fail || (h->lambda == 0.0 && totals[1] < (double)gp.ncol)) rc = SPLPAK_ERR_SOLVER;
-        h->solved = (rc == SPLPAK_OK);
-        h->cond_est = (prange[0] > 0.0 && prange[1] > 0.0) ? (prange[1] / prange[0]) * (prange[1] / prange[0]) : 0.0;
-        h->factor_valid = h->solved;
-        h->constraints_fired = (h->xtrap != 0.0) && (totals[1] > rows_before);
+    if (rc != SPLPAK_OK) return rc;
+    SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, d_sol, sizeof(double) * (size_t)gp.ncol, cudaMemcpyDeviceToDevice, st));
+    rc = write_coef(h, d_sol, coef, coef_on_device);
+    if (rc != SPLPAK_OK) return rc;
+    // smallest / largest diagonal entry of L (from the stored block inverses): a cheap LOWER bound of cond(G)
+    double prange[2] = {0.0, 0.0};
+    if (spl_pivot_range_launch(gp, h->d_AB + band_elems, h->d_dummy_tot, st) == SPLPAK_OK)
+        SPL_CUDA_TRY(cudaMemcpyAsync(prange, h->d_dummy_tot, sizeof(double) * 2, cudaMemcpyDeviceToHost, st));
+    rc = read_back_solve(h);
+    if (rc != SPLPAK_OK) return rc;
+    collect_assemble_timers(h);
+    add_ms(h, 3, h->ev[4], h->ev[5]);
+    add_ms(h, 4, sev[0], sev[1]);
+    add_ms(h, 5, sev[1], sev[2]);
+    add_ms(h, 6, sev[2], sev[3]);
+    h->cond_est = (prange[0] > 0.0 && prange[1] > 0.0) ? (prange[1] / prange[0]) * (prange[1] / prange[0]) : 0.0;
+    h->factor_valid = h->solved;
+    return h->solved ? SPLPAK_OK : SPLPAK_ERR_SOLVER;
+}
+
+static int fit_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_on_device, int64_t ncf,
+                            int64_t nwrk, int *ierror) {
+    int rc = valid(h) ? SPLPAK_OK : SPLPAK_ERR_HANDLE;
+    if (rc == SPLPAK_OK && h->gp.ncol > ncf) rc = SPLPAK_ERR_NCF;                // :751
+    if (rc == SPLPAK_OK && nwrk >= 0) {
+        // :757-781 and suprls :1443-1454
+        const long long ncol = h->gp.ncol;
+        const long long nwrk1 = (h->xtrap != 0.0) ? ncol + 1 : 1;
+        const long long nwlft = (long long)nwrk - nwrk1 + 1;
+        const long long nreq = ((ncol + 5) * ncol + 2) / 2;
+        if (nwlft < 1) rc = SPLPAK_ERR_NWRK;
+        else if (nwlft < nreq) rc = SPLPAK_ERR_SOLVER;
     }
-#undef FC_TRY
-    h->finalized = 1;
+    if (rc == SPLPAK_OK && h->finalized) rc = SPLPAK_ERR_HANDLE;
+    // a failed band allocation (204) leaves the handle open; every later outcome finalizes it
+    long long band_elems = 0, need = 0;
+    const bool ortho = rc == SPLPAK_OK && h->solver == SPLPAK_SOLVER_ORTHOGONAL;
+    if (rc == SPLPAK_OK && !ortho) rc = ensure_band(h, &band_elems, &need);
+    if (rc == SPLPAK_OK) {
+        h->finalized = 1;
+        h->solved = 0;
+        rc = ortho ? compute_orthogonal(h, coef, coef_on_device) : compute_cholesky(h, coef, coef_on_device, band_elems, need);
+    }
     if (ierror) *ierror = rc;
     return rc;
 }
@@ -1600,13 +1507,7 @@ static int refine_device_chunk(splpak_b200_fit_t h, const real_t *d_x, int l1x, 
                                const real_t *d_w, int weighted, long long n) {
     int rc = ensure_scratch(h, n);
     if (rc != SPLPAK_OK) return rc;
-    if (n > h->res_cap) {
-        if (h->d_res) cudaFree(h->d_res);
-        h->d_res = nullptr;
-        h->res_cap = 0;
-        SPL_CUDA_TRY(cudaMalloc((void **)&h->d_res, sizeof(real_t) * (size_t)n));
-        h->res_cap = n;
-    }
+    SPL_CUDA_TRY(grow(&h->d_res, &h->res_cap, n));
     // s(x_i) with the current coefficients, then r_i = y_i - s(x_i), then g += sum (w phi)(w r)
     rc = eval_device_impl(h->gp, h->di, nullptr, 0, d_x, l1x, n, reinterpret_cast<const real_t *>(h->d_coef64), h->d_res,
                           h->st);
@@ -1624,132 +1525,75 @@ extern "C" int splpak_b200_fit_refine_add_points_device(splpak_b200_fit_t h, con
     if (sizeof(real_t) != sizeof(double) || n <= 0) return SPLPAK_OK;
     if (l1x < h->gp.ndim) return SPLPAK_ERR_HANDLE;
     if (!d_w) weighted = 0;
-    for (long long i0 = 0; i0 < n; i0 += DEVICE_CHUNK) {
-        const long long nc = (n - i0 < DEVICE_CHUNK) ? n - i0 : DEVICE_CHUNK;
-        int rc = refine_device_chunk(h, d_x + i0 * (long long)l1x, l1x, d_y + i0, weighted ? d_w + i0 : nullptr,
-                                     weighted, nc);
-        if (rc != SPLPAK_OK) return rc;
-    }
-    return SPLPAK_OK;
+    return feed_device(h, d_x, l1x, d_y, d_w, weighted, n, refine_device_chunk);
 }
 
+// the staging buffers of add_points are reused (and grown if this call needs more)
 extern "C" int splpak_b200_fit_refine_add_points(splpak_b200_fit_t h, const real_t *x, int l1x,
                                                  const real_t *y, const real_t *w, int weighted, int64_t n) {
     if (!valid(h) || !h->refining) return SPLPAK_ERR_HANDLE;
     if (sizeof(real_t) != sizeof(double) || n <= 0) return SPLPAK_OK;
     if (l1x < h->gp.ndim) return SPLPAK_ERR_HANDLE;
     if (!w) weighted = 0;
-    const long long chunk = n < HOST_CHUNK ? n : HOST_CHUNK;
-    {   // the staging buffers of add_points are reused (and grown if this call needs more)
-        // the kernels of a previous call may still read them: frees are ordered by cudaFree's implicit sync
-        const int rcs = ensure_stage(h, chunk, l1x);
-        if (rcs != SPLPAK_OK) return rcs;
+    return feed_host(h, x, l1x, y, w, weighted, n, refine_device_chunk);
+}
+
+// One refinement step's solve: the constraint rows' and the penalty's share of the residual, then G dc = A^T r with the
+// factor compute left in d_AB, c += dc, and c to the caller.
+static int refine_solve(splpak_b200_fit_t h, real_t *coef, int coef_on_device) {
+    const GridParams &gp = h->gp;
+    cudaStream_t st = h->st;
+    if (sizeof(real_t) == sizeof(double)) {
+        int rc = SPLPAK_OK;
+        if (h->xtrap != 0.0) {
+            rc = spl_constraints_residual_launch(h->gp_fx.fxS ? h->gp_fx : gp, h->xtrap, h->d_cnt, h->d_totals, h->d_coef64, h->d_g, st, h->di.nsm);
+            if (rc != SPLPAK_OK) return rc;
+        }
+        if (h->lambda > 0.0) {
+            // the penalty's share of the residual, -lambda R c: without it the steps would converge to the unsmoothed fit
+            rc = spl_penalty_residual_launch(gp, h->lambda, h->penalty, h->d_pen, h->d_coef64, h->d_g, st, h->di.nsm);
+            if (rc != SPLPAK_OK) return rc;
+        }
+        const long long band_elems = spl_band_elems(gp);
+        const long long need = band_elems + spl_solve_workspace(gp);
+        if (need > h->ab_elems) return SPLPAK_ERR_HANDLE;               // compute allocated it
+        double *d_sol = nullptr;
+        // G is unchanged: reuse its factor (forward + back substitution only); re-factor only where the persistent
+        // substitution kernels are not available for this shape
+        rc = h->factor_valid ? spl_resolve_launch(gp, h->d_AB, h->d_g, h->d_AB + band_elems, &d_sol, h->d_fail, st, h->di.nsm)
+                             : SPLPAK_ERR_HANDLE;
+        if (rc != SPLPAK_OK) {
+            h->factor_valid = 0;
+            SPL_CUDA_TRY(cudaMemsetAsync(h->d_AB, 0, sizeof(double) * (size_t)need, st));
+            SPL_CUDA_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
+            rc = spl_solve_launch(gp, h->d_S, h->d_AB, h->d_g, h->d_AB + band_elems, &d_sol, h->d_fail, st, h->st_aux,
+                                  h->di.nsm, nullptr, &h->solve_cache);
+            if (rc != SPLPAK_OK) return rc;
+            h->factor_valid = 1;
+        }
+        spl_axpy_kernel<<<spl_div_up(gp.ncol, 256), 256, 0, st>>>(h->d_coef64, d_sol, gp.ncol);
+        ++g_spl_launches;
     }
-    int k = 0;
-    for (long long i0 = 0; i0 < n; i0 += chunk, k ^= 1) {
-        const long long nc = (n - i0 < chunk) ? n - i0 : chunk;
-        SPL_CUDA_TRY(cudaStreamWaitEvent(h->st_copy, h->ev_stage_free[k], 0));
-        SPL_CUDA_TRY(spl_h2d(h->d_stage[k][0], x + i0 * (long long)l1x, sizeof(real_t) * (size_t)nc * l1x, h->st_copy,
-                             h->di.dev));
-        SPL_CUDA_TRY(spl_h2d(h->d_stage[k][1], y + i0, sizeof(real_t) * (size_t)nc, h->st_copy, h->di.dev));
-        if (weighted)
-            SPL_CUDA_TRY(spl_h2d(h->d_stage[k][2], w + i0, sizeof(real_t) * (size_t)nc, h->st_copy, h->di.dev));
-        SPL_CUDA_TRY(cudaEventRecord(h->ev_stage_in[k], h->st_copy));
-        SPL_CUDA_TRY(cudaStreamWaitEvent(h->st, h->ev_stage_in[k], 0));
-        int rc = refine_device_chunk(h, h->d_stage[k][0], l1x, h->d_stage[k][1], weighted ? h->d_stage[k][2] : nullptr,
-                                     weighted, nc);
-        if (rc != SPLPAK_OK) return rc;
-        SPL_CUDA_TRY(cudaEventRecord(h->ev_stage_free[k], h->st));
-    }
-    return SPLPAK_OK;
+    int fail = 0;
+    SPL_CUDA_TRY(cudaMemcpyAsync(&fail, h->d_fail, sizeof(int), cudaMemcpyDeviceToHost, st));
+    const int rc = write_coef(h, h->d_coef64, coef, coef_on_device);
+    if (rc != SPLPAK_OK) return rc;
+    SPL_CUDA_TRY(cudaStreamSynchronize(st));
+    return fail ? SPLPAK_ERR_SOLVER : SPLPAK_OK;
 }
 
 static int fit_refine_compute_impl(splpak_b200_fit_t h, real_t *coef, int coef_on_device, int64_t ncf, int *ierror) {
     int rc = SPLPAK_OK;
     if (!valid(h) || !h->refining) rc = SPLPAK_ERR_HANDLE;
     else if (h->gp.ncol > ncf) rc = SPLPAK_ERR_NCF;
-    if (rc != SPLPAK_OK) {
-        if (ierror) *ierror = rc;
-        return rc;
-    }
-    const GridParams &gp = h->gp;
-    cudaStream_t st = h->st;
-    h->refining = 0;
-#define RC_TRY(expr)                                                                        \
-    do {                                                                                    \
-        cudaError_t _e = (expr);                                                            \
-        if (_e != cudaSuccess) {                                                            \
-            fprintf(stderr, "splpak_b200: CUDA error %s at %s:%d (%s)\n", cudaGetErrorString(_e), __FILE__, \
-                    __LINE__, #expr);                                                       \
-            h->factor_valid = 0;                                                            \
-            if (ierror) *ierror = SPLPAK_ERR_CUDA;                                          \
-            return SPLPAK_ERR_CUDA;                                                         \
-        }                                                                                   \
-    } while (0)
-    if (sizeof(real_t) == sizeof(double)) {
-        if (h->xtrap != 0.0) {
-            rc = spl_constraints_residual_launch(h->gp_fx.fxS ? h->gp_fx : gp, h->xtrap, h->d_cnt, h->d_totals, h->d_coef64, h->d_g, st, h->di.nsm);
-            if (rc != SPLPAK_OK) {
-                if (ierror) *ierror = rc;
-                return rc;
-            }
-        }
-        if (h->lambda > 0.0) {
-            // the penalty's share of the residual, -lambda R c: without it the steps would converge to the unsmoothed fit
-            rc = spl_penalty_residual_launch(gp, h->lambda, h->penalty, h->d_pen, h->d_coef64, h->d_g, st, h->di.nsm);
-            if (rc != SPLPAK_OK) {
-                if (ierror) *ierror = rc;
-                return rc;
-            }
-        }
-        const int bw = spl_half_bandwidth(gp);
-        const long long lda = spl_band_lda(bw);
-        const long long band_elems = (gp.ncol * (lda + 1) + 64 + 1) & ~1LL;     // even: the workspace behind stays 16-byte aligned
-        const long long need = band_elems + spl_solve_workspace(gp);
-        if (need > h->ab_elems) rc = SPLPAK_ERR_HANDLE;               // compute allocated it
-        if (rc == SPLPAK_OK) {
-            double *d_sol = nullptr;
-            // G is unchanged: reuse its factor (forward + back substitution only); re-factor only where the persistent
-            // substitution kernels are not available for this shape
-            int rs = h->factor_valid ? spl_resolve_launch(gp, h->d_AB, h->d_g, h->d_AB + band_elems, &d_sol, h->d_fail, st,
-                                                          h->di.nsm)
-                                     : SPLPAK_ERR_HANDLE;
-            if (rs != SPLPAK_OK) {
-                h->factor_valid = 0;
-                RC_TRY(cudaMemsetAsync(h->d_AB, 0, sizeof(double) * (size_t)need, st));
-                RC_TRY(cudaMemsetAsync(h->d_fail, 0, sizeof(int), st));
-                rs = spl_solve_launch(gp, h->d_S, h->d_AB, h->d_g, h->d_AB + band_elems, &d_sol, h->d_fail, st, h->st_aux,
-                                      h->di.nsm, nullptr, &h->solve_cache);
-                if (rs == SPLPAK_OK) h->factor_valid = 1;
-            }
-            rc = rs;
-            if (rc == SPLPAK_OK) {
-                spl_axpy_kernel<<<spl_div_up(gp.ncol, 256), 256, 0, st>>>(h->d_coef64, d_sol, gp.ncol);
-                ++g_spl_launches;
-            }
-        }
-    }
     if (rc == SPLPAK_OK) {
-        int fail = 0;
-        RC_TRY(cudaMemcpyAsync(&fail, h->d_fail, sizeof(int), cudaMemcpyDeviceToHost, st));
-        if (coef_on_device) {
-            spl_from_double_kernel<<<spl_div_up(gp.ncol, 256), 256, 0, st>>>(h->d_coef64, coef, gp.ncol);
-            ++g_spl_launches;
-        } else if (sizeof(real_t) == sizeof(double)) {
-            RC_TRY(cudaMemcpyAsync(coef, h->d_coef64, sizeof(double) * (size_t)gp.ncol, cudaMemcpyDeviceToHost, st));
-        } else {
-            real_t *tmp = h->d_out_tmp;
-            spl_from_double_kernel<<<spl_div_up(gp.ncol, 256), 256, 0, st>>>(h->d_coef64, tmp, gp.ncol);
-            ++g_spl_launches;
-            RC_TRY(cudaMemcpyAsync(coef, tmp, sizeof(real_t) * (size_t)gp.ncol, cudaMemcpyDeviceToHost, st));
-        }
-        RC_TRY(cudaStreamSynchronize(st));
-        if (fail) rc = SPLPAK_ERR_SOLVER;
+        h->refining = 0;
+        rc = refine_solve(h, coef, coef_on_device);
+        if (rc == SPLPAK_ERR_CUDA) h->factor_valid = 0;
     }
     if (ierror) *ierror = rc;
     return rc;
 }
-#undef RC_TRY
 
 extern "C" int splpak_b200_fit_refine_compute(splpak_b200_fit_t h, real_t *coef, int64_t ncf, int *ierror) {
     return fit_refine_compute_impl(h, coef, 0, ncf, ierror);
@@ -1771,17 +1615,23 @@ extern "C" int splpak_b200_fit_set_solver(splpak_b200_fit_t h, int solver) {
     return SPLPAK_ERR_HANDLE;
 }
 extern "C" int splpak_b200_fit_get_solver(splpak_b200_fit_t h) { return valid(h) ? h->solver : -1; }
+// The 1-D penalty tables (penalty.cu), allocated by the first call that needs them
+static int ensure_penalty_tables(splpak_b200_fit_t h) {
+    if (h->d_pen) return SPLPAK_OK;
+    if (cudaMalloc((void **)&h->d_pen, sizeof(double) * (size_t)spl_penalty_table_len(h->gp)) != cudaSuccess) {
+        cudaGetLastError();
+        h->d_pen = nullptr;
+        return SPLPAK_ERR_ALLOC;
+    }
+    return SPLPAK_OK;
+}
+
 extern "C" int splpak_b200_fit_set_smoothing(splpak_b200_fit_t h, double lambda, int penalty) {
     if (!valid(h) || h->finalized) return SPLPAK_ERR_HANDLE;
     if (!(lambda >= 0.0) || !isfinite(lambda)) return SPLPAK_ERR_HANDLE;                  // negative, NaN, inf
     if (penalty != SPLPAK_PENALTY_CURVATURE && penalty != SPLPAK_PENALTY_THIN_PLATE) return SPLPAK_ERR_HANDLE;
     if (lambda > 0.0 && h->solver == SPLPAK_SOLVER_ORTHOGONAL) return SPLPAK_ERR_HANDLE;
-    if (lambda > 0.0 && !h->d_pen &&
-        cudaMalloc((void **)&h->d_pen, sizeof(double) * (size_t)spl_penalty_table_len(h->gp)) != cudaSuccess) {
-        cudaGetLastError();
-        h->d_pen = nullptr;
-        return SPLPAK_ERR_ALLOC;
-    }
+    if (lambda > 0.0 && ensure_penalty_tables(h) != SPLPAK_OK) return SPLPAK_ERR_ALLOC;
     if (lambda != h->lambda || (lambda > 0.0 && penalty != h->penalty)) h->var_valid = 0;   // another system
     h->lambda = lambda;
     h->penalty = penalty;
@@ -1804,12 +1654,7 @@ extern "C" int splpak_b200_fit_enable_gcv(splpak_b200_fit_t h) {
     cudaFree(h->d_part);
     h->d_part = part;
     h->n_part += 1;
-    const GridParams &gp = h->gp;
-    h->d_S = h->d_part;
-    h->d_g = h->d_S + gp.ncol * gp.nsten;
-    h->d_cnt = h->d_g + gp.ncol;
-    h->d_totals = h->d_cnt + gp.ncol;
-    h->d_ywy = h->d_totals + 2;
+    layout_partial(h, true);
     SPL_CUDA_TRY(cudaMemsetAsync(h->d_part, 0, sizeof(double) * (size_t)h->n_part, h->st));
     h->gcv = 1;
     h->s1_valid = h->sigma_valid = h->var_valid = 0;
@@ -1855,13 +1700,7 @@ static int score_factor(splpak_b200_fit_t h, double lambda, int penalty, long lo
         }
         h->s1_valid = 0;
     }
-    if (lambda > 0.0 && !h->d_pen) {
-        if (cudaMalloc((void **)&h->d_pen, sizeof(double) * (size_t)spl_penalty_table_len(gp)) != cudaSuccess) {
-            cudaGetLastError();
-            h->d_pen = nullptr;
-            return SPLPAK_ERR_ALLOC;
-        }
-    }
+    if (lambda > 0.0 && ensure_penalty_tables(h) != SPLPAK_OK) return SPLPAK_ERR_ALLOC;
     const long long ns = gp.ncol * gp.nsten;
     double *d_S1 = h->d_gcv + L.S1, *d_S2 = h->d_gcv + L.S2, *d_g2 = h->d_gcv + L.g2, *d_tot1 = h->d_gcv + L.tot1;
     h->sigma_valid = 0;
@@ -2016,15 +1855,9 @@ static int select_smoothing_search(splpak_b200_fit_t h, int penalty, double lamb
     if (ntrace) *ntrace = 0;
     if (!(lambda_lo > 0.0) || !(lambda_hi > 0.0)) {
         // default range rho * [1e-10, 1e4], rho = sum G0_ii / sum R_ii on the device
-        if (!h->d_pen &&
-            cudaMalloc((void **)&h->d_pen, sizeof(double) * (size_t)spl_penalty_table_len(h->gp)) != cudaSuccess) {
-            cudaGetLastError();
-            h->d_pen = nullptr;
-            if (ierror) *ierror = SPLPAK_ERR_ALLOC;
-            return SPLPAK_ERR_ALLOC;
-        }
         double sums[2] = {0.0, 0.0};
-        rc = spl_penalty_diag_launch(h->gp, penalty, h->d_pen, h->d_S, h->d_dummy_tot, h->st);
+        rc = ensure_penalty_tables(h);
+        if (rc == SPLPAK_OK) rc = spl_penalty_diag_launch(h->gp, penalty, h->d_pen, h->d_S, h->d_dummy_tot, h->st);
         if (rc == SPLPAK_OK && (cudaMemcpyAsync(sums, h->d_dummy_tot, sizeof(sums), cudaMemcpyDeviceToHost, h->st) !=
                                     cudaSuccess ||
                                 cudaStreamSynchronize(h->st) != cudaSuccess))
@@ -2166,7 +1999,7 @@ extern "C" int splpak_b200_fit_get_cholesky_factor(splpak_b200_fit_t h, int whic
     const GridParams &gp = h->gp;
     if (which < 0 || which > 1 || first_col < 0 || ncols < 1 || first_col + ncols > gp.ncol) return SPLPAK_ERR_HANDLE;
     const long long lda = spl_band_lda(spl_half_bandwidth(gp));
-    const long long band_elems = (gp.ncol * (lda + 1) + 64 + 1) & ~1LL;
+    const long long band_elems = spl_band_elems(gp);
     const long long kb0 = first_col / 64, kb1 = (first_col + ncols - 1) / 64;
     const int64_t n = which == 0 ? ncols * lda : (kb1 - kb0 + 1) * 4096;
     if (count) *count = n;

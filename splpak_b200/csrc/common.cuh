@@ -105,6 +105,7 @@ struct HistScratch {
 struct AssembleScratch {
     unsigned *wincount, *winstart, *wincursor, *itemstart, *item_win, *item_seg, *meta;
     unsigned *perm;
+    long long cap;        // points the chunk-sized arrays hold (perm, perm2, yw, pairs, keys, item_win, item_seg)
     long long max_items;
     long long nbins;      // bins of the counting sort: windows (direct path) or cells (moment path)
     int moments;          // 1: 3-D assembly by cell moments (moments.cuh)

@@ -2259,7 +2259,14 @@ int spl_half_bandwidth(const GridParams &gp) {
     return (int)b;
 }
 
-// Workspace (doubles) next to the band matrix: block inverses (64*64 per panel) + ysol (n) + csol (n).
+// Doubles of the band matrix, i.e. the offset of the workspace behind it.  Element (i, j) lives at i + j*lda, so the
+// last one, (n-1, n-1), is at (n-1)*(lda+1); even, so that the workspace stays 16-byte aligned.
+long long spl_band_elems(const GridParams &gp) {
+    const long long lda = spl_band_lda(spl_half_bandwidth(gp));
+    return (gp.ncol * (lda + 1) + 64 + 1) & ~1LL;
+}
+
+// Workspace (doubles) next to the band matrix, at spl_band_elems: block inverses (64*64 per panel) + ysol (n) + csol (n).
 long long spl_solve_workspace(const GridParams &gp) {
     const long long nblk = (gp.ncol + SOLVE_NB - 1) / SOLVE_NB;
     return nblk * 64 * 64 + 2 * (gp.ncol + 64);

@@ -332,11 +332,33 @@ def test_3d_12_strided_device_points(monkeypatch):
     _check("3d12", "device l1x=5", d, ne)
 
 
-@pytest.mark.parametrize("name", ["3d12", "3d12_skew"])
-def test_refinement_rhs_reassembly(monkeypatch, oracle, name):
+def check_refine_rhs(name, label, d, c, rhs, oracle):
     """The rhs_only re-assembly of a refinement step (xtrap = 0: no constraint rows in g) against B^T W^2 (y - B c)
     on the host with the GPU's coefficients c; the residual's own rounding is relative to |y| and |B c|, so the
     tolerance adds TAU |B|^T W^2 |y| to TAU |B|^T W^2 |r|."""
+    t0 = time.perf_counter()
+    s, ierr = oracle.evaluate_batch(3, d["x"], c, d["xmin"], d["xmax"], d["nodes"])
+    assert ierr == 0
+    r = d["y"] - s
+    _, g_ref, gabs_r = assemble_stencil(3, d["x"], r, d["w"], d["xmin"], d["xmax"], d["nodes"], rhs_only=True)
+    SECONDS["reference"] += time.perf_counter() - t0
+    tol = TAU * (gabs_r + d["gabs"])
+    err = worst_ratio(rhs, g_ref, tol)
+    sens = []
+    for p in d["probes"]:
+        _, (gi, gv), _ = point_contribution(3, d["x"][p], r[p], d["w"][p], d["xmin"], d["xmax"], d["nodes"])
+        g1 = g_ref.copy()
+        np.add.at(g1, gi, -gv)
+        sens.append(worst_ratio(rhs, g1, tol))
+    REPORT.append(f"{name:11s} {label:34s} {err:9.2e}  one point out: {min(sens):9.2e}")
+    print(REPORT[-1], flush=True)
+    assert err <= 1.0
+    assert min(sens) >= 100.0
+
+
+@pytest.mark.parametrize("name", ["3d12", "3d12_skew"])
+def test_refinement_rhs_reassembly(monkeypatch, oracle, name):
+    """The rhs_only re-assembly of a refinement step with device points (check_refine_rhs)."""
     d = reference(name)
     _set_env(monkeypatch, {})
     t0 = time.perf_counter()
@@ -354,21 +376,4 @@ def test_refinement_rhs_reassembly(monkeypatch, oracle, name):
     rhs = snap[0].cpu().numpy()
     h.destroy()
     SECONDS["gpu"] += time.perf_counter() - t0
-    t0 = time.perf_counter()
-    s, ierr = oracle.evaluate_batch(3, d["x"], c, d["xmin"], d["xmax"], d["nodes"])
-    assert ierr == 0
-    r = d["y"] - s
-    _, g_ref, gabs_r = assemble_stencil(3, d["x"], r, d["w"], d["xmin"], d["xmax"], d["nodes"], rhs_only=True)
-    SECONDS["reference"] += time.perf_counter() - t0
-    tol = TAU * (gabs_r + d["gabs"])
-    err = worst_ratio(rhs, g_ref, tol)
-    sens = []
-    for p in d["probes"]:
-        _, (gi, gv), _ = point_contribution(3, d["x"][p], r[p], d["w"][p], d["xmin"], d["xmax"], d["nodes"])
-        g1 = g_ref.copy()
-        np.add.at(g1, gi, -gv)
-        sens.append(worst_ratio(rhs, g1, tol))
-    REPORT.append(f"{name:11s} {'refine rhs_only':34s} {err:9.2e}  one point out: {min(sens):9.2e}")
-    print(REPORT[-1], flush=True)
-    assert err <= 1.0
-    assert min(sens) >= 100.0
+    check_refine_rhs(name, "refine rhs_only", d, c, rhs, oracle)
