@@ -67,6 +67,7 @@
         procedure,public :: select_smoothing             !! (new) streaming fit: lambda minimising the GCV score, set on the fit
         procedure,public :: reml_score                   !! (new) streaming fit: REML score {V_R, D_p, log|M|, n, ywy, phi} of one lambda
         procedure,public :: select_smoothing_reml        !! (new) streaming fit: lambda minimising the REML score, set on the fit
+        procedure,public :: robust_fit                   !! (new) streaming fit: iteratively reweighted Huber / bisquare fit
         procedure,public :: prepare_variance             !! (new) streaming fit: tables of the posterior variances (before compute)
         procedure,public :: variance                     !! (new) streaming fit: b(x)^T Sigma b(x) at a batch of points
         procedure,private :: splcc
@@ -259,6 +260,19 @@
             integer(c_int),intent(out) :: ierror
             integer(c_int) :: rc
         end function c_fit_select_smoothing_reml
+        function c_fit_robust(h,x,l1x,y,w,weighted,n,psi,tuning,max_iter,tol,comm,coef,ncf,u,out,nout,ierror) &
+                 bind(C,name='splpak_b200_fit_robust') result(rc)
+            import :: c_int, c_int64_t, c_double, c_ptr, cwp
+            type(c_ptr),value :: h, comm, u
+            real(cwp),intent(in) :: x(*), y(*), w(*)
+            integer(c_int),value :: l1x, weighted, psi, max_iter, nout
+            integer(c_int64_t),value :: n, ncf
+            real(c_double),value :: tuning, tol
+            real(cwp) :: coef(*)
+            real(c_double),intent(out) :: out(*)
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_robust
         function c_fit_prepare_variance(h,out,nout,ierror) bind(C,name='splpak_b200_fit_prepare_variance') result(rc)
             import :: c_int, c_double, c_ptr
             type(c_ptr),value :: h
@@ -580,6 +594,43 @@
         rc = c_fit_variance(me%handle,x,int(l1x,c_int),int(nq,c_int64_t),pn,q,ie)
         ierror = int(rc)
     end subroutine variance
+
+    !> (new) robust fit of the points on a fresh (or reset) fit, by iteratively reweighted least squares:
+    !  psi = 0 Huber, 1 bisquare; tuning <= 0 selects the default constant (1.345 / 4.685); at most max_iter
+    !  reweightings, stop when max |dc| <= tol max |c|.  info = [iterations, sigma, last relative change, sum of u,
+    !  points rejected (u = 0), converged (0/1)]; u(ndata) (optional) receives the final weights u_i.
+    !  wdata absent (or wdata(1)<0) => all weights 1.  ierror: 203 when refused, 104, 105, 107 as compute.
+    subroutine robust_fit(me,xdata,l1xdat,ydata,ndata,psi,tuning,max_iter,tol,coef,ncf,info,ierror,wdata,u)
+        class(splpak_type),intent(inout) :: me
+        integer,intent(in) :: l1xdat, psi, max_iter, ncf
+        integer(int64),intent(in) :: ndata
+        real(wp),intent(in) :: xdata(l1xdat,ndata), ydata(ndata)
+        real(c_double),intent(in) :: tuning, tol
+        real(wp),intent(out) :: coef(ncf)
+        real(c_double),intent(out) :: info(6)
+        integer,intent(out) :: ierror
+        real(wp),intent(in),optional :: wdata(ndata)
+        real(wp),intent(out),optional,target :: u(ndata)
+        integer(c_int) :: weighted, rc, ie
+        real(wp) :: dummy(1)
+        type(c_ptr) :: pu
+        pu = c_null_ptr
+        if (present(u)) pu = c_loc(u)
+        weighted = 0
+        if (present(wdata)) then
+            if (wdata(1) >= 0.0_wp) weighted = 1
+            rc = c_fit_robust(me%handle,xdata,int(l1xdat,c_int),ydata,wdata,weighted,int(ndata,c_int64_t), &
+                              int(psi,c_int),tuning,int(max_iter,c_int),tol,c_null_ptr,coef,int(ncf,c_int64_t), &
+                              pu,info,6_c_int,ie)
+        else
+            dummy = -1.0_wp
+            rc = c_fit_robust(me%handle,xdata,int(l1xdat,c_int),ydata,dummy,weighted,int(ndata,c_int64_t), &
+                              int(psi,c_int),tuning,int(max_iter,c_int),tol,c_null_ptr,coef,int(ncf,c_int64_t), &
+                              pu,info,6_c_int,ie)
+        end if
+        ierror = int(rc)
+        call cfaerr(ierror,.false.)
+    end subroutine robust_fit
 
     !> (new) accumulate n more points; wdata absent (or wdata(1)<0) => all weights 1.
     subroutine add_points(me,xdata,l1xdat,ydata,ndata,ierror,wdata)

@@ -300,6 +300,51 @@ int splpak_b200_fit_variance(splpak_b200_fit_t h, const splpak_real *x, int l1x,
                              splpak_real *out, int *ierror);
 int splpak_b200_fit_variance_device(splpak_b200_fit_t h, const splpak_real *d_x, int l1x, int64_t nq, const int *nderiv,
                                     splpak_real *d_out, void *stream, int *ierror);
+/* Robust fit by iteratively reweighted least squares -- (new).  Data row i has coordinate x_i, value y_i and caller weight
+ * w_i (1 when weighted = 0); only points with w_i > 0 take part.
+ *   residual   r_i = w_i (y_i - s(x_i)), s evaluated as the refinement pass evaluates it
+ *   scale      sigma = MAD / 0.6744897501960817, MAD = the k-th smallest |r_i| over the m points with w_i > 0, k = ceil(m/2)
+ *              (the lower median, about 0; exact: MAD is one of the |r_i|, bit for bit)
+ *   weights    t = r_i / (c sigma);  Huber (c = 1.345 by default): u_i = min(1, 1/|t|);  bisquare (c = 4.685 by default):
+ *              u_i = (1 - t^2)^2 for |t| < 1, else 0;  u_i = 0 where w_i <= 0.  The next assembly uses row weights w_i sqrt(u_i).
+ *   iteration  c^0 is the fit fit_compute would return for the points (the handle's lambda and penalty, constraint rows
+ *              included); iteration k takes the residuals of c^(k-1) to get sigma_k and u^k, re-assembles S and g with the
+ *              new row weights, adds the constraint rows and lambda R, factors and solves for c^k.
+ *   stopping   max_j |c^k_j - c^(k-1)_j| <= tol max_j |c^k_j|, or k = max_iter.  MAD = 0 (the fit interpolates at least half
+ *              the points): stop with the current coefficients, converged.
+ *   constraint rows  the node histogram and [totlwt, nrows] come from the first assembly with the caller's weights and stay
+ *              fixed for the call: the data-sparse nodes, and so the constraint rows, are the same in every iteration.
+ *   refinement when constraint rows fired, two corrected-semi-normal-equation steps after the last solve, with the final row
+ *              weights (as splcw for an ordinary fit; none in the REAL32 library).
+ * out[0..5] = {iterations completed, the last sigma computed (0 when the MAD = 0 stop fired), the last relative change
+ * (0 before the first), sum of u_i, points with w_i > 0 and u_i = 0, converged (0/1)}, nout >= 6.  u (optional, NULL
+ * allowed): the u_i of the final solve.  tuning <= 0 selects the default c.
+ * Preconditions: a fresh or reset handle (no add_points yet), the Cholesky solver; the call does its own assembly.  After it
+ * the handle is finalized as after fit_compute, refine_begin returns 203 (it would re-feed the caller's weights) and the
+ * score and variance calls are refused as after fit_compute.
+ * Errors: 203 invalid or used handle, orthogonal solver, unknown psi, tuning NaN or inf, max_iter < 1, tol < 0 or NaN,
+ * nout < 6, l1x < ndim; 104 ncf < ncol; 105 n < 1; 107 a non-positive pivot in any iteration (coef then holds the last
+ * successful iterate, out[0] counts the completed iterations, u the weights of the failed solve); 204 the host entry
+ * cannot allocate device copies of the points (it copies them once for the whole call).
+ * Multi-GPU: nccl_comm NULL means one GPU; otherwise every rank passes its shard and its communicator (splpak_b200_comm_*)
+ * and the call all-reduces, on the handle's stream, the partial buffer after each assembly, the integer histograms of the
+ * median selection, the convergence numbers and the right-hand side of the refinement steps: every input of the replicated
+ * solve is the same on every rank, so the replicas stay bit-identical.  A process that drives several devices calls the
+ * function from one host thread per device.
+ * FP64 keys, scale and weights (the REAL32 library: float I/O, the residual from its working-precision splfe).
+ * Repeated calls with the same input return bit-identical coef, u and out in SPLPAK_B200_DETERMINISTIC=1 mode, and with
+ * the default assembly up to the order of its FP64 atomic sums. */
+#define SPLPAK_ROBUST_HUBER    0
+#define SPLPAK_ROBUST_BISQUARE 1
+int splpak_b200_fit_robust_device(splpak_b200_fit_t h, const splpak_real *d_x, int l1x, const splpak_real *d_y,
+                                  const splpak_real *d_w, int weighted, int64_t n, int psi, double tuning, int max_iter,
+                                  double tol, void *nccl_comm, splpak_real *d_coef, int64_t ncf, splpak_real *d_u,
+                                  double *out, int nout, int *ierror);
+/* Same with HOST x, y, w, coef and u. */
+int splpak_b200_fit_robust(splpak_b200_fit_t h, const splpak_real *x, int l1x, const splpak_real *y,
+                           const splpak_real *w, int weighted, int64_t n, int psi, double tuning, int max_iter,
+                           double tol, void *nccl_comm, splpak_real *coef, int64_t ncf, splpak_real *u, double *out,
+                           int nout, int *ierror);
 /* Parity-test hook of the orthogonal path: which = 0 -> per-window triangles [nwindows][4^ndim][4^ndim + 1] (R_w | z_w),
  * which = 1 -> band factor [ncol][b + 2] (row i: R[i][i..i+b], then (Q^T r)_i).  out may be NULL to query *count. */
 int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity, int64_t *count);

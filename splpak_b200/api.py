@@ -430,6 +430,64 @@ class FitHandle:
             raise SplpakError(f"prepare_variance failed: {rc}", rc)
         return dict(zip(self._SCORE_KEYS + ("sigma2",), (float(v) for v in out)))
 
+    PSI = {"huber": 0, "bisquare": 1}
+    _ROBUST_KEYS = ("iterations", "sigma", "change", "sum_u", "n_rejected", "converged")
+
+    def _psi_code(self, psi):
+        if psi not in self.PSI:
+            raise SplpakError(f"unknown psi {psi!r}: expected one of {sorted(self.PSI)}")
+        return self.PSI[psi]
+
+    def _robust_info(self, out):
+        info = dict(zip(self._ROBUST_KEYS, (float(v) for v in out)))
+        for k in ("iterations", "n_rejected"):
+            info[k] = int(info[k])
+        info["converged"] = bool(info["converged"])
+        return info
+
+    def robust_fit(self, x, y, w=None, psi="bisquare", tuning=None, max_iter=20, tol=1e-6, return_weights=False):
+        """Robust fit of HOST points on a fresh (or reset) handle by iteratively reweighted least squares: Huber or
+        Tukey bisquare weights from the residuals scaled by their exact median absolute value (header:
+        splpak_b200_fit_robust_device).  tuning None: 1.345 (Huber) / 4.685 (bisquare).  Returns (coef, info, ierror),
+        info = {iterations, sigma, change, sum_u, n_rejected, converged} and, with return_weights, "u": the weights u_i
+        of the final solve.  An unknown psi name raises SplpakError."""
+        self._check()
+        code = self._psi_code(psi)
+        xa = np.ascontiguousarray(x, dtype=self.dt)
+        if xa.ndim == 1:
+            xa = xa.reshape(-1, 1)
+        ya = _vec(y, self.dt)
+        wa = _vec(w, self.dt) if w is not None else None
+        n = xa.shape[0]
+        coef = np.zeros(self.ncol, dtype=self.dt)
+        u = np.zeros(max(n, 1), dtype=self.dt) if return_weights else None
+        out = np.zeros(6)
+        ierr = C.c_int(0)
+        self.lib.splpak_b200_fit_robust(self.h, _ptr(xa), xa.shape[1], _ptr(ya), _ptr(wa) if wa is not None else None,
+                                        int(wa is not None), n, code, 0.0 if tuning is None else float(tuning),
+                                        int(max_iter), float(tol), None, _ptr(coef), self.ncol,
+                                        _ptr(u) if u is not None else None, _ptr(out), 6, C.byref(ierr))
+        info = self._robust_info(out)
+        if return_weights:
+            info["u"] = u[:n]
+        return coef, info, ierr.value
+
+    def robust_fit_device(self, d_x, l1x, d_y, d_w, n, d_coef, psi="bisquare", tuning=None, max_iter=20, tol=1e-6,
+                          d_u=None, comm=None):
+        """robust_fit with torch CUDA tensors or raw device pointers (d_w None: all weights 1; d_u None: no weights
+        returned).  comm: a raw ncclComm_t (splpak_b200_comm_*) when every rank passes its shard, None on one GPU.
+        Returns (info, ierror)."""
+        self._check()
+        code = self._psi_code(psi)
+        out = np.zeros(6)
+        ierr = C.c_int(0)
+        self.lib.splpak_b200_fit_robust_device(self.h, _dev_ptr(d_x), int(l1x), _dev_ptr(d_y), _dev_ptr(d_w),
+                                               int(d_w is not None), int(n), code,
+                                               0.0 if tuning is None else float(tuning), int(max_iter), float(tol),
+                                               comm, _dev_ptr(d_coef), self.ncol, _dev_ptr(d_u), _ptr(out), 6,
+                                               C.byref(ierr))
+        return self._robust_info(out), ierr.value
+
     def variance(self, x, nderiv=None):
         """q(x) = b(x)^T Sigma b(x) at HOST points x (nq, l1x), after prepare_variance: the posterior variance of the
         fitted value (nderiv: of that partial derivative) divided by sigma2.  Returns (q[nq], ierror)."""

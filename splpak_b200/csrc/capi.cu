@@ -94,6 +94,17 @@ int spl_variance_table_launch(const GridParams &gp, const double *d_AB, long lon
                               int nsm);
 int spl_variance_launch(const GridParams &gp, const int *nderiv, const real_t *d_x, int l1x, long long nq,
                         const double *d_W, real_t *d_out, cudaStream_t st, int nsm);
+int spl_robust_scratch_init(RobustScratch &rs, long long n, long long ncol, int nsm);
+void spl_robust_scratch_free(RobustScratch &rs);
+int spl_robust_key_launch(const RobustScratch &rs, const real_t *d_y, const real_t *d_w, int weighted, cudaStream_t st,
+                          int nsm);
+int spl_robust_passes();
+long long spl_robust_bins();
+int spl_robust_hist_launch(const RobustScratch &rs, int pass, cudaStream_t st, int nsm);
+int spl_robust_select_launch(const RobustScratch &rs, int pass, cudaStream_t st);
+int spl_robust_weight_launch(const RobustScratch &rs, const real_t *d_w, int weighted, int psi, double c, int unit,
+                             real_t *d_u, cudaStream_t st, int nsm);
+int spl_robust_change_launch(const RobustScratch &rs, const double *d_c, long long ncol, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------
 // small conversion kernels
@@ -945,6 +956,7 @@ struct splpak_b200_fit_s {
     real_t *d_out_tmp;            // ncol reals: working-precision copy of the solution for the D2H of real32 builds
     int refining;
     int constraints_fired;        // derivative-constraint rows were added by compute
+    int robust;                   // the fit was a robust fit: refine_begin would re-feed the caller's weights, so it refuses
     // smoothing (penalty.cu): lambda * R is added to S by compute when lambda > 0; kept across fit_reset
     double lambda;
     int penalty;                  // SPLPAK_PENALTY_CURVATURE or SPLPAK_PENALTY_THIN_PLATE
@@ -1095,7 +1107,7 @@ extern "C" int splpak_b200_fit_reset(splpak_b200_fit_t h) {
     h->finalized = 0;
     h->timers_pending = 0;
     h->total_points = 0;
-    h->solved = h->refining = h->constraints_fired = h->factor_valid = 0;
+    h->solved = h->refining = h->constraints_fired = h->factor_valid = h->robust = 0;
     h->s1_valid = h->sigma_valid = h->var_valid = 0;
     h->cond_est = 0.0;
     if (h->os) return spl_ortho_reset(h->gp, *h->os, h->st);
@@ -1495,7 +1507,7 @@ extern "C" int splpak_b200_fit_compute_device(splpak_b200_fit_t h, real_t *d_coe
 // recovers the accuracy of the orthogonal method as long as eps*cond(G) < 1.
 // ------------------------------------------------------------------------------------------
 extern "C" int splpak_b200_fit_refine_begin(splpak_b200_fit_t h) {
-    if (!valid(h) || !h->finalized || !h->solved) return SPLPAK_ERR_HANDLE;
+    if (!valid(h) || !h->finalized || !h->solved || h->robust) return SPLPAK_ERR_HANDLE;
     if (h->solver == SPLPAK_SOLVER_ORTHOGONAL) return SPLPAK_ERR_HANDLE;   // already at cond(A): nothing to refine
     if (sizeof(real_t) != sizeof(double)) return SPLPAK_OK;            // fp32 I/O: nothing to gain
     SPL_CUDA_TRY(cudaMemsetAsync(h->d_g, 0, sizeof(double) * (size_t)h->gp.ncol, h->st));
@@ -1601,6 +1613,244 @@ extern "C" int splpak_b200_fit_refine_compute(splpak_b200_fit_t h, real_t *coef,
 extern "C" int splpak_b200_fit_refine_compute_device(splpak_b200_fit_t h, real_t *d_coef, int64_t ncf, int *ierror) {
     return fit_refine_compute_impl(h, d_coef, 1, ncf, ierror);
 }
+// ------------------------------------------------------------------------------------------
+// robust fit: iteratively reweighted least squares with an exact device median of |residual| (robust.cu; DESIGN §4.15)
+// ------------------------------------------------------------------------------------------
+// ncclDataType_t / ncclRedOp_t codes of nccl.h
+#define NCCL_UINT64 5
+#define NCCL_FLOAT64 8
+#define NCCL_SUM 0
+#define NCCL_MAX 2
+// In-place all-reduce of count elements on the handle's stream; nothing to do on one GPU (comm NULL)
+static int robust_allreduce(splpak_b200_fit_t h, void *comm, void *buf, size_t count, int dtype, int op) {
+    if (!comm) return SPLPAK_OK;
+    NcclApi &api = nccl_api();
+    if (!api.ok) return SPLPAK_ERR_NCCL;
+    return api.AllReduce(buf, buf, count, dtype, op, comm, h->st) == 0 ? SPLPAK_OK : SPLPAK_ERR_NCCL;
+}
+
+static int robust_check(splpak_b200_fit_t h, int l1x, int64_t n, int psi, double tuning, int max_iter, double tol,
+                        int64_t ncf, const double *out, int nout) {
+    if (!valid(h) || h->finalized || h->total_points != 0 || h->solver != SPLPAK_SOLVER_CHOLESKY) return SPLPAK_ERR_HANDLE;
+    if (psi != SPLPAK_ROBUST_HUBER && psi != SPLPAK_ROBUST_BISQUARE) return SPLPAK_ERR_HANDLE;
+    if (!isfinite(tuning) || max_iter < 1 || !(tol >= 0.0) || !out || nout < 6 || l1x < h->gp.ndim) return SPLPAK_ERR_HANDLE;
+    if (h->gp.ncol > ncf) return SPLPAK_ERR_NCF;
+    if (n < 1) return SPLPAK_ERR_NDATA;
+    return SPLPAK_OK;
+}
+
+// s(x_i) of the current solution d_coef64 into rs.s, in the chunks and with the evaluation of the refinement pass
+static int robust_eval(splpak_b200_fit_t h, RobustScratch &rs, const real_t *d_x, int l1x, long long n) {
+    const real_t *coef = reinterpret_cast<const real_t *>(h->d_coef64);
+    if (sizeof(real_t) != sizeof(double)) {
+        // the REAL32 library's splfe works in float: the solution rounded to working precision first
+        spl_from_double_kernel<<<spl_div_up(h->gp.ncol, 256), 256, 0, h->st>>>(h->d_coef64, h->d_out_tmp, h->gp.ncol);
+        ++g_spl_launches;
+        coef = h->d_out_tmp;
+    }
+    for (long long i0 = 0; i0 < n; i0 += DEVICE_CHUNK) {
+        const long long nc = (n - i0 < DEVICE_CHUNK) ? n - i0 : DEVICE_CHUNK;
+        const int rc = eval_device_impl(h->gp, h->di, nullptr, 0, d_x + i0 * (long long)l1x, l1x, nc, coef, rs.s + i0,
+                                        h->st);
+        if (rc != SPLPAK_OK) return rc;
+    }
+    return SPLPAK_OK;
+}
+
+// keys |w (y - s)|, then the radix select of the lower median: sigma in device memory (rs.state), no host synchronisation
+static int robust_scale(splpak_b200_fit_t h, RobustScratch &rs, const real_t *d_y, const real_t *d_w, int weighted,
+                        void *comm) {
+    int rc = spl_robust_key_launch(rs, d_y, d_w, weighted, h->st, h->di.nsm);
+    for (int pass = 0; pass < spl_robust_passes() && rc == SPLPAK_OK; ++pass) {
+        rc = spl_robust_hist_launch(rs, pass, h->st, h->di.nsm);
+        if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, rs.hist, (size_t)spl_robust_bins(), NCCL_UINT64, NCCL_SUM);
+        if (rc == SPLPAK_OK) rc = spl_robust_select_launch(rs, pass, h->st);
+    }
+    return rc;
+}
+
+// one chunk of a re-assembly with the robust row weights: S and g only (the histogram and totals stay those of the
+// first assembly; classify's totals go to the discarded slots, as in the refinement pass)
+static int reassemble_device_chunk(splpak_b200_fit_t h, const real_t *d_x, int l1x, const real_t *d_y,
+                                   const real_t *d_w, int weighted, long long n) {
+    const int rc = ensure_scratch(h, n);
+    if (rc != SPLPAK_OK) return rc;
+    return spl_assemble_chunk(h->gp, d_x, l1x, d_y, d_w, weighted, n, 0, 0, h->sc, h->d_S, h->d_g, h->d_cnt,
+                              h->d_dummy_tot, h->st, h->di.nsm, nullptr);
+}
+
+// The loop of splpak_b200_fit_robust_device (semantics: the header).  res = out[0..5]; on 107 the caller's coef holds
+// the last successful iterate.
+static int robust_run(splpak_b200_fit_t h, RobustScratch &rs, const real_t *d_x, int l1x, const real_t *d_y,
+                      const real_t *d_w, int weighted, long long n, int psi, double c, int max_iter, double tol,
+                      void *comm, real_t *coef, int coef_on_device, real_t *d_u, double res[6]) {
+    cudaStream_t st = h->st;
+    const long long ncol = h->gp.ncol;
+    long long band_elems = 0, need = 0;
+    int rc = ensure_band(h, &band_elems, &need);
+    // c^0: the ordinary fit, whose node histogram and totals stay for the whole call
+    if (rc == SPLPAK_OK) rc = feed_device(h, d_x, l1x, d_y, d_w, weighted, n, add_device_chunk);
+    if (rc != SPLPAK_OK) return rc;
+    h->total_points += n;
+    h->finalized = 1;
+    h->robust = 1;
+    h->solved = 0;
+    rc = robust_allreduce(h, comm, h->d_part, (size_t)h->n_part, NCCL_FLOAT64, NCCL_SUM);
+    if (rc != SPLPAK_OK) return rc;
+    SPL_CUDA_TRY(cudaMemcpyAsync(rs.tot0, h->d_totals, sizeof(double) * 2, cudaMemcpyDeviceToDevice, st));
+    rc = compute_cholesky(h, coef, coef_on_device, band_elems, need);
+    if (rc != SPLPAK_OK) return rc;
+    // row weights of the last solve (the refinement steps use them)
+    const real_t *fw = d_w;
+    int fweighted = weighted;
+    bool stats = false;
+    const long long nsg = ncol * h->gp.nsten + ncol;          // [S | g] at the start of the partial buffer
+    for (int k = 1; k <= max_iter; ++k) {
+        rc = robust_eval(h, rs, d_x, l1x, n);
+        if (rc == SPLPAK_OK) rc = robust_scale(h, rs, d_y, d_w, weighted, comm);
+        if (rc != SPLPAK_OK) return rc;
+        double sigma = 0.0;
+        SPL_CUDA_TRY(cudaMemcpyAsync(&sigma, rs.state + 3, sizeof(double), cudaMemcpyDeviceToHost, st));
+        SPL_CUDA_TRY(cudaStreamSynchronize(st));
+        res[1] = sigma;
+        if (!(sigma > 0.0)) {
+            // MAD = 0: the fit interpolates at least half the points.  Converged; at k = 1 the weights of the solve
+            // were the caller's (u = 1 where w > 0)
+            res[5] = 1.0;
+            if (k == 1) {
+                rc = spl_robust_weight_launch(rs, d_w, weighted, psi, c, 1, d_u, st, h->di.nsm);
+                if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, rs.stats, 2, NCCL_FLOAT64, NCCL_SUM);
+                if (rc != SPLPAK_OK) return rc;
+                stats = true;
+            }
+            break;
+        }
+        rc = spl_robust_weight_launch(rs, d_w, weighted, psi, c, 0, d_u, st, h->di.nsm);
+        if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, rs.stats, 2, NCCL_FLOAT64, NCCL_SUM);
+        if (rc != SPLPAK_OK) return rc;
+        stats = true;
+        fw = rs.rw;
+        fweighted = 1;
+        SPL_CUDA_TRY(cudaMemcpyAsync(rs.cprev, h->d_coef64, sizeof(double) * (size_t)ncol, cudaMemcpyDeviceToDevice, st));
+        SPL_CUDA_TRY(cudaMemsetAsync(h->d_part, 0, sizeof(double) * (size_t)nsg, st));
+        rc = feed_device(h, d_x, l1x, d_y, rs.rw, 1, n, reassemble_device_chunk);
+        if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, h->d_part, (size_t)nsg, NCCL_FLOAT64, NCCL_SUM);
+        if (rc != SPLPAK_OK) return rc;
+        SPL_CUDA_TRY(cudaMemcpyAsync(h->d_totals, rs.tot0, sizeof(double) * 2, cudaMemcpyDeviceToDevice, st));
+        rc = compute_cholesky(h, coef, coef_on_device, band_elems, need);
+        if (rc == SPLPAK_ERR_SOLVER) {
+            // the last successful iterate back to the caller
+            SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, rs.cprev, sizeof(double) * (size_t)ncol, cudaMemcpyDeviceToDevice, st));
+            rc = write_coef(h, h->d_coef64, coef, coef_on_device);
+            if (rc == SPLPAK_OK) rc = SPLPAK_ERR_SOLVER;
+            break;
+        }
+        if (rc != SPLPAK_OK) return rc;
+        res[0] = k;
+        rc = spl_robust_change_launch(rs, h->d_coef64, ncol, st);
+        if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, rs.change, 2, NCCL_FLOAT64, NCCL_MAX);
+        if (rc != SPLPAK_OK) return rc;
+        double chg[2] = {0.0, 0.0};
+        SPL_CUDA_TRY(cudaMemcpyAsync(chg, rs.change, sizeof(chg), cudaMemcpyDeviceToHost, st));
+        SPL_CUDA_TRY(cudaStreamSynchronize(st));
+        res[2] = chg[1] > 0.0 ? chg[0] / chg[1] : 0.0;
+        if (chg[0] <= tol * chg[1]) {
+            res[5] = 1.0;
+            break;
+        }
+    }
+    if (stats) {
+        SPL_CUDA_TRY(cudaMemcpyAsync(res + 3, rs.stats, sizeof(double) * 2, cudaMemcpyDeviceToHost, st));
+        SPL_CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    if (rc != SPLPAK_OK) return rc;
+    // the refinement steps of splcw, with the row weights of the last solve and the factor compute left in d_AB
+    if (sizeof(real_t) == sizeof(double) && h->constraints_fired) {
+        for (int step = 0; step < SPLPAK_REFINE_STEPS && rc == SPLPAK_OK; ++step) {
+            SPL_CUDA_TRY(cudaMemsetAsync(h->d_g, 0, sizeof(double) * (size_t)ncol, st));
+            rc = feed_device(h, d_x, l1x, d_y, fw, fweighted, n, refine_device_chunk);
+            if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, h->d_g, (size_t)ncol, NCCL_FLOAT64, NCCL_SUM);
+            if (rc == SPLPAK_OK) rc = refine_solve(h, coef, coef_on_device);
+        }
+    }
+    return rc;
+}
+
+static int fit_robust_impl(splpak_b200_fit_t h, const real_t *d_x, int l1x, const real_t *d_y, const real_t *d_w,
+                           int weighted, long long n, int psi, double tuning, int max_iter, double tol, void *comm,
+                           real_t *coef, int coef_on_device, real_t *d_u, double *out) {
+    const double c = tuning > 0.0 ? tuning : (psi == SPLPAK_ROBUST_HUBER ? 1.345 : 4.685);
+    double res[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    RobustScratch rs;
+    int rc = spl_robust_scratch_init(rs, n, h->gp.ncol, h->di.nsm);
+    if (rc == SPLPAK_OK) {
+        rc = robust_run(h, rs, d_x, l1x, d_y, d_w, weighted, n, psi, c, max_iter, tol, comm, coef, coef_on_device, d_u,
+                        res);
+        if (cudaStreamSynchronize(h->st) != cudaSuccess) {
+            cudaGetLastError();
+            if (rc == SPLPAK_OK) rc = SPLPAK_ERR_CUDA;
+        }
+        spl_robust_scratch_free(rs);
+    }
+    memcpy(out, res, sizeof(res));
+    return rc;
+}
+
+extern "C" int splpak_b200_fit_robust_device(splpak_b200_fit_t h, const real_t *d_x, int l1x, const real_t *d_y,
+                                             const real_t *d_w, int weighted, int64_t n, int psi, double tuning,
+                                             int max_iter, double tol, void *nccl_comm, real_t *d_coef, int64_t ncf,
+                                             real_t *d_u, double *out, int nout, int *ierror) {
+    int rc = robust_check(h, l1x, n, psi, tuning, max_iter, tol, ncf, out, nout);
+    if (!d_w) weighted = 0;
+    if (rc == SPLPAK_OK)
+        rc = fit_robust_impl(h, d_x, l1x, d_y, d_w, weighted, n, psi, tuning, max_iter, tol, nccl_comm, d_coef, 1, d_u,
+                             out);
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+// HOST arrays: the points go to device buffers once for the whole call (through the pinned staging of spl_h2d)
+extern "C" int splpak_b200_fit_robust(splpak_b200_fit_t h, const real_t *x, int l1x, const real_t *y, const real_t *w,
+                                      int weighted, int64_t n, int psi, double tuning, int max_iter, double tol,
+                                      void *nccl_comm, real_t *coef, int64_t ncf, real_t *u, double *out, int nout,
+                                      int *ierror) {
+    int rc = robust_check(h, l1x, n, psi, tuning, max_iter, tol, ncf, out, nout);
+    if (!w) weighted = 0;
+    real_t *d[4] = {nullptr, nullptr, nullptr, nullptr};          // x, y, w, u
+    if (rc == SPLPAK_OK) {
+        const size_t len[4] = {(size_t)n * (size_t)l1x, (size_t)n, weighted ? (size_t)n : 0, u ? (size_t)n : 0};
+        for (int a = 0; a < 4 && rc == SPLPAK_OK; ++a)
+            if (len[a] && cudaMalloc((void **)&d[a], sizeof(real_t) * len[a]) != cudaSuccess) {
+                cudaGetLastError();
+                d[a] = nullptr;
+                rc = SPLPAK_ERR_ALLOC;
+            }
+        if (rc == SPLPAK_OK && d[3] && cudaMemsetAsync(d[3], 0, sizeof(real_t) * len[3], h->st) != cudaSuccess) {
+            cudaGetLastError();
+            rc = SPLPAK_ERR_CUDA;
+        }
+        const real_t *src[3] = {x, y, w};
+        for (int a = 0; a < 3 && rc == SPLPAK_OK; ++a)
+            if (len[a] && spl_h2d(d[a], src[a], sizeof(real_t) * len[a], h->st, h->di.dev) != cudaSuccess) {
+                cudaGetLastError();
+                rc = SPLPAK_ERR_CUDA;
+            }
+        if (rc == SPLPAK_OK)
+            rc = fit_robust_impl(h, d[0], l1x, d[1], d[2], weighted, n, psi, tuning, max_iter, tol, nccl_comm, coef, 0,
+                                 d[3], out);
+        if (u && (rc == SPLPAK_OK || rc == SPLPAK_ERR_SOLVER) &&
+            (spl_d2h(u, d[3], sizeof(real_t) * (size_t)n, h->st, h->di.dev) != cudaSuccess ||
+             spl_d2h_flush(h->di.dev) != cudaSuccess || cudaStreamSynchronize(h->st) != cudaSuccess)) {
+            cudaGetLastError();
+            rc = SPLPAK_ERR_CUDA;
+        }
+        for (int a = 0; a < 4; ++a)
+            if (d[a]) cudaFree(d[a]);
+    }
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
 extern "C" int splpak_b200_fit_set_solver(splpak_b200_fit_t h, int solver) {
     if (!valid(h) || h->total_points != 0 || h->finalized) return SPLPAK_ERR_HANDLE;    // before the first point
     if (solver == SPLPAK_SOLVER_CHOLESKY) {

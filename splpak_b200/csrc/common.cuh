@@ -143,6 +143,20 @@ struct OrthoScratch {
     int ready = 0;
 };
 
+// Scratch of one robust fit call (robust.cu): per point the |residual| keys, the spline values and the row weights;
+// the selection's histogram + state, the weight kernel's partial sums, the previous coefficients and the small results.
+struct RobustScratch {
+    long long n;
+    int nparts;                           // CTAs of the weight kernel (one partial sum each)
+    unsigned long long *key;              // n
+    real_t *s;                            // n: s(x_i), then the keys are formed from it
+    real_t *rw;                           // n: row weights w_i sqrt(u_i) of the next assembly
+    unsigned long long *hist, *state, *nzero;   // one allocation: bins, 4 state words, the rejected count
+    // one allocation: [cprev (ncol) | change {max |dc|, max |c|} | stats {sum u, rejected} | tot0 | part (nparts)];
+    // tot0: [totlwt, nrows] of the first assembly, restored before every solve so that the constraint rows stay fixed
+    double *small, *cprev, *change, *stats, *tot0, *part;
+};
+
 extern unsigned long long g_spl_launches;   // host-side launch counter (capi.cu)
 
 #define SPL_CUDA_TRY(expr)                                                              \
