@@ -68,6 +68,7 @@
         procedure,public :: reml_score                   !! (new) streaming fit: REML score {V_R, D_p, log|M|, n, ywy, phi} of one lambda
         procedure,public :: select_smoothing_reml        !! (new) streaming fit: lambda minimising the REML score, set on the fit
         procedure,public :: robust_fit                   !! (new) streaming fit: iteratively reweighted Huber / bisquare fit
+        procedure,public :: glm_fit                      !! (new) streaming fit: penalized IRLS, Poisson / binomial / Gamma response
         procedure,public :: prepare_variance             !! (new) streaming fit: tables of the posterior variances (before compute)
         procedure,public :: variance                     !! (new) streaming fit: b(x)^T Sigma b(x) at a batch of points
         procedure,private :: splcc
@@ -273,6 +274,19 @@
             integer(c_int),intent(out) :: ierror
             integer(c_int) :: rc
         end function c_fit_robust
+        function c_fit_glm(h,x,l1x,y,w,weighted,offset,n,family,max_iter,tol,comm,coef,ncf,mu,out,nout,ierror) &
+                 bind(C,name='splpak_b200_fit_glm') result(rc)
+            import :: c_int, c_int64_t, c_double, c_ptr, cwp
+            type(c_ptr),value :: h, offset, comm, mu
+            real(cwp),intent(in) :: x(*), y(*), w(*)
+            integer(c_int),value :: l1x, weighted, family, max_iter, nout
+            integer(c_int64_t),value :: n, ncf
+            real(c_double),value :: tol
+            real(cwp) :: coef(*)
+            real(c_double),intent(out) :: out(*)
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_glm
         function c_fit_prepare_variance(h,out,nout,ierror) bind(C,name='splpak_b200_fit_prepare_variance') result(rc)
             import :: c_int, c_double, c_ptr
             type(c_ptr),value :: h
@@ -631,6 +645,48 @@
         ierror = int(rc)
         call cfaerr(ierror,.false.)
     end subroutine robust_fit
+
+    !> (new) generalized smoothing fit of the points on a fresh (or reset) fit, by penalized iteratively reweighted
+    !  least squares: family = 0 Poisson (log link), 1 binomial (logit; ydata a proportion, wdata = sqrt(trials)),
+    !  2 Gamma (log); eta = s(x) + offset.  At most max_iter solves (glm.control: 25), stop when
+    !  |D_k - D_(k-1)| / (|D_k| + 0.1) < tol (1e-8).  info = [iterations, deviance, Pearson X^2, last relative deviance
+    !  change, step halvings, converged (0/1), points with w > 0]; mu(ndata) (optional) receives the fitted means.
+    !  wdata absent (or wdata(1)<0) => all weights 1.  ierror: 203 when refused (a y outside the family's domain
+    !  included), 104, 105, 107 as compute.
+    subroutine glm_fit(me,xdata,l1xdat,ydata,ndata,family,max_iter,tol,coef,ncf,info,ierror,wdata,offset,mu)
+        class(splpak_type),intent(inout) :: me
+        integer,intent(in) :: l1xdat, family, max_iter, ncf
+        integer(int64),intent(in) :: ndata
+        real(wp),intent(in) :: xdata(l1xdat,ndata), ydata(ndata)
+        real(c_double),intent(in) :: tol
+        real(wp),intent(out) :: coef(ncf)
+        real(c_double),intent(out) :: info(7)
+        integer,intent(out) :: ierror
+        real(wp),intent(in),optional :: wdata(ndata)
+        real(wp),intent(in),optional,target :: offset(ndata)
+        real(wp),intent(out),optional,target :: mu(ndata)
+        integer(c_int) :: weighted, rc, ie
+        real(wp) :: dummy(1)
+        type(c_ptr) :: po, pm
+        po = c_null_ptr
+        pm = c_null_ptr
+        if (present(offset)) po = c_loc(offset)
+        if (present(mu)) pm = c_loc(mu)
+        weighted = 0
+        if (present(wdata)) then
+            if (wdata(1) >= 0.0_wp) weighted = 1
+            rc = c_fit_glm(me%handle,xdata,int(l1xdat,c_int),ydata,wdata,weighted,po,int(ndata,c_int64_t), &
+                           int(family,c_int),int(max_iter,c_int),tol,c_null_ptr,coef,int(ncf,c_int64_t), &
+                           pm,info,7_c_int,ie)
+        else
+            dummy = -1.0_wp
+            rc = c_fit_glm(me%handle,xdata,int(l1xdat,c_int),ydata,dummy,weighted,po,int(ndata,c_int64_t), &
+                           int(family,c_int),int(max_iter,c_int),tol,c_null_ptr,coef,int(ncf,c_int64_t), &
+                           pm,info,7_c_int,ie)
+        end if
+        ierror = int(rc)
+        call cfaerr(ierror,.false.)
+    end subroutine glm_fit
 
     !> (new) accumulate n more points; wdata absent (or wdata(1)<0) => all weights 1.
     subroutine add_points(me,xdata,l1xdat,ydata,ndata,ierror,wdata)

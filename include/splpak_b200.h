@@ -345,6 +345,64 @@ int splpak_b200_fit_robust(splpak_b200_fit_t h, const splpak_real *x, int l1x, c
                            const splpak_real *w, int weighted, int64_t n, int psi, double tuning, int max_iter,
                            double tol, void *nccl_comm, splpak_real *coef, int64_t ncf, splpak_real *u, double *out,
                            int nout, int *ierror);
+/* Generalized smoothing fit by penalized iteratively reweighted least squares (PIRLS) -- (new).  Data row i has
+ * coordinate x_i, response y_i, caller weight w_i (1 when weighted = 0) and offset o_i (0 when offset is NULL); only
+ * points with w_i > 0 take part.
+ *   prior weight      a_i = w_i^2 (row i of a least-squares fit contributes (w_i (y_i - s))^2).  Binomial: y_i is a
+ *                     proportion and a_i the number of trials, so pass w_i = sqrt(trials).
+ *   linear predictor  eta_i = s(x_i) + o_i, s evaluated as the refinement pass evaluates it.
+ *   family            link   mu(eta) and dmu/deta                              V(mu)        valid y     start mu0
+ *     POISSON  (0)    log    max(exp(eta), eps), same                          mu           y >= 0      y + 0.1
+ *     BINOMIAL (1)    logit  R's logit_linkinv / logit_mu_eta (+-30, eps, 1/eps) mu (1 - mu)  0 <= y <= 1 (a y + 0.5)/(a + 1)
+ *     GAMMA    (2)    log    max(exp(eta), eps), same                          mu^2         y > 0       y
+ *                     eps = 2^-52: the clamps of R's make.link, the starts of glm.fit.  eta itself is not clamped.
+ *   working values    z_i = eta_i - o_i + (y_i - mu_i) / mu'_i, W_i = a_i mu'_i^2 / V(mu_i); the assembly takes the
+ *                     response z_i with row weight sqrt(W_i) = w_i mu'_i / sqrt(V); z_i = 0 and row weight 0 where
+ *                     w_i <= 0 (y_i is not read there).
+ *   deviance          D = sum over w_i > 0 of R's unit deviances (y log y = 0 at y = 0): Poisson 2 a (y log(y/mu) -
+ *                     (y - mu)), binomial 2 a (y log(y/mu) + (1-y) log((1-y)/(1-mu))), Gamma -2 a (log(y/mu) -
+ *                     (y - mu)/mu);  Pearson X^2 = sum a (y - mu)^2 / V(mu).
+ *   iteration k = 1, 2, ...  z and W from the current mu (k = 1: mu0, eta0 = g(mu0), the offset ignored as glm.fit
+ *                     does); assemble (k = 1: the ordinary first assembly, whose node histogram and [totlwt, nrows]
+ *                     stay fixed for the call; later: S and g only); the constraint rows and lambda R (the handle's
+ *                     lambda and penalty); factor and solve for c^k; evaluate eta^k, mu^k and D_k.
+ *   step halving      while D_k is not finite: c^k = (c^k + c^(k-1)) / 2 and evaluate again, at most 10 times (glm.fit).
+ *                     Still not finite, or not finite at k = 1: 107, coef = the last iterate with a finite deviance
+ *                     (c^1 at k = 1).
+ *   stopping          |D_k - D_(k-1)| / (|D_k| + 0.1) < tol (D_0: the deviance of mu0), or k = max_iter.  glm.control's
+ *                     defaults are tol = 1e-8, max_iter = 25.
+ *   refinement        when constraint rows fired and the last iteration took its full step, two corrected-semi-normal-
+ *                     equation steps of splcw follow the last solve, with that solve's z and row weights (none in the
+ *                     REAL32 library), then one more evaluation: out and mu describe the returned coefficients.
+ * out[0..6] = {iterations (solves completed), D, X^2, the last relative deviance change, step halvings in all,
+ * converged (0/1), m = points with w_i > 0}, nout >= 7.  mu (optional, NULL allowed): the fitted means at the points.
+ * Preconditions: a fresh or reset handle (no add_points yet), the Cholesky solver; the call does its own assembly.  After
+ * it the handle is finalized as after fit_compute, refine_begin returns 203 and the score and variance calls are refused
+ * as after fit_compute.
+ * Errors: 203 invalid or used handle, orthogonal solver, unknown family, max_iter < 1, tol < 0 or NaN, nout < 7,
+ * l1x < ndim, or any y_i outside its family's domain (or not finite) where w_i > 0 -- checked on the device before the
+ * first assembly, after which the handle is still fresh; 104 ncf < ncol; 105 n < 1 or m = 0; 107 as above, or a
+ * non-positive pivot (coef then holds the last successful iterate); 204 the host entry cannot allocate its device
+ * copies (it copies the points once for the whole call).
+ * Multi-GPU: nccl_comm NULL means one GPU; otherwise every rank passes its shard and the call all-reduces, on the
+ * handle's stream, the domain-check counts, the partial buffer after the first assembly, [S | g] after each
+ * re-assembly, {D, X^2} of each evaluation and the right-hand side of the refinement steps: every rank makes the same
+ * halving and stopping decisions and the replicas stay bit-identical.
+ * All reductions are fixed-order per-CTA partial sums (no FP64 atomics): with SPLPAK_B200_DETERMINISTIC=1 repeated calls
+ * and the host and device entries return bit-identical coef, mu and out.  REAL32: float I/O (and float z and row
+ * weights for its assembly), FP64 everything else. */
+#define SPLPAK_GLM_POISSON  0
+#define SPLPAK_GLM_BINOMIAL 1
+#define SPLPAK_GLM_GAMMA    2
+int splpak_b200_fit_glm_device(splpak_b200_fit_t h, const splpak_real *d_x, int l1x, const splpak_real *d_y,
+                               const splpak_real *d_w, int weighted, const splpak_real *d_offset, int64_t n, int family,
+                               int max_iter, double tol, void *nccl_comm, splpak_real *d_coef, int64_t ncf,
+                               splpak_real *d_mu, double *out, int nout, int *ierror);
+/* Same with HOST x, y, w, offset, coef and mu. */
+int splpak_b200_fit_glm(splpak_b200_fit_t h, const splpak_real *x, int l1x, const splpak_real *y, const splpak_real *w,
+                        int weighted, const splpak_real *offset, int64_t n, int family, int max_iter, double tol,
+                        void *nccl_comm, splpak_real *coef, int64_t ncf, splpak_real *mu, double *out, int nout,
+                        int *ierror);
 /* Parity-test hook of the orthogonal path: which = 0 -> per-window triangles [nwindows][4^ndim][4^ndim + 1] (R_w | z_w),
  * which = 1 -> band factor [ncol][b + 2] (row i: R[i][i..i+b], then (Q^T r)_i).  out may be NULL to query *count. */
 int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity, int64_t *count);

@@ -59,6 +59,8 @@ SYMBOLS = [
     "splpak_b200_fit_select_smoothing_reml",
     "splpak_b200_fit_robust_device",
     "splpak_b200_fit_robust",
+    "splpak_b200_fit_glm_device",
+    "splpak_b200_fit_glm",
     "splpak_b200_fit_prepare_variance",
     "splpak_b200_fit_variance",
     "splpak_b200_fit_variance_device",
@@ -169,6 +171,10 @@ def load(real32: bool = False) -> C.CDLL:
                                                     C.c_double, vp, vp, i64, vp, vp, C.c_int, ip]),
         "splpak_b200_fit_robust": (C.c_int, [vp, vp, C.c_int, vp, vp, C.c_int, i64, C.c_int, C.c_double, C.c_int,
                                              C.c_double, vp, vp, i64, vp, vp, C.c_int, ip]),
+        "splpak_b200_fit_glm_device": (C.c_int, [vp, vp, C.c_int, vp, vp, C.c_int, vp, i64, C.c_int, C.c_int, C.c_double,
+                                                 vp, vp, i64, vp, vp, C.c_int, ip]),
+        "splpak_b200_fit_glm": (C.c_int, [vp, vp, C.c_int, vp, vp, C.c_int, vp, i64, C.c_int, C.c_int, C.c_double, vp,
+                                          vp, i64, vp, vp, C.c_int, ip]),
         "splpak_b200_fit_prepare_variance": (C.c_int, [vp, vp, C.c_int, ip]),
         "splpak_b200_fit_variance": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, ip]),
         "splpak_b200_fit_variance_device": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, vp, ip]),

@@ -488,6 +488,64 @@ class FitHandle:
                                                C.byref(ierr))
         return self._robust_info(out), ierr.value
 
+    FAMILY = {"poisson": 0, "binomial": 1, "gamma": 2}
+    _GLM_KEYS = ("iterations", "deviance", "pearson", "change", "halvings", "converged", "m")
+
+    def _family_code(self, family):
+        if family not in self.FAMILY:
+            raise SplpakError(f"unknown family {family!r}: expected one of {sorted(self.FAMILY)}")
+        return self.FAMILY[family]
+
+    def _glm_info(self, out):
+        info = dict(zip(self._GLM_KEYS, (float(v) for v in out)))
+        for k in ("iterations", "halvings", "m"):
+            info[k] = int(info[k])
+        info["converged"] = bool(info["converged"])
+        return info
+
+    def glm_fit(self, x, y, w=None, family="poisson", offset=None, max_iter=25, tol=1e-8, return_mu=False):
+        """Generalized smoothing fit of HOST points on a fresh (or reset) handle by penalized IRLS: Poisson (log link),
+        binomial (logit; y a proportion, w = sqrt(trials)) or Gamma (log) responses, eta = s(x) + offset (header:
+        splpak_b200_fit_glm_device).  Returns (coef, info, ierror), info = {iterations, deviance, pearson, change,
+        halvings, converged, m} and, with return_mu, "mu": the fitted means at the points.  An unknown family name
+        raises SplpakError."""
+        code = self._family_code(family)
+        self._check()
+        xa = np.ascontiguousarray(x, dtype=self.dt)
+        if xa.ndim == 1:
+            xa = xa.reshape(-1, 1)
+        n = xa.shape[0]
+        ya = _vec(y, self.dt, n)
+        wa = _vec(w, self.dt, n) if w is not None else None
+        oa = _vec(offset, self.dt, n) if offset is not None else None
+        coef = np.zeros(self.ncol, dtype=self.dt)
+        mu = np.zeros(max(n, 1), dtype=self.dt) if return_mu else None
+        out = np.zeros(7)
+        ierr = C.c_int(0)
+        self.lib.splpak_b200_fit_glm(self.h, _ptr(xa), xa.shape[1], _ptr(ya), _ptr(wa) if wa is not None else None,
+                                     int(wa is not None), _ptr(oa) if oa is not None else None, n, code,
+                                     int(max_iter), float(tol), None, _ptr(coef), self.ncol,
+                                     _ptr(mu) if mu is not None else None, _ptr(out), 7, C.byref(ierr))
+        info = self._glm_info(out)
+        if return_mu:
+            info["mu"] = mu[:n]
+        return coef, info, ierr.value
+
+    def glm_fit_device(self, d_x, l1x, d_y, d_w, n, d_coef, family="poisson", d_offset=None, max_iter=25, tol=1e-8,
+                       d_mu=None, comm=None):
+        """glm_fit with torch CUDA tensors or raw device pointers (d_w None: all weights 1; d_offset None: no offset;
+        d_mu None: no fitted means returned).  comm: a raw ncclComm_t (splpak_b200_comm_*) when every rank passes its
+        shard, None on one GPU.  Returns (info, ierror)."""
+        code = self._family_code(family)
+        self._check()
+        out = np.zeros(7)
+        ierr = C.c_int(0)
+        self.lib.splpak_b200_fit_glm_device(self.h, _dev_ptr(d_x), int(l1x), _dev_ptr(d_y), _dev_ptr(d_w),
+                                            int(d_w is not None), _dev_ptr(d_offset), int(n), code, int(max_iter),
+                                            float(tol), comm, _dev_ptr(d_coef), self.ncol, _dev_ptr(d_mu), _ptr(out), 7,
+                                            C.byref(ierr))
+        return self._glm_info(out), ierr.value
+
     def variance(self, x, nderiv=None):
         """q(x) = b(x)^T Sigma b(x) at HOST points x (nq, l1x), after prepare_variance: the posterior variance of the
         fitted value (nderiv: of that partial derivative) divided by sigma2.  Returns (q[nq], ierror)."""

@@ -105,6 +105,13 @@ int spl_robust_select_launch(const RobustScratch &rs, int pass, cudaStream_t st)
 int spl_robust_weight_launch(const RobustScratch &rs, const real_t *d_w, int weighted, int psi, double c, int unit,
                              real_t *d_u, cudaStream_t st, int nsm);
 int spl_robust_change_launch(const RobustScratch &rs, const double *d_c, long long ncol, cudaStream_t st);
+int spl_glm_scratch_init(GlmScratch &gs, long long n, long long ncol, int nsm);
+void spl_glm_scratch_free(GlmScratch &gs);
+int spl_glm_check_launch(const GlmScratch &gs, int family, const real_t *d_y, const real_t *d_w, int weighted,
+                         cudaStream_t st, int nsm);
+int spl_glm_work_launch(const GlmScratch &gs, int family, int start, const real_t *d_y, const real_t *d_w, int weighted,
+                        const real_t *d_o, real_t *d_mu, cudaStream_t st);
+int spl_glm_halve_launch(const GlmScratch &gs, double *d_c, long long ncol, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------
 // small conversion kernels
@@ -956,7 +963,8 @@ struct splpak_b200_fit_s {
     real_t *d_out_tmp;            // ncol reals: working-precision copy of the solution for the D2H of real32 builds
     int refining;
     int constraints_fired;        // derivative-constraint rows were added by compute
-    int robust;                   // the fit was a robust fit: refine_begin would re-feed the caller's weights, so it refuses
+    int irls;                     // the fit was a robust or GLM fit: refine_begin would re-feed the caller's data, so it
+                                  // refuses
     // smoothing (penalty.cu): lambda * R is added to S by compute when lambda > 0; kept across fit_reset
     double lambda;
     int penalty;                  // SPLPAK_PENALTY_CURVATURE or SPLPAK_PENALTY_THIN_PLATE
@@ -1107,7 +1115,7 @@ extern "C" int splpak_b200_fit_reset(splpak_b200_fit_t h) {
     h->finalized = 0;
     h->timers_pending = 0;
     h->total_points = 0;
-    h->solved = h->refining = h->constraints_fired = h->factor_valid = h->robust = 0;
+    h->solved = h->refining = h->constraints_fired = h->factor_valid = h->irls = 0;
     h->s1_valid = h->sigma_valid = h->var_valid = 0;
     h->cond_est = 0.0;
     if (h->os) return spl_ortho_reset(h->gp, *h->os, h->st);
@@ -1507,7 +1515,7 @@ extern "C" int splpak_b200_fit_compute_device(splpak_b200_fit_t h, real_t *d_coe
 // recovers the accuracy of the orthogonal method as long as eps*cond(G) < 1.
 // ------------------------------------------------------------------------------------------
 extern "C" int splpak_b200_fit_refine_begin(splpak_b200_fit_t h) {
-    if (!valid(h) || !h->finalized || !h->solved || h->robust) return SPLPAK_ERR_HANDLE;
+    if (!valid(h) || !h->finalized || !h->solved || h->irls) return SPLPAK_ERR_HANDLE;
     if (h->solver == SPLPAK_SOLVER_ORTHOGONAL) return SPLPAK_ERR_HANDLE;   // already at cond(A): nothing to refine
     if (sizeof(real_t) != sizeof(double)) return SPLPAK_OK;            // fp32 I/O: nothing to gain
     SPL_CUDA_TRY(cudaMemsetAsync(h->d_g, 0, sizeof(double) * (size_t)h->gp.ncol, h->st));
@@ -1639,8 +1647,8 @@ static int robust_check(splpak_b200_fit_t h, int l1x, int64_t n, int psi, double
     return SPLPAK_OK;
 }
 
-// s(x_i) of the current solution d_coef64 into rs.s, in the chunks and with the evaluation of the refinement pass
-static int robust_eval(splpak_b200_fit_t h, RobustScratch &rs, const real_t *d_x, int l1x, long long n) {
+// s(x_i) of the current solution d_coef64 into s[n], in the chunks and with the evaluation of the refinement pass
+static int robust_eval(splpak_b200_fit_t h, real_t *s, const real_t *d_x, int l1x, long long n) {
     const real_t *coef = reinterpret_cast<const real_t *>(h->d_coef64);
     if (sizeof(real_t) != sizeof(double)) {
         // the REAL32 library's splfe works in float: the solution rounded to working precision first
@@ -1650,7 +1658,7 @@ static int robust_eval(splpak_b200_fit_t h, RobustScratch &rs, const real_t *d_x
     }
     for (long long i0 = 0; i0 < n; i0 += DEVICE_CHUNK) {
         const long long nc = (n - i0 < DEVICE_CHUNK) ? n - i0 : DEVICE_CHUNK;
-        const int rc = eval_device_impl(h->gp, h->di, nullptr, 0, d_x + i0 * (long long)l1x, l1x, nc, coef, rs.s + i0,
+        const int rc = eval_device_impl(h->gp, h->di, nullptr, 0, d_x + i0 * (long long)l1x, l1x, nc, coef, s + i0,
                                         h->st);
         if (rc != SPLPAK_OK) return rc;
     }
@@ -1669,7 +1677,7 @@ static int robust_scale(splpak_b200_fit_t h, RobustScratch &rs, const real_t *d_
     return rc;
 }
 
-// one chunk of a re-assembly with the robust row weights: S and g only (the histogram and totals stay those of the
+// one chunk of a re-assembly with new row weights (robust or GLM fit): S and g only (the histogram and totals stay those of the
 // first assembly; classify's totals go to the discarded slots, as in the refinement pass)
 static int reassemble_device_chunk(splpak_b200_fit_t h, const real_t *d_x, int l1x, const real_t *d_y,
                                    const real_t *d_w, int weighted, long long n) {
@@ -1693,7 +1701,7 @@ static int robust_run(splpak_b200_fit_t h, RobustScratch &rs, const real_t *d_x,
     if (rc != SPLPAK_OK) return rc;
     h->total_points += n;
     h->finalized = 1;
-    h->robust = 1;
+    h->irls = 1;
     h->solved = 0;
     rc = robust_allreduce(h, comm, h->d_part, (size_t)h->n_part, NCCL_FLOAT64, NCCL_SUM);
     if (rc != SPLPAK_OK) return rc;
@@ -1706,7 +1714,7 @@ static int robust_run(splpak_b200_fit_t h, RobustScratch &rs, const real_t *d_x,
     bool stats = false;
     const long long nsg = ncol * h->gp.nsten + ncol;          // [S | g] at the start of the partial buffer
     for (int k = 1; k <= max_iter; ++k) {
-        rc = robust_eval(h, rs, d_x, l1x, n);
+        rc = robust_eval(h, rs.s, d_x, l1x, n);
         if (rc == SPLPAK_OK) rc = robust_scale(h, rs, d_y, d_w, weighted, comm);
         if (rc != SPLPAK_OK) return rc;
         double sigma = 0.0;
@@ -1845,6 +1853,222 @@ extern "C" int splpak_b200_fit_robust(splpak_b200_fit_t h, const real_t *x, int 
             rc = SPLPAK_ERR_CUDA;
         }
         for (int a = 0; a < 4; ++a)
+            if (d[a]) cudaFree(d[a]);
+    }
+    if (ierror) *ierror = rc;
+    return rc;
+}
+// ------------------------------------------------------------------------------------------
+// GLM fit: penalized IRLS for Poisson, binomial and Gamma responses (glm.cu; DESIGN §4.16)
+// ------------------------------------------------------------------------------------------
+#define GLM_MAX_HALVINGS 10                                     // glm.fit's limit
+
+static int glm_check(splpak_b200_fit_t h, int l1x, int64_t n, int family, int max_iter, double tol, int64_t ncf,
+                     const double *out, int nout) {
+    if (!valid(h) || h->finalized || h->total_points != 0 || h->solver != SPLPAK_SOLVER_CHOLESKY) return SPLPAK_ERR_HANDLE;
+    if (family != SPLPAK_GLM_POISSON && family != SPLPAK_GLM_BINOMIAL && family != SPLPAK_GLM_GAMMA)
+        return SPLPAK_ERR_HANDLE;
+    if (max_iter < 1 || !(tol >= 0.0) || !out || nout < 7 || l1x < h->gp.ndim) return SPLPAK_ERR_HANDLE;
+    if (h->gp.ncol > ncf) return SPLPAK_ERR_NCF;
+    if (n < 1) return SPLPAK_ERR_NDATA;
+    return SPLPAK_OK;
+}
+
+// the caller's device arrays of one GLM call (o and mu may be null)
+struct GlmData {
+    const real_t *x;
+    int l1x;
+    const real_t *y, *w;
+    int weighted;
+    const real_t *o;
+    long long n;
+    int family;
+    real_t *mu;
+};
+
+// One evaluation: s(x_i) of d_coef64 (start: mu0 instead), then z, row weights, mu and dev = {D, X^2}, all-reduced and
+// read back (one synchronisation)
+static int glm_eval(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int start, void *comm, double dev[2]) {
+    int rc = start ? SPLPAK_OK : robust_eval(h, gs.s, d.x, d.l1x, d.n);
+    if (rc == SPLPAK_OK) rc = spl_glm_work_launch(gs, d.family, start, d.y, d.w, d.weighted, d.o, d.mu, h->st);
+    if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, gs.dev, 2, NCCL_FLOAT64, NCCL_SUM);
+    if (rc != SPLPAK_OK) return rc;
+    SPL_CUDA_TRY(cudaMemcpyAsync(dev, gs.dev, sizeof(double) * 2, cudaMemcpyDeviceToHost, h->st));
+    SPL_CUDA_TRY(cudaStreamSynchronize(h->st));
+    return SPLPAK_OK;
+}
+
+// The loop of splpak_b200_fit_glm_device (semantics: the header).  res = out[0..6]; on 107 the caller's coef holds the
+// last iterate with a finite deviance (c^1 when the first has none).
+static int glm_run(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int max_iter, double tol, void *comm,
+                   real_t *coef, int coef_on_device, double res[7]) {
+    cudaStream_t st = h->st;
+    const long long ncol = h->gp.ncol;
+    const size_t cbytes = sizeof(double) * (size_t)ncol;
+    // the domain check and m, before anything touches the handle: a refused call leaves it fresh
+    int rc = spl_glm_check_launch(gs, d.family, d.y, d.w, d.weighted, st, h->di.nsm);
+    if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, gs.count, 2, NCCL_UINT64, NCCL_SUM);
+    if (rc != SPLPAK_OK) return rc;
+    unsigned long long cnt[2] = {0, 0};
+    SPL_CUDA_TRY(cudaMemcpyAsync(cnt, gs.count, sizeof(cnt), cudaMemcpyDeviceToHost, st));
+    SPL_CUDA_TRY(cudaStreamSynchronize(st));
+    res[6] = (double)cnt[1];
+    if (cnt[0]) return SPLPAK_ERR_HANDLE;
+    if (cnt[1] == 0) return SPLPAK_ERR_NDATA;
+    long long band_elems = 0, need = 0;
+    rc = ensure_band(h, &band_elems, &need);
+    // z and W of mu0 (and D_0), then the first assembly with them: its node histogram and totals stay for the call
+    double dev[2] = {0.0, 0.0};
+    if (rc == SPLPAK_OK) rc = glm_eval(h, gs, d, 1, comm, dev);
+    if (rc == SPLPAK_OK) rc = feed_device(h, d.x, d.l1x, gs.z, gs.rw, 1, d.n, add_device_chunk);
+    if (rc != SPLPAK_OK) return rc;
+    h->total_points += d.n;
+    h->finalized = 1;
+    h->irls = 1;
+    h->solved = 0;
+    rc = robust_allreduce(h, comm, h->d_part, (size_t)h->n_part, NCCL_FLOAT64, NCCL_SUM);
+    if (rc != SPLPAK_OK) return rc;
+    SPL_CUDA_TRY(cudaMemcpyAsync(gs.tot0, h->d_totals, sizeof(double) * 2, cudaMemcpyDeviceToDevice, st));
+    res[1] = dev[0];
+    res[2] = dev[1];
+    double dold = dev[0];
+    bool halved = false;                                      // the last iteration halved its step
+    const long long nsg = ncol * h->gp.nsten + ncol;          // [S | g] at the start of the partial buffer
+    int k = 1;
+    for (; k <= max_iter; ++k) {
+        if (k > 1) {
+            SPL_CUDA_TRY(cudaMemcpyAsync(gs.cprev, h->d_coef64, cbytes, cudaMemcpyDeviceToDevice, st));
+            SPL_CUDA_TRY(cudaMemsetAsync(h->d_part, 0, sizeof(double) * (size_t)nsg, st));
+            rc = feed_device(h, d.x, d.l1x, gs.z, gs.rw, 1, d.n, reassemble_device_chunk);
+            if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, h->d_part, (size_t)nsg, NCCL_FLOAT64, NCCL_SUM);
+            if (rc != SPLPAK_OK) return rc;
+            SPL_CUDA_TRY(cudaMemcpyAsync(h->d_totals, gs.tot0, sizeof(double) * 2, cudaMemcpyDeviceToDevice, st));
+        }
+        rc = compute_cholesky(h, coef, coef_on_device, band_elems, need);
+        if (rc == SPLPAK_ERR_SOLVER && k > 1) {
+            // the last successful iterate back to the caller; out and mu already describe it
+            SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cprev, cbytes, cudaMemcpyDeviceToDevice, st));
+            rc = write_coef(h, h->d_coef64, coef, coef_on_device);
+            return rc == SPLPAK_OK ? SPLPAK_ERR_SOLVER : rc;
+        }
+        if (rc != SPLPAK_OK) return rc;
+        res[0] = k;
+        rc = glm_eval(h, gs, d, 0, comm, dev);
+        int nh = 0;
+        for (; rc == SPLPAK_OK && !isfinite(dev[0]) && k > 1 && nh < GLM_MAX_HALVINGS; ++nh) {
+            rc = spl_glm_halve_launch(gs, h->d_coef64, ncol, st);
+            if (rc == SPLPAK_OK) rc = glm_eval(h, gs, d, 0, comm, dev);
+        }
+        res[4] += nh;
+        if (rc != SPLPAK_OK) return rc;
+        halved = nh > 0;
+        if (!isfinite(dev[0])) {
+            // no finite deviance: keep c^1 at k = 1, else go back to c^(k-1) and evaluate it again for out and mu
+            if (k > 1) {
+                SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cprev, cbytes, cudaMemcpyDeviceToDevice, st));
+                rc = glm_eval(h, gs, d, 0, comm, dev);
+            }
+            res[1] = dev[0];
+            res[2] = dev[1];
+            if (rc == SPLPAK_OK) rc = write_coef(h, h->d_coef64, coef, coef_on_device);
+            return rc == SPLPAK_OK ? SPLPAK_ERR_SOLVER : rc;
+        }
+        res[1] = dev[0];
+        res[2] = dev[1];
+        res[3] = fabs(dev[0] - dold) / (fabs(dev[0]) + 0.1);
+        dold = dev[0];
+        if (res[3] < tol) {
+            res[5] = 1.0;
+            break;
+        }
+    }
+    if (k > max_iter) k = max_iter;
+    // The refinement steps of splcw refine the last solve, so they need its z and row weights (the evaluation since has
+    // overwritten them: they come back from c^(k-1), or mu0) and its full step (skipped after a halving)
+    if (sizeof(real_t) == sizeof(double) && h->constraints_fired && !halved) {
+        SPL_CUDA_TRY(cudaMemcpyAsync(gs.cfin, h->d_coef64, cbytes, cudaMemcpyDeviceToDevice, st));
+        if (k > 1) SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cprev, cbytes, cudaMemcpyDeviceToDevice, st));
+        rc = glm_eval(h, gs, d, k == 1, comm, dev);
+        if (rc != SPLPAK_OK) return rc;
+        SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cfin, cbytes, cudaMemcpyDeviceToDevice, st));
+        for (int step = 0; step < SPLPAK_REFINE_STEPS && rc == SPLPAK_OK; ++step) {
+            SPL_CUDA_TRY(cudaMemsetAsync(h->d_g, 0, cbytes, st));
+            rc = feed_device(h, d.x, d.l1x, gs.z, gs.rw, 1, d.n, refine_device_chunk);
+            if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, h->d_g, (size_t)ncol, NCCL_FLOAT64, NCCL_SUM);
+            if (rc == SPLPAK_OK) rc = refine_solve(h, coef, coef_on_device);
+        }
+        // the final evaluation: out and mu describe the refined coefficients
+        if (rc == SPLPAK_OK) rc = glm_eval(h, gs, d, 0, comm, dev);
+        res[1] = dev[0];
+        res[2] = dev[1];
+        return rc;
+    }
+    return write_coef(h, h->d_coef64, coef, coef_on_device);
+}
+
+static int fit_glm_impl(splpak_b200_fit_t h, const GlmData &d, int max_iter, double tol, void *comm, real_t *coef,
+                        int coef_on_device, double *out) {
+    double res[7] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    GlmScratch gs;
+    int rc = spl_glm_scratch_init(gs, d.n, h->gp.ncol, h->di.nsm);
+    if (rc == SPLPAK_OK) {
+        rc = glm_run(h, gs, d, max_iter, tol, comm, coef, coef_on_device, res);
+        if (cudaStreamSynchronize(h->st) != cudaSuccess) {
+            cudaGetLastError();
+            if (rc == SPLPAK_OK) rc = SPLPAK_ERR_CUDA;
+        }
+        spl_glm_scratch_free(gs);
+    }
+    memcpy(out, res, sizeof(res));
+    return rc;
+}
+
+extern "C" int splpak_b200_fit_glm_device(splpak_b200_fit_t h, const real_t *d_x, int l1x, const real_t *d_y,
+                                          const real_t *d_w, int weighted, const real_t *d_offset, int64_t n,
+                                          int family, int max_iter, double tol, void *nccl_comm, real_t *d_coef,
+                                          int64_t ncf, real_t *d_mu, double *out, int nout, int *ierror) {
+    int rc = glm_check(h, l1x, n, family, max_iter, tol, ncf, out, nout);
+    if (!d_w) weighted = 0;
+    if (rc == SPLPAK_OK)
+        rc = fit_glm_impl(h, GlmData{d_x, l1x, d_y, d_w, weighted, d_offset, n, family, d_mu}, max_iter, tol, nccl_comm,
+                          d_coef, 1, out);
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+// HOST arrays: the points go to device buffers once for the whole call (through the pinned staging of spl_h2d)
+extern "C" int splpak_b200_fit_glm(splpak_b200_fit_t h, const real_t *x, int l1x, const real_t *y, const real_t *w,
+                                   int weighted, const real_t *offset, int64_t n, int family, int max_iter, double tol,
+                                   void *nccl_comm, real_t *coef, int64_t ncf, real_t *mu, double *out, int nout,
+                                   int *ierror) {
+    int rc = glm_check(h, l1x, n, family, max_iter, tol, ncf, out, nout);
+    if (!w) weighted = 0;
+    real_t *d[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};          // x, y, w, offset, mu
+    if (rc == SPLPAK_OK) {
+        const size_t len[5] = {(size_t)n * (size_t)l1x, (size_t)n, weighted ? (size_t)n : 0, offset ? (size_t)n : 0,
+                               mu ? (size_t)n : 0};
+        for (int a = 0; a < 5 && rc == SPLPAK_OK; ++a)
+            if (len[a] && cudaMalloc((void **)&d[a], sizeof(real_t) * len[a]) != cudaSuccess) {
+                cudaGetLastError();
+                d[a] = nullptr;
+                rc = SPLPAK_ERR_ALLOC;
+            }
+        const real_t *src[4] = {x, y, w, offset};
+        for (int a = 0; a < 4 && rc == SPLPAK_OK; ++a)
+            if (len[a] && spl_h2d(d[a], src[a], sizeof(real_t) * len[a], h->st, h->di.dev) != cudaSuccess) {
+                cudaGetLastError();
+                rc = SPLPAK_ERR_CUDA;
+            }
+        if (rc == SPLPAK_OK)
+            rc = fit_glm_impl(h, GlmData{d[0], l1x, d[1], d[2], weighted, d[3], n, family, d[4]}, max_iter, tol,
+                              nccl_comm, coef, 0, out);
+        if (mu && (rc == SPLPAK_OK || rc == SPLPAK_ERR_SOLVER) &&
+            (spl_d2h(mu, d[4], sizeof(real_t) * (size_t)n, h->st, h->di.dev) != cudaSuccess ||
+             spl_d2h_flush(h->di.dev) != cudaSuccess || cudaStreamSynchronize(h->st) != cudaSuccess)) {
+            cudaGetLastError();
+            rc = SPLPAK_ERR_CUDA;
+        }
+        for (int a = 0; a < 5; ++a)
             if (d[a]) cudaFree(d[a]);
     }
     if (ierror) *ierror = rc;

@@ -157,6 +157,18 @@ struct RobustScratch {
     double *small, *cprev, *change, *stats, *tot0, *part;
 };
 
+// Scratch of one GLM fit call (glm.cu): per point the spline values, the working response and the row weights; the
+// domain-check counts, the previous and the final coefficients, the deviance and the working kernel's partial sums.
+struct GlmScratch {
+    long long n;
+    int nparts;                           // CTAs of the working kernel (one pair of partial sums each)
+    real_t *s;                            // n: s(x_i) of the coefficients being evaluated
+    real_t *z, *rw;                       // n: working response z_i and row weight sqrt(W_i) of the next assembly
+    unsigned long long *count;            // {y outside the family's domain where w > 0, m = points with w > 0}
+    // one allocation: [cprev (ncol) | cfin (ncol) | dev {D, X^2} | tot0 | part (2 nparts)]; tot0 as in RobustScratch
+    double *small, *cprev, *cfin, *dev, *tot0, *part;
+};
+
 extern unsigned long long g_spl_launches;   // host-side launch counter (capi.cu)
 
 #define SPL_CUDA_TRY(expr)                                                              \
