@@ -69,6 +69,7 @@
         procedure,public :: select_smoothing_reml        !! (new) streaming fit: lambda minimising the REML score, set on the fit
         procedure,public :: robust_fit                   !! (new) streaming fit: iteratively reweighted Huber / bisquare fit
         procedure,public :: glm_fit                      !! (new) streaming fit: penalized IRLS, Poisson / binomial / Gamma response
+        procedure,public :: glm_select                   !! (new) streaming fit: glm_fit with lambda chosen by REML or UBRE / GCV
         procedure,public :: prepare_variance             !! (new) streaming fit: tables of the posterior variances (before compute)
         procedure,public :: variance                     !! (new) streaming fit: b(x)^T Sigma b(x) at a batch of points
         procedure,private :: splcc
@@ -287,6 +288,21 @@
             integer(c_int),intent(out) :: ierror
             integer(c_int) :: rc
         end function c_fit_glm
+        function c_fit_glm_select(h,x,l1x,y,w,weighted,offset,n,family,criterion,penalty,lambda_lo,lambda_hi, &
+                                  max_select,variance,max_iter,tol,comm,coef,ncf,mu,out,nout,trace,trace_cap,ntrace, &
+                                  ierror) bind(C,name='splpak_b200_fit_glm_select') result(rc)
+            import :: c_int, c_int64_t, c_double, c_ptr, cwp
+            type(c_ptr),value :: h, offset, comm, mu, trace
+            real(cwp),intent(in) :: x(*), y(*), w(*)
+            integer(c_int),value :: l1x, weighted, family, criterion, penalty, max_select, variance, max_iter, nout
+            integer(c_int64_t),value :: n, ncf, trace_cap
+            real(c_double),value :: lambda_lo, lambda_hi, tol
+            real(cwp) :: coef(*)
+            real(c_double),intent(out) :: out(*)
+            integer(c_int64_t),intent(out) :: ntrace
+            integer(c_int),intent(out) :: ierror
+            integer(c_int) :: rc
+        end function c_fit_glm_select
         function c_fit_prepare_variance(h,out,nout,ierror) bind(C,name='splpak_b200_fit_prepare_variance') result(rc)
             import :: c_int, c_double, c_ptr
             type(c_ptr),value :: h
@@ -687,6 +703,60 @@
         ierror = int(rc)
         call cfaerr(ierror,.false.)
     end subroutine glm_fit
+
+    !> (new) glm_fit with lambda chosen on each working system: criterion 0 = REML, 1 = UBRE (Poisson, binomial) /
+    !! GCV (Gamma); lambda_lo or lambda_hi <= 0 => rho * [1e-10, 1e4].  info(1:13) = glm_fit's seven, then lambda,
+    !! the criterion, edf, scale, selecting iterations, settled.  trace(5, :) (optional): one column per iteration,
+    !! [lambda, criterion, scores, deviance, halvings]; ntrace = columns written.  variance /= 0 builds the tables of
+    !! the variance calls.
+    subroutine glm_select(me,xdata,l1xdat,ydata,ndata,family,criterion,penalty,lambda_lo,lambda_hi,max_select,variance, &
+                          max_iter,tol,coef,ncf,info,ierror,wdata,offset,mu,trace,ntrace)
+        class(splpak_type),intent(inout) :: me
+        integer,intent(in) :: l1xdat, family, criterion, penalty, max_select, variance, max_iter, ncf
+        integer(int64),intent(in) :: ndata
+        real(wp),intent(in) :: xdata(l1xdat,ndata), ydata(ndata)
+        real(c_double),intent(in) :: lambda_lo, lambda_hi, tol
+        real(wp),intent(out) :: coef(ncf)
+        real(c_double),intent(out) :: info(13)
+        integer,intent(out) :: ierror
+        real(wp),intent(in),optional :: wdata(ndata)
+        real(wp),intent(in),optional,target :: offset(ndata)
+        real(wp),intent(out),optional,target :: mu(ndata)
+        real(c_double),intent(out),optional,target,contiguous :: trace(:,:)
+        integer(int64),intent(out),optional :: ntrace
+        integer(c_int) :: weighted, rc, ie
+        integer(c_int64_t) :: cap, nt
+        real(wp) :: dummy(1)
+        type(c_ptr) :: po, pm, pt
+        po = c_null_ptr
+        pm = c_null_ptr
+        pt = c_null_ptr
+        cap = 0
+        if (present(offset)) po = c_loc(offset)
+        if (present(mu)) pm = c_loc(mu)
+        if (present(trace)) then
+            if (size(trace,1) /= 5) error stop 'glm_select: trace must be (5, cap)'
+            pt = c_loc(trace)
+            cap = int(size(trace,2),c_int64_t)
+        end if
+        weighted = 0
+        if (present(wdata)) then
+            if (wdata(1) >= 0.0_wp) weighted = 1
+            rc = c_fit_glm_select(me%handle,xdata,int(l1xdat,c_int),ydata,wdata,weighted,po,int(ndata,c_int64_t), &
+                                  int(family,c_int),int(criterion,c_int),int(penalty,c_int),lambda_lo,lambda_hi, &
+                                  int(max_select,c_int),int(variance,c_int),int(max_iter,c_int),tol,c_null_ptr, &
+                                  coef,int(ncf,c_int64_t),pm,info,13_c_int,pt,cap,nt,ie)
+        else
+            dummy = -1.0_wp
+            rc = c_fit_glm_select(me%handle,xdata,int(l1xdat,c_int),ydata,dummy,weighted,po,int(ndata,c_int64_t), &
+                                  int(family,c_int),int(criterion,c_int),int(penalty,c_int),lambda_lo,lambda_hi, &
+                                  int(max_select,c_int),int(variance,c_int),int(max_iter,c_int),tol,c_null_ptr, &
+                                  coef,int(ncf,c_int64_t),pm,info,13_c_int,pt,cap,nt,ie)
+        end if
+        if (present(ntrace)) ntrace = int(nt,int64)
+        ierror = int(rc)
+        call cfaerr(ierror,.false.)
+    end subroutine glm_select
 
     !> (new) accumulate n more points; wdata absent (or wdata(1)<0) => all weights 1.
     subroutine add_points(me,xdata,l1xdat,ydata,ndata,ierror,wdata)

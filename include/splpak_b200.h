@@ -386,7 +386,7 @@ int splpak_b200_fit_robust(splpak_b200_fit_t h, const splpak_real *x, int l1x, c
  * copies (it copies the points once for the whole call).
  * Multi-GPU: nccl_comm NULL means one GPU; otherwise every rank passes its shard and the call all-reduces, on the
  * handle's stream, the domain-check counts, the partial buffer after the first assembly, [S | g] after each
- * re-assembly, {D, X^2} of each evaluation and the right-hand side of the refinement steps: every rank makes the same
+ * re-assembly, {D, X^2, ywy} of each evaluation and the right-hand side of the refinement steps: every rank makes the same
  * halving and stopping decisions and the replicas stay bit-identical.
  * All reductions are fixed-order per-CTA partial sums (no FP64 atomics): with SPLPAK_B200_DETERMINISTIC=1 repeated calls
  * and the host and device entries return bit-identical coef, mu and out.  REAL32: float I/O (and float z and row
@@ -403,6 +403,62 @@ int splpak_b200_fit_glm(splpak_b200_fit_t h, const splpak_real *x, int l1x, cons
                         int weighted, const splpak_real *offset, int64_t n, int family, int max_iter, double tol,
                         void *nccl_comm, splpak_real *coef, int64_t ncf, splpak_real *mu, double *out, int nout,
                         int *ierror);
+/* GLM fit with the smoothing parameter chosen on each PIRLS working system ("performance iteration") -- (new).
+ * Everything fit_glm_device says holds (data, families, working values, deviance, halving, stopping, the fixed node
+ * histogram and totals, refinement, multi-GPU, determinism), except that lambda is chosen inside the loop.
+ *   working system    iteration k assembles S_k, g_k from z and sqrt(W), and ywy_k = sum (sqrt(W_i) z_i)^2;
+ *                     M(lambda) = G0_k + C + lambda R with the given penalty.
+ *   criterion         the scores of smoothing_score / reml_score on that system (same quantities and counting: REML
+ *                     counts the constraint rows as observations, GCV / UBRE count them as part of the regulariser),
+ *                     the family deciding whether the scale is known:
+ *                                     Poisson, binomial (phi = 1)              Gamma (phi unknown)
+ *                       REML          V = D_p + log|M| - (p - Mp) log lambda   the profiled V_R of reml_score
+ *                       PREDICTION    UBRE U = RSS / N - 1 + 2 edf / N          GCV V = N RSS / (N - edf)^2
+ *   phase 1 (selecting)  k = 1: the search of select_smoothing over [lambda_lo, lambda_hi] (either <= 0: rho [1e-10,
+ *                     1e4] with rho from the first working system): a grid at 2 points per decade, golden section to
+ *                     0.02 decades, ties to the larger lambda.  k >= 2: the same search over log10 lambda_(k-1) +- 1
+ *                     decade clipped to the range, repeated over the whole range when its best grid point is an end of
+ *                     the window but not of the range.  Points with a non-positive pivot count as +inf (107 when all
+ *                     of a search do).  lambda_k then goes on the handle and the iteration solves with it.
+ *   phase 2           phase 1 ends at the first k >= 2 with |log10 lambda_k - log10 lambda_(k-1)| <= 0.05 (settled), or
+ *                     after max_select selecting iterations (not settled).  lambda-hat = lambda_k is then frozen and the
+ *                     loop continues as fit_glm's fixed-lambda PIRLS; `converged` needs a fixed-lambda iteration to
+ *                     meet the stopping rule.  max_iter counts all solves (tol = 0, max_iter = k: iterate k).  A
+ *                     converged, settled result is the fixed-lambda GLM fit at lambda-hat.
+ *   after the loop    the refinement steps (when constraint rows fired); then the system of the last solve is rebuilt
+ *                     (z and sqrt(W) from c^(k-1), or mu0) and one GCV score at lambda-hat gives edf = tr(M^-1 G0) and
+ *                     leaves Sigma = M^-1 in the band storage; with variance = 1 the tables of prepare_variance are
+ *                     built from it, so fit_variance[_device] return q(x) = b(x)^T M^-1 b(x) of the final working
+ *                     system and phi-hat q(x) is the Bayesian variance of eta(x) (mgcv's Vp).  The final evaluation of
+ *                     the returned coefficients fills out and mu.
+ * out[0..6] as fit_glm; out[7..12] = {lambda-hat, the criterion at lambda-hat in the last selecting iteration, edf,
+ * phi-hat, selecting iterations, settled (0/1)}, nout >= 13; phi-hat = 1 (Poisson, binomial) or X^2 / (m - edf) (Gamma;
+ * +inf when m <= edf).  trace (may be NULL): one row per iteration, [lambda_k, the criterion at lambda_k (NaN when
+ * frozen), scores evaluated, D_k, halvings_k], at most trace_cap rows; *ntrace = rows written.
+ * On return the handle's lambda is lambda-hat with the given penalty, GCV is enabled on it (the call enables it on the
+ * fresh handle), and get_cholesky_factor returns 203 (Sigma has overwritten the factor).
+ * Errors: those of fit_glm_device, and 203 for an unknown criterion or penalty, NaN or inf bounds, lambda_lo > lambda_hi
+ * with both > 0, max_select < 1, trace_cap < 0, nout < 13 (a refused call leaves the handle fresh; the domain check
+ * still runs before anything touches it); 204 when the score scratch or the variance tables cannot be allocated (before
+ * the first assembly: the handle stays fresh).
+ * Multi-GPU: every score is computed from the all-reduced system with fixed-order reductions, so every rank takes the
+ * same search path and the replicas stay bit-identical.  With SPLPAK_B200_DETERMINISTIC=1 repeated calls and the host
+ * and device entries return bit-identical coef, mu, out and trace. */
+#define SPLPAK_GLM_SELECT_REML       0
+#define SPLPAK_GLM_SELECT_PREDICTION 1   /* UBRE for Poisson / binomial, GCV for Gamma */
+int splpak_b200_fit_glm_select_device(splpak_b200_fit_t h, const splpak_real *d_x, int l1x, const splpak_real *d_y,
+                                      const splpak_real *d_w, int weighted, const splpak_real *d_offset, int64_t n,
+                                      int family, int criterion, int penalty, double lambda_lo, double lambda_hi,
+                                      int max_select, int variance, int max_iter, double tol, void *nccl_comm,
+                                      splpak_real *d_coef, int64_t ncf, splpak_real *d_mu, double *out, int nout,
+                                      double *trace, int64_t trace_cap, int64_t *ntrace, int *ierror);
+/* Same with HOST x, y, w, offset, coef and mu. */
+int splpak_b200_fit_glm_select(splpak_b200_fit_t h, const splpak_real *x, int l1x, const splpak_real *y,
+                               const splpak_real *w, int weighted, const splpak_real *offset, int64_t n, int family,
+                               int criterion, int penalty, double lambda_lo, double lambda_hi, int max_select,
+                               int variance, int max_iter, double tol, void *nccl_comm, splpak_real *coef, int64_t ncf,
+                               splpak_real *mu, double *out, int nout, double *trace, int64_t trace_cap,
+                               int64_t *ntrace, int *ierror);
 /* Parity-test hook of the orthogonal path: which = 0 -> per-window triangles [nwindows][4^ndim][4^ndim + 1] (R_w | z_w),
  * which = 1 -> band factor [ncol][b + 2] (row i: R[i][i..i+b], then (Q^T r)_i).  out may be NULL to query *count. */
 int splpak_b200_fit_get_orthogonal_factor(splpak_b200_fit_t h, int which, double *out, int64_t capacity, int64_t *count);

@@ -61,6 +61,8 @@ SYMBOLS = [
     "splpak_b200_fit_robust",
     "splpak_b200_fit_glm_device",
     "splpak_b200_fit_glm",
+    "splpak_b200_fit_glm_select_device",
+    "splpak_b200_fit_glm_select",
     "splpak_b200_fit_prepare_variance",
     "splpak_b200_fit_variance",
     "splpak_b200_fit_variance_device",
@@ -175,6 +177,13 @@ def load(real32: bool = False) -> C.CDLL:
                                                  vp, vp, i64, vp, vp, C.c_int, ip]),
         "splpak_b200_fit_glm": (C.c_int, [vp, vp, C.c_int, vp, vp, C.c_int, vp, i64, C.c_int, C.c_int, C.c_double, vp,
                                           vp, i64, vp, vp, C.c_int, ip]),
+        "splpak_b200_fit_glm_select_device": (C.c_int, [vp, vp, C.c_int, vp, vp, C.c_int, vp, i64, C.c_int, C.c_int,
+                                                        C.c_int, C.c_double, C.c_double, C.c_int, C.c_int, C.c_int,
+                                                        C.c_double, vp, vp, i64, vp, vp, C.c_int, vp, i64,
+                                                        C.POINTER(i64), ip]),
+        "splpak_b200_fit_glm_select": (C.c_int, [vp, vp, C.c_int, vp, vp, C.c_int, vp, i64, C.c_int, C.c_int, C.c_int,
+                                                 C.c_double, C.c_double, C.c_int, C.c_int, C.c_int, C.c_double, vp, vp,
+                                                 i64, vp, vp, C.c_int, vp, i64, C.POINTER(i64), ip]),
         "splpak_b200_fit_prepare_variance": (C.c_int, [vp, vp, C.c_int, ip]),
         "splpak_b200_fit_variance": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, ip]),
         "splpak_b200_fit_variance_device": (C.c_int, [vp, vp, C.c_int, i64, ip, vp, vp, ip]),

@@ -546,6 +546,78 @@ class FitHandle:
                                             C.byref(ierr))
         return self._glm_info(out), ierr.value
 
+    GLM_CRITERIA = {"reml": 0, "prediction": 1}
+    _GLM_SELECT_KEYS = ("lam", "score", "edf", "scale", "select_iterations", "settled")
+
+    def _glm_select_args(self, family, criterion, penalty, lo, hi):
+        code = self._family_code(family)
+        if criterion not in self.GLM_CRITERIA:
+            raise SplpakError(f"unknown criterion {criterion!r}: expected one of {sorted(self.GLM_CRITERIA)}")
+        return (code, self.GLM_CRITERIA[criterion], self._penalty_code(penalty), 0.0 if lo is None else float(lo),
+                0.0 if hi is None else float(hi))
+
+    def _glm_select_info(self, out):
+        info = self._glm_info(out[:7])
+        info.update(zip(self._GLM_SELECT_KEYS, (float(v) for v in out[7:13])))
+        info["select_iterations"] = int(info["select_iterations"])
+        info["settled"] = bool(info["settled"])
+        return info
+
+    def glm_select(self, x, y, w=None, family="poisson", offset=None, criterion="reml", penalty="curvature", lo=None,
+                   hi=None, max_select=10, variance=False, max_iter=25, tol=1e-8, return_mu=False, trace_cap=64):
+        """glm_fit with lambda chosen on each PIRLS working system (header: splpak_b200_fit_glm_select_device):
+        criterion "reml" or "prediction" (UBRE for Poisson / binomial, GCV for Gamma) over [lo, hi] (default rho *
+        [1e-10, 1e4]).  With variance=True the variance calls then return q(x) of the final working system; scale * q
+        is the posterior variance of eta(x).  Returns (coef, info, trace, ierror), info = the glm_fit keys plus {lam,
+        score, edf, scale, select_iterations, settled} (and "mu" with return_mu), trace: (k, 5) rows [lambda,
+        criterion (NaN when frozen), scores, deviance, halvings].  Unknown family, criterion or penalty names raise
+        SplpakError."""
+        code, crit, pen, lo, hi = self._glm_select_args(family, criterion, penalty, lo, hi)
+        self._check()
+        xa = np.ascontiguousarray(x, dtype=self.dt)
+        if xa.ndim == 1:
+            xa = xa.reshape(-1, 1)
+        n = xa.shape[0]
+        ya = _vec(y, self.dt, n)
+        wa = _vec(w, self.dt, n) if w is not None else None
+        oa = _vec(offset, self.dt, n) if offset is not None else None
+        coef = np.zeros(self.ncol, dtype=self.dt)
+        mu = np.zeros(max(n, 1), dtype=self.dt) if return_mu else None
+        out = np.zeros(13)
+        trace = np.zeros((max(int(trace_cap), 1), 5))
+        nt = C.c_int64(0)
+        ierr = C.c_int(0)
+        self.lib.splpak_b200_fit_glm_select(self.h, _ptr(xa), xa.shape[1], _ptr(ya),
+                                            _ptr(wa) if wa is not None else None, int(wa is not None),
+                                            _ptr(oa) if oa is not None else None, n, code, crit, pen, lo, hi,
+                                            int(max_select), int(bool(variance)), int(max_iter), float(tol), None,
+                                            _ptr(coef), self.ncol, _ptr(mu) if mu is not None else None, _ptr(out), 13,
+                                            _ptr(trace), int(trace_cap), C.byref(nt), C.byref(ierr))
+        info = self._glm_select_info(out)
+        if return_mu:
+            info["mu"] = mu[:n]
+        return coef, info, trace[: nt.value].copy(), ierr.value
+
+    def glm_select_device(self, d_x, l1x, d_y, d_w, n, d_coef, family="poisson", d_offset=None, criterion="reml",
+                          penalty="curvature", lo=None, hi=None, max_select=10, variance=False, max_iter=25, tol=1e-8,
+                          d_mu=None, trace_cap=64, comm=None):
+        """glm_select with torch CUDA tensors or raw device pointers (d_w None: all weights 1; d_offset None: no offset;
+        d_mu None: no fitted means returned).  comm: a raw ncclComm_t (splpak_b200_comm_*) when every rank passes its
+        shard, None on one GPU.  Returns (info, trace, ierror)."""
+        code, crit, pen, lo, hi = self._glm_select_args(family, criterion, penalty, lo, hi)
+        self._check()
+        out = np.zeros(13)
+        trace = np.zeros((max(int(trace_cap), 1), 5))
+        nt = C.c_int64(0)
+        ierr = C.c_int(0)
+        self.lib.splpak_b200_fit_glm_select_device(self.h, _dev_ptr(d_x), int(l1x), _dev_ptr(d_y), _dev_ptr(d_w),
+                                                   int(d_w is not None), _dev_ptr(d_offset), int(n), code, crit, pen,
+                                                   lo, hi, int(max_select), int(bool(variance)), int(max_iter),
+                                                   float(tol), comm, _dev_ptr(d_coef), self.ncol, _dev_ptr(d_mu),
+                                                   _ptr(out), 13, _ptr(trace), int(trace_cap), C.byref(nt),
+                                                   C.byref(ierr))
+        return self._glm_select_info(out), trace[: nt.value].copy(), ierr.value
+
     def variance(self, x, nderiv=None):
         """q(x) = b(x)^T Sigma b(x) at HOST points x (nq, l1x), after prepare_variance: the posterior variance of the
         fitted value (nderiv: of that partial derivative) divided by sigma2.  Returns (q[nq], ierror)."""

@@ -1886,26 +1886,21 @@ struct GlmData {
     real_t *mu;
 };
 
-// One evaluation: s(x_i) of d_coef64 (start: mu0 instead), then z, row weights, mu and dev = {D, X^2}, all-reduced and
-// read back (one synchronisation)
-static int glm_eval(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int start, void *comm, double dev[2]) {
+// One evaluation: s(x_i) of d_coef64 (start: mu0 instead), then z, row weights, mu and dev = {D, X^2, ywy}, all-reduced
+// and read back (one synchronisation)
+static int glm_eval(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int start, void *comm, double dev[3]) {
     int rc = start ? SPLPAK_OK : robust_eval(h, gs.s, d.x, d.l1x, d.n);
     if (rc == SPLPAK_OK) rc = spl_glm_work_launch(gs, d.family, start, d.y, d.w, d.weighted, d.o, d.mu, h->st);
-    if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, gs.dev, 2, NCCL_FLOAT64, NCCL_SUM);
+    if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, gs.dev, 3, NCCL_FLOAT64, NCCL_SUM);
     if (rc != SPLPAK_OK) return rc;
-    SPL_CUDA_TRY(cudaMemcpyAsync(dev, gs.dev, sizeof(double) * 2, cudaMemcpyDeviceToHost, h->st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(dev, gs.dev, sizeof(double) * 3, cudaMemcpyDeviceToHost, h->st));
     SPL_CUDA_TRY(cudaStreamSynchronize(h->st));
     return SPLPAK_OK;
 }
 
-// The loop of splpak_b200_fit_glm_device (semantics: the header).  res = out[0..6]; on 107 the caller's coef holds the
-// last iterate with a finite deviance (c^1 when the first has none).
-static int glm_run(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int max_iter, double tol, void *comm,
-                   real_t *coef, int coef_on_device, double res[7]) {
+// The domain check and m (res[6]), before anything touches the handle: a refused call leaves it fresh
+static int glm_domain(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, void *comm, double res[7]) {
     cudaStream_t st = h->st;
-    const long long ncol = h->gp.ncol;
-    const size_t cbytes = sizeof(double) * (size_t)ncol;
-    // the domain check and m, before anything touches the handle: a refused call leaves it fresh
     int rc = spl_glm_check_launch(gs, d.family, d.y, d.w, d.weighted, st, h->di.nsm);
     if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, gs.count, 2, NCCL_UINT64, NCCL_SUM);
     if (rc != SPLPAK_OK) return rc;
@@ -1915,11 +1910,21 @@ static int glm_run(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int ma
     res[6] = (double)cnt[1];
     if (cnt[0]) return SPLPAK_ERR_HANDLE;
     if (cnt[1] == 0) return SPLPAK_ERR_NDATA;
-    long long band_elems = 0, need = 0;
-    rc = ensure_band(h, &band_elems, &need);
-    // z and W of mu0 (and D_0), then the first assembly with them: its node histogram and totals stay for the call
-    double dev[2] = {0.0, 0.0};
-    if (rc == SPLPAK_OK) rc = glm_eval(h, gs, d, 1, comm, dev);
+    return SPLPAK_OK;
+}
+
+// The working system's ywy (gs.dev[2] of the evaluation that produced z and the row weights) into the handle's ywy slot
+// after an assembly, and S1 = G0 + C of the score calls stale
+static int glm_assembled(splpak_b200_fit_t h, GlmScratch &gs) {
+    h->s1_valid = 0;
+    if (h->d_ywy)
+        SPL_CUDA_TRY(cudaMemcpyAsync(h->d_ywy, gs.dev + 2, sizeof(double), cudaMemcpyDeviceToDevice, h->st));
+    return SPLPAK_OK;
+}
+
+// z and W of mu0 (and dev of mu0), then the first assembly with them: its node histogram and totals stay for the call
+static int glm_first_assembly(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, void *comm, double dev[3]) {
+    int rc = glm_eval(h, gs, d, 1, comm, dev);
     if (rc == SPLPAK_OK) rc = feed_device(h, d.x, d.l1x, gs.z, gs.rw, 1, d.n, add_device_chunk);
     if (rc != SPLPAK_OK) return rc;
     h->total_points += d.n;
@@ -1928,21 +1933,71 @@ static int glm_run(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int ma
     h->solved = 0;
     rc = robust_allreduce(h, comm, h->d_part, (size_t)h->n_part, NCCL_FLOAT64, NCCL_SUM);
     if (rc != SPLPAK_OK) return rc;
-    SPL_CUDA_TRY(cudaMemcpyAsync(gs.tot0, h->d_totals, sizeof(double) * 2, cudaMemcpyDeviceToDevice, st));
+    SPL_CUDA_TRY(cudaMemcpyAsync(gs.tot0, h->d_totals, sizeof(double) * 2, cudaMemcpyDeviceToDevice, h->st));
+    return glm_assembled(h, gs);
+}
+
+// [S | g] again from gs.z and gs.rw, all-reduced, with the totals of the first assembly restored
+static int glm_reassemble(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, void *comm) {
+    const long long nsg = h->gp.ncol * h->gp.nsten + h->gp.ncol;   // [S | g] at the start of the partial buffer
+    SPL_CUDA_TRY(cudaMemsetAsync(h->d_part, 0, sizeof(double) * (size_t)nsg, h->st));
+    int rc = feed_device(h, d.x, d.l1x, gs.z, gs.rw, 1, d.n, reassemble_device_chunk);
+    if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, h->d_part, (size_t)nsg, NCCL_FLOAT64, NCCL_SUM);
+    if (rc != SPLPAK_OK) return rc;
+    SPL_CUDA_TRY(cudaMemcpyAsync(h->d_totals, gs.tot0, sizeof(double) * 2, cudaMemcpyDeviceToDevice, h->st));
+    return glm_assembled(h, gs);
+}
+
+// z and the row weights of the last solve (iteration k) back into gs: the evaluations since have overwritten them, so
+// they come again from c^(k-1), or from mu0 at k = 1.  d_coef64 is unchanged; gs.cfin holds a copy of it.
+static int glm_last_system(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int k, void *comm, double dev[3]) {
+    const size_t cbytes = sizeof(double) * (size_t)h->gp.ncol;
+    SPL_CUDA_TRY(cudaMemcpyAsync(gs.cfin, h->d_coef64, cbytes, cudaMemcpyDeviceToDevice, h->st));
+    if (k > 1) SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cprev, cbytes, cudaMemcpyDeviceToDevice, h->st));
+    const int rc = glm_eval(h, gs, d, k == 1, comm, dev);
+    if (rc != SPLPAK_OK) return rc;
+    SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cfin, cbytes, cudaMemcpyDeviceToDevice, h->st));
+    return SPLPAK_OK;
+}
+
+// The refinement steps of splcw on the last solve, with its z and row weights in gs (glm_last_system) and its factor
+// in d_AB
+static int glm_refine(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, void *comm, real_t *coef,
+                      int coef_on_device) {
+    int rc = SPLPAK_OK;
+    for (int step = 0; step < SPLPAK_REFINE_STEPS && rc == SPLPAK_OK; ++step) {
+        SPL_CUDA_TRY(cudaMemsetAsync(h->d_g, 0, sizeof(double) * (size_t)h->gp.ncol, h->st));
+        rc = feed_device(h, d.x, d.l1x, gs.z, gs.rw, 1, d.n, refine_device_chunk);
+        if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, h->d_g, (size_t)h->gp.ncol, NCCL_FLOAT64, NCCL_SUM);
+        if (rc == SPLPAK_OK) rc = refine_solve(h, coef, coef_on_device);
+    }
+    return rc;
+}
+
+// The loop of splpak_b200_fit_glm_device (semantics: the header).  res = out[0..6]; on 107 the caller's coef holds the
+// last iterate with a finite deviance (c^1 when the first has none).
+static int glm_run(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int max_iter, double tol, void *comm,
+                   real_t *coef, int coef_on_device, double res[7]) {
+    cudaStream_t st = h->st;
+    const long long ncol = h->gp.ncol;
+    const size_t cbytes = sizeof(double) * (size_t)ncol;
+    int rc = glm_domain(h, gs, d, comm, res);
+    if (rc != SPLPAK_OK) return rc;
+    long long band_elems = 0, need = 0;
+    rc = ensure_band(h, &band_elems, &need);
+    double dev[3] = {0.0, 0.0, 0.0};
+    if (rc == SPLPAK_OK) rc = glm_first_assembly(h, gs, d, comm, dev);
+    if (rc != SPLPAK_OK) return rc;
     res[1] = dev[0];
     res[2] = dev[1];
     double dold = dev[0];
     bool halved = false;                                      // the last iteration halved its step
-    const long long nsg = ncol * h->gp.nsten + ncol;          // [S | g] at the start of the partial buffer
     int k = 1;
     for (; k <= max_iter; ++k) {
         if (k > 1) {
             SPL_CUDA_TRY(cudaMemcpyAsync(gs.cprev, h->d_coef64, cbytes, cudaMemcpyDeviceToDevice, st));
-            SPL_CUDA_TRY(cudaMemsetAsync(h->d_part, 0, sizeof(double) * (size_t)nsg, st));
-            rc = feed_device(h, d.x, d.l1x, gs.z, gs.rw, 1, d.n, reassemble_device_chunk);
-            if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, h->d_part, (size_t)nsg, NCCL_FLOAT64, NCCL_SUM);
+            rc = glm_reassemble(h, gs, d, comm);
             if (rc != SPLPAK_OK) return rc;
-            SPL_CUDA_TRY(cudaMemcpyAsync(h->d_totals, gs.tot0, sizeof(double) * 2, cudaMemcpyDeviceToDevice, st));
         }
         rc = compute_cholesky(h, coef, coef_on_device, band_elems, need);
         if (rc == SPLPAK_ERR_SOLVER && k > 1) {
@@ -1983,20 +2038,11 @@ static int glm_run(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int ma
         }
     }
     if (k > max_iter) k = max_iter;
-    // The refinement steps of splcw refine the last solve, so they need its z and row weights (the evaluation since has
-    // overwritten them: they come back from c^(k-1), or mu0) and its full step (skipped after a halving)
+    // The refinement steps of splcw refine the last solve, so they need its z and row weights and its full step
+    // (skipped after a halving)
     if (sizeof(real_t) == sizeof(double) && h->constraints_fired && !halved) {
-        SPL_CUDA_TRY(cudaMemcpyAsync(gs.cfin, h->d_coef64, cbytes, cudaMemcpyDeviceToDevice, st));
-        if (k > 1) SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cprev, cbytes, cudaMemcpyDeviceToDevice, st));
-        rc = glm_eval(h, gs, d, k == 1, comm, dev);
-        if (rc != SPLPAK_OK) return rc;
-        SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cfin, cbytes, cudaMemcpyDeviceToDevice, st));
-        for (int step = 0; step < SPLPAK_REFINE_STEPS && rc == SPLPAK_OK; ++step) {
-            SPL_CUDA_TRY(cudaMemsetAsync(h->d_g, 0, cbytes, st));
-            rc = feed_device(h, d.x, d.l1x, gs.z, gs.rw, 1, d.n, refine_device_chunk);
-            if (rc == SPLPAK_OK) rc = robust_allreduce(h, comm, h->d_g, (size_t)ncol, NCCL_FLOAT64, NCCL_SUM);
-            if (rc == SPLPAK_OK) rc = refine_solve(h, coef, coef_on_device);
-        }
+        rc = glm_last_system(h, gs, d, k, comm, dev);
+        if (rc == SPLPAK_OK) rc = glm_refine(h, gs, d, comm, coef, coef_on_device);
         // the final evaluation: out and mu describe the refined coefficients
         if (rc == SPLPAK_OK) rc = glm_eval(h, gs, d, 0, comm, dev);
         res[1] = dev[0];
@@ -2006,21 +2052,30 @@ static int glm_run(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, int ma
     return write_coef(h, h->d_coef64, coef, coef_on_device);
 }
 
-static int fit_glm_impl(splpak_b200_fit_t h, const GlmData &d, int max_iter, double tol, void *comm, real_t *coef,
-                        int coef_on_device, double *out) {
-    double res[7] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+// One GLM call with its scratch: run(gs, res) fills res, whose first nres values go to out
+#define GLM_NRES_MAX 13
+template <class Run>
+static int glm_call(splpak_b200_fit_t h, const GlmData &d, double *out, int nres, Run run) {
+    double res[GLM_NRES_MAX] = {0.0};
     GlmScratch gs;
     int rc = spl_glm_scratch_init(gs, d.n, h->gp.ncol, h->di.nsm);
     if (rc == SPLPAK_OK) {
-        rc = glm_run(h, gs, d, max_iter, tol, comm, coef, coef_on_device, res);
+        rc = run(gs, res);
         if (cudaStreamSynchronize(h->st) != cudaSuccess) {
             cudaGetLastError();
             if (rc == SPLPAK_OK) rc = SPLPAK_ERR_CUDA;
         }
         spl_glm_scratch_free(gs);
     }
-    memcpy(out, res, sizeof(res));
+    memcpy(out, res, sizeof(double) * (size_t)nres);
     return rc;
+}
+
+static int fit_glm_impl(splpak_b200_fit_t h, const GlmData &d, int max_iter, double tol, void *comm, real_t *coef,
+                        int coef_on_device, double *out) {
+    return glm_call(h, d, out, 7, [&](GlmScratch &gs, double *res) {
+        return glm_run(h, gs, d, max_iter, tol, comm, coef, coef_on_device, res);
+    });
 }
 
 extern "C" int splpak_b200_fit_glm_device(splpak_b200_fit_t h, const real_t *d_x, int l1x, const real_t *d_y,
@@ -2036,13 +2091,11 @@ extern "C" int splpak_b200_fit_glm_device(splpak_b200_fit_t h, const real_t *d_x
     return rc;
 }
 
-// HOST arrays: the points go to device buffers once for the whole call (through the pinned staging of spl_h2d)
-extern "C" int splpak_b200_fit_glm(splpak_b200_fit_t h, const real_t *x, int l1x, const real_t *y, const real_t *w,
-                                   int weighted, const real_t *offset, int64_t n, int family, int max_iter, double tol,
-                                   void *nccl_comm, real_t *coef, int64_t ncf, real_t *mu, double *out, int nout,
-                                   int *ierror) {
-    int rc = glm_check(h, l1x, n, family, max_iter, tol, ncf, out, nout);
-    if (!w) weighted = 0;
+// The host entries of the GLM calls: the points go to device buffers once for the whole call (through the pinned
+// staging of spl_h2d), run(d) runs the call on them, and mu comes back.  rc: the caller's checks.
+template <class Run>
+static int glm_host(splpak_b200_fit_t h, int rc, const real_t *x, int l1x, const real_t *y, const real_t *w,
+                    int weighted, const real_t *offset, int64_t n, int family, real_t *mu, Run run) {
     real_t *d[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};          // x, y, w, offset, mu
     if (rc == SPLPAK_OK) {
         const size_t len[5] = {(size_t)n * (size_t)l1x, (size_t)n, weighted ? (size_t)n : 0, offset ? (size_t)n : 0,
@@ -2059,9 +2112,7 @@ extern "C" int splpak_b200_fit_glm(splpak_b200_fit_t h, const real_t *x, int l1x
                 cudaGetLastError();
                 rc = SPLPAK_ERR_CUDA;
             }
-        if (rc == SPLPAK_OK)
-            rc = fit_glm_impl(h, GlmData{d[0], l1x, d[1], d[2], weighted, d[3], n, family, d[4]}, max_iter, tol,
-                              nccl_comm, coef, 0, out);
+        if (rc == SPLPAK_OK) rc = run(GlmData{d[0], l1x, d[1], d[2], weighted, d[3], n, family, d[4]});
         if (mu && (rc == SPLPAK_OK || rc == SPLPAK_ERR_SOLVER) &&
             (spl_d2h(mu, d[4], sizeof(real_t) * (size_t)n, h->st, h->di.dev) != cudaSuccess ||
              spl_d2h_flush(h->di.dev) != cudaSuccess || cudaStreamSynchronize(h->st) != cudaSuccess)) {
@@ -2071,6 +2122,18 @@ extern "C" int splpak_b200_fit_glm(splpak_b200_fit_t h, const real_t *x, int l1x
         for (int a = 0; a < 5; ++a)
             if (d[a]) cudaFree(d[a]);
     }
+    return rc;
+}
+
+extern "C" int splpak_b200_fit_glm(splpak_b200_fit_t h, const real_t *x, int l1x, const real_t *y, const real_t *w,
+                                   int weighted, const real_t *offset, int64_t n, int family, int max_iter, double tol,
+                                   void *nccl_comm, real_t *coef, int64_t ncf, real_t *mu, double *out, int nout,
+                                   int *ierror) {
+    int rc = glm_check(h, l1x, n, family, max_iter, tol, ncf, out, nout);
+    if (!w) weighted = 0;
+    rc = glm_host(h, rc, x, l1x, y, w, weighted, offset, n, family, mu, [&](const GlmData &d) {
+        return fit_glm_impl(h, d, max_iter, tol, nccl_comm, coef, 0, out);
+    });
     if (ierror) *ierror = rc;
     return rc;
 }
@@ -2156,6 +2219,18 @@ static GcvScratch gcv_scratch_layout(const GridParams &gp) {
     return L;
 }
 
+// The score scratch (gcv_scratch_layout), allocated by the first call that needs it
+static int ensure_score_scratch(splpak_b200_fit_t h) {
+    if (h->d_gcv) return SPLPAK_OK;
+    if (cudaMalloc((void **)&h->d_gcv, sizeof(double) * (size_t)gcv_scratch_layout(h->gp).len) != cudaSuccess) {
+        cudaGetLastError();
+        h->d_gcv = nullptr;
+        return SPLPAK_ERR_ALLOC;
+    }
+    h->s1_valid = 0;
+    return SPLPAK_OK;
+}
+
 // The part both scores share: M = S1 + lambda R into S2 (S1 = G0 + C cached per assembly), then the factor and solve
 // of M c = g in d_AB / the workspace behind it (band_elems doubles in), c at *d_sol.  Leaves S, g, cnt and totals as
 // they are.  Clears sigma_valid: d_AB no longer holds Sigma.  SPLPAK_ERR_SOLVER for a non-positive pivot.
@@ -2165,15 +2240,9 @@ static int score_factor(splpak_b200_fit_t h, double lambda, int penalty, long lo
     long long band_elems = 0, need = 0;
     int rc = ensure_band(h, &band_elems, &need);
     if (rc != SPLPAK_OK) return rc;
+    rc = ensure_score_scratch(h);
+    if (rc != SPLPAK_OK) return rc;
     const GcvScratch L = gcv_scratch_layout(gp);
-    if (!h->d_gcv) {
-        if (cudaMalloc((void **)&h->d_gcv, sizeof(double) * (size_t)L.len) != cudaSuccess) {
-            cudaGetLastError();
-            h->d_gcv = nullptr;
-            return SPLPAK_ERR_ALLOC;
-        }
-        h->s1_valid = 0;
-    }
     if (lambda > 0.0 && ensure_penalty_tables(h) != SPLPAK_OK) return SPLPAK_ERR_ALLOC;
     const long long ns = gp.ncol * gp.nsten;
     double *d_S1 = h->d_gcv + L.S1, *d_S2 = h->d_gcv + L.S2, *d_g2 = h->d_gcv + L.g2, *d_tot1 = h->d_gcv + L.tot1;
@@ -2310,47 +2379,61 @@ extern "C" int splpak_b200_fit_reml_score(splpak_b200_fit_t h, double lambda, in
     return rc;
 }
 
-// The search of select_smoothing and select_smoothing_reml: `score` writes nres outputs, the criterion first, and
-// returns SPLPAK_ERR_SOLVER for a non-positive pivot.  rescore: when the best point was not the last one evaluated,
-// score it again at the end (the GCV score leaves that point's Sigma behind).
+// Known-scale criteria for the GLM selection (phi = 1: Poisson and binomial).  UBRE on the GCV quantities,
+// {U, RSS, edf, N, ywy} with U = RSS / N - 1 + 2 edf / N
+static int ubre_score_impl(splpak_b200_fit_t h, double lambda, int penalty, double out5[5]) {
+    const int rc = gcv_score_impl(h, lambda, penalty, out5);
+    if (rc == SPLPAK_OK) out5[0] = out5[1] / out5[3] - 1.0 + 2.0 * out5[2] / out5[3];
+    return rc;
+}
+
+// REML with phi = 1 on the REML quantities, {V, D_p, log|M|, n, ywy, phi} with V = D_p + log|M| - (p - Mp) log lambda
+static int reml_known_score_impl(splpak_b200_fit_t h, double lambda, int penalty, double out6[6]) {
+    const int rc = reml_score_impl(h, lambda, penalty, out6);
+    if (rc == SPLPAK_OK) {
+        const double mp = (double)penalty_null_dim(h->gp.ndim, penalty), p = (double)h->gp.ncol;
+        out6[0] = out6[1] + out6[2] - (p - mp) * log(lambda);
+    }
+    return rc;
+}
+
+// The default search range rho * [1e-10, 1e4], rho = sum G0_ii / sum R_ii of the assembled S (before compute)
+static int default_smoothing_range(splpak_b200_fit_t h, int penalty, double *lambda_lo, double *lambda_hi) {
+    double sums[2] = {0.0, 0.0};
+    int rc = ensure_penalty_tables(h);
+    if (rc == SPLPAK_OK) rc = spl_penalty_diag_launch(h->gp, penalty, h->d_pen, h->d_S, h->d_dummy_tot, h->st);
+    if (rc != SPLPAK_OK) return rc;
+    SPL_CUDA_TRY(cudaMemcpyAsync(sums, h->d_dummy_tot, sizeof(sums), cudaMemcpyDeviceToHost, h->st));
+    SPL_CUDA_TRY(cudaStreamSynchronize(h->st));
+    const double rho = (sums[0] > 0.0 && sums[1] > 0.0) ? sums[0] / sums[1] : 1.0;
+    *lambda_lo = rho * 1e-10;
+    *lambda_hi = rho * 1e4;
+    return SPLPAK_OK;
+}
+
+// `score` writes nres outputs, the criterion first, and returns SPLPAK_ERR_SOLVER for a non-positive pivot.
 typedef int (*ScoreFn)(splpak_b200_fit_t, double, int, double *);
-static int select_smoothing_search(splpak_b200_fit_t h, int penalty, double lambda_lo, double lambda_hi, ScoreFn score,
-                                   int nres, bool rescore, double *lambda, double *out, int nout, double *trace,
-                                   int64_t trace_cap, int64_t *ntrace, int *ierror) {
-    int rc = gcv_check(h, penalty);
-    if (rc == SPLPAK_OK && (isnan(lambda_lo) || isnan(lambda_hi) || isinf(lambda_lo) || isinf(lambda_hi)))
-        rc = SPLPAK_ERR_HANDLE;
-    if (rc == SPLPAK_OK && lambda_lo > lambda_hi) rc = SPLPAK_ERR_HANDLE;
-    if (rc == SPLPAK_OK && out && nout < nres) rc = SPLPAK_ERR_HANDLE;
-    if (rc != SPLPAK_OK) {
-        if (ierror) *ierror = rc;
-        return rc;
-    }
-    if (ntrace) *ntrace = 0;
-    if (!(lambda_lo > 0.0) || !(lambda_hi > 0.0)) {
-        // default range rho * [1e-10, 1e4], rho = sum G0_ii / sum R_ii on the device
-        double sums[2] = {0.0, 0.0};
-        rc = ensure_penalty_tables(h);
-        if (rc == SPLPAK_OK) rc = spl_penalty_diag_launch(h->gp, penalty, h->d_pen, h->d_S, h->d_dummy_tot, h->st);
-        if (rc == SPLPAK_OK && (cudaMemcpyAsync(sums, h->d_dummy_tot, sizeof(sums), cudaMemcpyDeviceToHost, h->st) !=
-                                    cudaSuccess ||
-                                cudaStreamSynchronize(h->st) != cudaSuccess))
-            rc = SPLPAK_ERR_CUDA;
-        if (rc != SPLPAK_OK) {
-            if (ierror) *ierror = rc;
-            return rc;
-        }
-        const double rho = (sums[0] > 0.0 && sums[1] > 0.0) ? sums[0] / sums[1] : 1.0;
-        lambda_lo = rho * 1e-10;
-        lambda_hi = rho * 1e4;
-    }
-    // every evaluated point, in order; the best is the smallest V, ties to the larger lambda
-    int64_t neval = 0;
-    double best_t = 0.0, best_v = INFINITY, best_out[6] = {0, 0, 0, 0, 0, 0}, last_t = 0.0;
-    bool any_ok = false, have_best = false;
+
+// One search: the best point t (log10 lambda) and its outputs, the points evaluated, whether any had a positive pivot,
+// the last point evaluated, and whether the best grid point was the lower or the upper end of the grid
+struct SearchResult {
+    double t, out[6], last_t;
+    int64_t neval;
+    bool any_ok, grid_lo, grid_hi;
+};
+
+// The search over log10 lambda in [t_lo, t_hi]: a grid at 2 points per decade, then golden section on the grid bracket
+// of the best point down to 0.02 decades.  The best is the smallest criterion, ties to the larger lambda; points with a
+// non-positive pivot count as +inf.  trace (may be null): [lambda, out[0..2]] of every point in evaluation order, up to
+// trace_cap rows.
+static int smoothing_search(splpak_b200_fit_t h, int penalty, double t_lo, double t_hi, ScoreFn score, int nres,
+                            double *trace, int64_t trace_cap, SearchResult &res) {
+    res = SearchResult{0.0, {0, 0, 0, 0, 0, 0}, 0.0, 0, false, false, false};
+    double best_v = INFINITY;
+    bool have_best = false;
     auto eval = [&](double t, double *v) -> int {
         const double lam = pow(10.0, t);
-        last_t = t;
+        res.last_t = t;
         double o[6];
         const int r = score(h, lam, penalty, o);
         if (r != SPLPAK_OK && r != SPLPAK_ERR_SOLVER) return r;
@@ -2358,25 +2441,25 @@ static int select_smoothing_search(splpak_b200_fit_t h, int penalty, double lamb
             o[0] = INFINITY;
             o[1] = o[2] = NAN;
         } else {
-            any_ok = true;
+            res.any_ok = true;
         }
-        if (trace && neval < trace_cap) {
-            trace[4 * neval + 0] = lam;
-            trace[4 * neval + 1] = o[0];
-            trace[4 * neval + 2] = o[1];
-            trace[4 * neval + 3] = o[2];
+        if (trace && res.neval < trace_cap) {
+            trace[4 * res.neval + 0] = lam;
+            trace[4 * res.neval + 1] = o[0];
+            trace[4 * res.neval + 2] = o[1];
+            trace[4 * res.neval + 3] = o[2];
         }
-        ++neval;
-        if (r == SPLPAK_OK && (!have_best || o[0] < best_v || (o[0] == best_v && t > best_t))) {
+        ++res.neval;
+        if (r == SPLPAK_OK && (!have_best || o[0] < best_v || (o[0] == best_v && t > res.t))) {
             have_best = true;
-            best_t = t;
+            res.t = t;
             best_v = o[0];
-            memcpy(best_out, o, sizeof(double) * (size_t)nres);
+            memcpy(res.out, o, sizeof(double) * (size_t)nres);
         }
         *v = o[0];
         return SPLPAK_OK;
     };
-    const double t_lo = log10(lambda_lo), t_hi = log10(lambda_hi);
+    int rc = SPLPAK_OK;
     int K = (int)ceil(2.0 * (t_hi - t_lo) - 1e-9);
     if (K < 0) K = 0;
     int kbest = 0;
@@ -2390,6 +2473,8 @@ static int select_smoothing_search(splpak_b200_fit_t h, int penalty, double lamb
             kbest = k;
         }
     }
+    res.grid_lo = K > 0 && kbest == 0;
+    res.grid_hi = K > 0 && kbest == K;
     if (rc == SPLPAK_OK && K > 0) {
         // golden section on the grid bracket of the best point
         auto grid_t = [&](int k) { return t_lo + (t_hi - t_lo) * k / K; };
@@ -2414,20 +2499,47 @@ static int select_smoothing_search(splpak_b200_fit_t h, int penalty, double lamb
             }
         }
     }
-    if (ntrace) *ntrace = (trace && neval > trace_cap) ? trace_cap : neval;
-    if (rc == SPLPAK_OK && !any_ok) rc = SPLPAK_ERR_SOLVER;
-    if (rescore && rc == SPLPAK_OK && last_t != best_t) {
+    return rc;
+}
+
+// select_smoothing and select_smoothing_reml: the checks, the range, the search, then set_smoothing.  rescore: when the
+// best point was not the last one evaluated, score it again at the end (the GCV score leaves that point's Sigma behind).
+static int select_smoothing_search(splpak_b200_fit_t h, int penalty, double lambda_lo, double lambda_hi, ScoreFn score,
+                                   int nres, bool rescore, double *lambda, double *out, int nout, double *trace,
+                                   int64_t trace_cap, int64_t *ntrace, int *ierror) {
+    int rc = gcv_check(h, penalty);
+    if (rc == SPLPAK_OK && (isnan(lambda_lo) || isnan(lambda_hi) || isinf(lambda_lo) || isinf(lambda_hi)))
+        rc = SPLPAK_ERR_HANDLE;
+    if (rc == SPLPAK_OK && lambda_lo > lambda_hi) rc = SPLPAK_ERR_HANDLE;
+    if (rc == SPLPAK_OK && out && nout < nres) rc = SPLPAK_ERR_HANDLE;
+    if (rc != SPLPAK_OK) {
+        if (ierror) *ierror = rc;
+        return rc;
+    }
+    if (ntrace) *ntrace = 0;
+    if (!(lambda_lo > 0.0) || !(lambda_hi > 0.0)) {
+        rc = default_smoothing_range(h, penalty, &lambda_lo, &lambda_hi);
+        if (rc != SPLPAK_OK) {
+            if (ierror) *ierror = rc;
+            return rc;
+        }
+    }
+    SearchResult sr;
+    rc = smoothing_search(h, penalty, log10(lambda_lo), log10(lambda_hi), score, nres, trace, trace_cap, sr);
+    if (ntrace) *ntrace = (trace && sr.neval > trace_cap) ? trace_cap : sr.neval;
+    if (rc == SPLPAK_OK && !sr.any_ok) rc = SPLPAK_ERR_SOLVER;
+    if (rescore && rc == SPLPAK_OK && sr.last_t != sr.t) {
         // d_AB holds Sigma of the last point evaluated: score the selected lambda again, so that get_selected_inverse
         // returns the inverse of the system the handle now carries (the same inputs: the same scores, bit for bit)
         double o[5];
-        rc = gcv_score_impl(h, pow(10.0, best_t), penalty, o);
+        rc = gcv_score_impl(h, pow(10.0, sr.t), penalty, o);
     }
     if (rc == SPLPAK_OK) {
-        const double lam = pow(10.0, best_t);
+        const double lam = pow(10.0, sr.t);
         rc = splpak_b200_fit_set_smoothing(h, lam, penalty);
         if (rc == SPLPAK_OK) {
             if (lambda) *lambda = lam;
-            if (out) memcpy(out, best_out, sizeof(double) * (size_t)nres);
+            if (out) memcpy(out, sr.out, sizeof(double) * (size_t)nres);
         }
     }
     if (ierror) *ierror = rc;
@@ -2491,6 +2603,17 @@ extern "C" int splpak_b200_fit_get_cholesky_factor(splpak_b200_fit_t h, int whic
 }
 
 // ---- posterior variances (variance.cu; DESIGN §4.13) ----
+// The table buffer, allocated by the first call that needs it
+static int ensure_variance_tables(splpak_b200_fit_t h) {
+    if (h->d_var) return SPLPAK_OK;
+    if (cudaMalloc((void **)&h->d_var, sizeof(double) * (size_t)spl_variance_table_len(h->gp)) != cudaSuccess) {
+        cudaGetLastError();
+        h->d_var = nullptr;
+        return SPLPAK_ERR_ALLOC;
+    }
+    return SPLPAK_OK;
+}
+
 extern "C" int splpak_b200_fit_prepare_variance(splpak_b200_fit_t h, double *out, int nout, int *ierror) {
     int rc = SPLPAK_OK;
     if (!valid(h) || h->finalized || !h->gcv || h->solver == SPLPAK_SOLVER_ORTHOGONAL || !out || nout < 6)
@@ -2504,12 +2627,7 @@ extern "C" int splpak_b200_fit_prepare_variance(splpak_b200_fit_t h, double *out
         if (same) memcpy(o, h->sigma_out, sizeof(o));
         else rc = gcv_score_impl(h, h->lambda, h->penalty, o);
     }
-    if (rc == SPLPAK_OK && !h->d_var &&
-        cudaMalloc((void **)&h->d_var, sizeof(double) * (size_t)spl_variance_table_len(h->gp)) != cudaSuccess) {
-        cudaGetLastError();
-        h->d_var = nullptr;
-        rc = SPLPAK_ERR_ALLOC;
-    }
+    if (rc == SPLPAK_OK) rc = ensure_variance_tables(h);
     if (rc == SPLPAK_OK) {
         const long long lda = spl_band_lda(spl_half_bandwidth(h->gp));
         rc = spl_variance_table_launch(h->gp, h->d_AB, lda, h->d_var, h->st, h->di.nsm);
@@ -2555,6 +2673,223 @@ extern "C" int splpak_b200_fit_variance(splpak_b200_fit_t h, const real_t *x, in
                                   return spl_variance_launch(h->gp, nderiv, d_x, l1x, n, h->d_var, d_out, st,
                                                              h->di.nsm);
                               });
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+// ---- GLM fit with the smoothing parameter chosen on each working system (DESIGN §4.17) ----
+struct GlmSelect {
+    int criterion, penalty;
+    double lambda_lo, lambda_hi;
+    int max_select, variance;
+    double *trace;                                            // rows [lambda_k, criterion, scores, D_k, halvings_k]
+    int64_t trace_cap, ntrace;
+};
+
+static int glm_select_check(splpak_b200_fit_t h, int l1x, int64_t n, int family, const GlmSelect &sel, int max_iter,
+                            double tol, int64_t ncf, const double *out, int nout) {
+    const int rc = glm_check(h, l1x, n, family, max_iter, tol, ncf, out, nout);
+    if (rc == SPLPAK_ERR_HANDLE || !valid(h)) return rc;
+    if (sel.criterion != SPLPAK_GLM_SELECT_REML && sel.criterion != SPLPAK_GLM_SELECT_PREDICTION) return SPLPAK_ERR_HANDLE;
+    if (sel.penalty != SPLPAK_PENALTY_CURVATURE && sel.penalty != SPLPAK_PENALTY_THIN_PLATE) return SPLPAK_ERR_HANDLE;
+    if (!isfinite(sel.lambda_lo) || !isfinite(sel.lambda_hi)) return SPLPAK_ERR_HANDLE;
+    if (sel.lambda_lo > 0.0 && sel.lambda_hi > 0.0 && sel.lambda_lo > sel.lambda_hi) return SPLPAK_ERR_HANDLE;
+    if (sel.max_select < 1 || sel.trace_cap < 0 || nout < 13) return SPLPAK_ERR_HANDLE;
+    return rc;
+}
+
+// The loop of splpak_b200_fit_glm_select_device (semantics: the header).  res = out[0..12].
+static int glm_select_run(splpak_b200_fit_t h, GlmScratch &gs, const GlmData &d, GlmSelect &sel, int max_iter,
+                          double tol, void *comm, real_t *coef, int coef_on_device, double res[13]) {
+    cudaStream_t st = h->st;
+    const long long ncol = h->gp.ncol;
+    const size_t cbytes = sizeof(double) * (size_t)ncol;
+    const bool known_scale = d.family != SPLPAK_GLM_GAMMA;
+    const bool reml = sel.criterion == SPLPAK_GLM_SELECT_REML;
+    const ScoreFn score = reml ? (known_scale ? reml_known_score_impl : reml_score_impl)
+                               : (known_scale ? ubre_score_impl : gcv_score_impl);
+    const int nres = reml ? 6 : 5;
+    int rc = glm_domain(h, gs, d, comm, res);
+    if (rc != SPLPAK_OK) return rc;
+    // every buffer of the call before the first assembly, so that a 204 leaves the handle fresh
+    long long band_elems = 0, need = 0;
+    rc = splpak_b200_fit_enable_gcv(h);
+    if (rc == SPLPAK_OK) rc = ensure_band(h, &band_elems, &need);
+    if (rc == SPLPAK_OK) rc = ensure_score_scratch(h);
+    if (rc == SPLPAK_OK) rc = ensure_penalty_tables(h);
+    if (rc == SPLPAK_OK && sel.variance) rc = ensure_variance_tables(h);
+    double dev[3] = {0.0, 0.0, 0.0};
+    if (rc == SPLPAK_OK) rc = glm_first_assembly(h, gs, d, comm, dev);
+    if (rc != SPLPAK_OK) return rc;
+    h->penalty = sel.penalty;
+    h->var_valid = 0;
+    double lo = sel.lambda_lo, hi = sel.lambda_hi;
+    if (!(lo > 0.0) || !(hi > 0.0)) {
+        rc = default_smoothing_range(h, sel.penalty, &lo, &hi);
+        if (rc != SPLPAK_OK) return rc;
+    }
+    const double t_lo = log10(lo), t_hi = log10(hi);
+    res[1] = dev[0];
+    res[2] = dev[1];
+    double dold = dev[0], t_prev = 0.0;
+    bool halved = false, selecting = true;
+    int k = 1;
+    for (; k <= max_iter; ++k) {
+        if (k > 1) {
+            SPL_CUDA_TRY(cudaMemcpyAsync(gs.cprev, h->d_coef64, cbytes, cudaMemcpyDeviceToDevice, st));
+            rc = glm_reassemble(h, gs, d, comm);
+            if (rc != SPLPAK_OK) return rc;
+        }
+        // phase 1: lambda_k from the working system just assembled (before compute adds C and lambda R to S)
+        const bool searched = selecting;
+        double crit = NAN;
+        int64_t nscore = 0;
+        if (searched) {
+            SearchResult sr;
+            const double a = k > 1 ? fmax(t_lo, t_prev - 1.0) : t_lo, b = k > 1 ? fmin(t_hi, t_prev + 1.0) : t_hi;
+            rc = smoothing_search(h, sel.penalty, a, b, score, nres, nullptr, 0, sr);
+            nscore = sr.neval;
+            // the best grid point at an end of the window that is not an end of the range: the whole range
+            if (rc == SPLPAK_OK && ((sr.grid_lo && a > t_lo) || (sr.grid_hi && b < t_hi))) {
+                rc = smoothing_search(h, sel.penalty, t_lo, t_hi, score, nres, nullptr, 0, sr);
+                nscore += sr.neval;
+            }
+            if (rc == SPLPAK_OK && !sr.any_ok) {
+                // no point with a positive pivot: the last iterate (c^(k-1), not yet replaced) to the caller
+                rc = k > 1 ? write_coef(h, h->d_coef64, coef, coef_on_device) : SPLPAK_OK;
+                return rc == SPLPAK_OK ? SPLPAK_ERR_SOLVER : rc;
+            }
+            if (rc != SPLPAK_OK) return rc;
+            crit = sr.out[0];
+            h->lambda = pow(10.0, sr.t);
+            res[7] = h->lambda;
+            res[8] = crit;
+            res[11] += 1.0;
+            if (k > 1 && fabs(sr.t - t_prev) <= 0.05) {
+                selecting = false;
+                res[12] = 1.0;
+            } else if (res[11] >= sel.max_select) {
+                selecting = false;
+            }
+            t_prev = sr.t;
+        }
+        double *row = (sel.trace && sel.ntrace < sel.trace_cap) ? sel.trace + 5 * sel.ntrace : nullptr;
+        if (row) {
+            row[0] = h->lambda;
+            row[1] = crit;
+            row[2] = (double)nscore;
+            row[3] = NAN;
+            row[4] = 0.0;
+            ++sel.ntrace;
+        }
+        rc = compute_cholesky(h, coef, coef_on_device, band_elems, need);
+        if (rc == SPLPAK_ERR_SOLVER && k > 1) {
+            // the last successful iterate back to the caller; out and mu already describe it
+            SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cprev, cbytes, cudaMemcpyDeviceToDevice, st));
+            rc = write_coef(h, h->d_coef64, coef, coef_on_device);
+            return rc == SPLPAK_OK ? SPLPAK_ERR_SOLVER : rc;
+        }
+        if (rc != SPLPAK_OK) return rc;
+        res[0] = k;
+        rc = glm_eval(h, gs, d, 0, comm, dev);
+        int nh = 0;
+        for (; rc == SPLPAK_OK && !isfinite(dev[0]) && k > 1 && nh < GLM_MAX_HALVINGS; ++nh) {
+            rc = spl_glm_halve_launch(gs, h->d_coef64, ncol, st);
+            if (rc == SPLPAK_OK) rc = glm_eval(h, gs, d, 0, comm, dev);
+        }
+        res[4] += nh;
+        if (rc != SPLPAK_OK) return rc;
+        halved = nh > 0;
+        if (row) {
+            row[3] = dev[0];
+            row[4] = nh;
+        }
+        if (!isfinite(dev[0])) {
+            // no finite deviance: keep c^1 at k = 1, else go back to c^(k-1) and evaluate it again for out and mu
+            if (k > 1) {
+                SPL_CUDA_TRY(cudaMemcpyAsync(h->d_coef64, gs.cprev, cbytes, cudaMemcpyDeviceToDevice, st));
+                rc = glm_eval(h, gs, d, 0, comm, dev);
+            }
+            res[1] = dev[0];
+            res[2] = dev[1];
+            if (rc == SPLPAK_OK) rc = write_coef(h, h->d_coef64, coef, coef_on_device);
+            return rc == SPLPAK_OK ? SPLPAK_ERR_SOLVER : rc;
+        }
+        res[1] = dev[0];
+        res[2] = dev[1];
+        res[3] = fabs(dev[0] - dold) / (fabs(dev[0]) + 0.1);
+        dold = dev[0];
+        // phase 2 only: a change measured across a change of lambda says nothing about convergence
+        if (!searched && res[3] < tol) {
+            res[5] = 1.0;
+            break;
+        }
+    }
+    if (k > max_iter) k = max_iter;
+    // the last solve's z and row weights; with them the refinement steps (which need the factor in d_AB) and then the
+    // last solve's system again, whose GCV score at the selected lambda gives edf and leaves Sigma in d_AB
+    rc = glm_last_system(h, gs, d, k, comm, dev);
+    if (rc == SPLPAK_OK && sizeof(real_t) == sizeof(double) && h->constraints_fired && !halved)
+        rc = glm_refine(h, gs, d, comm, coef, coef_on_device);
+    if (rc == SPLPAK_OK) rc = glm_reassemble(h, gs, d, comm);
+    double o5[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    if (rc == SPLPAK_OK) rc = gcv_score_impl(h, h->lambda, h->penalty, o5);
+    if (rc == SPLPAK_OK && sel.variance) {
+        rc = spl_variance_table_launch(h->gp, h->d_AB, spl_band_lda(spl_half_bandwidth(h->gp)), h->d_var, st,
+                                       h->di.nsm);
+        h->var_valid = rc == SPLPAK_OK;
+    }
+    // the final evaluation: out and mu describe the returned coefficients
+    if (rc == SPLPAK_OK) rc = glm_eval(h, gs, d, 0, comm, dev);
+    if (rc == SPLPAK_OK) rc = write_coef(h, h->d_coef64, coef, coef_on_device);
+    if (rc != SPLPAK_OK) return rc;
+    res[1] = dev[0];
+    res[2] = dev[1];
+    res[9] = o5[2];
+    res[10] = known_scale ? 1.0 : (res[6] > o5[2] ? dev[1] / (res[6] - o5[2]) : INFINITY);
+    return SPLPAK_OK;
+}
+
+static int fit_glm_select_impl(splpak_b200_fit_t h, const GlmData &d, GlmSelect &sel, int max_iter, double tol,
+                               void *comm, real_t *coef, int coef_on_device, double *out, int64_t *ntrace) {
+    const int rc = glm_call(h, d, out, 13, [&](GlmScratch &gs, double *res) {
+        return glm_select_run(h, gs, d, sel, max_iter, tol, comm, coef, coef_on_device, res);
+    });
+    if (ntrace) *ntrace = sel.ntrace;
+    return rc;
+}
+
+extern "C" int splpak_b200_fit_glm_select_device(splpak_b200_fit_t h, const real_t *d_x, int l1x, const real_t *d_y,
+                                                 const real_t *d_w, int weighted, const real_t *d_offset, int64_t n,
+                                                 int family, int criterion, int penalty, double lambda_lo,
+                                                 double lambda_hi, int max_select, int variance, int max_iter,
+                                                 double tol, void *nccl_comm, real_t *d_coef, int64_t ncf, real_t *d_mu,
+                                                 double *out, int nout, double *trace, int64_t trace_cap,
+                                                 int64_t *ntrace, int *ierror) {
+    GlmSelect sel{criterion, penalty, lambda_lo, lambda_hi, max_select, variance, trace, trace_cap, 0};
+    if (ntrace) *ntrace = 0;
+    int rc = glm_select_check(h, l1x, n, family, sel, max_iter, tol, ncf, out, nout);
+    if (!d_w) weighted = 0;
+    if (rc == SPLPAK_OK)
+        rc = fit_glm_select_impl(h, GlmData{d_x, l1x, d_y, d_w, weighted, d_offset, n, family, d_mu}, sel, max_iter,
+                                 tol, nccl_comm, d_coef, 1, out, ntrace);
+    if (ierror) *ierror = rc;
+    return rc;
+}
+
+extern "C" int splpak_b200_fit_glm_select(splpak_b200_fit_t h, const real_t *x, int l1x, const real_t *y,
+                                          const real_t *w, int weighted, const real_t *offset, int64_t n, int family,
+                                          int criterion, int penalty, double lambda_lo, double lambda_hi,
+                                          int max_select, int variance, int max_iter, double tol, void *nccl_comm,
+                                          real_t *coef, int64_t ncf, real_t *mu, double *out, int nout, double *trace,
+                                          int64_t trace_cap, int64_t *ntrace, int *ierror) {
+    GlmSelect sel{criterion, penalty, lambda_lo, lambda_hi, max_select, variance, trace, trace_cap, 0};
+    if (ntrace) *ntrace = 0;
+    int rc = glm_select_check(h, l1x, n, family, sel, max_iter, tol, ncf, out, nout);
+    if (!w) weighted = 0;
+    rc = glm_host(h, rc, x, l1x, y, w, weighted, offset, n, family, mu, [&](const GlmData &d) {
+        return fit_glm_select_impl(h, d, sel, max_iter, tol, nccl_comm, coef, 0, out, ntrace);
+    });
     if (ierror) *ierror = rc;
     return rc;
 }

@@ -161,11 +161,11 @@ struct RobustScratch {
 // domain-check counts, the previous and the final coefficients, the deviance and the working kernel's partial sums.
 struct GlmScratch {
     long long n;
-    int nparts;                           // CTAs of the working kernel (one pair of partial sums each)
+    int nparts;                           // CTAs of the working kernel (three partial sums each)
     real_t *s;                            // n: s(x_i) of the coefficients being evaluated
     real_t *z, *rw;                       // n: working response z_i and row weight sqrt(W_i) of the next assembly
     unsigned long long *count;            // {y outside the family's domain where w > 0, m = points with w > 0}
-    // one allocation: [cprev (ncol) | cfin (ncol) | dev {D, X^2} | tot0 | part (2 nparts)]; tot0 as in RobustScratch
+    // one allocation: [cprev (ncol) | cfin (ncol) | dev {D, X^2, ywy} | tot0 | part (3 nparts)]; tot0 as in RobustScratch
     double *small, *cprev, *cfin, *dev, *tot0, *part;
 };
 

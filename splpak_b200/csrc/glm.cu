@@ -5,7 +5,9 @@
 //                                    mu_i, mu'_i, V(mu_i) with the clamps of R's make.link; the working response
 //                                    z_i = eta_i - o_i + (y_i - mu_i) / mu'_i and row weight sqrt(W_i) = w_i mu'_i / sqrt(V)
 //                                    of the next assembly (0 and 0 where w_i <= 0, y_i not read there), mu_i on request,
-//                                    and per-CTA partial sums of the deviance D and of Pearson's X^2
+//                                    and per-CTA partial sums of the deviance D, of Pearson's X^2 and of
+//                                    ywy = sum (sqrt(W_i) z_i)^2 (from z and the row weight as stored, so that in the
+//                                    REAL32 library it is the sum of what the next assembly reads)
 //   spl_glm_dev_kernel               the partial sums added in CTA order: bit-identical from call to call
 // and, once before the first assembly, spl_glm_check_kernel: an integer count of the y_i outside the family's domain
 // (or not finite) where w_i > 0, and m, the points with w_i > 0.  spl_glm_halve_kernel is the step halving
@@ -92,7 +94,7 @@ spl_glm_work_kernel(const real_t *__restrict__ y, const real_t *__restrict__ w, 
                     const real_t *__restrict__ o, const real_t *__restrict__ s, long long n, real_t *__restrict__ z,
                     real_t *__restrict__ rw, real_t *__restrict__ mu_out, double *__restrict__ part) {
     typedef GlmFamily<FAM> F;
-    double dsum = 0.0, xsum = 0.0;
+    double dsum = 0.0, xsum = 0.0, ysum = 0.0;
     const long long stride = (long long)gridDim.x * blockDim.x;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const double wv = weighted ? (double)w[i] : 1.0;
@@ -116,42 +118,51 @@ spl_glm_work_kernel(const real_t *__restrict__ y, const real_t *__restrict__ w, 
             dsum += F::dev(yv, mu, a);
             xsum += a * rr * rr;
         }
-        z[i] = (real_t)zi;
-        rw[i] = (real_t)rwi;
+        const real_t zs = (real_t)zi, rws = (real_t)rwi;
+        z[i] = zs;
+        rw[i] = rws;
         if (mu_out) mu_out[i] = (real_t)mu;
+        const double t = (double)rws * (double)zs;
+        ysum = fma(t, t, ysum);
     }
-    __shared__ double s_d[GLM_NT / 32], s_x[GLM_NT / 32];
+    __shared__ double s_d[GLM_NT / 32], s_x[GLM_NT / 32], s_y[GLM_NT / 32];
 #pragma unroll
     for (int k = 16; k > 0; k >>= 1) {
         dsum += __shfl_xor_sync(0xffffffffu, dsum, k);
         xsum += __shfl_xor_sync(0xffffffffu, xsum, k);
+        ysum += __shfl_xor_sync(0xffffffffu, ysum, k);
     }
     if ((threadIdx.x & 31) == 0) {
         s_d[threadIdx.x >> 5] = dsum;
         s_x[threadIdx.x >> 5] = xsum;
+        s_y[threadIdx.x >> 5] = ysum;
     }
     __syncthreads();
     if (threadIdx.x == 0) {
-        double d = 0.0, x = 0.0;
+        double d = 0.0, x = 0.0, yy = 0.0;
         for (int k = 0; k < GLM_NT / 32; ++k) {
             d += s_d[k];
             x += s_x[k];
+            yy += s_y[k];
         }
-        part[2 * blockIdx.x] = d;
-        part[2 * blockIdx.x + 1] = x;
+        part[3 * blockIdx.x] = d;
+        part[3 * blockIdx.x + 1] = x;
+        part[3 * blockIdx.x + 2] = yy;
     }
 }
 
-// dev = {D, X^2}: the CTA partials in CTA order
+// dev = {D, X^2, ywy}: the CTA partials in CTA order
 __global__ void spl_glm_dev_kernel(const double *__restrict__ part, int nparts, double *__restrict__ dev) {
     if (threadIdx.x == 0) {
-        double d = 0.0, x = 0.0;
+        double d = 0.0, x = 0.0, yy = 0.0;
         for (int k = 0; k < nparts; ++k) {
-            d += part[2 * k];
-            x += part[2 * k + 1];
+            d += part[3 * k];
+            x += part[3 * k + 1];
+            yy += part[3 * k + 2];
         }
         dev[0] = d;
         dev[1] = x;
+        dev[2] = yy;
     }
 }
 
@@ -171,7 +182,7 @@ static int glm_grid(long long n, int nsm) {
 
 void spl_glm_scratch_free(GlmScratch &gs);
 
-// Scratch of one call: s, z and row weights of the n points, the two counts, [cprev | cfin | dev | tot0 | partials].
+// Scratch of one call: s, z and row weights of the n points, the two counts, [cprev | cfin | dev(3) | tot0 | partials].
 int spl_glm_scratch_init(GlmScratch &gs, long long n, long long ncol, int nsm) {
     memset(&gs, 0, sizeof(gs));
     gs.n = n;
@@ -180,7 +191,7 @@ int spl_glm_scratch_init(GlmScratch &gs, long long n, long long ncol, int nsm) {
     ok = ok && cudaMalloc((void **)&gs.z, sizeof(real_t) * (size_t)n) == cudaSuccess;
     ok = ok && cudaMalloc((void **)&gs.rw, sizeof(real_t) * (size_t)n) == cudaSuccess;
     ok = ok && cudaMalloc((void **)&gs.count, sizeof(unsigned long long) * 2) == cudaSuccess;
-    ok = ok && cudaMalloc((void **)&gs.small, sizeof(double) * (size_t)(2 * ncol + 4 + 2 * gs.nparts)) == cudaSuccess;
+    ok = ok && cudaMalloc((void **)&gs.small, sizeof(double) * (size_t)(2 * ncol + 5 + 3 * gs.nparts)) == cudaSuccess;
     if (!ok) {
         cudaGetLastError();
         spl_glm_scratch_free(gs);
@@ -189,7 +200,7 @@ int spl_glm_scratch_init(GlmScratch &gs, long long n, long long ncol, int nsm) {
     gs.cprev = gs.small;
     gs.cfin = gs.cprev + ncol;
     gs.dev = gs.cfin + ncol;
-    gs.tot0 = gs.dev + 2;
+    gs.tot0 = gs.dev + 3;
     gs.part = gs.tot0 + 2;
     return SPLPAK_OK;
 }
@@ -229,7 +240,7 @@ static void glm_work(const GlmScratch &gs, int start, const real_t *d_y, const r
                                                                      d_mu, gs.part);
 }
 
-// start != 0: the working quantities of mu0 (gs.s is not read); otherwise of s = gs.s.  {D, X^2} into gs.dev.
+// start != 0: the working quantities of mu0 (gs.s is not read); otherwise of s = gs.s.  {D, X^2, ywy} into gs.dev.
 int spl_glm_work_launch(const GlmScratch &gs, int family, int start, const real_t *d_y, const real_t *d_w, int weighted,
                         const real_t *d_o, real_t *d_mu, cudaStream_t st) {
     if (family == SPLPAK_GLM_POISSON) glm_work<SPLPAK_GLM_POISSON>(gs, start, d_y, d_w, weighted, d_o, d_mu, st);
