@@ -1369,7 +1369,7 @@ static int assemble_chunk_t(const GridParams &gp, const real_t *d_x, int l1x, co
         g_spl_launches += 6;
     } else if constexpr (CELL) {
         static_assert(NDIM == 3, "the moment path is 3-D and 4-D");
-        const size_t smem = sizeof(double) * (size_t)MOM_PB * MOM_RS;
+        const size_t smem = sizeof(double) * (size_t)MOM_NWARP * MOM_PB * MOM_RS;
         auto kern = rhs_only ? spl_moments_kernel<true> : spl_moments_kernel<false>;
         SPL_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int per_sm = 1;

@@ -28,9 +28,9 @@
 #define MOM_NR 64                     // moments of g per cell
 #define MOM_MG 408                    // doubles per cell of the moment array (407 used)
 #ifndef MOM_NT
-#define MOM_NT 128                    // threads per CTA of the moment kernel (thread = point when staging)
+#define MOM_NT 128                    // threads per CTA of the moment kernel (lane = point when staging)
 #endif
-#define MOM_PB MOM_NT                 // points per staged batch
+#define MOM_PB 32                     // points per staged sub-batch (one warp's batch)
 #ifndef MOM_MINB
 #define MOM_MINB 4                    // CTAs per SM the register allocation aims at
 #endif
@@ -115,9 +115,11 @@ __device__ __forceinline__ void spl_mom_dmma(double &c0, double &c1, double a, d
                  : "d"(a), "d"(b));
 }
 
-// Persistent CTAs over work items (cell, segment of <= MOM_CH points).  Per batch of MOM_PB points:
-//   stage   thread = point: gather through the permutation (prefetched one batch ahead, the permutation
-//           two ahead), Legendre values of the three local coordinates -> P1, P2, w^2 P3, w^2 y P3 into
+// Persistent CTAs over work items (cell, segment of <= MOM_CH points).  A work item is cut into sub-batches of MOM_PB = 32
+// points; warp w owns sub-batches w, w + MOM_NWARP, w + 2 MOM_NWARP, ... (a static split, so the order of every warp's
+// sums, and with it the deterministic mode, does not depend on timing).  Per sub-batch the warp alone runs
+//   stage   lane = point: gather through the permutation (prefetched one sub-batch ahead, the permutation two ahead),
+//           Legendre values of the three local coordinates -> P1, P2, w^2 P3, w^2 y P3 into the warp's private slice of
 //           shared memory (28 doubles per point);
 //   accumulate   the moment sums are a GEMM over the points, M[(e3,e2)][e1] = sum_p (A3[e3] P2[e2])_p P1[e1]_p,
 //           run on the FP64 tensor cores (mma.sync.m8n8k4.f64 -> DMMA.8x8x4): k = 4 points, n = e1 (7 of 8
@@ -125,7 +127,11 @@ __device__ __forceinline__ void spl_mom_dmma(double &c0, double &c1, double a, d
 //           right-hand side.  Lane (r, k) multiplies its own A fragment A3[e3]*P2[r] of point k; the B
 //           fragment P1[r] is ONE shared-memory load per 4 points, where the DFMA form needed 7 broadcast
 //           loads per point -- the kernel is bound by the shared-memory pipe, not by FP64 issue.
-// Several CTAs are resident per SM, so one CTA's staging overlaps another's MMA stream.
+// The two phases are separated by __syncwarp only; the CTA meets at a barrier just at the work-item claim and at the
+// reduction.  Warps therefore drift apart, and the scheduler overlaps one warp's FP64 staging with another's DMMA
+// stream.  (A CTA-wide batch through one buffer, with two barriers per batch, held every warp to the slowest one twice
+// per batch.)  One slice per warp, not two: 2 x 32 x MOM_RS doubles per warp would not fit 16 warps per SM in shared
+// memory, and holding the next sub-batch's Legendre values in registers across the DMMA stream would spill.
 template <bool RHS_ONLY>
 __global__ void __launch_bounds__(MOM_NT, MOM_MINB)
 spl_moments_kernel(const __grid_constant__ GridParams gp, const real_t *__restrict__ x, int l1x,
@@ -135,11 +141,12 @@ spl_moments_kernel(const __grid_constant__ GridParams gp, const real_t *__restri
                    const unsigned *__restrict__ item_seg, unsigned *__restrict__ meta,
                    double *__restrict__ MG, const unsigned ch) {
     // ch: points per work item (MOM_CH; deterministic mode: a whole cell, so that every moment receives ONE addition)
-    extern __shared__ __align__(16) double s_pts[];          // MOM_PB x MOM_RS, reused for the reduction
+    extern __shared__ __align__(16) double s_pts[];          // MOM_NWARP x MOM_PB x MOM_RS, reused for the reduction
     __shared__ unsigned s_item;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int fr = lane >> 2, fk = lane & 3;                // MMA fragment coordinates of this lane
     const int frr = fr & 3, frh = fr >> 2;
+    double *const s_warp = s_pts + warp * (MOM_PB * MOM_RS);
     const unsigned nitems = meta[0];
     const int nc1 = gp.nodes[0] + 1, nc2 = gp.nodes[1] + 1;
     for (;;) {
@@ -152,7 +159,7 @@ spl_moments_kernel(const __grid_constant__ GridParams gp, const real_t *__restri
         const unsigned seg = item_seg[item];
         const long long first = (long long)binstart[cell] + (long long)seg * ch;
         const int npts = (int)min(ch, bincount[cell] - seg * ch);
-        const int nbatch = (npts + MOM_PB - 1) / MOM_PB;
+        const int nsub = (npts + MOM_PB - 1) / MOM_PB;
         double xc[3];                                        // left end of the cell per dimension (:246 form)
         {
             const int c1 = (int)(cell % (unsigned)nc1), c2 = (int)((cell / (unsigned)nc1) % (unsigned)nc2),
@@ -166,14 +173,14 @@ spl_moments_kernel(const __grid_constant__ GridParams gp, const real_t *__restri
         for (int e = 0; e < MOM_NE; ++e) acc[e][0] = acc[e][1] = 0.0;
         racc[0][0] = racc[0][1] = racc[1][0] = racc[1][1] = 0.0;
 
-        // pn: permutation entry of the batch AFTER the one held in px/py/pw.  The entry a gather uses is
+        // pn: permutation entry of the sub-batch AFTER the one held in px/py/pw.  The entry a gather uses is
         // first copied to a fresh register: overwriting the register the in-flight gathers were addressed
         // from made the next permutation load wait on their scoreboard (a full memory latency per batch).
         unsigned pn;
         double px[3], py, pw;
-        auto load_perm = [&](int b) {
-            const int p = b * MOM_PB + tid;
-            pn = (b < nbatch && p < npts) ? perm[first + p] : 0xffffffffu;
+        auto load_perm = [&](int k) {
+            const int p = k * MOM_PB + lane;
+            pn = (k < nsub && p < npts) ? perm[first + p] : 0xffffffffu;
         };
         auto load_data = [&](unsigned pc) {
             px[0] = px[1] = px[2] = 0.0;
@@ -194,20 +201,20 @@ spl_moments_kernel(const __grid_constant__ GridParams gp, const real_t *__restri
                 }
             }
         };
-        load_perm(0);
+        load_perm(warp);
         load_data(pn);
-        load_perm(1);
-        for (int b = 0; b < nbatch; ++b) {
-            const int nb = min(MOM_PB, npts - b * MOM_PB);
+        load_perm(warp + MOM_NWARP);
+        for (int k = warp; k < nsub; k += MOM_NWARP) {
+            const int nb = min(MOM_PB, npts - k * MOM_PB);
             // ---- stage ----
-            if (tid < nb) {
+            if (lane < nb) {
                 double P1[MOM_NE], P2[MOM_NE], P3[MOM_NE];
                 spl_legendre<MOM_NE>(spl_mul(gp.dxin[0], spl_sub(px[0], xc[0])), P1);
                 spl_legendre<MOM_NE>(spl_mul(gp.dxin[1], spl_sub(px[1], xc[1])), P2);
                 spl_legendre<MOM_NE>(spl_mul(gp.dxin[2], spl_sub(px[2], xc[2])), P3);
                 const double w2 = pw * pw;                       // row = w*phi, rhs = w*y (:806, :837)
                 const double w2y = w2 * py;
-                double *rec = s_pts + tid * MOM_RS;
+                double *rec = s_warp + lane * MOM_RS;
 #pragma unroll
                 for (int e = 0; e < 8; e += 2) {
                     *reinterpret_cast<double2 *>(rec + e) = make_double2(P1[e], e + 1 < MOM_NE ? P1[e + 1] : 0.0);
@@ -221,23 +228,29 @@ spl_moments_kernel(const __grid_constant__ GridParams gp, const real_t *__restri
                 }
                 *reinterpret_cast<double2 *>(rec + MOM_OFF_B3) = make_double2(w2y * P3[0], w2y * P3[1]);
                 *reinterpret_cast<double2 *>(rec + MOM_OFF_B3 + 2) = make_double2(w2y * P3[2], w2y * P3[3]);
-            } else if (tid < ((nb + 7) & ~7)) {
+            } else if (lane < ((nb + 7) & ~7)) {
                 // the MMA consumes whole groups of 8 points: pad the last group with zero records
-                double *rec = s_pts + tid * MOM_RS;
+                double *rec = s_warp + lane * MOM_RS;
 #pragma unroll
                 for (int e = 0; e < 28; e += 2) *reinterpret_cast<double2 *>(rec + e) = make_double2(0.0, 0.0);
             }
-            __syncthreads();
+            __syncwarp();
             {
                 const unsigned pc = pn;
-                load_perm(b + 2);                                // permutation two batches ahead
-                if (b + 1 < nbatch) load_data(pc);               // gathers of the next batch fly under the DFMAs
+                load_perm(k + 2 * MOM_NWARP);                    // permutation two sub-batches ahead
+                if (k + MOM_NWARP < nsub) load_data(pc);         // gathers of the next sub-batch fly under the DMMAs
             }
             // ---- accumulate ----
-            for (int p0 = warp * 8; p0 < nb; p0 += MOM_NWARP * 8) {
+            // unrolled over the (at most four) groups of 8 points, so the fragment loads of one group are issued under
+            // the DMMAs of the previous one: 4.81 -> 4.54 ms at cfg3 (B200, 1000 W) against a loop bounded by nb
+            const int ng = (nb + 7) >> 3;
+#pragma unroll
+            for (int g = 0; g < MOM_PB / 8; ++g) {
+                if (g >= ng) break;
+                const int p0 = 8 * g;
 #pragma unroll
                 for (int half = 0; half < 2; ++half) {
-                    const double *rec = s_pts + (p0 + half + 2 * fk) * MOM_RS;      // point of this lane's k
+                    const double *rec = s_warp + (p0 + half + 2 * fk) * MOM_RS;     // point of this lane's k
                     const double bfrag = rec[fr];                                    // B[k][n = fr] = P1[fr]
                     const double p2r = rec[MOM_OFF_P2 + frr];
                     const double b30 = rec[MOM_OFF_B3 + frh], b31 = rec[MOM_OFF_B3 + 2 + frh];
@@ -257,9 +270,10 @@ spl_moments_kernel(const __grid_constant__ GridParams gp, const real_t *__restri
                     }
                 }
             }
-            __syncthreads();
+            __syncwarp();                                        // every lane has read the slice before it is restaged
         }
-        // ---- reduce the four warps through shared memory, flush once per work item ----
+        // ---- reduce the warps through shared memory (over their slices: all must be done), flush once per work item ----
+        __syncthreads();
         {
             // C fragment: rows fr, columns 2 fk + {0, 1}
             double *red = s_pts + warp * MOM_MG;
